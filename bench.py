@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W          # this repo's CUDA path
     python bench.py --impl reference ...                     # the CPU path (oracle port) on the host cores
+    python bench.py --dump-outputs DIR ...                   # also write the last timed step's boxes as DIR/*.npy
 
 A step = one pass of the whole path over one batch of independent chains of 67 frames (= 64 windows per chain):
     --config c2 (default)  720p,  80x45 macroblocks, 128 chains per GPU = 8192 windows per step
@@ -207,11 +208,45 @@ def time_cpu(w, steps, warmup, h_mb, w_mb, max_streams, target_s=5.0, one_core=T
     return out, dt / max(steps, 1) * 1e3, n1
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(pipe, out_dir):
+    """Writes the boxes of the last step the pipeline ran, as a caller of run() receives them from fetch_boxes_raw(), so
+    that two builds can be compared output for output:
+        boxes.npy             float32 [n, 5]: left, top, width, height, area of every box, window by window
+        boxes_per_window.npy  float64 [w]: how many of those rows belong to each window
+        windows.npy           float64 [w]: which windows these are
+    All windows, unless that would exceed DUMP_BYTES; then a sample of windows drawn with a fixed seed."""
+    blob, offs, lens = pipe.fetch_boxes_raw()
+    n_box = (lens.astype(np.int64) - 8) // 24                       # bincode Vec<Bbox>: u64 count, 24 bytes per box
+    windows = np.arange(len(lens))
+    if int((20 * n_box + 16).sum()) > DUMP_BYTES:
+        order = np.random.default_rng(0).permutation(len(lens))
+        windows = np.sort(order[np.cumsum(20 * n_box[order] + 16) <= DUMP_BYTES])
+    boxes = []
+    for i in windows:
+        o, k = int(offs[i]), int(n_box[i])
+        assert int(blob[o: o + 8].view("<u8")[0]) == k
+        boxes.append(blob[o + 8: o + 8 + 24 * k].reshape(k, 24)[:, :20].copy().view("<f4"))   # drop the 4 None tags
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "boxes.npy"), np.concatenate(boxes) if boxes else np.zeros((0, 5), np.float32))
+    np.save(os.path.join(out_dir, "boxes_per_window.npy"), n_box[windows].astype(np.float64))
+    np.save(os.path.join(out_dir, "windows.npy"), windows.astype(np.float64))
+
+
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be at least 1")
+    return v
+
+
 # ------------------------------------------------------------------------------------------------ main
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=positive_int, default=20, help="timed steps of the device-resident and of each end-to-end loop")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="cova_b200", choices=["cova_b200", "reference"])
     ap.add_argument("--config", default="c2", choices=sorted(CONFIGS))
@@ -219,6 +254,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-packed", action="store_true", help="skip the packed-input end-to-end leg")
     ap.add_argument("--chunks", type=int, default=1, help="chunks per batch inside the library (1 = whole-batch kernels)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the boxes of the last timed device-resident step (rank 0) as DIR/*.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "cova_b200" else args.warmup
     h_mb, w_mb, cfg_streams, head_bias, cfg_desc = CONFIGS[args.config]
@@ -233,6 +270,8 @@ def main():
                 f"(64-window batch per chain) per GPU")
 
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the CUDA path's boxes; the reference arm keeps none")
         if rank != 0:
             return
         # exactly --steps timed steps after --warmup untimed ones; the per-step sample is sized so that the whole run takes
@@ -307,6 +346,8 @@ def main():
     ms_total = ev0.elapsed_time(ev1)
     launches = pipe.launch_count() - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(pipe, args.dump_outputs)
     t = torch.tensor([ms_total], device="cuda")
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -336,7 +377,7 @@ def main():
     for _ in host_frames:
         pipe.collect(raw=True)
     barrier()
-    e2e_steps = max(6, args.steps)      # as many steps as the device-resident measurement: the two-batch pipeline fill is amortised alike
+    e2e_steps = args.steps              # as many steps as the device-resident measurement: the pipeline fill is amortised alike
     t0 = time.perf_counter()
     for k in range(min(AHEAD, e2e_steps)):
         pipe.submit(host_frames[k % len(host_frames)])

@@ -13,7 +13,33 @@ from oracle import demux_ref
 HERE = os.path.dirname(os.path.abspath(__file__))
 MOOV = open(os.path.join(HERE, "golden", "demo_1m_moov.bin"), "rb").read()
 META = np.load(os.path.join(HERE, "golden", "demo_1m_meta.npz"))
-DEMO = "/root/reference/demo/1m.mp4"   # only in the build container; never on the GPU box
+
+
+def demo_clip_with_synthetic_media(seed=0):
+    """The demo clip as a whole MP4 file: its own ftyp and moov boxes around an mdat whose samples sit at the offsets and
+    have the sizes the clip's sample table gives.  The media bytes are synthetic: each sample is a run of 4-byte
+    length-prefixed NAL units (an optional SEI, then one to three IDR or non-IDR slices, first_mb_in_slice = 0 only
+    on the first) with random non-zero bodies, so that no start code appears inside a NAL unit, as in a real stream."""
+    samples, _ = demux_ref.mp4_video_samples(MOOV)
+    ftyp_size = struct.unpack_from(">I", MOOV)[0]
+    assert samples[0][0] == ftyp_size + 16                   # the clip has an 8-byte free box, then the mdat header
+    rng = np.random.default_rng(seed)
+    mdat = bytearray()
+    for off, size, key, _dts, _pts in samples:
+        assert off == samples[0][0] + len(mdat)
+        n_slices = int(rng.integers(1, 4)) if size >= 64 else 1
+        kinds = ([6] if size >= 64 and rng.random() < 0.2 else []) + [5 if key else 1] * n_slices
+        cuts = np.sort(rng.choice(np.arange(1, size - 12 * len(kinds)), len(kinds) - 1, replace=False)) if len(kinds) > 1 else []
+        bodies = np.diff(np.r_[0, cuts, size - 12 * len(kinds)]) + 8   # every NAL body at least 8 bytes
+        for i, (typ, n) in enumerate(zip(kinds, bodies)):
+            body = rng.integers(1, 256, int(n), dtype=np.uint8)
+            body[0] = (0x60 if typ == 5 else 0x40 if typ == 1 else 0) | typ
+            if typ in (1, 5):                                  # ue(first_mb_in_slice): '1' = 0, '01..' > 0
+                body[1] = 0x80 | body[1] if kinds.index(typ) == i else max(1, body[1] & 0x7F)
+            mdat += struct.pack(">I", int(n)) + body.tobytes()
+        assert len(mdat) == off + size - samples[0][0]
+    return (MOOV[:ftyp_size] + struct.pack(">I4s", 8, b"free") + struct.pack(">I4s", 8 + len(mdat), b"mdat") + bytes(mdat)
+            + MOOV[ftyp_size:])
 
 
 def test_mp4_sample_table_on_the_demo_clip():
@@ -87,11 +113,10 @@ def test_annexb_access_units_synthetic():
     assert shard.demux_annexb(b"") == [] and shard.demux_annexb(b"\x00\x00\x01\x67\x42") == []   # parameter sets only
 
 
-@pytest.mark.skipif(not os.path.exists(DEMO), reason="reference demo clip only exists in the build container")
-def test_annexb_scan_recovers_the_real_clip():
-    """AVCC samples of the real clip rewritten as an Annex-B stream (length prefixes -> start codes): the scanner must
-    find the same 1802 frames and the same 8 key frames the MP4 tables list."""
-    d = open(DEMO, "rb").read()
+def test_annexb_scan_recovers_the_demo_clip_layout():
+    """AVCC samples of the demo clip (its sample table, synthetic media bytes) rewritten as an Annex-B stream (length
+    prefixes -> start codes): the scanner must find the same 1802 frames and the same 8 key frames the MP4 tables list."""
+    d = demo_clip_with_synthetic_media()
     samples, info = shard.demux_mp4(d)
     assert (samples, info) == demux_ref.mp4_video_samples(d)
     stream, starts = bytearray(), []
