@@ -13,6 +13,14 @@ OK, DROPPED = 0, 1
 E_INVAL, E_CUDA, E_NOMEM, E_TOOSMALL, E_WEIGHTS, E_UNSUPPORTED, E_NODEVICE, E_NUMERIC, E_STATE = -1, -2, -3, -4, -5, -6, -7, -8, -9
 IMPL_TCGEN05, IMPL_SIMT = 0, 1
 FLAG_KEEP_LOGITS, FLAG_KEEP_STACKED, FLAG_INPUT_PACKED16 = 0x100, 0x200, 0x400
+FLAG_CCL_CLUSTER = 0x800
+
+
+def flag_ccl_bands(k: int) -> int:
+    """COVA_FLAG_CCL_BANDS(k): force the cluster CCL with k bands (k = 2..8; needs FLAG_CCL_CLUSTER)."""
+    return (k & 0xF) << 24
+
+
 SUBMIT_CONTINUE = 1
 
 
@@ -46,6 +54,7 @@ SIGNATURES = {
     "cova_metapreprocess_out_caps": (ctypes.c_int, [_vp, _u32p, _u32p, _szp]),
     "cova_metapreprocess_transform": (ctypes.c_int, [_vp, _vp, ctypes.c_size_t, _vp, ctypes.c_size_t]),
     "cova_bboxcc_new": (ctypes.c_int, [_vpp, ctypes.c_int, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32]),
+    "cova_bboxcc_new2": (ctypes.c_int, [_vpp, ctypes.c_int, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32]),
     "cova_bboxcc_free": (None, [_vp]),
     "cova_bboxcc_set_cc_threshold": (ctypes.c_int, [_vp, ctypes.c_uint32]),
     "cova_bboxcc_get_cc_threshold": (ctypes.c_int, [_vp, _u32p]),

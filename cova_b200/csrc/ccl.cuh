@@ -16,6 +16,8 @@
 #pragma once
 #include <type_traits>
 
+#include <cooperative_groups.h>
+
 #include "common.cuh"
 
 namespace cova {
@@ -191,21 +193,14 @@ struct CclMem {
     __device__ __forceinline__ int label(int b) const { return COMPACT ? (int)area[b] : stat[5 * b + 4]; }
 };
 
+// Phases 1 and 2 over one CTA's grid of blocks - the whole mask in ccl_bbox_kernel, one band of it in ccl_cluster_kernel.
+// Afterwards parent[] is a forest over the grid whose roots are the first blocks (raster order) of its components, and
+// my_list / the return value are the calling warp's list of foreground blocks.
 template <bool COMPACT>
-__global__ void ccl_bbox_kernel(CclArgs A) {
-    extern __shared__ __align__(16) unsigned char ccl_smem[];
-    const int nb = A.nbx * A.nby;
-    const CclMem<COMPACT> M(ccl_smem, nb, (int)blockDim.x);
-    uint8_t *code = M.code;
-    int *scan = M.scan;
-    __shared__ unsigned long long s_off;
-
-    const int frame = blockIdx.x;
+__device__ __forceinline__ int ccl_codes_and_merge(const CclArgs &A, const CclMem<COMPACT> &M, const uint8_t *m, int nb,
+                                                   unsigned short *&my_list) {
     const int tid = threadIdx.x, nt = blockDim.x;
-    pdl_launch_dependents();
-    pdl_wait();              // the mask comes from the preceding kernel of the stream (common.cuh, "Programmatic dependent launch")
-    const uint8_t *m = A.masks + (size_t)frame * A.H * A.W;
-
+    uint8_t *code = M.code;
     // 1. 2x2 block codes: bit0 (0,0) bit1 (0,1) bit2 (1,0) bit3 (1,1).  Horizontal runs are linked here, without
     //    union-find: consecutive lanes hold consecutive blocks, so a warp ballot of "not connected to my west
     //    neighbour" gives every block the first block of its run inside the warp's 32-block segment as parent
@@ -221,7 +216,7 @@ __global__ void ccl_bbox_kernel(CclArgs A) {
     // for 32.  A warp owns the 32-block segments base + 32*wid .. of every pass over the grid, i.e. a fine interleave of the
     // whole mask, so the lists are balanced.
     const int iters = (nb + nt - 1) / nt;
-    unsigned short *my_list = M.list + (size_t)(tid >> 5) * iters * 32;
+    my_list = M.list + (size_t)(tid >> 5) * iters * 32;
     int n_fg = 0;                                    // warp-uniform: entries in my_list
     int run_by = by_first, run_bx = bx_first;
     for (int base = 0; base < nb; base += nt) {
@@ -390,6 +385,27 @@ __global__ void ccl_bbox_kernel(CclArgs A) {
     __syncthreads();
 
     }
+    return n_fg;
+}
+
+template <bool COMPACT>
+__global__ void ccl_bbox_kernel(CclArgs A) {
+    extern __shared__ __align__(16) unsigned char ccl_smem[];
+    const int nb = A.nbx * A.nby;
+    const CclMem<COMPACT> M(ccl_smem, nb, (int)blockDim.x);
+    uint8_t *code = M.code;
+    int *scan = M.scan;
+    __shared__ unsigned long long s_off;
+
+    const int frame = blockIdx.x;
+    const int tid = threadIdx.x, nt = blockDim.x;
+    pdl_launch_dependents();
+    pdl_wait();              // the mask comes from the preceding kernel of the stream (common.cuh, "Programmatic dependent launch")
+    const uint8_t *m = A.masks + (size_t)frame * A.H * A.W;
+
+    unsigned short *my_list;
+    const int n_fg = ccl_codes_and_merge<COMPACT>(A, M, m, nb, my_list);
+    const int lane = tid & 31;
 
     // 3. flatten + per-root statistics.  parent[b] is lowered to the root while other threads may still walk through b in
     //    their own find: they read either b's old parent (an ancestor) or its root and reach the same root either way.
@@ -513,5 +529,253 @@ __global__ void ccl_bbox_kernel(CclArgs A) {
 }
 
 inline int ccl_threads_for(int nb) { return nb <= 1024 ? 256 : (nb <= 4096 ? 512 : 1024); }
+
+// =====================================================================================================================
+// Thread-block-cluster CCL for masks whose blocks do not fit one CTA's shared memory (8K video: 480 x 270 macroblocks =
+// 32,400 blocks, 876 KB in the wide layout).  One cluster of k CTAs per mask; rank r owns the block rows
+// [r * rows, min((r + 1) * rows, nby)), a band that is itself a grid of the single-CTA kind (at 8K: 4 bands of at most
+// 34 x 240 = 8,160 blocks, exactly the 4K problem).  Phases 1-2 run per band with ccl_codes_and_merge on band-local
+// indices; then the parents become GLOBAL block indices (band offset + local index) and everything else works on the
+// whole mask through distributed shared memory: the seams between bands are linked by the same lock-free union-find
+// (compare-and-swap links of the larger root under the smaller, compression only towards ancestors), so a component's
+// root is still its first block in raster order over the whole mask and the label order stays OpenCV's with no sort.
+// Every CTA lays its shared memory out for a full band (CclMem of rows * nbx blocks), the last one included, so a
+// global index g lives at offset g - q * band_nb of rank q = g / band_nb's arrays, at the same addresses in every CTA.
+// =====================================================================================================================
+struct CclClusterArgs {
+    CclArgs band[2];          // [0]: ranks 0 .. k-2 (`rows` block rows, 2 * rows pixel rows), [1]: the last rank
+    int H;                    // pixel rows of the whole mask
+    int nb;                   // blocks of the whole mask
+    int rows, band_nb;        // block rows and blocks of every band but the last
+    FastDiv div_band;         // by band_nb (when band_nb >= 2)
+};
+
+namespace ccl_cluster_detail {
+namespace cg = cooperative_groups;
+
+// union-find and statistics over the global block indices of the cluster's mask; every access may land in a peer CTA
+struct Global {
+    cg::cluster_group cl;
+    int *parent, *stat;       // this CTA's arrays (the same offsets in every CTA of the cluster)
+    int band_nb;
+    FastDiv div_band;
+
+    __device__ __forceinline__ int owner(int g) const { return band_nb > 1 ? (int)fast_div((uint32_t)g, div_band) : g; }
+    __device__ __forceinline__ int *par(int g) const {
+        const int q = owner(g);
+        return cl.map_shared_rank(parent, (unsigned)q) + (g - q * band_nb);
+    }
+    __device__ __forceinline__ int *st(int g) const {
+        const int q = owner(g);
+        return cl.map_shared_rank(stat, (unsigned)q) + 5 * (g - q * band_nb);
+    }
+    __device__ __forceinline__ int load(int g) const { return *reinterpret_cast<volatile int *>(par(g)); }
+    __device__ __forceinline__ int find(int g) const {
+        int p;
+        while ((p = load(g)) != g) g = p;
+        return g;
+    }
+    // CclMem::find_compress / unite over the whole mask: the same invariants (see there)
+    __device__ __forceinline__ int find_compress(int i) const {
+        int r = load(i);
+        if (r == i) return i;
+        int p, hops = 0;
+        while ((p = load(r)) != r) { r = p; hops++; }
+        if (hops) {
+            int j = i;
+            while ((p = load(j)) > r) {
+                atomicMin(par(j), r);
+                j = p;
+            }
+        }
+        return r;
+    }
+    __device__ __forceinline__ void unite(int a, int b) const {
+        while (true) {
+            a = find_compress(a);
+            b = find_compress(b);
+            if (a == b) return;
+            if (a < b) { int t = a; a = b; b = t; }
+            const int old = atomicCAS(par(a), a, b);
+            if (old == a) return;
+            a = old;
+        }
+    }
+    __device__ __forceinline__ void stat_add(int r, int x0, int y0, int x1, int y1, int cnt) const {
+        int *sr = st(r);
+        atomicMin(&sr[0], x0); atomicMax(&sr[2], x1);
+        atomicMin(&sr[1], y0); atomicMax(&sr[3], y1);
+        atomicAdd(&sr[4], cnt);
+    }
+    __device__ __forceinline__ int label(int g) const { return st(g)[4]; }
+};
+}  // namespace ccl_cluster_detail
+
+__global__ void ccl_cluster_kernel(const __grid_constant__ CclClusterArgs C) {
+    namespace cg = cooperative_groups;
+    extern __shared__ __align__(16) unsigned char ccl_smem[];
+    __shared__ unsigned long long s_off;
+    __shared__ int s_cnt[2];            // roots of this band: all, passing the area filter (read by the peers)
+    __shared__ int s_base[4];           // components of the earlier bands (all, kept) and of the whole mask (all, kept)
+    const cg::cluster_group cl = cg::this_cluster();
+    const int rank = (int)cl.block_rank(), k = (int)cl.num_blocks();
+    const CclArgs &A = C.band[rank == k - 1 ? 1 : 0];
+    const int nb = A.nbx * A.nby;                      // blocks of this band
+    const CclMem<false> M(ccl_smem, C.band_nb, (int)blockDim.x);
+    int *scan = M.scan;
+    const ccl_cluster_detail::Global G{cl, M.parent, M.stat, C.band_nb, C.div_band};
+
+    const int frame = blockIdx.x / k;                  // a cluster is k consecutive CTAs along x
+    const int tid = threadIdx.x, nt = blockDim.x;
+    const int row0 = rank * C.rows, off = row0 * A.nbx;
+    pdl_launch_dependents();
+    pdl_wait();
+    const uint8_t *m = A.masks + (size_t)frame * C.H * A.W + (size_t)2 * row0 * A.W;
+
+    // 1-2. codes, runs and merge inside the band, on band-local indices (in-band links never leave the band)
+    unsigned short *my_list;
+    const int n_fg = ccl_codes_and_merge<false>(A, M, m, nb, my_list);
+    const int lane = tid & 31;
+    for (int i = lane; i < n_fg; i += 32) M.parent[my_list[i] & 0x7fff] += off;    // -> global indices, order kept
+    cl.sync();                                         // also: every peer has started, its shared memory may be touched
+
+    // 2c. seams: this band's first block row against the last row of the band above (north, north-west, north-east)
+    if (rank > 0) {
+        const uint8_t *up = cl.map_shared_rank(M.code, (unsigned)(rank - 1)) + (C.rows - 1) * A.nbx;
+        for (int bx = tid; bx < A.nbx; bx += nt) {
+            const int c = M.code[bx];
+            if (!c) continue;
+            const int g = off + bx, gu = off - A.nbx + bx;
+            if ((c & 0x3) && (up[bx] & 0xC)) G.unite(g, gu);
+            if (bx > 0 && (c & 0x1) && (up[bx - 1] & 0x8)) G.unite(g, gu - 1);
+            if (bx + 1 < A.nbx && (c & 0x2) && (up[bx + 1] & 0x4)) G.unite(g, gu + 1);
+        }
+    }
+    cl.sync();
+
+    // 3. flatten + statistics into the owner CTA's slots (as in ccl_bbox_kernel; the warp combining matters more here:
+    //    a component across a seam would otherwise send thousands of remote atomics to the same five words)
+    for (int k0 = 0; k0 < n_fg; k0 += 32) {
+        const int kk = k0 + lane;
+        const bool live = kk < n_fg;
+        int r = -1 - lane, x0 = 0x7fffffff, y0 = 0x7fffffff, x1 = -1, y1 = -1, cnt = 0;
+        if (live) {
+            const int b = my_list[kk] & 0x7fff;
+            const int c = M.code[b];
+            const int by = A.nbx > 1 ? (int)fast_div((uint32_t)b, A.div_nbx) : b, bx = b - by * A.nbx;
+            r = G.find(off + b);
+            atomicMin(&M.parent[b], r);
+            x0 = 2 * bx + ((c & 0x5) ? 0 : 1); x1 = 2 * bx + ((c & 0xA) ? 1 : 0);
+            y0 = 2 * (row0 + by) + ((c & 0x3) ? 0 : 1); y1 = 2 * (row0 + by) + ((c & 0xC) ? 1 : 0);
+            cnt = __popc(c);
+        }
+        const int r_lead = __shfl_sync(0xffffffffu, r, 0);
+        const unsigned grp = __ballot_sync(0xffffffffu, r == r_lead);
+        bool speak = live;
+        if (__popc(grp) >= 8) {
+            if (r == r_lead) {
+                x0 = __reduce_min_sync(grp, x0); y0 = __reduce_min_sync(grp, y0);
+                x1 = __reduce_max_sync(grp, x1); y1 = __reduce_max_sync(grp, y1);
+                cnt = __reduce_add_sync(grp, cnt);
+                speak = lane == 0;
+            }
+        }
+        if (speak) G.stat_add(r, x0, y0, x1, y1, cnt);
+    }
+    cl.sync();
+
+    // 4. rank this band's roots (hi16 all, lo16 kept: a band has fewer than 2^15 blocks), then across the cluster in 32 bits
+    const int ipt = (nb + nt - 1) / nt;
+    const int b0 = min(tid * ipt, nb), b1 = min(b0 + ipt, nb);
+    int cnt = 0;
+    for (int b = b0; b < b1; b++)
+        if (M.parent[b] == off + b) cnt += 0x10000 + (M.stat[5 * b + 4] >= A.area_thresh ? 1 : 0);
+    int incl = cnt;
+    const int wid = tid >> 5;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        int v = __shfl_up_sync(0xffffffffu, incl, d);
+        if (lane >= d) incl += v;
+    }
+    if (lane == 31) scan[wid] = incl;
+    __syncthreads();
+    if (wid == 0) {
+        int nw = nt >> 5;
+        int v = lane < nw ? scan[lane] : 0, s = v;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            int u = __shfl_up_sync(0xffffffffu, s, d);
+            if (lane >= d) s += u;
+        }
+        if (lane < nw) scan[lane] = s - v;
+        if (lane == 31) { s_cnt[0] = s >> 16; s_cnt[1] = s & 0xffff; }
+    }
+    cl.sync();
+    const int excl = scan[wid] + incl - cnt;
+    if (tid == 0) {
+        int all_before = 0, keep_before = 0, n_all = 0, n_keep = 0;
+        for (int q = 0; q < k; q++) {
+            const int *pc = cl.map_shared_rank(s_cnt, (unsigned)q);
+            const int a = pc[0], kp = pc[1];
+            if (q < rank) { all_before += a; keep_before += kp; }
+            n_all += a; n_keep += kp;
+        }
+        s_base[0] = all_before; s_base[1] = keep_before; s_base[2] = n_all; s_base[3] = n_keep;
+        // 5. rank 0 reserves the mask's output range and publishes its offset into every CTA of the cluster
+        if (rank == 0) {
+            const unsigned long long need = 8ull + 24ull * (unsigned long long)n_keep;
+            const unsigned long long o = atomicAdd(A.cursor, need);
+            A.offsets[frame] = o;
+            A.lens[frame] = need;
+            if (o + need > A.blob_cap) atomicExch(A.cursor + 1, 1ull);
+            if (A.n_labels) A.n_labels[frame] = n_all + 1;
+            if (o + need <= A.blob_cap) *reinterpret_cast<unsigned long long *>(A.blob + o) = (unsigned long long)n_keep;
+            for (int q = 0; q < k; q++) *cl.map_shared_rank(&s_off, (unsigned)q) = o;
+        }
+    }
+    cl.sync();
+    const unsigned long long off_out = s_off;
+    const unsigned long long need = 8ull + 24ull * (unsigned long long)s_base[3];
+    const bool fits = off_out + need <= A.blob_cap;
+    int32_t *st = A.stats ? A.stats + (size_t)frame * (C.nb + 1) * 5 : nullptr;
+    if (st && rank == 0 && tid < 5) st[tid] = 0;
+
+    // 6. emit this band's boxes at its base; the area slot of a root becomes the root -> label map
+    int rank_all = s_base[0] + (excl >> 16), rank_keep = s_base[1] + (excl & 0xffff);
+    for (int b = b0; b < b1; b++) {
+        if (M.parent[b] != off + b) continue;
+        int x0, y0, x1, y1;
+        M.stat_get(b, x0, y0, x1, y1);
+        const int w = x1 - x0 + 1, h = y1 - y0 + 1, ar = M.stat_area(b);
+        rank_all++;
+        if (st) {
+            int32_t *s5 = st + (size_t)rank_all * 5;
+            s5[0] = x0; s5[1] = y0; s5[2] = w; s5[3] = h; s5[4] = ar;
+        }
+        if (ar >= A.area_thresh) {
+            if (fits) {
+                uint32_t *rec = reinterpret_cast<uint32_t *>(A.blob + off_out + 8 + 24ull * rank_keep);
+                float fw = (float)w, fh = (float)h;
+                rec[0] = __float_as_uint((float)x0);
+                rec[1] = __float_as_uint((float)y0);
+                rec[2] = __float_as_uint(fw);
+                rec[3] = __float_as_uint(fh);
+                rec[4] = __float_as_uint(fw * fh);   // bbox.rs:23
+                rec[5] = 0u;
+            }
+            rank_keep++;
+        }
+        M.set_label(b, rank_all);
+    }
+    if (!A.labels) return;             // no CTA reads a peer's shared memory after the last barrier
+    cl.sync();                         // every label map of the cluster is written
+    int32_t *lab = A.labels + (size_t)frame * C.H * A.W + (size_t)2 * row0 * A.W;
+    for (int p = tid; p < A.H * A.W; p += nt) {
+        int y = p / A.W, x = p - y * A.W;
+        int b = (y >> 1) * A.nbx + (x >> 1);
+        lab[p] = (m[p] != 0) ? G.label(M.parent[b]) : 0;
+    }
+    cl.sync();                         // no CTA leaves while a peer may still read its label map
+}
 
 }  // namespace cova

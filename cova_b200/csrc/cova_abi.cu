@@ -238,11 +238,45 @@ struct CclBuffers {
     size_t smem = 0;
     int threads = 0;
     bool compact = false;     // 13-byte-per-block shared-memory layout (ccl.cuh): two CTAs per SM at 4K
+    int k = 1, rows = 0;      // k > 1: ccl_cluster_kernel, one cluster of k CTAs per mask, bands of `rows` block rows
 };
 
 constexpr int kCclSmemLimit = tc::kSmemLimit - 1024;   // dynamic part: the kernel also has a few bytes of static shared memory
 
-static int ccl_alloc(CclBuffers &b, int H, int W, int max_masks, bool own_masks) {
+// COVA_FLAG_CCL_CLUSTER / COVA_FLAG_CCL_BANDS: checked before any device call
+static int ccl_check_flags(uint32_t flags) {
+    const uint32_t bands = (flags >> 24) & 0xfu;
+    if (bands && !(flags & COVA_FLAG_CCL_CLUSTER)) return set_err(COVA_E_INVAL, "COVA_FLAG_CCL_BANDS needs COVA_FLAG_CCL_CLUSTER");
+    if (bands == 1 || bands > 8) return set_err(COVA_E_INVAL, "COVA_FLAG_CCL_BANDS(k) takes k = 2..8");
+    return COVA_OK;
+}
+static int ccl_check_bands(uint32_t flags, uint32_t height) {
+    if (((flags >> 24) & 0xfu) > (height + 1) / 2) return set_err(COVA_E_INVAL, "COVA_FLAG_CCL_BANDS(k) needs k <= ceil(height / 2) block rows");
+    return COVA_OK;
+}
+
+// Can one cluster of b.k CTAs of b.smem bytes be resident at all?  (k CTAs of ~220 KB on SMs of one GPC, which the
+// single-CTA kernel never needs.)
+static int ccl_cluster_ok(const CclBuffers &b) {
+    COVA_CUDA(cudaFuncSetAttribute(ccl_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kCclSmemLimit));
+    cudaLaunchConfig_t cfg;
+    memset(&cfg, 0, sizeof(cfg));
+    cfg.gridDim = dim3((unsigned)b.k); cfg.blockDim = dim3((unsigned)b.threads); cfg.dynamicSmemBytes = b.smem;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension;
+    at[0].val.clusterDim.x = (unsigned)b.k; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+    cfg.attrs = at; cfg.numAttrs = 1;
+    int n = 0;
+    COVA_CUDA(cudaOccupancyMaxActiveClusters(&n, ccl_cluster_kernel, &cfg));
+    if (n < 1) {
+        char msg[160];
+        snprintf(msg, sizeof(msg), "no cluster of %d CTAs with %zu bytes of shared memory each fits this device", b.k, b.smem);
+        return set_err(COVA_E_UNSUPPORTED, "%s", msg);
+    }
+    return COVA_OK;
+}
+
+static int ccl_alloc(CclBuffers &b, int H, int W, int max_masks, bool own_masks, uint32_t flags = 0) {
     b.H = H; b.W = W; b.nbx = (W + 1) / 2; b.nby = (H + 1) / 2; b.nb = b.nbx * b.nby; b.max_masks = max_masks;
     b.threads = ccl_threads_for(b.nb);
     // The compact layout would give 4K masks two CTAs per SM (204 KB -> 106 KB), but measured it does not pay: its
@@ -253,8 +287,24 @@ static int ccl_alloc(CclBuffers &b, int H, int W, int max_masks, bool own_masks)
     if (force && (force[0] == '0' || force[0] == '1')) b.compact = force[0] == '1';
     b.smem = ccl_smem_bytes(b.nb, b.threads, b.compact);
     if (b.smem > (size_t)kCclSmemLimit && !b.compact) { b.compact = true; b.smem = ccl_smem_bytes(b.nb, b.threads, true); }
-    if (b.smem > (size_t)kCclSmemLimit || b.nb >= 0x7FFF)       // block indices travel in 15 bits of the foreground lists
+    const bool one_cta = b.smem <= (size_t)kCclSmemLimit && b.nb < 0x7FFF;   // block indices travel in 15 bits of the foreground lists
+    const int forced = (int)((flags >> 24) & 0xfu);
+    b.k = 1;
+    if ((flags & COVA_FLAG_CCL_CLUSTER) && (forced || !one_cta)) {
+        // bands in the wide layout: the fewest (2..8) that fit, or exactly the forced count of rows ceil(nby / k) - which
+        // may leave fewer than k bands when the rows run out (nby = 5, k = 4: 2 + 2 + 1)
+        for (int k = forced ? forced : 2; k <= (forced ? forced : 8) && b.k == 1; k++) {
+            const int rows = (b.nby + k - 1) / k, band_nb = rows * b.nbx, threads = ccl_threads_for(band_nb);
+            const size_t smem = ccl_smem_bytes(band_nb, threads, false);
+            if (smem > (size_t)kCclSmemLimit || band_nb >= 0x7FFF) continue;
+            b.k = (b.nby + rows - 1) / rows; b.rows = rows; b.threads = threads; b.smem = smem; b.compact = false;
+        }
+        if (b.k == 1) return set_err(COVA_E_UNSUPPORTED, "mask grid too large for the cluster CCL kernel (8 bands of the shared-memory layout)");
+        int rc = ccl_cluster_ok(b);
+        if (rc) return rc;
+    } else if (!one_cta) {
         return set_err(COVA_E_UNSUPPORTED, "mask grid too large for the shared-memory CCL kernel");
+    }
     b.blob_cap = (size_t)max_masks * (8 + 24 * (size_t)b.nb);
     if (own_masks) COVA_CUDA(cudaMalloc(&b.d_masks, (size_t)max_masks * H * W));
     COVA_CUDA(cudaMalloc(&b.d_blob, b.blob_cap));
@@ -273,32 +323,62 @@ static void ccl_free(CclBuffers &b, bool own_masks) {
     if (b.d_stats) cudaFree(b.d_stats);
     if (b.d_nlabels) cudaFree(b.d_nlabels);
 }
-static int ccl_launch(CclBuffers &b, const uint8_t *d_masks, int n, uint32_t cc_threshold, bool want_labels, cudaStream_t st,
-                      size_t first = 0, bool reset_cursor = true, bool pdl = true) {
-    if (n <= 0) return COVA_OK;
-    CclArgs a;
-    a.masks = d_masks + first * (size_t)b.H * b.W; a.H = b.H; a.W = b.W; a.nbx = b.nbx; a.nby = b.nby;
-    a.area_thresh = (int)cc_threshold;   // `settings.cc_threshold as i32` (imp.rs:248)
-    a.blob = b.d_blob; a.blob_cap = b.blob_cap; a.cursor = b.d_cursor; a.offsets = b.d_offsets + first; a.lens = b.d_lens + first;
-    a.labels = want_labels ? b.d_labels : nullptr;
-    a.stats = want_labels ? b.d_stats : nullptr;
-    a.n_labels = want_labels ? b.d_nlabels : nullptr;
-    a.div_nbx = make_fastdiv((uint32_t)std::max(2, b.nbx));
-    a.step_by = b.threads / b.nbx; a.step_bx = b.threads % b.nbx;
+// merge-phase choice and tiling of a grid of a.nbx x nby blocks (the whole mask, or one band of it)
+static void ccl_grid_args(CclArgs &a, int nby, int threads) {
+    a.nby = nby;
+    const int nb = a.nbx * nby;
+    a.div_nbx = make_fastdiv((uint32_t)std::max(2, a.nbx));
+    a.step_by = threads / a.nbx; a.step_bx = threads % a.nbx;
     // merge phase: tile scan (ccl.cuh, 2a/2b; about one tile of 32 columns per warp) for large grids, the concurrent
     // union-find over all foreground blocks for small ones.  Measured per 1024 4K masks (tools/ccl_timing.py): network masks
     // 0.35 -> 0.31 ms, dense network masks 0.86 -> 0.66, dense noise 0.88 -> 0.74 (all-ones 0.35 -> 0.55, empty 0.09 -> 0.11);
     // at 720p / 1080p the row-serial scan loses to the union-find (0.160 -> 0.189 / 0.156 -> 0.191 ms), so it is off there.
     // COVA_CCL_SCAN=0/1 forces either (development knob; both pass the golden and stress suites).
     static const char *scan_env = getenv("COVA_CCL_SCAN");
-    a.scan = b.nb >= 4096;
+    a.scan = nb >= 4096;
     if (scan_env && (scan_env[0] == '0' || scan_env[0] == '1')) a.scan = scan_env[0] == '1';
-    a.tiles_x = (b.nbx + 31) / 32;
-    a.tiles_y = std::max(1, std::min(b.nby, (b.threads / 32) / a.tiles_x));
-    a.tile_rows = (b.nby + a.tiles_y - 1) / a.tiles_y;
-    a.tiles_y = (b.nby + a.tile_rows - 1) / a.tile_rows;
+    a.tiles_x = (a.nbx + 31) / 32;
+    a.tiles_y = std::max(1, std::min(nby, (threads / 32) / a.tiles_x));
+    a.tile_rows = (nby + a.tiles_y - 1) / a.tiles_y;
+    a.tiles_y = (nby + a.tile_rows - 1) / a.tile_rows;
     a.div_tile_rows = make_fastdiv((uint32_t)std::max(2, a.tile_rows));
+}
+
+static int ccl_launch(CclBuffers &b, const uint8_t *d_masks, int n, uint32_t cc_threshold, bool want_labels, cudaStream_t st,
+                      size_t first = 0, bool reset_cursor = true, bool pdl = true) {
+    if (n <= 0) return COVA_OK;
+    CclArgs a;
+    a.masks = d_masks + first * (size_t)b.H * b.W; a.H = b.H; a.W = b.W; a.nbx = b.nbx;
+    a.area_thresh = (int)cc_threshold;   // `settings.cc_threshold as i32` (imp.rs:248)
+    a.blob = b.d_blob; a.blob_cap = b.blob_cap; a.cursor = b.d_cursor; a.offsets = b.d_offsets + first; a.lens = b.d_lens + first;
+    a.labels = want_labels ? b.d_labels : nullptr;
+    a.stats = want_labels ? b.d_stats : nullptr;
+    a.n_labels = want_labels ? b.d_nlabels : nullptr;
     if (reset_cursor) COVA_CUDA(cudaMemsetAsync(b.d_cursor, 0, 2 * sizeof(unsigned long long), st));
+    if (b.k > 1) {
+        CclClusterArgs c;
+        c.H = b.H; c.nb = b.nb; c.rows = b.rows; c.band_nb = b.rows * b.nbx;
+        c.div_band = make_fastdiv((uint32_t)std::max(2, c.band_nb));
+        c.band[0] = a; c.band[0].H = 2 * b.rows;
+        ccl_grid_args(c.band[0], b.rows, b.threads);
+        const int last_rows = b.nby - (b.k - 1) * b.rows;
+        c.band[1] = a; c.band[1].H = b.H - 2 * (b.k - 1) * b.rows;
+        ccl_grid_args(c.band[1], last_rows, b.threads);
+        // same attribute policy as below: always the architectural maximum
+        COVA_CUDA(cudaFuncSetAttribute(ccl_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kCclSmemLimit));
+        cudaLaunchConfig_t cfg;
+        memset(&cfg, 0, sizeof(cfg));
+        cfg.gridDim = dim3((unsigned)(n * b.k)); cfg.blockDim = dim3((unsigned)b.threads); cfg.dynamicSmemBytes = b.smem; cfg.stream = st;
+        cudaLaunchAttribute at[2];
+        at[0].id = cudaLaunchAttributeClusterDimension;
+        at[0].val.clusterDim.x = (unsigned)b.k; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+        at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        at[1].val.programmaticStreamSerializationAllowed = 1;
+        cfg.attrs = at; cfg.numAttrs = pdl ? 2 : 1;
+        COVA_CUDA(cudaLaunchKernelEx(&cfg, ccl_cluster_kernel, c));
+        return COVA_OK;
+    }
+    ccl_grid_args(a, b.nby, b.threads);
     // the attribute is per function AND per device, last write wins: handles of different grids (or on different devices,
     // or on different threads) share ccl_bbox_kernel, so it is set for every launch and always to the same value, the
     // architectural maximum (see tc::try_launch)
@@ -313,26 +393,34 @@ static int ccl_launch(CclBuffers &b, const uint8_t *d_masks, int n, uint32_t cc_
 // =================================================================================================
 struct cova_bboxcc {
     int device;
-    uint32_t width, height, cc_threshold;
+    uint32_t width, height, cc_threshold, flags;
     CclBuffers b;
     cudaStream_t stream = nullptr;
 };
 
-extern "C" int cova_bboxcc_new(cova_bboxcc **out, int device, uint32_t width, uint32_t height, uint32_t cc_threshold) {
+extern "C" int cova_bboxcc_new2(cova_bboxcc **out, int device, uint32_t width, uint32_t height, uint32_t cc_threshold,
+                                uint32_t flags) {
     if (!out) return set_err(COVA_E_INVAL, "null out");
     *out = nullptr;
     if (!width || !height) return set_err(COVA_E_INVAL, "empty mask");
-    int rc = check_device(device);
+    if (flags & ~(COVA_FLAG_CCL_CLUSTER | COVA_FLAG_CCL_BANDS(0xf))) return set_err(COVA_E_INVAL, "unknown bboxcc flag");
+    int rc = ccl_check_flags(flags);
+    if (!rc) rc = ccl_check_bands(flags, height);
+    if (rc) return rc;
+    rc = check_device(device);
     if (rc) return rc;
     auto *cc = new (std::nothrow) cova_bboxcc();
     if (!cc) return set_err(COVA_E_NOMEM, "host allocation failed");
-    cc->device = device; cc->width = width; cc->height = height; cc->cc_threshold = cc_threshold;
-    rc = ccl_alloc(cc->b, (int)height, (int)width, 1, true);
+    cc->device = device; cc->width = width; cc->height = height; cc->cc_threshold = cc_threshold; cc->flags = flags;
+    rc = ccl_alloc(cc->b, (int)height, (int)width, 1, true, flags);
     if (rc == COVA_OK && cudaStreamCreateWithFlags(&cc->stream, cudaStreamNonBlocking) != cudaSuccess)
         rc = set_err(COVA_E_CUDA, "stream creation failed");
     if (rc) { cova_bboxcc_free(cc); return rc; }
     *out = cc;
     return COVA_OK;
+}
+extern "C" int cova_bboxcc_new(cova_bboxcc **out, int device, uint32_t width, uint32_t height, uint32_t cc_threshold) {
+    return cova_bboxcc_new2(out, device, width, height, cc_threshold, 0);
 }
 extern "C" void cova_bboxcc_free(cova_bboxcc *cc) {
     if (!cc) return;
@@ -518,6 +606,12 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
     if (gamma < 1 || !max_streams || max_fps < timestep) return set_err(COVA_E_INVAL, "need gamma >= 1, max_streams >= 1, max_frames_per_stream >= timestep");
     if (w_mb < 16 || h_mb < 16) return set_err(COVA_E_UNSUPPORTED, "macroblock grid must be at least 16x16 for four 2x poolings");
     if ((flags & 0xffu) > COVA_IMPL_SIMT) return set_err(COVA_E_INVAL, "unknown implementation selector");
+    if (flags & ~(0xffu | COVA_FLAG_KEEP_LOGITS | COVA_FLAG_KEEP_STACKED | COVA_FLAG_INPUT_PACKED16 | COVA_FLAG_CCL_CLUSTER |
+                  COVA_FLAG_CHUNKS(0xff) | COVA_FLAG_CCL_BANDS(0xf)))
+        return set_err(COVA_E_INVAL, "unknown pipeline flag");
+    int rc = ccl_check_flags(flags);
+    if (!rc) rc = ccl_check_bands(flags, h_mb);
+    if (rc) return rc;
     if (flags & COVA_FLAG_INPUT_PACKED16) {
         if (flags & COVA_FLAG_KEEP_STACKED) return set_err(COVA_E_INVAL, "the stacked RGBA windows cannot be rebuilt from packed input (byte 3 and values above 6 are gone)");
         if ((flags & 0xffu) == COVA_IMPL_SIMT) return set_err(COVA_E_UNSUPPORTED, "the validation kernels read the 4-byte input format");
@@ -527,7 +621,7 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
     if ((flags & 0xffu) == COVA_IMPL_SIMT)
         return set_err(COVA_E_UNSUPPORTED, "the validation kernels (COVA_IMPL_SIMT) are not part of this build; use libcova_b200_val.so");
 #endif
-    int rc = check_device(device);
+    rc = check_device(device);
     if (rc) return rc;
     auto *p = new (std::nothrow) cova_pipeline();
     if (!p) return set_err(COVA_E_NOMEM, "host allocation failed");
@@ -605,7 +699,7 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
     if (e == cudaSuccess) e = cudaMallocHost(&p->h_pinned, sizeof(unsigned long long) * (2 + 2 * (size_t)std::max(1, NB) + 2 * 64));
     if (e != cudaSuccess) return fail(set_err(COVA_E_CUDA, "pipeline allocation: %s", cudaGetErrorString(e)));
     p->slot[0].ccl.d_masks = p->d_mask;
-    if ((rc = ccl_alloc(p->slot[0].ccl, (int)h_mb, (int)w_mb, std::max(1, NB), false))) return fail(rc);
+    if ((rc = ccl_alloc(p->slot[0].ccl, (int)h_mb, (int)w_mb, std::max(1, NB), false, flags))) return fail(rc);
     p->slot[0].ready = true;
     p->ccl = p->slot[0].ccl;
     for (auto &sl : p->slot)
@@ -1052,7 +1146,7 @@ static int ccl_range(cova_pipeline *p, size_t first, int n, bool reset_cursor) {
     if (rc) return rc;
     if (n > 0) {
         p->launches++;
-        prof_mark(p, "ccl_bbox");
+        prof_mark(p, p->ccl.k > 1 ? "ccl_bbox_cluster" : "ccl_bbox");
     }
     return COVA_OK;
 }
@@ -1174,7 +1268,7 @@ static int ensure_slot(cova_pipeline *p, int k) {
     if (!sl.d_frames) COVA_CUDA(cudaMalloc(&sl.d_frames, p->frame_bytes * p->max_streams * p->max_fps));
     if (!sl.ccl.d_blob) {
         sl.ccl.d_masks = p->d_mask;
-        int rc = ccl_alloc(sl.ccl, (int)p->H, (int)p->W, std::max<int>(1, (int)p->max_windows), false);
+        int rc = ccl_alloc(sl.ccl, (int)p->H, (int)p->W, std::max<int>(1, (int)p->max_windows), false, p->flags);
         if (rc) { ccl_free(sl.ccl, false); sl.ccl = CclBuffers(); return rc; }    // a later submit retries from scratch
     }
     sl.ready = true;

@@ -145,9 +145,13 @@ class BboxCc:
 
     ELEMENT_NAME = "bboxcc"
 
-    def __init__(self, width: int, height: int, cc_threshold: int = DEFAULT_CC_THRESHOLD, device: int = 0):
+    def __init__(self, width: int, height: int, cc_threshold: int = DEFAULT_CC_THRESHOLD, device: int = 0,
+                 cluster: bool = False, bands: int = 0):
+        # cluster=True: grids beyond one CTA's shared memory (8K) run the thread-block-cluster CCL instead of being
+        # refused; bands=k forces that kernel with k bands on any grid (COVA_FLAG_CCL_CLUSTER / COVA_FLAG_CCL_BANDS)
         self._h = ctypes.c_void_p()
-        check(_lib.load().cova_bboxcc_new(ctypes.byref(self._h), device, width, height, cc_threshold))
+        flags = (_lib.FLAG_CCL_CLUSTER if cluster else 0) | (_lib.flag_ccl_bands(bands) if bands else 0)
+        check(_lib.load().cova_bboxcc_new2(ctypes.byref(self._h), device, width, height, cc_threshold, flags))
         self.width, self.height = width, height
         self._cap = _lib.load().cova_bboxcc_max_out_size(self._h)
 
@@ -366,7 +370,7 @@ class BlobPipeline:
     def __init__(self, w_mb: int, h_mb: int, weights_blob: bytes, max_streams: int, max_frames_per_stream: int,
                  timestep: int = 4, gamma: int = 1, cc_threshold: int = 1, device: int = 0,
                  impl: int = _lib.IMPL_TCGEN05, keep_logits: bool = False, keep_stacked: bool = False, n_chunks: int = 0,
-                 validation: bool = False, packed_input: bool = False):
+                 validation: bool = False, packed_input: bool = False, ccl_cluster: bool = False, ccl_bands: int = 0):
         # validation=True (or impl=IMPL_SIMT) binds this handle to libcova_b200_val.so, the build that also holds the
         # fp32 validation kernels; the product library refuses IMPL_SIMT
         self._L = _lib.load_validation() if (validation or impl == _lib.IMPL_SIMT) else _lib.load()
@@ -374,6 +378,8 @@ class BlobPipeline:
         flags = impl | (_lib.FLAG_KEEP_LOGITS if keep_logits else 0) | (_lib.FLAG_KEEP_STACKED if keep_stacked else 0)
         flags |= (n_chunks & 0xff) << 16
         flags |= _lib.FLAG_INPUT_PACKED16 if packed_input else 0
+        # ccl_cluster / ccl_bands: as BboxCc's cluster / bands
+        flags |= (_lib.FLAG_CCL_CLUSTER if ccl_cluster else 0) | (_lib.flag_ccl_bands(ccl_bands) if ccl_bands else 0)
         # packed_input: every frames argument is [n_streams, frames, h_mb, w_mb] u16 (FramePacker) instead of [.., 4] u8
         self.packed_input = packed_input
         self._wbuf = ctypes.create_string_buffer(weights_blob, len(weights_blob))

@@ -29,7 +29,7 @@ extern "C" {
 #define COVA_E_NOMEM (-3)
 #define COVA_E_TOOSMALL (-4)    /* output buffer too small; the required size is reported */
 #define COVA_E_WEIGHTS (-5)     /* not a CVBN v1 weight container */
-#define COVA_E_UNSUPPORTED (-6) /* e.g. timestep != 4 for BlobNet, grid too large for the CCL kernel */
+#define COVA_E_UNSUPPORTED (-6) /* e.g. timestep != 4 for BlobNet, grid too large for the CCL kernel (see COVA_FLAG_CCL_CLUSTER) */
 #define COVA_E_NODEVICE (-7)    /* no CUDA device: there is no CPU fallback */
 #define COVA_E_NUMERIC (-8)     /* host tracker: Kalman innovation covariance not positive definite */
 #define COVA_E_STATE (-9)       /* host frame selection: a state the reference asserts can never happen */
@@ -81,6 +81,10 @@ int cova_metapreprocess_transform(cova_metapreprocess *mp, const uint8_t *inbuf,
 typedef struct cova_bboxcc cova_bboxcc;
 
 int cova_bboxcc_new(cova_bboxcc **out, int device, uint32_t width, uint32_t height, uint32_t cc_threshold);
+/* as cova_bboxcc_new (which is new2 with flags 0), with COVA_FLAG_CCL_CLUSTER / COVA_FLAG_CCL_BANDS(k) (see below);
+ * any other bit is COVA_E_INVAL */
+int cova_bboxcc_new2(cova_bboxcc **out, int device, uint32_t width, uint32_t height, uint32_t cc_threshold,
+                     uint32_t flags);
 void cova_bboxcc_free(cova_bboxcc *cc);
 int cova_bboxcc_set_cc_threshold(cova_bboxcc *cc, uint32_t cc_threshold);
 int cova_bboxcc_get_cc_threshold(const cova_bboxcc *cc, uint32_t *cc_threshold);
@@ -120,6 +124,20 @@ typedef struct cova_pipeline cova_pipeline;
  * [n_streams][frames][h_mb][w_mb] u16.  Not combinable with COVA_FLAG_KEEP_STACKED; w_mb must be even. */
 #define COVA_FLAG_INPUT_PACKED16 0x400u
 #define COVA_FLAG_CHUNKS(n) (((uint32_t)(n) & 0xffu) << 16) /* process a batch in n chunks of whole chains (0 = auto) */
+/* Masks larger than one CTA's shared memory (8K video: 480x270 macroblocks = 32,400 2x2 blocks).  The CCL normally holds a
+ * whole mask in one CTA's shared memory and such grids are refused with COVA_E_UNSUPPORTED at creation.  With this flag
+ * (for cova_pipeline_new and cova_bboxcc_new2) a grid that fits one CTA still runs the single-CTA kernel; a larger one
+ * runs a thread-block-cluster kernel: one cluster of k = 2..8 CTAs per mask, each CTA owning a band of ceil(nby/k) block
+ * rows and reaching its peers through distributed shared memory (8K: k = 4).  Outputs are byte-identical to what the
+ * single-CTA kernel would produce; under profiling the kernel is named "ccl_bbox_cluster".  Still COVA_E_UNSUPPORTED: a
+ * grid that needs more than 8 bands (about 65,000 blocks), and a device on which no such cluster can be resident
+ * (creation checks cudaOccupancyMaxActiveClusters).  Opt-in because the cluster kernel needs k CTAs of up to ~220 KB of
+ * shared memory to be co-resident in one GPC, which the single-CTA kernel never does. */
+#define COVA_FLAG_CCL_CLUSTER 0x800u
+/* Forces the cluster kernel with bands of ceil(ceil(H/2) / k) block rows (k bands, fewer when the rows run out) on any
+ * grid, so that tests and measurements can put seams into small masks.  COVA_E_INVAL, before any device call: without
+ * COVA_FLAG_CCL_CLUSTER, k = 1 or k > 8, k > ceil(H/2), and any flag bit that no COVA_FLAG_* / COVA_IMPL_* defines. */
+#define COVA_FLAG_CCL_BANDS(k) (((uint32_t)(k) & 0xfu) << 24)
 
 int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb, uint32_t h_mb, uint32_t timestep,
                       uint32_t gamma, uint32_t max_streams, uint32_t max_frames_per_stream, const void *weights,
