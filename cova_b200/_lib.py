@@ -22,6 +22,7 @@ def flag_ccl_bands(k: int) -> int:
 
 
 SUBMIT_CONTINUE = 1
+SUBMIT_STAGGERED = 2       # with SUBMIT_CONTINUE: the continued streams of a batch may differ in history and gamma phase
 
 
 class CovaError(RuntimeError):

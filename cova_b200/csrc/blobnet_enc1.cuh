@@ -33,7 +33,11 @@ constexpr int kThreads1 = 64 + 32 * kEpiWarps1;
 constexpr int kPairRows = 2 * kTileM;
 
 struct Enc1Extra {
-    int n_chains, fps, wps, gamma, first;   // chains of this chunk, frames per chain, windows per chain, sub-sampling, T - 1
+    int n_chains, fps, gamma;               // chains of this chunk, frames per chain, sub-sampling
+    // per chain of the chunk: (index of the newest frame of its first window, index of that window in the chunk).  Chains
+    // of a staggered batch differ in both (cova_abi.cu, set_batch_shape); a chain's window n + k has its newest frame at
+    // first + k * gamma
+    const int2 *tab;
     int ntp;                                // tile pairs per frame
     int n_items;                            // (chain, tile pair) items = n_chains * ntp, each fps frame steps long
     int full_items;                         // items handed out whole, round-robin: a multiple of the grid size
@@ -186,10 +190,15 @@ __global__ void __launch_bounds__(kThreads1, 1) enc1_fused_kernel(const __grid_c
             const int y2 = r / gi.P, x2 = r - y2 * gi.P;
             const bool valid = r < gi.S && y2 < (gi.H >> 1) && x2 < (gi.W >> 1);
             const bool warp_live = __any_sync(0xffffffffu, valid);       // warps that only cover padding rows skip the arithmetic
+            // (first, window 0) of the chain: one load per item; window 0 goes into the base addresses, only first stays live
+            const int2 cw = ex.tab[w.chain];
             const int Y = y2 + (gi.H & 1), X = x2 + (gi.W & 1);          // zero-pad top / left when odd (encoder.py:68-76)
             const int pho = ((Y & 1) << 1) | (X & 1);
-            const long long base_o = (long long)(cg * 4 + pho) * p.gout.Lp + p.gout.guard + ((long long)(Y >> 1) * p.gout.P + (X >> 1)) * kT;
-            const long long base_s = (long long)((p.out2_cb + cg) * 4 + pho) * p.gout2.Lp + p.gout2.guard + (long long)(Y >> 1) * p.gout2.P + (X >> 1);
+            const long long base_o = (long long)(cg * 4 + pho) * p.gout.Lp + p.gout.guard + ((long long)(Y >> 1) * p.gout.P + (X >> 1)) * kT +
+                                   (long long)cw.y * p.gout.S * kT;
+            const long long base_s = (long long)((p.out2_cb + cg) * 4 + pho) * p.gout2.Lp + p.gout2.guard + (long long)(Y >> 1) * p.gout2.P + (X >> 1) +
+                                   (long long)cw.y * p.gout2.S;
+            const int first = cw.x;
             // Ring of the last four pooled frames: ring[s][k] = channel pair (2k, 2k+1) of the frame whose index is s mod 4,
             // as fp32 values already rounded to fp16 (what the two-kernel path stores and re-reads).  The frame loop is
             // unrolled four times over the ring phase R, so "frame i - t" is the compile-time slot (R - t) & 3: no
@@ -238,10 +247,10 @@ __global__ void __launch_bounds__(kThreads1, 1) enc1_fused_kernel(const __grid_c
                         ring[R][k] = __half22float2(__floats2half2_rn(o.x, o.y));   // the pooled activation is an fp16 tensor
                     }
                 }
-                const int rel = i - ex.first;
+                const int rel = i - first;
                 const bool emit = i >= w.i0 && rel >= 0 && (ex.gamma == 1 || rel % ex.gamma == 0);   // warp-uniform
                 if (emit && valid) {
-                    const long long n = (long long)w.chain * ex.wps + (ex.gamma == 1 ? rel : rel / ex.gamma);
+                    const long long n = ex.gamma == 1 ? rel : rel / ex.gamma;           // window of the chain
                     uint32_t o32[4][4];
 #pragma unroll
                     for (int k = 0; k < 4; k++) {                        // channel pair (2k, 2k+1) in the two packed fp32 lanes

@@ -503,17 +503,13 @@ struct cova_pipeline {
     size_t frame_bytes = 0;              // bytes of one frame in the pool: 4 per macroblock, or 2 with COVA_FLAG_INPUT_PACKED16
     bool packed = false;
     uint8_t *d_frames = nullptr;
-    int *d_newest = nullptr;
-    uint32_t cur_streams = 0, cur_fps = 0, cur_windows = 0, table_streams = 0, table_fps = 0, table_first = 0;
-    // index (inside a device chain) of the newest frame of the chain's first window, and windows per chain: T - 1 and
-    // (fps - T) / gamma + 1 for a chain that starts with an empty window; a CONTINUED chain (submit_host2) starts with the
-    // carried T - 1 frames of its stream and its first window sits where the stream's gamma phase puts it
-    uint32_t cur_first = 0, cur_wps = 0;
+    uint32_t cur_streams = 0, cur_fps = 0, cur_windows = 0;
     // per-stream state for CONTINUED batches (metapreprocess/imp.rs:38-42: prev_buffers and gamma_idx live as long as the
     // stream): the last T - 1 frames of every stream id on the device, frames seen so far on the host
     uint8_t *d_carry = nullptr;
     std::vector<uint64_t> n_seen, id_mark;
     uint64_t id_epoch = 0;
+    std::vector<uint32_t> first_scratch, hist_scratch;   // per chain of the batch being submitted
     // A batch is processed in chunks of whole chains: the activation buffers are sized for ONE chunk, and
     // process_host() overlaps the H2D copy of chunk c+1, the kernels of chunk c and the D2H of chunk c-1.
     uint32_t chunk_streams = 0;          // chains per chunk (capacity)
@@ -529,11 +525,24 @@ struct cova_pipeline {
         CclBuffers ccl;
         std::vector<cudaEvent_t> ev_in, ev_done;
         unsigned long long *h_cursor = nullptr;      // pinned: per-chunk cursor snapshots (2 words each)
-        uint32_t n_streams = 0, fps = 0, n_windows = 0, wps = 0;
+        uint32_t n_streams = 0, fps = 0, n_windows = 0;
         bool busy = false, failed = false, ready = false;
         uint32_t *h_ids = nullptr, *d_ids = nullptr;   // stream ids of a submit_host2 batch (pinned staging + device copy)
         std::vector<uint64_t> win_pts;                 // per window: PTS of its newest frame / stream id (submit_host2)
         std::vector<uint32_t> win_ids;
+        // Window shape of the slot's batch (set_batch_shape).  Chain s yields windows [win0[s], win0[s+1]) of the batch; its
+        // first one has its newest frame at device index first_s, the next ones follow every gamma frames.
+        //   tab[s]     = (first_s, win0[s] - win0[first chain of s's chunk])      read by enc1_fused_kernel
+        //   newest[w]  = index of window w's newest frame among its chunk's frames  read by the gather kernels
+        // Each slot owns pinned staging and a device copy, uploaded on the compute stream in order with the batch's
+        // kernels: batches of different shapes can be in flight together without draining the pipeline.
+        std::vector<uint32_t> win0;
+        int2 *h_tab = nullptr, *d_tab = nullptr;
+        int *h_newest = nullptr, *d_newest = nullptr;
+        cudaEvent_t ev_tab = nullptr;                  // recorded after the upload: the staging may be rewritten after it
+        std::vector<uint32_t> tab_first;               // what the tables hold: per-chain first, frames per chain, stream
+        uint32_t tab_fps = 0;
+        cudaStream_t tab_stream = nullptr;
     } slot[kSlots];
     int cur_slot = 0, next_submit = 0, next_collect = 0;
     int sizes_h[5], sizes_w[5];          // extents: [0] input, [1..4] encoder outputs
@@ -541,7 +550,6 @@ struct cova_pipeline {
     Geom gd[4];                          // D0in..D3in (Tn = 1): inputs of dec0..dec3
     Geom gx0f, gp1;                      // per-FRAME first-conv input (x-pair packed) and pooled output (Tn = 1, N = frames)
     uint4 *x0f = nullptr, *p1 = nullptr;
-    std::vector<int> h_newest;
     uint4 *x[4] = {nullptr, nullptr, nullptr, nullptr};
     uint4 *d[4] = {nullptr, nullptr, nullptr, nullptr};
     uint8_t *d_mask = nullptr, *d_stacked = nullptr;
@@ -651,6 +659,8 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
             cudaStreamCreateWithFlags(&p->s_out, cudaStreamNonBlocking) != cudaSuccess)
             return fail(set_err(COVA_E_CUDA, "stream creation failed"));
         for (auto &sl : p->slot) {
+            if (cudaEventCreateWithFlags(&sl.ev_tab, cudaEventDisableTiming) != cudaSuccess)
+                return fail(set_err(COVA_E_CUDA, "event creation failed"));
             sl.ev_in.resize(chunks); sl.ev_done.resize(chunks);
             for (uint32_t c = 0; c < chunks; c++)
                 if (cudaEventCreateWithFlags(&sl.ev_in[c], cudaEventDisableTiming) != cudaSuccess ||
@@ -689,7 +699,12 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
     p->frame_bytes = (size_t)w_mb * h_mb * (p->packed ? 2 : 4);
     cudaError_t e = cudaMalloc(&p->slot[0].d_frames, p->frame_bytes * max_streams * max_fps);
     p->d_frames = p->slot[0].d_frames;
-    if (e == cudaSuccess) e = cudaMalloc(&p->d_newest, sizeof(int) * std::max(1, N));
+    for (auto &sl : p->slot) {
+        if (e == cudaSuccess) e = cudaMallocHost(&sl.h_tab, sizeof(int2) * max_streams);
+        if (e == cudaSuccess) e = cudaMalloc(&sl.d_tab, sizeof(int2) * max_streams);
+        if (e == cudaSuccess) e = cudaMallocHost(&sl.h_newest, sizeof(int) * std::max(1, NB));
+        if (e == cudaSuccess) e = cudaMalloc(&sl.d_newest, sizeof(int) * std::max(1, NB));
+    }
     if (e == cudaSuccess) e = cudaMalloc(&p->d_mask, (size_t)std::max(1, NB) * w_mb * h_mb);
     if (e == cudaSuccess) e = cudaMemset(p->d_mask, 0, (size_t)std::max(1, NB) * w_mb * h_mb);
     if (e == cudaSuccess && (flags & COVA_FLAG_KEEP_LOGITS)) e = cudaMalloc(&p->d_logits, sizeof(float) * (size_t)NB * w_mb * h_mb);
@@ -750,10 +765,14 @@ extern "C" void cova_pipeline_free(cova_pipeline *p) {
         if (sl.h_cursor) cudaFreeHost(sl.h_cursor);
         if (sl.h_ids) cudaFreeHost(sl.h_ids);
         if (sl.d_ids) cudaFree(sl.d_ids);
+        if (sl.h_tab) cudaFreeHost(sl.h_tab);
+        if (sl.d_tab) cudaFree(sl.d_tab);
+        if (sl.h_newest) cudaFreeHost(sl.h_newest);
+        if (sl.d_newest) cudaFree(sl.d_newest);
+        if (sl.ev_tab) cudaEventDestroy(sl.ev_tab);
         for (auto e : sl.ev_in) cudaEventDestroy(e);
         for (auto e : sl.ev_done) cudaEventDestroy(e);
     }
-    if (p->d_newest) cudaFree(p->d_newest);
     if (p->d_carry) cudaFree(p->d_carry);
     if (p->d_mask) cudaFree(p->d_mask);
     if (p->d_logits) cudaFree(p->d_logits);
@@ -785,37 +804,53 @@ extern "C" int cova_pipeline_n_windows(const cova_pipeline *p, uint32_t n_stream
     return COVA_OK;
 }
 
-static int set_batch_shape(cova_pipeline *p, uint32_t n_streams, uint32_t fps, uint32_t first = 0xffffffffu) {
+// Window shape of a batch of n_streams device chains of fps frames each, into the tables of slot k.  first[s] is the index
+// (inside device chain s) of the newest frame of the chain's first window; nullptr = T - 1 for every chain, i.e. chains
+// that start with an empty window.  CONTINUED chains (submit_host2) start later, where their carried history and gamma
+// phase put them.  Lock-step and staggered batches go through the same tables and kernels.
+static int set_batch_shape(cova_pipeline *p, int k, uint32_t n_streams, uint32_t fps, const uint32_t *first = nullptr) {
     if (!n_streams || n_streams > p->max_streams || fps > p->max_fps)
         return set_err(COVA_E_INVAL, "batch exceeds max_streams / max_frames_per_stream of the pipeline");
-    if (first == 0xffffffffu) first = p->T - 1;                   // chains that start with an empty window
-    const uint32_t wps = windows_from(fps, first, p->gamma);
-    if ((uint64_t)n_streams * wps > p->max_windows) return set_err(COVA_E_INVAL, "batch produces more windows than the pipeline was sized for");
-    p->cur_streams = n_streams; p->cur_fps = fps; p->cur_windows = n_streams * wps;
-    p->cur_first = first; p->cur_wps = wps;
-    const uint32_t tstreams = std::min(n_streams, p->chunk_streams);
-    if (p->table_streams != tstreams || p->table_fps != fps || p->table_first != first) {
-        // chunk-relative table: window k of a chunk -> index (inside the chunk's frames) of its newest frame
-        std::vector<int> &newest = p->h_newest;
-        newest.assign(std::max<size_t>(1, (size_t)tstreams * wps), 0);
-        size_t k = 0;
-        for (uint32_t s = 0; s < tstreams; s++)
-            for (uint32_t w = 0; w < wps; w++) newest[k++] = (int)(s * fps + first + w * p->gamma);
-        if (k) COVA_CUDA(cudaMemcpyAsync(p->d_newest, newest.data(), sizeof(int) * k, cudaMemcpyHostToDevice, p->stream));
-        COVA_CUDA(cudaStreamSynchronize(p->stream));
-        p->table_streams = tstreams; p->table_fps = fps; p->table_first = first;
+    auto &sl = p->slot[k];
+    const uint32_t t1 = p->T - 1, cs = p->chunk_streams;
+    uint64_t total = 0;
+    for (uint32_t s = 0; s < n_streams; s++) total += windows_from(fps, first ? first[s] : t1, p->gamma);
+    if (total > p->max_windows) return set_err(COVA_E_INVAL, "batch produces more windows than the pipeline was sized for");
+    sl.win0.resize(n_streams + 1);
+    sl.win0[0] = 0;
+    for (uint32_t s = 0; s < n_streams; s++) sl.win0[s + 1] = sl.win0[s] + windows_from(fps, first ? first[s] : t1, p->gamma);
+    p->cur_streams = n_streams; p->cur_fps = fps; p->cur_windows = (uint32_t)total;
+    bool same = sl.tab_fps == fps && sl.tab_stream == p->stream && sl.tab_first.size() == n_streams;
+    for (uint32_t s = 0; same && s < n_streams; s++) same = sl.tab_first[s] == (first ? first[s] : t1);
+    if (same) return COVA_OK;                                      // the slot's device tables already hold this shape
+    // The staging may still be read by this slot's previous upload when synchronous entry points reuse slot 0 back to back.
+    // On the submit path that upload has completed: the slot's previous batch was collected.
+    COVA_CUDA(cudaEventSynchronize(sl.ev_tab));
+    sl.tab_first.clear();                                          // invalid until the upload below is enqueued
+    for (uint32_t s = 0; s < n_streams; s++) {
+        const uint32_t f = first ? first[s] : t1, c0 = s / cs * cs;
+        sl.h_tab[s] = make_int2((int)f, (int)(sl.win0[s] - sl.win0[c0]));
+        for (uint32_t w = sl.win0[s]; w < sl.win0[s + 1]; w++)
+            sl.h_newest[w] = (int)((s - c0) * fps + f + (w - sl.win0[s]) * p->gamma);
     }
+    COVA_CUDA(cudaMemcpyAsync(sl.d_tab, sl.h_tab, sizeof(int2) * n_streams, cudaMemcpyHostToDevice, p->stream));
+    if (total) COVA_CUDA(cudaMemcpyAsync(sl.d_newest, sl.h_newest, sizeof(int) * total, cudaMemcpyHostToDevice, p->stream));
+    COVA_CUDA(cudaEventRecord(sl.ev_tab, p->stream));
+    if (first) sl.tab_first.assign(first, first + n_streams);
+    else sl.tab_first.assign(n_streams, t1);
+    sl.tab_fps = fps; sl.tab_stream = p->stream;
     return COVA_OK;
 }
 
 static void use_slot(cova_pipeline *p, int k);
 static uint32_t n_chunks_of(const cova_pipeline *p) { return (p->cur_streams + p->chunk_streams - 1) / p->chunk_streams; }
 static void select_chunk(cova_pipeline *p, uint32_t c) {
-    const uint32_t wps = p->cur_wps;
+    const std::vector<uint32_t> &win0 = p->slot[p->cur_slot].win0;
     p->ck_stream0 = c * p->chunk_streams;
     p->ck_n_streams = std::min(p->chunk_streams, p->cur_streams - p->ck_stream0);
-    p->ck_window0 = p->ck_stream0 * wps;
-    p->ck_windows = p->ck_n_streams * wps;
+    if (!p->ck_n_streams) { p->ck_window0 = p->ck_windows = 0; return; }      // masks loaded directly: no chains
+    p->ck_window0 = win0[p->ck_stream0];
+    p->ck_windows = win0[p->ck_stream0 + p->ck_n_streams] - p->ck_window0;
 }
 static int require_single_chunk(cova_pipeline *p) {
     if (p->cur_streams > p->chunk_streams)
@@ -827,7 +862,7 @@ static int require_single_chunk(cova_pipeline *p) {
 extern "C" int cova_pipeline_load_frames(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, uint32_t fps, int is_device) {
     if (!p || !frames) return set_err(COVA_E_INVAL, "null argument");
     COVA_CUDA(cudaSetDevice(p->device));
-    int rc = set_batch_shape(p, n_streams, fps);
+    int rc = set_batch_shape(p, 0, n_streams, fps);
     if (rc) return rc;
     use_slot(p, 0);
     COVA_CUDA(cudaMemcpyAsync(p->d_frames, frames, p->frame_bytes * n_streams * fps,
@@ -849,18 +884,19 @@ static int tensorise_chunk(cova_pipeline *p) {
     const int N = (int)p->ck_windows;
     if (!N) return COVA_OK;
     const uint8_t *frames = p->d_frames + (size_t)p->ck_stream0 * p->cur_fps * p->frame_bytes;
+    const int *newest = p->slot[p->cur_slot].d_newest + p->ck_window0;      // chunk-relative, like the frames
     if (p->d_stacked) {
         const size_t S = p->frame_bytes;
         uint8_t *dst = p->d_stacked + (size_t)p->ck_window0 * p->T * S;
         if (S % 16 == 0) {
             long long total = (long long)N * p->T * (S / 16);
             int blocks = (int)std::min<long long>((total + 255) / 256, (long long)p->n_sms * 16);
-            stack_rgba_kernel<uint4><<<blocks, 256, 0, p->stream>>>(reinterpret_cast<const uint4 *>(frames), p->d_newest,
+            stack_rgba_kernel<uint4><<<blocks, 256, 0, p->stream>>>(reinterpret_cast<const uint4 *>(frames), newest,
                                                                    reinterpret_cast<uint4 *>(dst), (int)(S / 16), (int)p->T, total);
         } else {
             long long total = (long long)N * p->T * (S / 4);
             int blocks = (int)std::min<long long>((total + 255) / 256, (long long)p->n_sms * 16);
-            stack_rgba_kernel<uint32_t><<<blocks, 256, 0, p->stream>>>(reinterpret_cast<const uint32_t *>(frames), p->d_newest,
+            stack_rgba_kernel<uint32_t><<<blocks, 256, 0, p->stream>>>(reinterpret_cast<const uint32_t *>(frames), newest,
                                                                       reinterpret_cast<uint32_t *>(dst), (int)(S / 4), (int)p->T, total);
         }
         COVA_CUDA(cudaGetLastError());
@@ -882,7 +918,7 @@ static int tensorise_chunk(cova_pipeline *p) {
     if (p->x[0]) {   // window-layout input of the validation kernels
         long long total = (long long)N * p->H * p->gx[0].Wh * kT;
         int blocks = (int)std::min<long long>((total + 255) / 256, (long long)p->n_sms * 32);
-        tensorise_x0_kernel<<<blocks, 256, 0, p->stream>>>(reinterpret_cast<const uint32_t *>(frames), p->d_newest, p->x[0], p->gx[0], N);
+        tensorise_x0_kernel<<<blocks, 256, 0, p->stream>>>(reinterpret_cast<const uint32_t *>(frames), newest, p->x[0], p->gx[0], N);
         COVA_CUDA(cudaGetLastError());
         p->launches++;
         prof_mark(p, "tensorise_x0");
@@ -1032,8 +1068,8 @@ static int tc_layer(cova_pipeline *p, int layer) {
                 fp.in = p->x0f; fp.gin = p->gx0f; fp.out = p->x[1]; fp.gout = p->gx[1]; fp.N = F;
                 tc1::Enc1Extra ex;
                 memset(&ex, 0, sizeof(ex));
-                ex.n_chains = (int)p->ck_n_streams; ex.fps = (int)p->cur_fps; ex.wps = (int)p->cur_wps;
-                ex.gamma = (int)p->gamma; ex.first = (int)p->cur_first;
+                ex.n_chains = (int)p->ck_n_streams; ex.fps = (int)p->cur_fps; ex.gamma = (int)p->gamma;
+                ex.tab = p->slot[p->cur_slot].d_tab + p->ck_stream0;
                 cudaError_t err = cudaSuccess;
                 if (tc1::try_launch_enc1(fp, ex, p->n_sms, p->stream, err)) {
                     if (err != cudaSuccess) return set_err(COVA_E_CUDA, "fused enc1 launch: %s", cudaGetErrorString(err));
@@ -1050,8 +1086,8 @@ static int tc_layer(cova_pipeline *p, int layer) {
             prof_mark(p, "tc_enc1_conv");
             TnArgs ta;
             ta.p1 = p->p1; ta.gp1 = p->gp1; ta.x1 = p->x[1]; ta.gx1 = p->gx[1]; ta.skip = p->d[3]; ta.gskip = p->gd[3];
-            ta.skip_cb = kDecCout[2] / 8; ta.newest = p->d_newest; ta.n_windows = N;
-            ta.wps = p->cur_wps; ta.fps = p->cur_fps; ta.gamma = p->gamma; ta.first = p->cur_first; ta.CB = kEncCout[0] / 8;
+            ta.skip_cb = kDecCout[2] / 8; ta.newest = p->slot[p->cur_slot].d_newest + p->ck_window0; ta.n_windows = N;
+            ta.CB = kEncCout[0] / 8;
             memcpy(ta.w1, p->hw.enc[0].tn_w1, 64);
             memcpy(ta.w2, p->hw.enc[0].tn_w2, 64);
             long long total = (long long)ta.CB * 4 * N * p->gx[1].S;
@@ -1302,10 +1338,17 @@ __global__ void __launch_bounds__(256) carry_kernel(uint32_t *__restrict__ pool,
 // COVA_SUBMIT_CONTINUE the chains of this batch continue the streams `stream_ids` from where their previous batch left
 // them - the carried T - 1 frames are put in front of the new ones on the device and the gamma phase continues, so a
 // stream cut into batches yields exactly the windows of the uncut stream.
+//
+// COVA_SUBMIT_STAGGERED lets the continued streams of one batch differ in history h_s = min(seen_s, T - 1) and gamma phase.
+// Every device chain then has fps + lead frames, lead = max_s h_s: the new frames start at index lead, the carried ones sit
+// right-aligned in front of them at [lead - h_s, lead), and what lies before that is never read by an emitted window.  So
+// the copies and the per-frame kernels see one uniform chain length, and only the window -> frame tables differ per chain.
 static int submit_impl(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, uint32_t fps, const uint32_t *stream_ids,
                        const uint64_t *pts, uint32_t flags, bool stateful) {
     if (!p || !frames) return set_err(COVA_E_INVAL, "null argument");
-    if (flags & ~COVA_SUBMIT_CONTINUE) return set_err(COVA_E_INVAL, "unknown submit flag");
+    if (flags & ~(COVA_SUBMIT_CONTINUE | COVA_SUBMIT_STAGGERED)) return set_err(COVA_E_INVAL, "unknown submit flag");
+    if ((flags & COVA_SUBMIT_STAGGERED) && !(flags & COVA_SUBMIT_CONTINUE))
+        return set_err(COVA_E_INVAL, "COVA_SUBMIT_STAGGERED needs COVA_SUBMIT_CONTINUE");
     COVA_CUDA(cudaSetDevice(p->device));
     const int k = p->next_submit;
     if (p->slot[k].busy) return set_err(COVA_E_INVAL, "four batches are already in flight: collect one first");
@@ -1314,7 +1357,10 @@ static int submit_impl(cova_pipeline *p, const uint8_t *frames, uint32_t n_strea
     if (!n_streams || n_streams > p->max_streams) return set_err(COVA_E_INVAL, "batch exceeds max_streams of the pipeline");
     auto &sl = p->slot[k];
     const uint32_t t1 = p->T - 1;
-    uint32_t h = 0, first = t1;
+    uint32_t lead = 0;                                              // carried frames in front of every device chain
+    std::vector<uint32_t> &first = p->first_scratch, &hist = p->hist_scratch;
+    first.assign(n_streams, t1);
+    hist.assign(n_streams, 0);
     if (stateful) {
         if (!fps) return set_err(COVA_E_INVAL, "a stream batch needs at least one frame per stream");
         if (p->n_seen.empty()) { p->n_seen.assign(p->max_streams, 0); p->id_mark.assign(p->max_streams, 0); }
@@ -1326,18 +1372,20 @@ static int submit_impl(cova_pipeline *p, const uint8_t *frames, uint32_t n_strea
             p->id_mark[id] = p->id_epoch;
         }
         if (flags & COVA_SUBMIT_CONTINUE) {
-            // the kernels take one window shape per batch: every chain must carry the same number of frames and sit at the
-            // same gamma phase, i.e. the streams of a batch advance in lock-step (start new streams in a batch of their own)
             for (uint32_t s = 0; s < n_streams; s++) {
                 const uint64_t seen = p->n_seen[stream_ids ? stream_ids[s] : s];
                 const uint32_t hs = (uint32_t)std::min<uint64_t>(seen, t1);
-                const uint64_t base = seen - hs;                    // frames of the stream in front of the device chain
-                // smallest index i' >= T-1 of the device chain with (base + i' - (T-1)) % gamma == 0 (imp.rs:321-330)
-                const uint32_t fs = t1 + (uint32_t)((p->gamma - base % p->gamma) % p->gamma);
-                if (s == 0) { h = hs; first = fs; }
-                else if (hs != h || fs != first)
-                    return set_err(COVA_E_INVAL, "streams of one CONTINUED batch must have the same history length and gamma phase");
+                const uint64_t base = seen - hs;                    // frames of the stream in front of its carried ones
+                // smallest index i' >= T-1 of the unpadded chain with (base + i' - (T-1)) % gamma == 0 (imp.rs:321-330)
+                hist[s] = hs;
+                first[s] = t1 + (uint32_t)((p->gamma - base % p->gamma) % p->gamma);
+                lead = std::max(lead, hs);
+                // without COVA_SUBMIT_STAGGERED the streams of a batch advance in lock-step: same history, same gamma phase
+                if (!(flags & COVA_SUBMIT_STAGGERED) && s && (hs != hist[0] || first[s] != first[0]))
+                    return set_err(COVA_E_INVAL, "streams of one CONTINUED batch must have the same history length and gamma phase "
+                                                 "(or pass COVA_SUBMIT_STAGGERED)");
             }
+            for (uint32_t s = 0; s < n_streams; s++) first[s] += lead - hist[s];   // chain s is padded by lead - h_s frames
         }
         if (!p->d_carry && t1) {
             COVA_CUDA(cudaMalloc(&p->d_carry, (size_t)p->max_streams * t1 * p->frame_bytes));
@@ -1348,23 +1396,23 @@ static int submit_impl(cova_pipeline *p, const uint8_t *frames, uint32_t n_strea
             COVA_CUDA(cudaMalloc(&sl.d_ids, sizeof(uint32_t) * p->max_streams));
         }
     }
-    const uint32_t fps_dev = fps + h;                               // frames per chain on the device
+    const uint32_t fps_dev = fps + lead;                            // frames per chain on the device
     if (fps_dev > p->max_fps)
         return set_err(COVA_E_INVAL, "carried frames + new frames exceed max_frames_per_stream of the pipeline");
-    if ((rc = set_batch_shape(p, n_streams, fps_dev, first))) return rc;
+    if ((rc = set_batch_shape(p, k, n_streams, fps_dev, first.data()))) return rc;
     use_slot(p, k);
-    sl.n_streams = n_streams; sl.fps = fps_dev; sl.n_windows = p->cur_windows; sl.wps = p->cur_wps;
+    sl.n_streams = n_streams; sl.fps = fps_dev; sl.n_windows = p->cur_windows;
     sl.win_pts.clear(); sl.win_ids.clear();
     if (stateful) {
-        // window w of chain s has its newest frame at device index first + w*gamma = new-frame index first + w*gamma - h
+        // window w of chain s has its newest frame at device index first_s + w*gamma = new-frame index first_s + w*gamma - lead
         sl.win_ids.resize(sl.n_windows);
         if (pts) sl.win_pts.resize(sl.n_windows);
         for (uint32_t s = 0; s < n_streams; s++) {
             const uint32_t id = stream_ids ? stream_ids[s] : s;
             sl.h_ids[s] = id;
-            for (uint32_t w = 0; w < sl.wps; w++) {
-                sl.win_ids[(size_t)s * sl.wps + w] = id;
-                if (pts) sl.win_pts[(size_t)s * sl.wps + w] = pts[(size_t)s * fps + (first + w * p->gamma - h)];
+            for (uint32_t w = sl.win0[s]; w < sl.win0[s + 1]; w++) {
+                sl.win_ids[w] = id;
+                if (pts) sl.win_pts[w] = pts[(size_t)s * fps + (first[s] + (w - sl.win0[s]) * p->gamma - lead)];
             }
             p->n_seen[id] = ((flags & COVA_SUBMIT_CONTINUE) ? p->n_seen[id] : 0) + fps;
         }
@@ -1381,11 +1429,11 @@ static int submit_impl(cova_pipeline *p, const uint8_t *frames, uint32_t n_strea
         if (_e != cudaSuccess) return fail(cova::set_err(COVA_E_CUDA, "%s: %s", #expr, cudaGetErrorString(_e)));    \
     } while (0)
     const uint32_t nc = n_chunks_of(p);
-    const size_t src_chain = p->frame_bytes * fps, dst_chain = p->frame_bytes * fps_dev, lead = p->frame_bytes * h;
+    const size_t src_chain = p->frame_bytes * fps, dst_chain = p->frame_bytes * fps_dev, lead_bytes = p->frame_bytes * lead;
     for (uint32_t c = 0; c < nc; c++) {
         const size_t s0 = (size_t)c * p->chunk_streams, ns = std::min<size_t>(p->chunk_streams, n_streams - s0);
-        if (!h) COVA_CUDA_SLOT(cudaMemcpyAsync(sl.d_frames + s0 * dst_chain, frames + s0 * src_chain, ns * src_chain, cudaMemcpyHostToDevice, p->s_in));
-        else COVA_CUDA_SLOT(cudaMemcpy2DAsync(sl.d_frames + s0 * dst_chain + lead, dst_chain, frames + s0 * src_chain, src_chain, src_chain, ns,
+        if (!lead) COVA_CUDA_SLOT(cudaMemcpyAsync(sl.d_frames + s0 * dst_chain, frames + s0 * src_chain, ns * src_chain, cudaMemcpyHostToDevice, p->s_in));
+        else COVA_CUDA_SLOT(cudaMemcpy2DAsync(sl.d_frames + s0 * dst_chain + lead_bytes, dst_chain, frames + s0 * src_chain, src_chain, src_chain, ns,
                                               cudaMemcpyHostToDevice, p->s_in));
         COVA_CUDA_SLOT(cudaEventRecord(sl.ev_in[c], p->s_in));
     }
@@ -1398,11 +1446,11 @@ static int submit_impl(cova_pipeline *p, const uint8_t *frames, uint32_t n_strea
             const int ns = (int)std::min<size_t>(p->chunk_streams, n_streams - s0);
             uint32_t *pool = reinterpret_cast<uint32_t *>(sl.d_frames + s0 * dst_chain);
             const int blocks = std::min(p->n_sms * 8, std::max(1, (int)(((long long)ns * t1 * wpf + 255) / 256)));
-            if (h) {
-                carry_kernel<<<blocks, 256, 0, p->stream>>>(pool, reinterpret_cast<uint32_t *>(p->d_carry), sl.d_ids + s0, ns, wpf, (int)fps_dev, (int)h, (int)t1, 0);
+            if (lead) {     // lead frames for every chain: a chain with less history gets older carry bytes no window reads
+                carry_kernel<<<blocks, 256, 0, p->stream>>>(pool, reinterpret_cast<uint32_t *>(p->d_carry), sl.d_ids + s0, ns, wpf, (int)fps_dev, (int)lead, (int)t1, 0);
                 p->launches++;
             }
-            carry_kernel<<<blocks, 256, 0, p->stream>>>(pool, reinterpret_cast<uint32_t *>(p->d_carry), sl.d_ids + s0, ns, wpf, (int)fps_dev, (int)h, (int)t1, 1);
+            carry_kernel<<<blocks, 256, 0, p->stream>>>(pool, reinterpret_cast<uint32_t *>(p->d_carry), sl.d_ids + s0, ns, wpf, (int)fps_dev, (int)lead, (int)t1, 1);
             p->launches++;
             COVA_CUDA_SLOT(cudaGetLastError());
         }
@@ -1460,15 +1508,14 @@ static int collect_impl(cova_pipeline *p, uint8_t *blob, size_t blob_cap, size_t
         if (nc && cudaEventSynchronize(sl.ev_done[nc - 1]) != cudaSuccess) return sync_stream(p, p->stream);
         return COVA_OK;
     }
-    const uint32_t wps = sl.wps;
     unsigned long long prev = 0;
     bool too_small = false;
     for (uint32_t c = 0; c < nc; c++) {
         if (cudaEventSynchronize(sl.ev_done[c]) != cudaSuccess) return sync_stream(p, p->stream);
         if (sl.h_cursor[2 * c + 1]) return set_err(COVA_E_CUDA, "device box arena overflow (internal sizing error)");
         const unsigned long long end = sl.h_cursor[2 * c];
-        const size_t w0 = (size_t)c * p->chunk_streams * wps;
-        const size_t nw = (size_t)std::min<uint32_t>(p->chunk_streams, sl.n_streams - c * p->chunk_streams) * wps;
+        const size_t w0 = sl.win0[c * p->chunk_streams];
+        const size_t nw = sl.win0[std::min<uint32_t>((c + 1) * p->chunk_streams, sl.n_streams)] - w0;
         if (offsets) COVA_CUDA(cudaMemcpyAsync(offsets + w0, sl.ccl.d_offsets + w0, nw * sizeof(uint64_t), cudaMemcpyDeviceToHost, p->s_out));
         if (lens) COVA_CUDA(cudaMemcpyAsync(lens + w0, sl.ccl.d_lens + w0, nw * sizeof(uint64_t), cudaMemcpyDeviceToHost, p->s_out));
         if (blob && end <= blob_cap) {
@@ -1561,7 +1608,7 @@ extern "C" int cova_pipeline_read_activation(cova_pipeline *p, int layer, float 
                 for (int t = 0; t < kT; t++)
                     for (int y = 0; y < gf.H; y++)
                         for (int x = 0; x < gf.W; x++) {
-                            const int f = p->h_newest[nn] - t;
+                            const int f = p->slot[p->cur_slot].h_newest[p->ck_window0 + nn] - t;
                             const Row8 &r = host[(size_t)geom_row(gf, 0, (y & 1) << 1, geom_pos(gf, f, y >> 1, x >> 1, 0))];
                             out[((((size_t)nn * 3 + c) * kT + t) * gf.H + y) * gf.W + x] = __half2float(r.v[(x & 1) * 4 + c]);
                         }

@@ -151,8 +151,7 @@ struct TnArgs {
     uint4 *x1; Geom gx1;             // next encoder input (Tn = 4)
     uint4 *skip; Geom gskip;         // decoder concat buffer (Tn = 1)
     int skip_cb;
-    const int *newest;
-    uint32_t wps, fps, gamma, first;   // windows per chain, frames per chain, sub-sampling: newest[n] in closed form
+    const int *newest;               // per window of the chunk: index of its newest frame among the chunk's frames
     float w1[16], w2[16];
     int n_windows, CB;
 };
@@ -166,8 +165,7 @@ __global__ void __launch_bounds__(256) pointwise_tn_kernel(const __grid_constant
         const uint32_t y2 = s / P, x2 = s - y2 * P;
         const uint32_t ph = pl & 3u;
         if (2 * y2 + (ph >> 1) >= (uint32_t)A.gx1.H || 2 * x2 + (ph & 1) >= (uint32_t)A.gx1.W) continue;   // shared zero row / column
-        const uint32_t chain = n / A.wps;
-        const int f0 = (int)(chain * A.fps + A.first + (n - chain * A.wps) * A.gamma);   // == A.newest[n], without the dependent load
+        const int f0 = __ldg(A.newest + n);      // chains of a staggered batch have different window shapes
         const uint4 *src = A.p1 + ((long long)pl * A.gp1.Lp + A.gp1.guard + (long long)f0 * S + s);
         uint4 in[4];
 #pragma unroll

@@ -480,16 +480,18 @@ class BlobPipeline:
         return n_windows * (8 + 24 * ((self.h_mb + 1) // 2) * ((self.w_mb + 1) // 2))
 
     # ---- asynchronous streaming form: at most four batches in flight
-    def submit(self, frames: np.ndarray, blob_cap: int | None = None, stream_ids=None, pts=None, cont: bool | None = None):
+    def submit(self, frames: np.ndarray, blob_cap: int | None = None, stream_ids=None, pts=None, cont: bool | None = None,
+               staggered: bool = False):
         """Enqueue one batch (copies + kernels) and return immediately.  `frames` should live in page-locked
         memory (PinnedBuffer) and must stay untouched until the matching collect().
 
         With `stream_ids` / `pts` / `cont` the batch goes through cova_pipeline_submit_host2: chain s belongs to stream
         stream_ids[s] (default 0, 1, ...), `pts[s, f]` is echoed per window by collect(meta=True), and cont=True continues
         the streams from their previous batch (carried timestep-1 frames + gamma phase) like one long-lived metapreprocess
-        element would."""
+        element would.  staggered=True (with cont=True) lets those streams differ in history and gamma phase: each continues
+        from its own state, so chains may yield different numbers of windows (collect(meta=True) maps them to streams)."""
         a = self._frames(frames)
-        if stream_ids is None and pts is None and cont is None:
+        if stream_ids is None and pts is None and cont is None and not staggered:
             self._ensure_out(blob_cap or self._worst_case_cap(self.windows_for(a.shape[0], a.shape[1])))
             self._check(self._L.cova_pipeline_submit_host(self._h, _ptr(a), a.shape[0], a.shape[1]))
         else:
@@ -500,7 +502,8 @@ class BlobPipeline:
             assert ids is None or ids.shape == (a.shape[0],)
             assert p is None or p.shape == a.shape[:2]
             self._check(self._L.cova_pipeline_submit_host2(self._h, _ptr(a), a.shape[0], a.shape[1], None if ids is None else _ptr(ids),
-                                                         None if p is None else _ptr(p), _lib.SUBMIT_CONTINUE if cont else 0))
+                                                         None if p is None else _ptr(p),
+                                                         (_lib.SUBMIT_CONTINUE if cont else 0) | (_lib.SUBMIT_STAGGERED if staggered else 0)))
         self._inflight = getattr(self, "_inflight", []) + [a]
 
     def reset_streams(self, stream_ids=None):

@@ -188,13 +188,21 @@ int cova_pipeline_collect_host(cova_pipeline *p, uint8_t *blob, size_t blob_cap,
  *          the device) precede the new ones and the gamma phase carries on, so the batch yields exactly the windows the
  *          uncut stream would have produced for these frames (frames_per_stream windows per chain at gamma 1).
  *          Without the flag the named streams (re)start with an empty window.  Either way their state is recorded.
- * Constraints: the streams of one CONTINUED batch must advance in lock-step (same number of frames seen so far modulo
- * nothing: same history length min(seen, timestep-1) and same gamma phase) - COVA_E_INVAL otherwise; carried + new
- * frames must fit max_frames_per_stream.  Window order stays stream-major, time-minor.
+ *          COVA_SUBMIT_STAGGERED (only together with COVA_SUBMIT_CONTINUE): the streams of the batch need not be in
+ *          lock-step.  Each chain continues its stream from that stream's own state - its own history
+ *          h_s = min(seen_s, timestep-1) and its own gamma phase; a stream never seen (or reset) starts with an empty
+ *          window - and yields exactly the windows its uncut stream would yield for these frames.  Chains may therefore
+ *          yield different numbers of windows: map windows to streams with collect_host2's win_stream_ids.
+ *          Any other flag bit, or STAGGERED without CONTINUE: COVA_E_INVAL before any device call.
+ * Constraints: without COVA_SUBMIT_STAGGERED the streams of one CONTINUED batch must advance in lock-step (same history
+ * length min(seen, timestep-1) and same gamma phase) - COVA_E_INVAL otherwise; pass COVA_SUBMIT_STAGGERED to lift this
+ * rule.  frames_per_stream is the same for every stream of a call, and frames_per_stream + max_s h_s must fit
+ * max_frames_per_stream.  Window order stays stream-major, time-minor.
  * collect_host2: as collect_host, plus per window the stream id and the PTS of its newest frame (the PTS the
  * reference's metapreprocess output buffer carries, BaseTransform default; cova/imp.rs:110-112 requires it).
  * Both arrays have n_windows entries; win_pts is only written when the submit passed pts. */
 #define COVA_SUBMIT_CONTINUE 1u
+#define COVA_SUBMIT_STAGGERED 2u
 int cova_pipeline_submit_host2(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, uint32_t frames_per_stream,
                                const uint32_t *stream_ids, const uint64_t *pts, uint32_t flags);
 int cova_pipeline_collect_host2(cova_pipeline *p, uint8_t *blob, size_t blob_cap, size_t *blob_len, uint64_t *offsets,
