@@ -8,9 +8,8 @@
 // runs the 12 MMAs of the frame-level conv (same operand layout as tc::issue_tile<ENCF>), and the epilogue thread
 // that owns (position, channel block) keeps the pooled fp16 activations of the three previous frames in REGISTERS -
 // so the window's PointWiseTN input never touches shared memory or HBM.  Per step the kernel writes the window's
-// four time planes of X1 (next encoder input) and the t = 0 skip row of the decoder concat buffer; the per-frame
-// pooled tensor P1 and the separate gather kernel of the unfused path disappear (their traffic: 0.3 GB written +
-// 0.3 GB read per 8192 windows at 720p).
+// four time planes of X1 (next encoder input) and the t = 0 skip row of the decoder concat buffer; no per-frame pooled
+// tensor goes through HBM (it would be 0.3 GB written + 0.3 GB read per 8192 windows at 720p).
 //
 // Work item = (chain, tile pair, segment of frames); a segment after the first re-computes 3 warm-up frames.
 // Warp roles as in blobnet_tc.cuh: warp 0 producer, warp 1 TMEM owner + MMA issuer, 16 epilogue warps
@@ -200,7 +199,7 @@ __global__ void __launch_bounds__(kThreads1, 1) enc1_fused_kernel(const __grid_c
                                    (long long)cw.y * p.gout2.S;
             const int first = cw.x;
             // Ring of the last four pooled frames: ring[s][k] = channel pair (2k, 2k+1) of the frame whose index is s mod 4,
-            // as fp32 values already rounded to fp16 (what the two-kernel path stores and re-reads).  The frame loop is
+            // as fp32 values already rounded to fp16 (the pooled activation is an fp16 tensor).  The frame loop is
             // unrolled four times over the ring phase R, so "frame i - t" is the compile-time slot (R - t) & 3: no
             // rotation moves, and one fp16 round trip per frame instead of one conversion per frame and window.
             float2 ring[4][4];

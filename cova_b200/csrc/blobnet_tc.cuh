@@ -22,7 +22,7 @@
 namespace cova {
 namespace tc {
 
-constexpr int MODE_ENC = 0, MODE_DEC = 1, MODE_HEAD = 2, MODE_ENCF = 3;   // ENCF: first conv, per FRAME (no PointWiseTN)
+constexpr int MODE_ENC = 0, MODE_DEC = 1, MODE_HEAD = 2, MODE_ENCF = 3;   // ENCF: first conv, per FRAME (MMAs of blobnet_enc1.cuh)
 constexpr int kMaxStage = 4;
 constexpr int kEpiWarps = 16;                 // 4 groups of 4 warps (one per TMEM lane quarter)
 constexpr int kThreads = 64 + 32 * kEpiWarps;
@@ -200,7 +200,7 @@ template <class C>
 __host__ __device__ constexpr int epi_floats() {
     // encoder: bias|scale|shift, two 4x4 TN matrices, then 256 floats of exchange scratch per epilogue warp
     return C::MODE == MODE_ENC ? 3 * C::COUT + 32 + kEpiWarps * 8 * kScratchPitch
-                               : (C::MODE == MODE_ENCF ? 3 * C::COUT : (C::MODE == MODE_DEC ? 2 * C::COUT + kEpiWarps * kDecScratchRows * 4 : 4));
+                               : (C::MODE == MODE_DEC ? 2 * C::COUT + kEpiWarps * kDecScratchRows * 4 : 4);
 }
 
 // ------------------------------------------------------------------------------------------------ MMA issue
@@ -427,50 +427,6 @@ __device__ __forceinline__ void epilogue_enc(const LayerParams &p, const float *
     }
 }
 
-// First conv, per frame: bias -> ReLU -> BatchNorm -> 2x2 max-pool, stored as fp16 rows (pre-PointWiseTN)
-template <class C>
-__device__ __forceinline__ void epilogue_encf(const LayerParams &p, const float *epi, uint32_t taddr, int pp, int cg) {
-    const Geom &gi = p.gin;
-    const int f = (int)fast_div((uint32_t)pp, p.divS);
-    const int r = pp - f * gi.S;
-    const int y2 = (int)fast_div((uint32_t)r, p.divP), x2 = r - y2 * gi.P;
-    const bool valid = f < p.N && y2 < (gi.H >> 1) && x2 < (gi.W >> 1);
-    const int Y = y2 + (gi.H & 1), X = x2 + (gi.W & 1);          // zero-pad top / left when odd (encoder.py:68-76)
-    long long row = 0;
-    if (valid) row = geom_row(p.gout, 0, ((Y & 1) << 1) | (X & 1), geom_pos(p.gout, f, Y >> 1, X >> 1, 0));
-    const float4 *bias4 = reinterpret_cast<const float4 *>(epi), *scale4 = reinterpret_cast<const float4 *>(epi + C::COUT),
-                 *shift4 = reinterpret_cast<const float4 *>(epi + 2 * C::COUT);
-    constexpr int CB_PER = (C::COUT / 8) / C::CG;
-#pragma unroll 1
-    for (int cb = cg * CB_PER; cb < (cg + 1) * CB_PER; cb++) {
-        uint32_t v[4][8];
-#pragma unroll
-        for (int ph = 0; ph < 4; ph++) tmem_ld8(taddr + (uint32_t)(ph * C::NCOLS + cb * 8), v[ph]);
-        float bs[8], sc[8], sh[8], o[8];
-        *reinterpret_cast<float4 *>(bs) = bias4[cb * 2]; *reinterpret_cast<float4 *>(bs + 4) = bias4[cb * 2 + 1];
-        *reinterpret_cast<float4 *>(sc) = scale4[cb * 2]; *reinterpret_cast<float4 *>(sc + 4) = scale4[cb * 2 + 1];
-        *reinterpret_cast<float4 *>(sh) = shift4[cb * 2]; *reinterpret_cast<float4 *>(sh + 4) = shift4[cb * 2 + 1];
-        tmem_wait_ld();
-#pragma unroll
-        for (int j = 0; j < 8; j++) {
-            const float a0 = __uint_as_float(v[0][j]), a1 = __uint_as_float(v[1][j]);
-            const float a2 = __uint_as_float(v[2][j]), a3 = __uint_as_float(v[3][j]);
-            float ext = fmaxf(fmaxf(a0, a1), fmaxf(a2, a3));      // see epilogue_enc: pool before the monotone ReLU/BN
-            if (!p.bn_nonneg) {
-                const float lo = fminf(fminf(a0, a1), fminf(a2, a3));
-                ext = sc[j] >= 0.f ? ext : lo;
-            }
-            o[j] = fmaf(fmaxf(ext + bs[j], 0.f), sc[j], sh[j]);
-        }
-        if (valid) {
-            uint4 rw;
-            rw.x = pack_half2(o[0], o[1]); rw.y = pack_half2(o[2], o[3]);
-            rw.z = pack_half2(o[4], o[5]); rw.w = pack_half2(o[6], o[7]);
-            p.out[row + (long long)cb * 4 * p.gout.Lp] = rw;
-        }
-    }
-}
-
 // Decoder tail.  Warp group g takes the input-row phase pa = g >> 1, BOTH column phases pb, and every second output parity
 // of the CTA (pl = g & 1, g & 1 + 2, ...).  Why both pb: output column X = 4*x2 + 2*pb + px - crop_l, so within one output
 // phase plane the rows of consecutive input positions x2 alternate between pb = 0 and pb = 1.  A warp that stores one pb
@@ -569,6 +525,7 @@ __device__ __forceinline__ void epilogue_head(const LayerParams &p, const float 
 // ------------------------------------------------------------------------------------------------ kernel
 template <class C>
 __global__ void __launch_bounds__(kThreads, 1) shiftgemm_kernel(const __grid_constant__ LayerParams p) {
+    static_assert(!C::ENCF, "the first block runs tc1::enc1_fused_kernel");
     extern __shared__ __align__(1024) unsigned char smem[];
     const SmemPlan sp = plan_smem<C>(p.Ls, p.n_stage, p.w_bytes, epi_floats<C>());
     const uint32_t smem_base = smem_u32(smem);
@@ -723,7 +680,6 @@ __global__ void __launch_bounds__(kThreads, 1) shiftgemm_kernel(const __grid_con
                     }
                     if (p.dbg & 2) {
                     }
-                    else if constexpr (C::MODE == MODE_ENCF) epilogue_encf<C>(p, epi, taddr, pp, cg);
                     else if constexpr (C::MODE == MODE_DEC)
                         epilogue_dec<C>(p, epi, reinterpret_cast<uint4 *>(epi + 2 * C::COUT) + (warp - 2) * kDecScratchRows, taddr, pp, half, cg, lane);
                     else epilogue_head<C>(p, epi, taddr, pp, cg);

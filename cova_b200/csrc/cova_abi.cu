@@ -548,8 +548,8 @@ struct cova_pipeline {
     int sizes_h[5], sizes_w[5];          // extents: [0] input, [1..4] encoder outputs
     Geom gx[4];                          // X0..X3 (Tn = 4): inputs of enc1..enc4
     Geom gd[4];                          // D0in..D3in (Tn = 1): inputs of dec0..dec3
-    Geom gx0f, gp1;                      // per-FRAME first-conv input (x-pair packed) and pooled output (Tn = 1, N = frames)
-    uint4 *x0f = nullptr, *p1 = nullptr;
+    Geom gx0f;                           // per-FRAME first-conv input (x-pair packed, Tn = 1, N = frames)
+    uint4 *x0f = nullptr;
     uint4 *x[4] = {nullptr, nullptr, nullptr, nullptr};
     uint4 *d[4] = {nullptr, nullptr, nullptr, nullptr};
     uint8_t *d_mask = nullptr, *d_stacked = nullptr;
@@ -692,9 +692,7 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
     }
     const int F = (int)(p->chunk_streams * max_fps);
     p->gx0f = make_geom(p->sizes_h[0], p->sizes_w[0], 8, 1, F);
-    p->gp1 = make_geom(p->sizes_h[1], p->sizes_w[1], kEncCout[0], 1, F);
     if ((rc = alloc_zero(&p->x0f, p->gx0f))) return fail(rc);
-    if ((rc = alloc_zero(&p->p1, p->gp1))) return fail(rc);
     p->packed = (flags & COVA_FLAG_INPUT_PACKED16) != 0;
     p->frame_bytes = (size_t)w_mb * h_mb * (p->packed ? 2 : 4);
     cudaError_t e = cudaMalloc(&p->slot[0].d_frames, p->frame_bytes * max_streams * max_fps);
@@ -750,7 +748,6 @@ extern "C" void cova_pipeline_free(cova_pipeline *p) {
     for (int i = 0; i < 4; i++) {
         if (p->x[i]) cudaFree(p->x[i]);
         if (i == 0 && p->x0f) cudaFree(p->x0f);
-        if (i == 0 && p->p1) cudaFree(p->p1);
         if (p->d[i]) cudaFree(p->d[i]);
         if (p->enc[i].wpack) cudaFree(p->enc[i].wpack);
         if (p->enc[i].epi) cudaFree(p->enc[i].epi);
@@ -1057,49 +1054,21 @@ static int tc_layer(cova_pipeline *p, int layer) {
         lp.bn_nonneg = 1;
         for (int c = 0; c < kEncCout[i]; c++)
             if (!(p->hw.enc[i].gamma[c] >= 0.f)) lp.bn_nonneg = 0;
-        //                                  MODE   CIN_CB NCOLS TPS KCH COUT
         if (i == 0) {
-            // first block: conv+ReLU+BN+pool once per FRAME, then PointWiseTN gathers the 4 frames of every window
-            const int F = (int)(p->ck_n_streams * p->cur_fps);
-            if (!(p->dbg & 16)) {
-                // fused: frame-level conv + PointWiseTN over a register ring of 4 frames, one kernel (blobnet_enc1.cuh);
-                // dbg bit 4 forces the two-kernel path below (also the fallback for grids the fused kernel cannot take)
-                LayerParams fp = lp;
-                fp.in = p->x0f; fp.gin = p->gx0f; fp.out = p->x[1]; fp.gout = p->gx[1]; fp.N = F;
-                tc1::Enc1Extra ex;
-                memset(&ex, 0, sizeof(ex));
-                ex.n_chains = (int)p->ck_n_streams; ex.fps = (int)p->cur_fps; ex.gamma = (int)p->gamma;
-                ex.tab = p->slot[p->cur_slot].d_tab + p->ck_stream0;
-                cudaError_t err = cudaSuccess;
-                if (tc1::try_launch_enc1(fp, ex, p->n_sms, p->stream, err)) {
-                    if (err != cudaSuccess) return set_err(COVA_E_CUDA, "fused enc1 launch: %s", cudaGetErrorString(err));
-                    p->launches++;
-                    prof_mark(p, "tc_enc1_fused");
-                    return COVA_OK;
-                }
-            }
-            lp.in = p->x0f; lp.gin = p->gx0f; lp.out = p->p1; lp.gout = p->gp1; lp.out2 = nullptr; lp.N = F;
-            rc = launch_first_fit<Cfg<MODE_ENCF, 1, 16, 8, 1, 16>, Cfg<MODE_ENCF, 1, 16, 4, 1, 16>, Cfg<MODE_ENCF, 1, 16, 2, 1, 16>,
-                                  Cfg<MODE_ENCF, 1, 16, 1, 1, 16>>(lp, p->n_sms, p->stream);
-            if (rc) return rc;
+            // first block: frame-level conv + PointWiseTN over a register ring of 4 frames, one kernel (blobnet_enc1.cuh).
+            // It takes every frame width up to 3172 macroblocks; block 2 already refuses beyond 800.
+            LayerParams fp = lp;
+            fp.in = p->x0f; fp.gin = p->gx0f; fp.out = p->x[1]; fp.gout = p->gx[1]; fp.N = (int)(p->ck_n_streams * p->cur_fps);
+            tc1::Enc1Extra ex;
+            memset(&ex, 0, sizeof(ex));
+            ex.n_chains = (int)p->ck_n_streams; ex.fps = (int)p->cur_fps; ex.gamma = (int)p->gamma;
+            ex.tab = p->slot[p->cur_slot].d_tab + p->ck_stream0;
+            cudaError_t err = cudaSuccess;
+            if (!tc1::try_launch_enc1(fp, ex, p->n_sms, p->stream, err))
+                return set_err(COVA_E_UNSUPPORTED, "no tcgen05 tile configuration fits shared memory for this macroblock grid");
+            if (err != cudaSuccess) return set_err(COVA_E_CUDA, "fused enc1 launch: %s", cudaGetErrorString(err));
             p->launches++;
-            prof_mark(p, "tc_enc1_conv");
-            TnArgs ta;
-            ta.p1 = p->p1; ta.gp1 = p->gp1; ta.x1 = p->x[1]; ta.gx1 = p->gx[1]; ta.skip = p->d[3]; ta.gskip = p->gd[3];
-            ta.skip_cb = kDecCout[2] / 8; ta.newest = p->slot[p->cur_slot].d_newest + p->ck_window0; ta.n_windows = N;
-            ta.CB = kEncCout[0] / 8;
-            memcpy(ta.w1, p->hw.enc[0].tn_w1, 64);
-            memcpy(ta.w2, p->hw.enc[0].tn_w2, 64);
-            long long total = (long long)ta.CB * 4 * N * p->gx[1].S;
-            if (total >= (1ll << 32)) return set_err(COVA_E_UNSUPPORTED, "chunk too large for the PointWiseTN gather kernel (32-bit index)");
-            // 64 CTAs per SM queued (4-5 resident) - measured sweep per 8192 windows at 720p: resident-only grid 0.49 ms,
-            // x16 0.43, x64 0.39, one iteration per thread 0.45
-            static const int tn_factor = getenv("COVA_TN_GRID") ? atoi(getenv("COVA_TN_GRID")) : 64;   // development knob
-            int blocks = (int)std::min<long long>((total + 255) / 256, (long long)p->n_sms * tn_factor);
-            pointwise_tn_kernel<<<blocks, 256, 0, p->stream>>>(ta);
-            COVA_CUDA(cudaGetLastError());
-            p->launches++;
-            prof_mark(p, "enc1_pointwise_tn");
+            prof_mark(p, "tc_enc1_fused");
             return COVA_OK;
         }
         // block 3 (Cout = 64) stays on the positions-as-M kernel: measured 0.335 ms vs 0.376 ms per 8192 windows at 720p
@@ -1120,6 +1089,7 @@ static int tc_layer(cova_pipeline *p, int layer) {
                 return COVA_OK;
             }
         }
+        //                                  MODE   CIN_CB NCOLS TPS KCH COUT
         if (i == 1) rc = launch_first_fit<Cfg<MODE_ENC, 2, 32, 4, 2, 32>, Cfg<MODE_ENC, 2, 32, 2, 2, 32>, Cfg<MODE_ENC, 2, 32, 1, 2, 32>>(lp, p->n_sms, p->stream);
         else if (i == 2) rc = launch_first_fit<Cfg<MODE_ENC, 4, 64, 2, 4, 64>, Cfg<MODE_ENC, 4, 64, 1, 4, 64>, Cfg<MODE_ENC, 4, 64, 1, 2, 64>>(lp, p->n_sms, p->stream);
         else rc = launch_first_fit<Cfg<MODE_ENC, 8, 128, 1, 2, 128>>(lp, p->n_sms, p->stream);

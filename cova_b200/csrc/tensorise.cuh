@@ -77,7 +77,7 @@ __global__ void __launch_bounds__(256) tensorise_x0_kernel(const uint32_t *__res
 //     [c0 c1 c2 0 | c0' c1' c2' 0] (fp16, clipped to 6), in the two row-parity planes (ph = 0 and 2) of a
 //     Tn = 1 phase-plane geometry whose "windows" are the frames of the pool.  The first convolution runs once
 //     per frame on this; the window structure (newest-first stacking of `timestep` frames) is applied afterwards
-//     by pointwise_tn_kernel through the `newest` table.
+//     by enc1_fused_kernel as it walks each chain through time (blobnet_enc1.cuh).
 // fp16 of the clipped bytes without integer->float conversions: 0x6400 | n is the half 1024 + n for n < 1024, and
 // subtracting 1024 in half arithmetic is exact.  q = [mb_weight, |mv_x|, |mv_y|, stale]; returns (c0 c1 | c2 0) as two half2.
 __device__ __forceinline__ uint2 quad_to_half4(uint32_t q) {
@@ -139,65 +139,6 @@ __global__ void __launch_bounds__(256) tensorise_frames_kernel(const uint32_t *_
             const uint2 a = quad_to_half4(q0[k]), b = quad_to_half4(q1[k]);
             x0f[geom_row(g, 0, (int)((y & 1u) << 1), geom_pos(g, (int)f, (int)(y >> 1), (int)xx[k], 0))] = make_uint4(a.x, a.y, b.x, b.y);
         }
-    }
-}
-
-// PointWiseTN of the first encoder block (reference utils/model/pointwise.py:10-26) as a gather over frames:
-// window n, time t reads the pooled per-frame activation of frame newest[n]-t.  Thread <-> (channel block,
-// phase plane, window, position): 4 x 128-bit loads, 8 channels x two 4x4 products, 4 consecutive 16-byte rows
-// out (t interleaved innermost) + the t = 0 row into the decoder's concat buffer.
-struct TnArgs {
-    const uint4 *p1; Geom gp1;       // per-frame pooled activations (Tn = 1, "windows" = frames)
-    uint4 *x1; Geom gx1;             // next encoder input (Tn = 4)
-    uint4 *skip; Geom gskip;         // decoder concat buffer (Tn = 1)
-    int skip_cb;
-    const int *newest;               // per window of the chunk: index of its newest frame among the chunk's frames
-    float w1[16], w2[16];
-    int n_windows, CB;
-};
-__global__ void __launch_bounds__(256) pointwise_tn_kernel(const __grid_constant__ TnArgs A) {
-    const uint32_t S = (uint32_t)A.gx1.S, P = (uint32_t)A.gx1.P, NW = (uint32_t)A.n_windows;
-    const uint32_t per_plane = NW * S, total = (uint32_t)A.CB * 4u * per_plane;      // host guarantees < 2^32
-    const uint32_t stride = gridDim.x * blockDim.x;
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
-        const uint32_t pl = i / per_plane, r = i - pl * per_plane;                    // pl = cb*4 + ph
-        const uint32_t n = r / S, s = r - n * S;
-        const uint32_t y2 = s / P, x2 = s - y2 * P;
-        const uint32_t ph = pl & 3u;
-        if (2 * y2 + (ph >> 1) >= (uint32_t)A.gx1.H || 2 * x2 + (ph & 1) >= (uint32_t)A.gx1.W) continue;   // shared zero row / column
-        const int f0 = __ldg(A.newest + n);      // chains of a staggered batch have different window shapes
-        const uint4 *src = A.p1 + ((long long)pl * A.gp1.Lp + A.gp1.guard + (long long)f0 * S + s);
-        uint4 in[4];
-#pragma unroll
-        for (int t = 0; t < 4; t++) in[t] = __ldg(src - (long long)t * S);
-        uint32_t o32[4][4];
-#pragma unroll
-        for (int k = 0; k < 4; k++) {                       // channel pair (2k, 2k+1); packed lanes = the two channels
-            float2 x[4];
-#pragma unroll
-            for (int t = 0; t < 4; t++) x[t] = __half22float2(reinterpret_cast<const __half2 *>(&in[t])[k]);
-            float2 h1[4];
-#pragma unroll
-            for (int m = 0; m < 4; m++) {
-                float2 h = fmul2(x[0], bc2(A.w1[m]));
-#pragma unroll
-                for (int t = 1; t < 4; t++) h = ffma2(x[t], bc2(A.w1[t * 4 + m]), h);
-                h1[m] = relu2(h);
-            }
-#pragma unroll
-            for (int to = 0; to < 4; to++) {
-                float2 h = x[to];                            // relu(x + relu(h2)) = max(x + h2, x, 0)
-#pragma unroll
-                for (int m = 0; m < 4; m++) h = ffma2(h1[m], bc2(A.w2[m * 4 + to]), h);
-                const __half2 hh = __floats2half2_rn(fmax3(h.x, x[to].x, 0.f), fmax3(h.y, x[to].y, 0.f));
-                o32[to][k] = *reinterpret_cast<const uint32_t *>(&hh);
-            }
-        }
-        uint4 *dst = A.x1 + ((long long)pl * A.gx1.Lp + A.gx1.guard + ((long long)n * S + s) * 4);
-#pragma unroll
-        for (int to = 0; to < 4; to++) dst[to] = make_uint4(o32[to][0], o32[to][1], o32[to][2], o32[to][3]);
-        A.skip[((long long)(A.skip_cb * 4) + pl) * A.gskip.Lp + A.gskip.guard + (long long)n * S + s] =
-            make_uint4(o32[0][0], o32[0][1], o32[0][2], o32[0][3]);
     }
 }
 

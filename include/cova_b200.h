@@ -234,9 +234,9 @@ int cova_pipeline_read_activation(cova_pipeline *p, int layer, float *out, size_
 int cova_pipeline_run_layer(cova_pipeline *p, int layer, uint32_t impl);
 /* development switches.  Results become garbage with bit 0 (skip the MMAs) or bit 1 (skip the epilogue math); the others
  * select alternative, equally correct code paths for A/B measurements (tools/ab_step.py, tools/layer_timing.py):
- * bit 2 positions-as-M kernels for encoder blocks 2 and 4, bit 3 weights-stationary kernel for block 3, bit 4 two-kernel
- * block 1, bit 5 plain stream-ordered launches instead of programmatic dependent launch (this handle only), bit 6 whole-tile
- * accumulators for dec0 / dec1 */
+ * bit 2 positions-as-M kernels for encoder blocks 2 and 4, bit 3 weights-stationary kernel for block 3, bit 5 plain
+ * stream-ordered launches instead of programmatic dependent launch (this handle only), bit 6 whole-tile accumulators for
+ * dec0 / dec1 */
 int cova_pipeline_set_debug(cova_pipeline *p, int flags);
 /* kernels launched by this handle since creation */
 int cova_pipeline_launch_count(const cova_pipeline *p, uint64_t *count);

@@ -229,24 +229,42 @@ def test_negative_batchnorm_scales_and_forced_weights_stationary_block3():
 
 @pytest.mark.parametrize("h,w,n_streams,fps,gamma", [(45, 80, 2, 21, 1), (45, 80, 3, 23, 3), (33, 47, 1, 18, 2),
                                                      (68, 120, 1, 9, 1), (135, 240, 1, 6, 1)])
-def test_fused_block1_equals_two_kernel_path(h, w, n_streams, fps, gamma):
-    """Block 1 as ONE kernel (frame-level conv + PointWiseTN over a register ring of frames, chains cut into frame
-    segments with 3 warm-up frames) must write exactly the bytes of the conv-per-frame + gather pair (debug bit 4):
-    X1, the t = 0 skip inside the decoder concat buffer, and therefore the logits."""
+def test_fused_block1_matches_validation_and_is_partition_independent(h, w, n_streams, fps, gamma):
+    """Block 1 as ONE kernel (frame-level conv + PointWiseTN over a register ring of frames).
+    (a) On identical input, X1 and the t = 0 skip inside the decoder concat buffer match the fp32 validation kernel.
+    (b) The chains give the same bytes (X1, skip, logits) run alone, where every (chain, tile pair) item is cut into
+    frame segments that re-compute 3 warm-up frames, and run as the first chains of a batch whose items fill the
+    grid at least once, where those chains' items are handed out whole."""
+    import torch
     wts = weights.random_weights(7, head_bias=-1.0)
     wts["enc0.bn_gamma"][::5] = -wts["enc0.bn_gamma"][::5]            # exercise the min-pool branch too
+    blob = weights.to_blob(wts)
     frames = synth.synth_streams(n_streams, fps, h, w, config_idx=8)
-    got = []
-    for dbg in (0, 16):
-        p = BlobPipeline(w, h, weights.to_blob(wts), n_streams, fps, gamma=gamma, keep_logits=True)
-        p.set_debug(dbg)
-        p.process(frames)
-        n_launch = p.launch_count()
-        got.append((p.read_activation(1), p.read_activation(7), p.read_logits(), n_launch, p.read_activation(0)))
-    assert got[0][3] + 1 == got[1][3]                                 # conv + gather instead of one kernel
-    assert (got[0][4] == got[1][4]).all()
-    for a, b in zip(got[0][:3], got[1][:3]):
-        assert a.shape == b.shape and (a == b).all()
+
+    p = BlobPipeline(w, h, blob, n_streams, fps, gamma=gamma, impl=_lib.IMPL_SIMT)
+    p.load_frames(frames)
+    p.tensorise()
+    got = {}
+    for impl in (_lib.IMPL_TCGEN05, _lib.IMPL_SIMT):
+        p.run_layer(0, impl)
+        got[impl] = (p.read_activation(1), p.read_activation(7))
+    for a, ref in zip(got[_lib.IMPL_TCGEN05], got[_lib.IMPL_SIMT]):
+        assert a.shape == ref.shape
+        assert np.abs(a - ref).max() <= ACT_REL_TOL * np.abs(ref).max()
+
+    # work items of enc1_fused_kernel: (chain, pair of 128-position tiles of a frame's phase planes, common.cuh make_geom)
+    tile_pairs = (((h + 1) // 2 + 1) * ((w + 1) // 2 + 1) + 255) // 256
+    n_sms = torch.cuda.get_device_properties(0).multi_processor_count
+    n_big = n_streams + (n_sms + tile_pairs - 1) // tile_pairs
+    assert n_streams * tile_pairs < n_sms <= n_big * tile_pairs      # alone: no whole round of items; big: at least one
+    big = np.concatenate([frames, synth.tiled_streams(n_big - n_streams, fps, h, w, config_idx=9)])
+    outs = []
+    for fr in (frames, big):
+        p = BlobPipeline(w, h, blob, fr.shape[0], fps, gamma=gamma, keep_logits=True, n_chunks=1)
+        p.process(fr)
+        outs.append((p.read_activation(0), p.read_activation(1), p.read_activation(7), p.read_logits()))
+    for a, b in zip(*outs):
+        assert (a == b[: a.shape[0]]).all()
 
 
 def test_gamma_subsampling_and_chain_restart():

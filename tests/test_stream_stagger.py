@@ -169,16 +169,14 @@ def test_four_staggered_batches_in_flight():
 
 @pytest.mark.gpu
 def test_block1_paths_agree_on_a_staggered_batch():
-    """One staggered batch, one chunk: the BlobNet input equals the element's windows, and the first block's output is the
-    same from the fused kernel, the two-kernel path (debug bit 4) and the fp32 validation kernel."""
+    """One staggered batch, one chunk: the BlobNet input equals the element's windows, and the first block's output from
+    the fused kernel agrees with the fp32 validation kernel."""
     gamma = 2
     frames = synth.synth_streams(4, 20, H, W, config_idx=40)
     pre = [0, 1, 3, 4]                             # frames fed before the batch: histories 0, 1, 3, 3 on two phases
     outs = []
-    for kind in ("fused", "two_kernel", "simt"):
-        p = BlobPipeline(W, H, _wts(), 4, 16, gamma=gamma, n_chunks=1, impl=_lib.IMPL_SIMT if kind == "simt" else _lib.IMPL_TCGEN05)
-        if kind == "two_kernel":
-            p.set_debug(16)
+    for impl in (_lib.IMPL_TCGEN05, _lib.IMPL_SIMT):
+        p = BlobPipeline(W, H, _wts(), 4, 16, gamma=gamma, n_chunks=1, impl=impl)
         for s, n in enumerate(pre):
             if n:
                 p.submit(frames[s: s + 1, :n], stream_ids=[s], cont=True, staggered=True)
@@ -194,11 +192,8 @@ def test_block1_paths_agree_on_a_staggered_batch():
     for wid, a0, _ in outs:
         assert (wid == outs[0][0]).all()
         assert a0.shape == x.shape and (a0 == x).all()
-    fused, two, simt = (o[2] for o in outs)
-    assert (fused == two).all()
-    scale = np.abs(simt).max()
-    assert np.abs(fused - simt).max() <= ACT_REL_TOL * scale
-    assert np.abs(two - simt).max() <= ACT_REL_TOL * scale
+    fused, simt = (o[2] for o in outs)
+    assert np.abs(fused - simt).max() <= ACT_REL_TOL * np.abs(simt).max()
 
 
 @pytest.mark.gpu

@@ -14,8 +14,8 @@ p.load_frames(synth.tiled_streams(n_streams, fps, h, w, 1))
 p.set_profiling(True)
 res = {}
 import time
-VARIANTS = (("normal", 0), ("no_epilogue", 2), ("no_mma", 1), ("neither", 3), ("old_enc", 4), ("unfused_enc1", 16),
-            ("no_pdl", 32), ("dec_whole", 64))
+VARIANTS = (("normal", 0), ("no_epilogue", 2), ("no_mma", 1), ("neither", 3), ("old_enc", 4), ("no_pdl", 32),
+            ("dec_whole", 64))
 if os.environ.get("VARIANTS"):          # e.g. VARIANTS="ws3:8,ws3_no_epi:10,ws3_no_mma:9"
     VARIANTS = tuple((v.split(":")[0], int(v.split(":")[1])) for v in os.environ["VARIANTS"].split(","))
 steps = {}
