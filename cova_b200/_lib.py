@@ -25,6 +25,11 @@ SUBMIT_CONTINUE = 1
 SUBMIT_STAGGERED = 2       # with SUBMIT_CONTINUE: the continued streams of a batch may differ in history and gamma phase
 
 
+def sparse_max_frame_bytes(n_mb: int) -> int:
+    """COVA_SPARSE_MAX_FRAME_BYTES(n_mb): the size of a sparse record in which every macroblock differs."""
+    return 8 + 4 * ((n_mb + 31) // 32) + 4 * ((n_mb + 1) // 2)
+
+
 class CovaError(RuntimeError):
     def __init__(self, code: int, detail: str):
         super().__init__(f"cova_b200 error {code}: {detail}")
@@ -84,6 +89,8 @@ SIGNATURES = {
     "cova_packer_new": (ctypes.c_int, [_vpp, ctypes.c_uint32]),
     "cova_packer_free": (None, [_vp]),
     "cova_packer_pack": (ctypes.c_int, [_vp, _vp, _vp, ctypes.c_size_t]),
+    "cova_packer_pack_sparse": (ctypes.c_int, [_vp, _vp, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32, _vp, ctypes.c_size_t, _szp]),
+    "cova_pipeline_submit_sparse": (ctypes.c_int, [_vp, _vp, ctypes.c_size_t, ctypes.c_uint32, ctypes.c_uint32, _vp, _vp, ctypes.c_uint32]),
     "cova_pipeline_load_masks": (ctypes.c_int, [_vp, _vp, ctypes.c_uint32, ctypes.c_int]),
     "cova_pipeline_read_stacked": (ctypes.c_int, [_vp, _vp, ctypes.c_size_t]),
     "cova_pipeline_read_mask": (ctypes.c_int, [_vp, _vp, ctypes.c_size_t]),

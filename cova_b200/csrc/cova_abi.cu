@@ -18,6 +18,7 @@
 #include "blobnet_enc1.cuh"
 #include "ccl.cuh"
 #include "common.cuh"
+#include "sparse_expand.cuh"
 #include "tensorise.cuh"
 #include "weights_pack.cuh"
 
@@ -510,6 +511,7 @@ struct cova_pipeline {
     std::vector<uint64_t> n_seen, id_mark;
     uint64_t id_epoch = 0;
     std::vector<uint32_t> first_scratch, hist_scratch;   // per chain of the batch being submitted
+    std::vector<uint64_t> off_scratch;                   // record offsets of the sparse batch being submitted
     // A batch is processed in chunks of whole chains: the activation buffers are sized for ONE chunk, and
     // process_host() overlaps the H2D copy of chunk c+1, the kernels of chunk c and the D2H of chunk c-1.
     uint32_t chunk_streams = 0;          // chains per chunk (capacity)
@@ -543,6 +545,11 @@ struct cova_pipeline {
         std::vector<uint32_t> tab_first;               // what the tables hold: per-chain first, frames per chain, stream
         uint32_t tab_fps = 0;
         cudaStream_t tab_stream = nullptr;
+        // sparse input (cova_pipeline_submit_sparse), allocated on the slot's first sparse submit: the batch's records at
+        // their host byte offsets, and the record offsets (pinned staging + device copy, uploaded on the compute stream)
+        uint8_t *d_sparse = nullptr;
+        unsigned long long *h_off = nullptr, *d_off = nullptr;
+        cudaEvent_t ev_off = nullptr;                  // recorded after the offsets upload: the staging may be rewritten after it
     } slot[kSlots];
     int cur_slot = 0, next_submit = 0, next_collect = 0;
     int sizes_h[5], sizes_w[5];          // extents: [0] input, [1..4] encoder outputs
@@ -767,6 +774,10 @@ extern "C" void cova_pipeline_free(cova_pipeline *p) {
         if (sl.h_newest) cudaFreeHost(sl.h_newest);
         if (sl.d_newest) cudaFree(sl.d_newest);
         if (sl.ev_tab) cudaEventDestroy(sl.ev_tab);
+        if (sl.d_sparse) cudaFree(sl.d_sparse);
+        if (sl.h_off) cudaFreeHost(sl.h_off);
+        if (sl.d_off) cudaFree(sl.d_off);
+        if (sl.ev_off) cudaEventDestroy(sl.ev_off);
         for (auto e : sl.ev_in) cudaEventDestroy(e);
         for (auto e : sl.ev_done) cudaEventDestroy(e);
     }
@@ -1313,12 +1324,31 @@ __global__ void __launch_bounds__(256) carry_kernel(uint32_t *__restrict__ pool,
 // Every device chain then has fps + lead frames, lead = max_s h_s: the new frames start at index lead, the carried ones sit
 // right-aligned in front of them at [lead - h_s, lead), and what lies before that is never read by an emitted window.  So
 // the copies and the per-frame kernels see one uniform chain length, and only the window -> frame tables differ per chain.
+//
+// Sparse input (submit_sparse, sparse_len != nullptr: `frames` is a batch of *sparse_len bytes of records) differs only in
+// the copy stage of a chunk: the host validates every record first and keeps their offsets; chunk c's records are one
+// contiguous byte range, copied as such, and sparse_expand_kernel writes them into the frame pool where the dense copy
+// would have put them.  Everything after that is shared.
 static int submit_impl(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, uint32_t fps, const uint32_t *stream_ids,
-                       const uint64_t *pts, uint32_t flags, bool stateful) {
+                       const uint64_t *pts, uint32_t flags, bool stateful, const size_t *sparse_len = nullptr) {
     if (!p || !frames) return set_err(COVA_E_INVAL, "null argument");
     if (flags & ~(COVA_SUBMIT_CONTINUE | COVA_SUBMIT_STAGGERED)) return set_err(COVA_E_INVAL, "unknown submit flag");
     if ((flags & COVA_SUBMIT_STAGGERED) && !(flags & COVA_SUBMIT_CONTINUE))
         return set_err(COVA_E_INVAL, "COVA_SUBMIT_STAGGERED needs COVA_SUBMIT_CONTINUE");
+    const bool sparse = sparse_len != nullptr;
+    const uint64_t n_frames = (uint64_t)n_streams * fps;
+    if (sparse) {           // the whole batch is checked before any device call
+        if (!p->packed) return set_err(COVA_E_INVAL, "sparse input needs a COVA_FLAG_INPUT_PACKED16 pipeline");
+        if (!n_streams || n_streams > p->max_streams || fps > p->max_fps)
+            return set_err(COVA_E_INVAL, "batch exceeds max_streams / max_frames_per_stream of the pipeline");
+        p->off_scratch.resize(n_frames + 1);
+        uint64_t bad = 0;
+        if (const char *why = sparse::validate_batch(frames, *sparse_len, n_frames, p->W * p->H, p->off_scratch.data(), &bad)) {
+            char frame[32];
+            snprintf(frame, sizeof(frame), "%llu", (unsigned long long)bad);
+            return set_err(COVA_E_INVAL, "malformed sparse batch at frame %s: %s", frame, why);
+        }
+    }
     COVA_CUDA(cudaSetDevice(p->device));
     const int k = p->next_submit;
     if (p->slot[k].busy) return set_err(COVA_E_INVAL, "four batches are already in flight: collect one first");
@@ -1366,6 +1396,13 @@ static int submit_impl(cova_pipeline *p, const uint8_t *frames, uint32_t n_strea
             COVA_CUDA(cudaMalloc(&sl.d_ids, sizeof(uint32_t) * p->max_streams));
         }
     }
+    if (sparse && !sl.ev_off) {        // dense users never pay for these
+        const size_t max_frames = (size_t)p->max_streams * p->max_fps;
+        if (!sl.d_sparse) COVA_CUDA(cudaMalloc(&sl.d_sparse, max_frames * COVA_SPARSE_MAX_FRAME_BYTES(p->W * p->H)));
+        if (!sl.h_off) COVA_CUDA(cudaMallocHost(&sl.h_off, sizeof(unsigned long long) * (max_frames + 1)));
+        if (!sl.d_off) COVA_CUDA(cudaMalloc(&sl.d_off, sizeof(unsigned long long) * (max_frames + 1)));
+        COVA_CUDA(cudaEventCreateWithFlags(&sl.ev_off, cudaEventDisableTiming));
+    }
     const uint32_t fps_dev = fps + lead;                            // frames per chain on the device
     if (fps_dev > p->max_fps)
         return set_err(COVA_E_INVAL, "carried frames + new frames exceed max_frames_per_stream of the pipeline");
@@ -1400,9 +1437,19 @@ static int submit_impl(cova_pipeline *p, const uint8_t *frames, uint32_t n_strea
     } while (0)
     const uint32_t nc = n_chunks_of(p);
     const size_t src_chain = p->frame_bytes * fps, dst_chain = p->frame_bytes * fps_dev, lead_bytes = p->frame_bytes * lead;
+    if (sparse) {
+        // the slot's previous offsets upload has completed (its batch was collected); the event makes that explicit
+        COVA_CUDA_SLOT(cudaEventSynchronize(sl.ev_off));
+        memcpy(sl.h_off, p->off_scratch.data(), sizeof(unsigned long long) * (n_frames + 1));
+        COVA_CUDA_SLOT(cudaMemcpyAsync(sl.d_off, sl.h_off, sizeof(unsigned long long) * (n_frames + 1), cudaMemcpyHostToDevice, p->stream));
+        COVA_CUDA_SLOT(cudaEventRecord(sl.ev_off, p->stream));
+    }
     for (uint32_t c = 0; c < nc; c++) {
         const size_t s0 = (size_t)c * p->chunk_streams, ns = std::min<size_t>(p->chunk_streams, n_streams - s0);
-        if (!lead) COVA_CUDA_SLOT(cudaMemcpyAsync(sl.d_frames + s0 * dst_chain, frames + s0 * src_chain, ns * src_chain, cudaMemcpyHostToDevice, p->s_in));
+        if (sparse) {      // chunk c's records: one contiguous byte range, to the same offset of the staging
+            const uint64_t b0 = p->off_scratch[s0 * fps], b1 = p->off_scratch[(s0 + ns) * fps];
+            COVA_CUDA_SLOT(cudaMemcpyAsync(sl.d_sparse + b0, frames + b0, b1 - b0, cudaMemcpyHostToDevice, p->s_in));
+        } else if (!lead) COVA_CUDA_SLOT(cudaMemcpyAsync(sl.d_frames + s0 * dst_chain, frames + s0 * src_chain, ns * src_chain, cudaMemcpyHostToDevice, p->s_in));
         else COVA_CUDA_SLOT(cudaMemcpy2DAsync(sl.d_frames + s0 * dst_chain + lead_bytes, dst_chain, frames + s0 * src_chain, src_chain, src_chain, ns,
                                               cudaMemcpyHostToDevice, p->s_in));
         COVA_CUDA_SLOT(cudaEventRecord(sl.ev_in[c], p->s_in));
@@ -1411,6 +1458,13 @@ static int submit_impl(cova_pipeline *p, const uint8_t *frames, uint32_t n_strea
     const int wpf = (int)(p->frame_bytes / 4);
     for (uint32_t c = 0; c < nc; c++) {
         COVA_CUDA_SLOT(cudaStreamWaitEvent(p->stream, sl.ev_in[c], 0));
+        if (sparse) {      // a plain launch: tensorise_frames_kernel waits for it (pdl_wait) before reading the pool
+            const uint32_t s0 = c * p->chunk_streams, ns = std::min(p->chunk_streams, n_streams - s0);
+            SparseExpandArgs ea{sl.d_sparse, sl.d_off, sl.d_frames, s0 * fps, fps, fps_dev, lead, p->W * p->H};
+            sparse_expand_kernel<<<ns * fps, kExpandThreads, 0, p->stream>>>(ea);
+            p->launches++;
+            COVA_CUDA_SLOT(cudaGetLastError());
+        }
         if (stateful && t1) {
             const size_t s0 = (size_t)c * p->chunk_streams;
             const int ns = (int)std::min<size_t>(p->chunk_streams, n_streams - s0);
@@ -1440,6 +1494,10 @@ extern "C" int cova_pipeline_submit_host(cova_pipeline *p, const uint8_t *frames
 extern "C" int cova_pipeline_submit_host2(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, uint32_t fps,
                                           const uint32_t *stream_ids, const uint64_t *pts, uint32_t flags) {
     return submit_impl(p, frames, n_streams, fps, stream_ids, pts, flags, true);
+}
+extern "C" int cova_pipeline_submit_sparse(cova_pipeline *p, const uint8_t *data, size_t data_len, uint32_t n_streams,
+                                           uint32_t fps, const uint32_t *stream_ids, const uint64_t *pts, uint32_t flags) {
+    return submit_impl(p, data, n_streams, fps, stream_ids, pts, flags, true, &data_len);
 }
 extern "C" int cova_pipeline_reset_streams(cova_pipeline *p, const uint32_t *stream_ids, uint32_t n) {
     if (!p) return set_err(COVA_E_INVAL, "null handle");

@@ -308,3 +308,20 @@ extern "C" int cova_packer_pack(cova_packer *pk, const uint8_t *quads, uint16_t 
     pk->pk.pack(quads, out, n_mb);
     return COVA_OK;
 }
+static_assert(COVA_SPARSE_MAX_FRAME_BYTES(3600) == cova::sparse::max_record_bytes(3600) &&
+                  COVA_SPARSE_MAX_FRAME_BYTES(8160) == cova::sparse::max_record_bytes(8160) &&
+                  COVA_SPARSE_MAX_FRAME_BYTES(129600) == cova::sparse::max_record_bytes(129600),
+              "COVA_SPARSE_MAX_FRAME_BYTES and sparse_format.hpp disagree");
+extern "C" int cova_packer_pack_sparse(cova_packer *pk, const uint8_t *quads, uint32_t n_frames, uint32_t w_mb, uint32_t h_mb,
+                                       uint8_t *out, size_t out_cap, size_t *out_len) {
+    if (!pk || !out_len || (!quads && n_frames)) return fail(COVA_E_INVAL, "null argument");
+    if (!w_mb || !h_mb) return fail(COVA_E_INVAL, "empty macroblock grid");
+    if ((uint64_t)w_mb * h_mb > UINT32_MAX / 2) return fail(COVA_E_INVAL, "macroblock grid too large");
+    try {
+        if (!pk->pk.pack_sparse(quads, n_frames, w_mb * h_mb, out, out_cap, out_len))
+            return fail(COVA_E_TOOSMALL, "output buffer too small for the sparse batch; *out_len is the size it needs");
+    } catch (const std::bad_alloc &) {
+        return fail(COVA_E_NOMEM, "staging allocation failed");
+    }
+    return COVA_OK;
+}

@@ -20,6 +20,7 @@ from __future__ import annotations
 
 import ctypes
 import struct
+from dataclasses import dataclass
 
 import numpy as np
 
@@ -61,9 +62,22 @@ class PinnedBuffer:
             pass
 
 
+@dataclass
+class SparseBatch:
+    """A batch in the sparse input format (include/cova_b200.h, COVA_SPARSE_MAX_FRAME_BYTES): the records of
+    n_streams x frames_per_stream frames, stream-major.  `data` is u8 and exactly the batch's bytes (it may be a view of
+    a PinnedBuffer array).  BlobPipeline(packed_input=True).submit() takes it like a dense frames array."""
+    data: np.ndarray
+    n_streams: int
+    frames_per_stream: int
+    h_mb: int
+    w_mb: int
+
+
 class FramePacker:
     """Host packer for BlobPipeline(packed_input=True): decoder quads [.., h, w, 4] u8 -> [.., h, w] u16
-    (cova_packer_pack: min(b, 6) of bytes 0-2 in 3 bits each; worker threads live as long as the packer)."""
+    (cova_packer_pack: min(b, 6) of bytes 0-2 in 3 bits each; worker threads live as long as the packer), or -> a
+    SparseBatch (pack_sparse)."""
 
     def __init__(self, n_threads: int = 0):
         self._h = ctypes.c_void_p()
@@ -77,6 +91,21 @@ class FramePacker:
         assert out.dtype == np.uint16 and out.size == a.size // 4 and out.flags.c_contiguous
         check(_lib.load().cova_packer_pack(self._h, _ptr(a), _ptr(out), out.size))
         return out
+
+    def pack_sparse(self, quads: np.ndarray, out: np.ndarray | None = None) -> SparseBatch:
+        """quads [n_streams, frames, h, w, 4] u8 -> SparseBatch (cova_packer_pack_sparse).  `out`: a u8 array to encode
+        into (e.g. PinnedBuffer(...).array); data is then a view of its first bytes.  Raises CovaError(E_TOOSMALL) when
+        it is too small."""
+        a = np.ascontiguousarray(quads, dtype=np.uint8)
+        assert a.ndim == 5 and a.shape[-1] == 4, a.shape
+        n_streams, fps, h_mb, w_mb = a.shape[:4]
+        n_frames = n_streams * fps
+        if out is None:
+            out = np.empty(n_frames * _lib.sparse_max_frame_bytes(h_mb * w_mb), dtype=np.uint8)
+        assert out.dtype == np.uint8 and out.flags.c_contiguous
+        ln = ctypes.c_size_t()
+        check(_lib.load().cova_packer_pack_sparse(self._h, _ptr(a), n_frames, w_mb, h_mb, _ptr(out), out.size, ctypes.byref(ln)))
+        return SparseBatch(out.reshape(-1)[: ln.value], n_streams, fps, h_mb, w_mb)
 
     def close(self):
         if self._h:
@@ -489,7 +518,13 @@ class BlobPipeline:
         stream_ids[s] (default 0, 1, ...), `pts[s, f]` is echoed per window by collect(meta=True), and cont=True continues
         the streams from their previous batch (carried timestep-1 frames + gamma phase) like one long-lived metapreprocess
         element would.  staggered=True (with cont=True) lets those streams differ in history and gamma phase: each continues
-        from its own state, so chains may yield different numbers of windows (collect(meta=True) maps them to streams)."""
+        from its own state, so chains may yield different numbers of windows (collect(meta=True) maps them to streams).
+
+        `frames` may be a SparseBatch (packed_input pipelines): it goes through cova_pipeline_submit_sparse with the same
+        stream semantics as cova_pipeline_submit_host2."""
+        if isinstance(frames, SparseBatch):
+            self._submit_sparse(frames, blob_cap, stream_ids, pts, cont, staggered)
+            return
         a = self._frames(frames)
         if stream_ids is None and pts is None and cont is None and not staggered:
             self._ensure_out(blob_cap or self._worst_case_cap(self.windows_for(a.shape[0], a.shape[1])))
@@ -505,6 +540,20 @@ class BlobPipeline:
                                                          None if p is None else _ptr(p),
                                                          (_lib.SUBMIT_CONTINUE if cont else 0) | (_lib.SUBMIT_STAGGERED if staggered else 0)))
         self._inflight = getattr(self, "_inflight", []) + [a]
+
+    def _submit_sparse(self, b: SparseBatch, blob_cap, stream_ids, pts, cont, staggered):
+        assert (b.h_mb, b.w_mb) == (self.h_mb, self.w_mb), (b.h_mb, b.w_mb)
+        d = b.data
+        assert d.dtype == np.uint8 and d.ndim == 1 and d.flags.c_contiguous
+        self._ensure_out(blob_cap or self._worst_case_cap(b.n_streams * b.frames_per_stream))
+        ids = None if stream_ids is None else np.ascontiguousarray(stream_ids, dtype=np.uint32)
+        p = None if pts is None else np.ascontiguousarray(pts, dtype=np.uint64)
+        assert ids is None or ids.shape == (b.n_streams,)
+        assert p is None or p.shape == (b.n_streams, b.frames_per_stream)
+        self._check(self._L.cova_pipeline_submit_sparse(self._h, _ptr(d), d.size, b.n_streams, b.frames_per_stream,
+                                                        None if ids is None else _ptr(ids), None if p is None else _ptr(p),
+                                                        (_lib.SUBMIT_CONTINUE if cont else 0) | (_lib.SUBMIT_STAGGERED if staggered else 0)))
+        self._inflight = getattr(self, "_inflight", []) + [d]
 
     def reset_streams(self, stream_ids=None):
         if stream_ids is None:

@@ -218,6 +218,31 @@ int cova_packer_new(cova_packer **out, uint32_t n_threads);
 void cova_packer_free(cova_packer *pk);
 int cova_packer_pack(cova_packer *pk, const uint8_t *quads, uint16_t *out, size_t n_mb);
 
+/* Sparse input for COVA_FLAG_INPUT_PACKED16 pipelines: only the macroblocks that differ from a per-frame background cross
+ * PCIe.  One frame = one record, 4-byte aligned, little-endian, n_mb = w_mb * h_mb macroblocks in raster order y*w_mb + x:
+ *   bytes 0-3   u32 background: a packed16 value in bits 0-8, bits 9-31 zero
+ *   bytes 4-7   u32 count: macroblocks whose value is not the background
+ *   then        u32 bitmap[ceil(n_mb / 32)]: bit i % 32 of word i / 32 set = macroblock i differs; bits >= n_mb zero
+ *   then        u16 values[count]: the packed16 values of the set macroblocks in raster order, zero-padded to 4 bytes
+ * Record size = 8 + 4*ceil(n_mb/32) + 4*ceil(count/2).  A batch is the records of n_streams x frames_per_stream frames,
+ * stream-major and time-minor like a dense frames argument, without gaps.  Any background is valid (a decoder can use its
+ * skip value); the values follow the packed16 contract, which is documented and not checked. */
+#define COVA_SPARSE_MAX_FRAME_BYTES(n_mb) \
+    (8u + 4u * (((size_t)(n_mb) + 31u) / 32u) + 4u * (((size_t)(n_mb) + 1u) / 2u)) /* a record with count = n_mb */
+/* Encodes n_frames frames of decoder quads [n_frames][h_mb][w_mb][4] into a sparse batch, reading every quad once, on the
+ * packer's threads (contiguous ranges of frames per thread).  Canonical output: background = the frame's most frequent
+ * packed16 value (ties: the smallest), zero padding.  *out_len = the batch size; COVA_E_TOOSMALL (nothing written) when it
+ * exceeds out_cap.  It never exceeds n_frames * COVA_SPARSE_MAX_FRAME_BYTES(w_mb * h_mb). */
+int cova_packer_pack_sparse(cova_packer *pk, const uint8_t *quads, uint32_t n_frames, uint32_t w_mb, uint32_t h_mb,
+                            uint8_t *out, size_t out_cap, size_t *out_len);
+/* As cova_pipeline_submit_host2 (stream ids, PTS echo, COVA_SUBMIT_CONTINUE / _STAGGERED, the same rules and errors;
+ * collect with collect_host / collect_host2), with the frames as a sparse batch of data_len bytes.  Only on a
+ * COVA_FLAG_INPUT_PACKED16 pipeline (COVA_E_INVAL otherwise).  Before any device call every record is checked - reserved
+ * background bits, count == popcount(bitmap), no bit at or past n_mb, zero padding, and records ending exactly at
+ * data_len - and a malformed batch is COVA_E_INVAL with nothing in flight.  data must stay valid until the collect. */
+int cova_pipeline_submit_sparse(cova_pipeline *p, const uint8_t *data, size_t data_len, uint32_t n_streams,
+                                uint32_t frames_per_stream, const uint32_t *stream_ids, const uint64_t *pts, uint32_t flags);
+
 /* feed a mask batch straight to the CCL stage (u8 [n][h_mb][w_mb]; is_device as above) */
 int cova_pipeline_load_masks(cova_pipeline *p, const uint8_t *masks, uint32_t n, int is_device);
 
