@@ -98,6 +98,8 @@ SIGNATURES = {
     "cova_pipeline_read_activation": (ctypes.c_int, [_vp, ctypes.c_int, _vp, ctypes.c_size_t, _u32p]),
     "cova_pipeline_run_layer": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_uint32]),
     "cova_pipeline_set_debug": (ctypes.c_int, [_vp, ctypes.c_int]),
+    "cova_blobnet_plan": (ctypes.c_int, [ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_int, ctypes.c_int, _vp]),
+    "cova_pipeline_last_plan": (ctypes.c_int, [_vp, _vp]),
     "cova_pipeline_launch_count": (ctypes.c_int, [_vp, _u64p]),
     "cova_pipeline_set_profiling": (ctypes.c_int, [_vp, ctypes.c_int]),
     "cova_pipeline_last_timings": (ctypes.c_int, [_vp, ctypes.c_char_p, ctypes.c_size_t, _f32p, _u32p]),
@@ -114,6 +116,27 @@ SIGNATURES = {
     "cova_sort_match_dets": (ctypes.c_int, [_vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32, ctypes.c_float, _vp, _u32p]),
 }
 
+
+
+PLAN_ENC1, PLAN_POS, PLAN_WS = 1, 2, 3
+N_LAYERS = 8
+
+
+class LayerPlan(ctypes.Structure):
+    """cova_layer_plan"""
+    _fields_ = [(k, ctypes.c_int32) for k in ("family", "config", "tps", "tile", "n_stage", "n_groups", "ctas")]
+
+    def as_dict(self) -> dict:
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
+def blobnet_plan(w_mb: int, h_mb: int, windows: int, debug: int = 0, n_sms: int = 148) -> list[dict]:
+    """cova_blobnet_plan: per layer the launch plan the library would pick (host arithmetic, no device).  Raises CovaError
+    (E_UNSUPPORTED) when a layer has no plan."""
+    lib = load()
+    out = (LayerPlan * N_LAYERS)()
+    check(lib.cova_blobnet_plan(w_mb, h_mb, windows, debug, n_sms, out), lib)
+    return [p.as_dict() for p in out]
 
 
 class PushedBuffer(ctypes.Structure):

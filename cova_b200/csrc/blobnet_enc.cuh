@@ -447,11 +447,11 @@ __global__ void __launch_bounds__(C::THREADS, 1) enc_ws_kernel(const __grid_cons
 }
 
 // ------------------------------------------------------------------------------------------------ launch
+// as tc::plan / tc::launch
 template <class C>
-inline bool try_launch_e(LayerParams p, int n_sms, cudaStream_t st, cudaError_t &err, int min_stage) {
+inline bool plan_e(LayerParams &p, int n_sms, int min_stage, tc::Grid &g) {
     const long long mtot = (long long)p.N * p.gin.S * p.gin.Tn;
     if (mtot >= (1ll << 31)) return false;
-    if ((p.out != nullptr) != C::HAS_OUT || !p.out2) return false;       // output set is part of the configuration (ECfg::HAS_OUT)
     p.n_tiles = (int)((mtot + C::NP - 1) / C::NP);
     p.n_groups = (p.n_tiles + C::TPS - 1) / C::TPS;
     p.Ls = C::TPS * C::NP + 2 * p.gin.halo;
@@ -460,16 +460,20 @@ inline bool try_launch_e(LayerParams p, int n_sms, cudaStream_t st, cudaError_t 
     for (p.n_stage = kMaxStage; p.n_stage >= 1; p.n_stage--)
         if (plan_smem_e<C>(p.Ls, p.n_stage).total <= (uint32_t)tc::kSmemLimit) break;
     if (p.n_stage < min_stage) return false;
-    const SmemPlanE sp = plan_smem_e<C>(p.Ls, p.n_stage);
-    err = cudaFuncSetAttribute(enc_ws_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::kSmemLimit);   // see tc::try_launch
-    if (err != cudaSuccess) return true;
+    g.smem = plan_smem_e<C>(p.Ls, p.n_stage).total;
+    g.ctas = std::max(1, std::min(n_sms, p.n_groups));
+    return true;
+}
+
+template <class C>
+inline cudaError_t launch_e(const LayerParams &p, const tc::Grid &g, cudaStream_t st) {
+    if ((p.out != nullptr) != C::HAS_OUT || !p.out2) return cudaErrorInvalidValue;   // output set is part of the configuration (ECfg::HAS_OUT)
+    cudaError_t err = cudaFuncSetAttribute(enc_ws_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::kSmemLimit);   // see tc::launch
+    if (err != cudaSuccess) return err;
     ELayerExtra ex;
     ex.divS = make_fastdiv((uint32_t)p.gin.S);
     ex.divP = make_fastdiv((uint32_t)p.gin.P);
-    int ctas = std::min(n_sms, p.n_groups);
-    if (ctas < 1) ctas = 1;
-    err = launch_pdl(enc_ws_kernel<C>, dim3((unsigned)ctas), dim3(C::THREADS), sp.total, st, !(p.dbg & kDbgNoPdl), p, ex);
-    return true;
+    return launch_pdl(enc_ws_kernel<C>, dim3((unsigned)g.ctas), dim3(C::THREADS), g.smem, st, !(p.dbg & kDbgNoPdl), p, ex);
 }
 
 }  // namespace tcs

@@ -290,7 +290,8 @@ __global__ void __launch_bounds__(kThreads1, 1) enc1_fused_kernel(const __grid_c
     if (warp == 1) tc::tmem_dealloc(tmem_base, 512);
 }
 
-inline bool try_launch_enc1(LayerParams p, Enc1Extra ex, int n_sms, cudaStream_t st, cudaError_t &err) {
+// as tc::plan / tc::launch: the ring depth is the only choice (as deep as fits, at least 2)
+inline bool plan_enc1(LayerParams &p, Enc1Extra &ex, int n_sms, tc::Grid &g) {
     p.Ls = kPairRows + 2 * p.gin.halo;
     if (p.gin.P >= 16384) return false;                                            // LBO field: 14 bits of 16-byte units
     ex.ntp = (p.gin.S + kPairRows - 1) / kPairRows;
@@ -309,11 +310,15 @@ inline bool try_launch_enc1(LayerParams p, Enc1Extra ex, int n_sms, cudaStream_t
         if (plan_smem1(p.Ls, p.n_stage, p.w_bytes).total <= (uint32_t)tc::kSmemLimit) break;
     if (p.n_stage < 2) return false;
     // more than half of the SM's shared memory: one CTA per SM (the CTA allocates all 512 TMEM columns)
-    const uint32_t total = std::max<uint32_t>(plan_smem1(p.Ls, p.n_stage, p.w_bytes).total, 120u * 1024u);
-    err = cudaFuncSetAttribute(enc1_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::kSmemLimit);   // see tc::try_launch
-    if (err != cudaSuccess) return true;
-    err = launch_pdl(enc1_fused_kernel, dim3((unsigned)ctas), dim3(kThreads1), total, st, !(p.dbg & kDbgNoPdl), p, ex);
+    g.smem = std::max<uint32_t>(plan_smem1(p.Ls, p.n_stage, p.w_bytes).total, 120u * 1024u);
+    g.ctas = ctas;
     return true;
+}
+
+inline cudaError_t launch_enc1(const LayerParams &p, const Enc1Extra &ex, const tc::Grid &g, cudaStream_t st) {
+    cudaError_t err = cudaFuncSetAttribute(enc1_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::kSmemLimit);   // see tc::launch
+    if (err != cudaSuccess) return err;
+    return launch_pdl(enc1_fused_kernel, dim3((unsigned)g.ctas), dim3(kThreads1), g.smem, st, !(p.dbg & kDbgNoPdl), p, ex);
 }
 
 }  // namespace tc1

@@ -699,8 +699,16 @@ __global__ void __launch_bounds__(kThreads, 1) shiftgemm_kernel(const __grid_con
 // ------------------------------------------------------------------------------------------------ launch
 constexpr int kSmemLimit = 227 * 1024;
 
+// Host-side part of a launch, split in two so that the choice can be queried without a device (cova_blobnet_plan).
+// plan: fills the tiling fields of p (n_tiles, n_groups, Ls, n_stage, w_bytes, divS, divP) and the grid; false when C
+// does not fit this geometry with at least min_stage strips in its ring.  launch: the attribute call and the launch.
+struct Grid {
+    int ctas;          // CTAs launched (all N-halves)
+    uint32_t smem;     // dynamic shared memory per CTA
+};
+
 template <class C>
-inline bool try_launch(LayerParams p, int n_sms, cudaStream_t st, cudaError_t &err, int min_stage) {
+inline bool plan(LayerParams &p, int n_sms, int min_stage, Grid &g) {
     const long long mtot = (long long)p.N * p.gin.S * p.gin.Tn;
     p.n_tiles = (int)((mtot + kTileM - 1) / kTileM);
     p.n_groups = (p.n_tiles + C::TPS - 1) / C::TPS;
@@ -716,18 +724,23 @@ inline bool try_launch(LayerParams p, int n_sms, cudaStream_t st, cudaError_t &e
     for (p.n_stage = target; p.n_stage >= 1; p.n_stage--)
         if (plan_smem<C>(p.Ls, p.n_stage, p.w_bytes, epi_floats<C>()).total <= (uint32_t)kSmemLimit) break;
     if (p.n_stage < min_stage) return false;
-    const SmemPlan sp = plan_smem<C>(p.Ls, p.n_stage, p.w_bytes, epi_floats<C>());
+    g.smem = plan_smem<C>(p.Ls, p.n_stage, p.w_bytes, epi_floats<C>()).total;
+    int ctas = n_sms / nsplit;
+    if (ctas > p.n_groups) ctas = p.n_groups;
+    if (ctas < 1) ctas = 1;
+    g.ctas = ctas * nsplit;
+    return true;
+}
+
+template <class C>
+inline cudaError_t launch(const LayerParams &p, const Grid &g, cudaStream_t st) {
     // The attribute belongs to the FUNCTION (per device), not to a launch, and the last write wins: two handles with
     // different grids on two threads would otherwise lower it under each other's feet between "set" and "launch"
     // (seen as cudaErrorInvalidValue by tests/test_gpu_parity.py::test_two_threads_two_handles...).  Always the same value,
     // the architectural maximum, makes the call idempotent; occupancy follows the size actually requested at launch.
-    err = cudaFuncSetAttribute(shiftgemm_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit);
-    if (err != cudaSuccess) return true;
-    int ctas = n_sms / nsplit;
-    if (ctas > p.n_groups) ctas = p.n_groups;
-    if (ctas < 1) ctas = 1;
-    err = launch_pdl(shiftgemm_kernel<C>, dim3((unsigned)(ctas * nsplit)), dim3(kThreads), sp.total, st, !(p.dbg & kDbgNoPdl), p);
-    return true;
+    cudaError_t err = cudaFuncSetAttribute(shiftgemm_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit);
+    if (err != cudaSuccess) return err;
+    return launch_pdl(shiftgemm_kernel<C>, dim3((unsigned)g.ctas), dim3(kThreads), g.smem, st, !(p.dbg & kDbgNoPdl), p);
 }
 
 }  // namespace tc

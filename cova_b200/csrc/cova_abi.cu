@@ -575,6 +575,7 @@ struct cova_pipeline {
     size_t ev_used = 0;
     uint64_t launches = 0;
     int dbg = 0;
+    cova_layer_plan last_plan[8] = {};   // per layer: the plan of its last tcgen05 launch (cova_pipeline_last_plan)
 };
 
 static uint32_t windows_per_stream(uint32_t fps, uint32_t T, uint32_t gamma) {
@@ -612,6 +613,17 @@ static int upload_layer(DevLayer &dl, const PackedLayer *halves, int n_halves) {
     return rc;
 }
 
+// chains per chunk: ~1024 windows per chunk, at most 16 chunks; tiny pipelines stay single-chunk
+static uint32_t chunk_streams_for(uint32_t max_streams, uint32_t max_windows, uint32_t flags) {
+    uint32_t chunks = std::min<uint32_t>(16, std::max<uint32_t>(1, max_windows / 1024));
+    const uint32_t hint = (flags >> 16) & 0xffu;
+    if (hint) chunks = hint;
+    chunks = std::min(chunks, max_streams);
+    return (max_streams + chunks - 1) / chunks;
+}
+static void blobnet_geoms(int h_mb, int w_mb, int N, int F, int sizes_h[5], int sizes_w[5], Geom gx[4], Geom gd[4], Geom &gx0f);
+static int plan_blobnet(int h_mb, int w_mb, int N, int n_chains, int fps, int gamma, int dbg, int n_sms, cova_layer_plan out[8]);
+
 extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb, uint32_t h_mb, uint32_t timestep,
                                  uint32_t gamma, uint32_t max_streams, uint32_t max_fps, const void *weights,
                                  size_t weights_len, uint32_t cc_threshold, uint32_t flags) {
@@ -627,6 +639,15 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
     int rc = ccl_check_flags(flags);
     if (!rc) rc = ccl_check_bands(flags, h_mb);
     if (rc) return rc;
+    const uint32_t max_windows = max_streams * windows_per_stream(max_fps, timestep, gamma);
+    const uint32_t chunk_streams = chunk_streams_for(max_streams, max_windows, flags);
+    {   // every layer must have a tile plan for a chunk of this grid (the widest grids run out of shared memory for the
+        // strips of block 4 first).  Whether a plan fits does not depend on the SM count.
+        cova_layer_plan plans[8];
+        rc = plan_blobnet((int)h_mb, (int)w_mb, (int)(chunk_streams * windows_per_stream(max_fps, timestep, gamma)), (int)chunk_streams,
+                          (int)max_fps, (int)gamma, 0, 1, plans);
+        if (rc) return rc;
+    }
     if (flags & COVA_FLAG_INPUT_PACKED16) {
         if (flags & COVA_FLAG_KEEP_STACKED) return set_err(COVA_E_INVAL, "the stacked RGBA windows cannot be rebuilt from packed input (byte 3 and values above 6 are gone)");
         if ((flags & 0xffu) == COVA_IMPL_SIMT) return set_err(COVA_E_UNSUPPORTED, "the validation kernels read the 4-byte input format");
@@ -643,7 +664,7 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
     p->device = device; p->W = w_mb; p->H = h_mb; p->T = timestep; p->gamma = gamma;
     p->max_streams = max_streams; p->max_fps = max_fps; p->flags = flags; p->impl = flags & 0xffu;
     p->cc_threshold = cc_threshold;
-    p->max_windows = max_streams * windows_per_stream(max_fps, timestep, gamma);
+    p->max_windows = max_windows;
     auto fail = [&](int code) { cova_pipeline_free(p); return code; };
     if ((rc = parse_weights(weights, weights_len, p->hw))) return fail(rc);
     cudaDeviceProp prop;
@@ -654,14 +675,9 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
     if (cudaStreamCreateWithFlags(&p->own_stream, cudaStreamNonBlocking) != cudaSuccess) return fail(set_err(COVA_E_CUDA, "stream creation failed"));
     p->stream = p->own_stream;
 
-    {   // chunking: ~1024 windows per chunk, at most 16 chunks; tiny pipelines stay single-chunk
-        const uint32_t wps = windows_per_stream(max_fps, timestep, gamma);
-        uint32_t chunks = std::min<uint32_t>(16, std::max<uint32_t>(1, p->max_windows / 1024));
-        const uint32_t hint = (flags >> 16) & 0xffu;
-        if (hint) chunks = hint;
-        chunks = std::min(chunks, max_streams);
-        p->chunk_streams = (max_streams + chunks - 1) / chunks;
-        chunks = (max_streams + p->chunk_streams - 1) / p->chunk_streams;
+    {
+        p->chunk_streams = chunk_streams;
+        const uint32_t chunks = (max_streams + p->chunk_streams - 1) / p->chunk_streams;
         if (cudaStreamCreateWithFlags(&p->s_in, cudaStreamNonBlocking) != cudaSuccess ||
             cudaStreamCreateWithFlags(&p->s_out, cudaStreamNonBlocking) != cudaSuccess)
             return fail(set_err(COVA_E_CUDA, "stream creation failed"));
@@ -674,17 +690,11 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
                     cudaEventCreateWithFlags(&sl.ev_done[c], cudaEventDisableTiming) != cudaSuccess)
                     return fail(set_err(COVA_E_CUDA, "event creation failed"));
         }
-        (void)wps;
     }
     const int N = (int)(p->chunk_streams * windows_per_stream(max_fps, timestep, gamma));   // windows per chunk
     const int NB = (int)p->max_windows;                                                       // windows per batch
-    p->sizes_h[0] = (int)h_mb; p->sizes_w[0] = (int)w_mb;
-    for (int i = 1; i <= 4; i++) { p->sizes_h[i] = (p->sizes_h[i - 1] + 1) / 2; p->sizes_w[i] = (p->sizes_w[i - 1] + 1) / 2; }
-    // encoder inputs (Tn = 4): X0 (8 ch incl. padding), X1 (16), X2 (32), X3 (64)
-    const int xc[4] = {8, 16, 32, 64};
-    for (int i = 0; i < 4; i++) p->gx[i] = make_geom(p->sizes_h[i], p->sizes_w[i], xc[i], kT, N);
-    // decoder inputs (Tn = 1): D0in = enc4 t0 (128 @ s4), D1in (128 @ s3), D2in (64 @ s2), D3in (32 @ s1)
-    for (int i = 0; i < 4; i++) p->gd[i] = make_geom(p->sizes_h[4 - i], p->sizes_w[4 - i], kDecCin[i], 1, N);
+    const int F = (int)(p->chunk_streams * max_fps);
+    blobnet_geoms((int)h_mb, (int)w_mb, N, F, p->sizes_h, p->sizes_w, p->gx, p->gd, p->gx0f);
     auto alloc_zero = [&](uint4 **ptr, const Geom &g) -> int {
         size_t bytes = (size_t)geom_rows(g) * 16;
         COVA_CUDA(cudaMalloc(ptr, bytes));
@@ -697,8 +707,6 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
             if ((rc = alloc_zero(&p->x[i], p->gx[i]))) return fail(rc);
         if ((rc = alloc_zero(&p->d[i], p->gd[i]))) return fail(rc);
     }
-    const int F = (int)(p->chunk_streams * max_fps);
-    p->gx0f = make_geom(p->sizes_h[0], p->sizes_w[0], 8, 1, F);
     if ((rc = alloc_zero(&p->x0f, p->gx0f))) return fail(rc);
     p->packed = (flags & COVA_FLAG_INPUT_PACKED16) != 0;
     p->frame_bytes = (size_t)w_mb * h_mb * (p->packed ? 2 : 4);
@@ -1007,128 +1015,235 @@ static int simt_layer(cova_pipeline *p, int layer) {
 }
 #endif
 
-// Candidate tile configurations in order of preference; a configuration that can double-buffer its strips
-// (ring depth >= 2) beats an earlier one that cannot.
-template <class C0, class... Cs>
-static int launch_fit(const tc::LayerParams &lp, int n_sms, cudaStream_t st, int min_stage) {
-    cudaError_t err = cudaSuccess;
-    if (tc::try_launch<C0>(lp, n_sms, st, err, min_stage)) {
-        if (err != cudaSuccess) return set_err(COVA_E_CUDA, "tcgen05 layer launch: %s", cudaGetErrorString(err));
-        return COVA_OK;
-    }
-    if constexpr (sizeof...(Cs) > 0) return launch_fit<Cs...>(lp, n_sms, st, min_stage);
-    else return COVA_E_UNSUPPORTED;
-}
+// ---- launch plans ------------------------------------------------------------------------------------
+// The candidate tile configurations of every tcgen05 layer, in order of preference.  Each list is written once:
+// plan_layer() picks an entry and launch_layer() launches that entry of the same list.
 template <class... Cs>
-static int launch_first_fit(const tc::LayerParams &lp, int n_sms, cudaStream_t st) {
-    int rc = launch_fit<Cs...>(lp, n_sms, st, 2);
-    if (rc == COVA_E_UNSUPPORTED) rc = launch_fit<Cs...>(lp, n_sms, st, 1);
-    if (rc == COVA_E_UNSUPPORTED) return set_err(COVA_E_UNSUPPORTED, "no tcgen05 tile configuration fits shared memory for this macroblock grid");
-    return rc;
+struct Cands {};
+using tc::Cfg;
+using tc::MODE_DEC;
+using tc::MODE_ENC;
+using tc::MODE_HEAD;
+using tcs::ECfg;
+//                       CIN_CB COUT LA LB NP TPS
+using Enc2Ws = Cands<ECfg<2, 32, 2, 2, 192, 3>, ECfg<2, 32, 2, 2, 192, 2>, ECfg<2, 32, 2, 2, 192, 1>>;
+using Enc3Ws = Cands<ECfg<4, 64, 1, 2, 128, 2>, ECfg<4, 64, 1, 2, 128, 1>>;
+using Enc4Ws = Cands<ECfg<8, 128, 1, 1, 64, 2>, ECfg<8, 128, 1, 1, 64, 1>>;
+//                    MODE   CIN_CB NCOLS TPS KCH COUT
+using Enc2Pos = Cands<Cfg<MODE_ENC, 2, 32, 4, 2, 32>, Cfg<MODE_ENC, 2, 32, 2, 2, 32>, Cfg<MODE_ENC, 2, 32, 1, 2, 32>>;
+using Enc3Pos = Cands<Cfg<MODE_ENC, 4, 64, 1, 4, 64>, Cfg<MODE_ENC, 4, 64, 1, 2, 64>>;
+using Enc4Pos = Cands<Cfg<MODE_ENC, 8, 128, 1, 2, 128>>;
+using Dec0Pos = Cands<Cfg<MODE_DEC, 16, 128, 1, 2, 64>>;
+using Dec1Pos = Cands<Cfg<MODE_DEC, 16, 128, 1, 2, 32>>;
+using Dec2Pos = Cands<Cfg<MODE_DEC, 8, 64, 1, 4, 16>, Cfg<MODE_DEC, 8, 64, 1, 2, 16>>;
+using Dec3Pos = Cands<Cfg<MODE_HEAD, 4, 16, 2, 4, 16>, Cfg<MODE_HEAD, 4, 16, 1, 4, 16>, Cfg<MODE_HEAD, 4, 16, 1, 2, 16>>;
+
+static const char *const kLayerName[8] = {"enc1", "enc2", "enc3", "enc4", "dec0", "dec1", "dec2", "dec3+head"};
+
+// One layer's plan: the public record, the layer parameters with their tiling fields filled, and the grid.
+struct LayerPlan {
+    cova_layer_plan info;
+    tc::LayerParams lp;
+    tc1::Enc1Extra ex;        // block 1 only
+    tc::Grid grid;
+};
+
+template <bool WS, class C0, class... Cs>
+static bool fit(LayerPlan &pl, int n_sms, int min_stage, int idx = 0) {
+    tc::LayerParams q = pl.lp;
+    bool ok;
+    if constexpr (WS) ok = tcs::plan_e<C0>(q, n_sms, min_stage, pl.grid);
+    else ok = tc::plan<C0>(q, n_sms, min_stage, pl.grid);
+    if (ok) {
+        pl.lp = q;
+        pl.info.config = idx;
+        pl.info.tps = C0::TPS;
+        if constexpr (WS) pl.info.tile = C0::NP;
+        else pl.info.tile = kTileM;
+        return true;
+    }
+    if constexpr (sizeof...(Cs) > 0) return fit<WS, Cs...>(pl, n_sms, min_stage, idx + 1);
+    else return false;
+}
+// first fit in list order, except that a configuration that can double-buffer its strips (ring depth >= 2) beats an
+// earlier one that cannot
+template <bool WS, class... Cs>
+static bool first_fit(Cands<Cs...>, LayerPlan &pl, int n_sms) {
+    pl.info.family = WS ? COVA_PLAN_WS : COVA_PLAN_POS;
+    return fit<WS, Cs...>(pl, n_sms, 2) || fit<WS, Cs...>(pl, n_sms, 1);
+}
+template <bool WS, class C0, class... Cs>
+static cudaError_t launch_nth(const LayerPlan &pl, int idx, cudaStream_t st) {
+    if (idx == 0) {
+        if constexpr (WS) return tcs::launch_e<C0>(pl.lp, pl.grid, st);
+        else return tc::launch<C0>(pl.lp, pl.grid, st);
+    }
+    if constexpr (sizeof...(Cs) > 0) return launch_nth<WS, Cs...>(pl, idx - 1, st);
+    else return cudaErrorInvalidValue;
+}
+template <bool WS, class... Cs>
+static cudaError_t launch_entry(Cands<Cs...>, const LayerPlan &pl, cudaStream_t st) {
+    return launch_nth<WS, Cs...>(pl, pl.info.config, st);
 }
 
-template <class C0, class... Cs>
-static int launch_fit_e(const tc::LayerParams &lp, int n_sms, cudaStream_t st, int min_stage) {
-    cudaError_t err = cudaSuccess;
-    if (tcs::try_launch_e<C0>(lp, n_sms, st, err, min_stage)) {
-        if (err != cudaSuccess) return set_err(COVA_E_CUDA, "tcgen05 encoder launch: %s", cudaGetErrorString(err));
-        return COVA_OK;
+// The geometry part of a layer's parameters, all a plan depends on: N windows (block 1: n_chains chains of fps frames).
+static void plan_input(LayerPlan &pl, int layer, const Geom gx[4], const Geom gd[4], const Geom &gx0f, int N, int n_chains,
+                       int fps, int gamma) {
+    memset(&pl, 0, sizeof(pl));
+    tc::LayerParams &lp = pl.lp;
+    lp.N = N;
+    lp.nsplit = 1;
+    if (layer == 0) {
+        lp.gin = gx0f; lp.gout = gx[1]; lp.gout2 = gd[3]; lp.N = n_chains * fps;
+        pl.ex.n_chains = n_chains; pl.ex.fps = fps; pl.ex.gamma = gamma;
+    } else if (layer < 4) {
+        const int i = layer;
+        lp.gin = gx[i]; lp.gout = i < 3 ? gx[i + 1] : gx[3]; lp.gout2 = gd[3 - i];
+    } else {
+        const int i = layer - 4;
+        lp.gin = gd[i]; lp.gout = i < 3 ? gd[i + 1] : gd[3];
+        lp.nsplit = i == 0 ? 2 : 1;
     }
-    if constexpr (sizeof...(Cs) > 0) return launch_fit_e<Cs...>(lp, n_sms, st, min_stage);
-    else return COVA_E_UNSUPPORTED;
-}
-template <class... Cs>
-static int launch_first_fit_e(const tc::LayerParams &lp, int n_sms, cudaStream_t st) {
-    int rc = launch_fit_e<Cs...>(lp, n_sms, st, 2);
-    if (rc == COVA_E_UNSUPPORTED) rc = launch_fit_e<Cs...>(lp, n_sms, st, 1);
-    return rc;
 }
 
-static int tc_layer(cova_pipeline *p, int layer) {
-    using namespace tc;
-    const int N = (int)p->ck_windows;
-    LayerParams lp;
-    memset(&lp, 0, sizeof(lp));
-    lp.N = N; lp.watchdog = p->d_watchdog; lp.dbg = p->dbg;
-    int rc;
+// THE launch decision of a tcgen05 layer: kernel family and candidate for the geometry in pl (plan_input).  tc_layer launches
+// what it returns, cova_blobnet_plan and cova_pipeline_new report or check it.  Depends on the grid width (the strip length
+// grows with the row pitch), the debug bits 2 and 3, and the window count only through the SM count and 32-bit limits.
+static int plan_layer(int layer, int dbg, int n_sms, LayerPlan &pl) {
+    bool ok = false;
+    if (layer == 0) {
+        // first block: frame-level conv + PointWiseTN over a register ring of 4 frames, one kernel (blobnet_enc1.cuh)
+        ok = tc1::plan_enc1(pl.lp, pl.ex, n_sms, pl.grid);
+        pl.info.family = COVA_PLAN_ENC1; pl.info.tps = 2; pl.info.tile = kTileM;
+    } else if (layer < 4) {
+        const int i = layer;
+        // block 3 (Cout = 64) stays on the positions-as-M kernel: measured 0.335 ms vs 0.376 ms per 8192 windows at 720p
+        // (profiles/r1c_layer_timing.txt); dbg bit 3 forces the weights-stationary variant for experiments, dbg bit 2 the
+        // positions-as-M kernel for blocks 2 and 4
+        if (!(dbg & 4) && (i != 2 || (dbg & 8))) {
+            // weights-stationary kernel first; the positions-as-M kernel below remains the fallback for grids
+            // whose strips do not fit shared memory
+            ok = i == 1 ? first_fit<true>(Enc2Ws{}, pl, n_sms) : i == 2 ? first_fit<true>(Enc3Ws{}, pl, n_sms) : first_fit<true>(Enc4Ws{}, pl, n_sms);
+        }
+        if (!ok) ok = i == 1 ? first_fit<false>(Enc2Pos{}, pl, n_sms) : i == 2 ? first_fit<false>(Enc3Pos{}, pl, n_sms) : first_fit<false>(Enc4Pos{}, pl, n_sms);
+    } else {
+        const int i = layer - 4;
+        ok = i == 0 ? first_fit<false>(Dec0Pos{}, pl, n_sms) : i == 1 ? first_fit<false>(Dec1Pos{}, pl, n_sms)
+           : i == 2 ? first_fit<false>(Dec2Pos{}, pl, n_sms) : first_fit<false>(Dec3Pos{}, pl, n_sms);
+    }
+    if (!ok) {
+        pl.info = cova_layer_plan{};
+        return set_err(COVA_E_UNSUPPORTED, "%s: no tcgen05 tile configuration fits shared memory for this macroblock grid", kLayerName[layer]);
+    }
+    pl.info.n_stage = pl.lp.n_stage;
+    pl.info.n_groups = layer == 0 ? pl.ex.total : pl.lp.n_groups;
+    pl.info.ctas = pl.grid.ctas;
+    return COVA_OK;
+}
+
+static cudaError_t launch_layer(int layer, const LayerPlan &pl, cudaStream_t st) {
+    const bool ws = pl.info.family == COVA_PLAN_WS;
+    switch (layer) {
+        case 0: return tc1::launch_enc1(pl.lp, pl.ex, pl.grid, st);
+        case 1: return ws ? launch_entry<true>(Enc2Ws{}, pl, st) : launch_entry<false>(Enc2Pos{}, pl, st);
+        case 2: return ws ? launch_entry<true>(Enc3Ws{}, pl, st) : launch_entry<false>(Enc3Pos{}, pl, st);
+        case 3: return ws ? launch_entry<true>(Enc4Ws{}, pl, st) : launch_entry<false>(Enc4Pos{}, pl, st);
+        case 4: return launch_entry<false>(Dec0Pos{}, pl, st);
+        case 5: return launch_entry<false>(Dec1Pos{}, pl, st);
+        case 6: return launch_entry<false>(Dec2Pos{}, pl, st);
+        default: return launch_entry<false>(Dec3Pos{}, pl, st);
+    }
+}
+
+// extents and activation geometries of a grid: N windows, F frames (block-1 input) per chunk
+static void blobnet_geoms(int h_mb, int w_mb, int N, int F, int sizes_h[5], int sizes_w[5], Geom gx[4], Geom gd[4], Geom &gx0f) {
+    sizes_h[0] = h_mb; sizes_w[0] = w_mb;
+    for (int i = 1; i <= 4; i++) { sizes_h[i] = (sizes_h[i - 1] + 1) / 2; sizes_w[i] = (sizes_w[i - 1] + 1) / 2; }
+    // encoder inputs (Tn = 4): X0 (8 ch incl. padding), X1 (16), X2 (32), X3 (64)
+    const int xc[4] = {8, 16, 32, 64};
+    for (int i = 0; i < 4; i++) gx[i] = make_geom(sizes_h[i], sizes_w[i], xc[i], kT, N);
+    // decoder inputs (Tn = 1): D0in = enc4 t0 (128 @ s4), D1in (128 @ s3), D2in (64 @ s2), D3in (32 @ s1)
+    for (int i = 0; i < 4; i++) gd[i] = make_geom(sizes_h[4 - i], sizes_w[4 - i], kDecCin[i], 1, N);
+    // per-FRAME first-conv input (x-pair packed, Tn = 1, N = frames)
+    gx0f = make_geom(sizes_h[0], sizes_w[0], 8, 1, F);
+}
+
+// plans of all eight layers for chunks of n_chains chains of fps frames that yield N windows
+static int plan_blobnet(int h_mb, int w_mb, int N, int n_chains, int fps, int gamma, int dbg, int n_sms, cova_layer_plan out[8]) {
+    int sh[5], sw[5];
+    Geom gx[4], gd[4], gx0f;
+    blobnet_geoms(h_mb, w_mb, N, n_chains * fps, sh, sw, gx, gd, gx0f);
+    for (int layer = 0; layer < 8; layer++) {
+        LayerPlan pl;
+        plan_input(pl, layer, gx, gd, gx0f, N, n_chains, fps, gamma);
+        int rc = plan_layer(layer, dbg, n_sms, pl);
+        if (rc) return rc;
+        out[layer] = pl.info;
+    }
+    return COVA_OK;
+}
+
+extern "C" int cova_blobnet_plan(uint32_t w_mb, uint32_t h_mb, uint32_t windows, int debug, int n_sms, cova_layer_plan out[8]) {
+    if (!out) return set_err(COVA_E_INVAL, "null argument");
+    memset(out, 0, 8 * sizeof(cova_layer_plan));
+    if (!windows || windows > (1u << 24) || n_sms < 1) return set_err(COVA_E_INVAL, "need 1 <= windows <= 2^24 and n_sms >= 1");
+    if (w_mb < 16 || h_mb < 16 || w_mb > (1u << 16) || h_mb > (1u << 16))
+        return set_err(COVA_E_UNSUPPORTED, "macroblock grid must be at least 16x16 for four 2x poolings");
+    // one chain of windows + timestep - 1 frames at gamma 1
+    return plan_blobnet((int)h_mb, (int)w_mb, (int)windows, 1, (int)windows + kT - 1, 1, debug, n_sms, out);
+}
+
+static int tc_plan(cova_pipeline *p, int layer, LayerPlan &pl) {
+    plan_input(pl, layer, p->gx, p->gd, p->gx0f, (int)p->ck_windows, (int)p->ck_n_streams, (int)p->cur_fps, (int)p->gamma);
+    return plan_layer(layer, p->dbg, p->n_sms, pl);
+}
+
+// launch a planned layer: everything but the plan's geometry and tiling fields is filled here
+static int tc_launch(cova_pipeline *p, int layer, LayerPlan &pl) {
+    tc::LayerParams &lp = pl.lp;
+    lp.watchdog = p->d_watchdog; lp.dbg = p->dbg;
     if (layer < 4) {
         const int i = layer;
-        lp.in = p->x[i]; lp.gin = p->gx[i];
+        lp.in = p->x[i];
         lp.out = i < 3 ? p->x[i + 1] : nullptr;
-        lp.gout = i < 3 ? p->gx[i + 1] : p->gx[3];
-        lp.out2 = p->d[3 - i]; lp.gout2 = p->gd[3 - i];
+        lp.out2 = p->d[3 - i];
         lp.out2_cb = i < 3 ? kDecCout[2 - i] / 8 : 0;
-        lp.wpack = p->enc[i].wpack; lp.epi = p->enc[i].epi;
+        const DevLayer &dl = pl.info.family == COVA_PLAN_WS ? p->encs[i] : p->enc[i];
+        lp.wpack = dl.wpack; lp.epi = dl.epi;
         memcpy(lp.tn_w1, p->hw.enc[i].tn_w1, 64);
         memcpy(lp.tn_w2, p->hw.enc[i].tn_w2, 64);
-        lp.nsplit = 1;
         lp.bn_nonneg = 1;
         for (int c = 0; c < kEncCout[i]; c++)
             if (!(p->hw.enc[i].gamma[c] >= 0.f)) lp.bn_nonneg = 0;
         if (i == 0) {
-            // first block: frame-level conv + PointWiseTN over a register ring of 4 frames, one kernel (blobnet_enc1.cuh).
-            // It takes every frame width up to 3172 macroblocks; block 2 already refuses beyond 800.
-            LayerParams fp = lp;
-            fp.in = p->x0f; fp.gin = p->gx0f; fp.out = p->x[1]; fp.gout = p->gx[1]; fp.N = (int)(p->ck_n_streams * p->cur_fps);
-            tc1::Enc1Extra ex;
-            memset(&ex, 0, sizeof(ex));
-            ex.n_chains = (int)p->ck_n_streams; ex.fps = (int)p->cur_fps; ex.gamma = (int)p->gamma;
-            ex.tab = p->slot[p->cur_slot].d_tab + p->ck_stream0;
-            cudaError_t err = cudaSuccess;
-            if (!tc1::try_launch_enc1(fp, ex, p->n_sms, p->stream, err))
-                return set_err(COVA_E_UNSUPPORTED, "no tcgen05 tile configuration fits shared memory for this macroblock grid");
-            if (err != cudaSuccess) return set_err(COVA_E_CUDA, "fused enc1 launch: %s", cudaGetErrorString(err));
-            p->launches++;
-            prof_mark(p, "tc_enc1_fused");
-            return COVA_OK;
+            lp.in = p->x0f;
+            pl.ex.tab = p->slot[p->cur_slot].d_tab + p->ck_stream0;
         }
-        // block 3 (Cout = 64) stays on the positions-as-M kernel: measured 0.335 ms vs 0.376 ms per 8192 windows at 720p
-        // (profiles/r1c_layer_timing.txt); dbg bit 3 forces the weights-stationary variant for experiments
-        if (!(p->dbg & 4) && (i != 2 || (p->dbg & 8))) {
-            // weights-stationary kernel first; the positions-as-M kernel below remains the fallback for grids
-            // whose strips do not fit shared memory
-            LayerParams ws = lp;
-            ws.wpack = p->encs[i].wpack; ws.epi = p->encs[i].epi;
-            using tcs::ECfg;
-            if (i == 1) rc = launch_first_fit_e<ECfg<2, 32, 2, 2, 192, 3>, ECfg<2, 32, 2, 2, 192, 2>, ECfg<2, 32, 2, 2, 192, 1>>(ws, p->n_sms, p->stream);
-            else if (i == 2) rc = launch_first_fit_e<ECfg<4, 64, 1, 2, 128, 2>, ECfg<4, 64, 1, 2, 128, 1>>(ws, p->n_sms, p->stream);
-            else rc = launch_first_fit_e<ECfg<8, 128, 1, 1, 64, 2>, ECfg<8, 128, 1, 1, 64, 1>>(ws, p->n_sms, p->stream);
-            if (rc != COVA_E_UNSUPPORTED) {
-                if (rc) return rc;
-                p->launches++;
-                prof_mark(p, i == 1 ? "tc_enc2" : i == 2 ? "tc_enc3" : "tc_enc4");
-                return COVA_OK;
-            }
-        }
-        //                                  MODE   CIN_CB NCOLS TPS KCH COUT
-        if (i == 1) rc = launch_first_fit<Cfg<MODE_ENC, 2, 32, 4, 2, 32>, Cfg<MODE_ENC, 2, 32, 2, 2, 32>, Cfg<MODE_ENC, 2, 32, 1, 2, 32>>(lp, p->n_sms, p->stream);
-        else if (i == 2) rc = launch_first_fit<Cfg<MODE_ENC, 4, 64, 2, 4, 64>, Cfg<MODE_ENC, 4, 64, 1, 4, 64>, Cfg<MODE_ENC, 4, 64, 1, 2, 64>>(lp, p->n_sms, p->stream);
-        else rc = launch_first_fit<Cfg<MODE_ENC, 8, 128, 1, 2, 128>>(lp, p->n_sms, p->stream);
-        if (rc) return rc;
-        p->launches++;
-        prof_mark(p, i == 1 ? "tc_enc2" : i == 2 ? "tc_enc3" : "tc_enc4");
-        return COVA_OK;
+    } else {
+        const int i = layer - 4;
+        lp.in = p->d[i];
+        lp.out = i < 3 ? p->d[i + 1] : nullptr;
+        lp.wpack = p->dec[i].wpack; lp.epi = p->dec[i].epi;
+        lp.psplit = (p->dbg & 64) ? 0 : 1;     // dbg bit 6: whole-tile accumulators for dec0 / dec1 (experiments)
+        lp.Ht = p->sizes_h[3 - i]; lp.Wt = p->sizes_w[3 - i];
+        crop_for(lp.gin.H, lp.Ht, lp.crop_t);
+        crop_for(lp.gin.W, lp.Wt, lp.crop_l);
+        lp.mask = p->d_mask + (size_t)p->ck_window0 * p->W * p->H;
+        lp.logits = p->d_logits ? p->d_logits + (size_t)p->ck_window0 * p->W * p->H : nullptr;
     }
-    const int i = layer - 4;
-    lp.in = p->d[i]; lp.gin = p->gd[i];
-    lp.out = i < 3 ? p->d[i + 1] : nullptr;
-    lp.gout = i < 3 ? p->gd[i + 1] : p->gd[3];
-    lp.wpack = p->dec[i].wpack; lp.epi = p->dec[i].epi;
-    lp.nsplit = i == 0 ? 2 : 1;
-    lp.psplit = (p->dbg & 64) ? 0 : 1;     // dbg bit 6: whole-tile accumulators for dec0 / dec1 (experiments)
-    lp.Ht = p->sizes_h[3 - i]; lp.Wt = p->sizes_w[3 - i];
-    crop_for(lp.gin.H, lp.Ht, lp.crop_t);
-    crop_for(lp.gin.W, lp.Wt, lp.crop_l);
-    lp.mask = p->d_mask + (size_t)p->ck_window0 * p->W * p->H;
-    lp.logits = p->d_logits ? p->d_logits + (size_t)p->ck_window0 * p->W * p->H : nullptr;
-    if (i == 0) rc = launch_first_fit<Cfg<MODE_DEC, 16, 128, 1, 2, 64>>(lp, p->n_sms, p->stream);
-    else if (i == 1) rc = launch_first_fit<Cfg<MODE_DEC, 16, 128, 1, 2, 32>>(lp, p->n_sms, p->stream);
-    else if (i == 2) rc = launch_first_fit<Cfg<MODE_DEC, 8, 64, 1, 4, 16>, Cfg<MODE_DEC, 8, 64, 1, 2, 16>>(lp, p->n_sms, p->stream);
-    else rc = launch_first_fit<Cfg<MODE_HEAD, 4, 16, 2, 4, 16>, Cfg<MODE_HEAD, 4, 16, 1, 4, 16>, Cfg<MODE_HEAD, 4, 16, 1, 2, 16>>(lp, p->n_sms, p->stream);
-    if (rc) return rc;
+    cudaError_t err = launch_layer(layer, pl, p->stream);
+    if (err != cudaSuccess) return set_err(COVA_E_CUDA, "%s launch: %s", kLayerName[layer], cudaGetErrorString(err));
+    p->last_plan[layer] = pl.info;
     p->launches++;
-    prof_mark(p, i == 0 ? "tc_dec0" : i == 1 ? "tc_dec1" : i == 2 ? "tc_dec2" : "tc_dec3_head");
+    static const char *const prof_name[8] = {"tc_enc1_fused", "tc_enc2", "tc_enc3", "tc_enc4", "tc_dec0", "tc_dec1", "tc_dec2", "tc_dec3_head"};
+    prof_mark(p, prof_name[layer]);
     return COVA_OK;
+}
+
+static int tc_layer(cova_pipeline *p, int layer) {
+    LayerPlan pl;
+    int rc = tc_plan(p, layer, pl);
+    return rc ? rc : tc_launch(p, layer, pl);
 }
 
 extern "C" int cova_pipeline_run_layer(cova_pipeline *p, int layer, uint32_t impl) {
@@ -1143,8 +1258,22 @@ extern "C" int cova_pipeline_run_layer(cova_pipeline *p, int layer, uint32_t imp
 
 static int blobnet_chunk(cova_pipeline *p) {
     if (!p->ck_windows) return COVA_OK;
+    if (p->impl == COVA_IMPL_SIMT) {
+        for (int layer = 0; layer < 8; layer++) {
+            int rc = simt_layer(p, layer);
+            if (rc) return rc;
+        }
+        return COVA_OK;
+    }
+    // every layer is planned before the first one is launched: a grid (or debug route) that one of them cannot take is
+    // refused on the host, with nothing of the chunk's network enqueued
+    LayerPlan plans[8];
     for (int layer = 0; layer < 8; layer++) {
-        int rc = p->impl == COVA_IMPL_SIMT ? simt_layer(p, layer) : tc_layer(p, layer);
+        int rc = tc_plan(p, layer, plans[layer]);
+        if (rc) return rc;
+    }
+    for (int layer = 0; layer < 8; layer++) {
+        int rc = tc_launch(p, layer, plans[layer]);
         if (rc) return rc;
     }
     return COVA_OK;
@@ -1660,6 +1789,11 @@ extern "C" int cova_pipeline_set_debug(cova_pipeline *p, int flags) {
     if (!p) return set_err(COVA_E_INVAL, "null handle");
     p->dbg = flags;
     // bit 5 (kDbgNoPdl): plain stream-ordered launches instead of programmatic dependent launch, for THIS handle only
+    return COVA_OK;
+}
+extern "C" int cova_pipeline_last_plan(const cova_pipeline *p, cova_layer_plan out[8]) {
+    if (!p || !out) return set_err(COVA_E_INVAL, "null argument");
+    memcpy(out, p->last_plan, sizeof(p->last_plan));
     return COVA_OK;
 }
 extern "C" int cova_pipeline_launch_count(const cova_pipeline *p, uint64_t *count) {

@@ -631,6 +631,12 @@ class BlobPipeline:
     def set_debug(self, flags: int):
         self._check(self._L.cova_pipeline_set_debug(self._h, flags))
 
+    def last_plan(self) -> list[dict]:
+        """cova_pipeline_last_plan: per layer the launch plan of its last tcgen05 launch (family 0: not launched yet)."""
+        out = (_lib.LayerPlan * _lib.N_LAYERS)()
+        self._check(self._L.cova_pipeline_last_plan(self._h, out))
+        return [p.as_dict() for p in out]
+
     def launch_count(self) -> int:
         c = ctypes.c_uint64()
         self._check(self._L.cova_pipeline_launch_count(self._h, ctypes.byref(c)))

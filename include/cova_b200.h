@@ -263,6 +263,33 @@ int cova_pipeline_run_layer(cova_pipeline *p, int layer, uint32_t impl);
  * stream-ordered launches instead of programmatic dependent launch (this handle only), bit 6 whole-tile accumulators for
  * dec0 / dec1 */
 int cova_pipeline_set_debug(cova_pipeline *p, int flags);
+
+/* Diagnostics: the launch plan of each tcgen05 BlobNet layer, out[layer] for the layers of cova_pipeline_run_layer.  Each
+ * layer picks its plan at run time from a list of candidate tile configurations, by what fits shared memory for the
+ * grid WIDTH (the operand strips hold TPS tiles plus two rows of halo); height does not matter, the window count only
+ * sets the number of tile groups and CTAs.  The widest grid every layer has a plan for at debug 0 is w_mb = 736
+ * macroblocks (block 4 runs out first); cova_pipeline_new refuses a wider one with COVA_E_UNSUPPORTED before it touches
+ * the device, and a debug route (cova_pipeline_set_debug bits 2 and 3) without a plan at the pipeline's width makes the
+ * run calls return COVA_E_UNSUPPORTED before they launch any BlobNet layer. */
+#define COVA_PLAN_ENC1 1 /* the fused block-1 kernel */
+#define COVA_PLAN_POS 2  /* positions-as-M kernel (output positions in the MMA's M) */
+#define COVA_PLAN_WS 3   /* weights-stationary kernel (blocks 2-4; weights in tensor memory) */
+typedef struct cova_layer_plan {
+    int32_t family;   /* COVA_PLAN_*; 0 = no plan / not launched yet */
+    int32_t config;   /* index of the tile configuration in the layer's candidate list for that family */
+    int32_t tps;      /* tiles per operand-ring stage */
+    int32_t tile;     /* output positions per tile */
+    int32_t n_stage;  /* operand-ring depth */
+    int32_t n_groups; /* tile groups (block 1: frame steps of tile pairs) that pass through the ring */
+    int32_t ctas;     /* CTAs launched */
+} cova_layer_plan;
+/* The plans the library would launch for a batch of `windows` windows (one chain of windows + timestep - 1 frames, gamma
+ * 1) of a w_mb x h_mb grid, with debug bits `debug`, on a device of n_sms SMs.  Host arithmetic only: needs no device.
+ * COVA_E_UNSUPPORTED, with the layer named in cova_last_error(), when some layer has no plan: out[] then holds the plans of
+ * the layers before it and zeros from it on. */
+int cova_blobnet_plan(uint32_t w_mb, uint32_t h_mb, uint32_t windows, int debug, int n_sms, cova_layer_plan out[8]);
+/* the plan each layer used at its last tcgen05 launch on this handle (family 0 for a layer not launched yet) */
+int cova_pipeline_last_plan(const cova_pipeline *p, cova_layer_plan out[8]);
 /* kernels launched by this handle since creation */
 int cova_pipeline_launch_count(const cova_pipeline *p, uint64_t *count);
 /* per-kernel device time of the last cova_pipeline_run* with profiling enabled: names is a
