@@ -496,6 +496,9 @@ struct DevLayer {
 
 constexpr int kSlots = 4;
 
+// chains [stream0, stream0 + n_streams) of a batch, which yield its windows [window0, window0 + windows)
+struct Chunk { uint32_t stream0, n_streams, window0, windows; };
+
 struct cova_pipeline {
     int device = 0, n_sms = 0;
     uint32_t W = 0, H = 0, T = 0, gamma = 1, max_streams = 0, max_fps = 0, max_windows = 0, flags = 0, impl = 0;
@@ -503,8 +506,6 @@ struct cova_pipeline {
     cudaStream_t own_stream = nullptr, stream = nullptr;
     size_t frame_bytes = 0;              // bytes of one frame in the pool: 4 per macroblock, or 2 with COVA_FLAG_INPUT_PACKED16
     bool packed = false;
-    uint8_t *d_frames = nullptr;
-    uint32_t cur_streams = 0, cur_fps = 0, cur_windows = 0;
     // per-stream state for CONTINUED batches (metapreprocess/imp.rs:38-42: prev_buffers and gamma_idx live as long as the
     // stream): the last T - 1 frames of every stream id on the device, frames seen so far on the host
     uint8_t *d_carry = nullptr;
@@ -515,7 +516,7 @@ struct cova_pipeline {
     // A batch is processed in chunks of whole chains: the activation buffers are sized for ONE chunk, and
     // process_host() overlaps the H2D copy of chunk c+1, the kernels of chunk c and the D2H of chunk c-1.
     uint32_t chunk_streams = 0;          // chains per chunk (capacity)
-    uint32_t ck_stream0 = 0, ck_n_streams = 0, ck_window0 = 0, ck_windows = 0;   // chunk being processed
+    Chunk last_chunk = {};               // the chunk whose activations the buffers hold (cova_pipeline_read_activation)
     cudaStream_t s_in = nullptr, s_out = nullptr;
     // Four batch slots (frame pool + box arena + events): submit_host(k+3) can be queued before collect_host(k).  A
     // batch's host-visible latency is H2D + kernels + D2H of the boxes (whose size the host must first learn): measured
@@ -527,8 +528,8 @@ struct cova_pipeline {
         CclBuffers ccl;
         std::vector<cudaEvent_t> ev_in, ev_done;
         unsigned long long *h_cursor = nullptr;      // pinned: per-chunk cursor snapshots (2 words each)
-        uint32_t n_streams = 0, fps = 0, n_windows = 0;
-        bool busy = false, failed = false, ready = false;
+        uint32_t n_streams = 0, fps = 0, n_windows = 0;  // n_streams = 0, n_windows = n: masks loaded directly, no chains
+        bool busy = false, failed = false;
         uint32_t *h_ids = nullptr, *d_ids = nullptr;   // stream ids of a submit_host2 batch (pinned staging + device copy)
         std::vector<uint64_t> win_pts;                 // per window: PTS of its newest frame / stream id (submit_host2)
         std::vector<uint32_t> win_ids;
@@ -551,7 +552,7 @@ struct cova_pipeline {
         unsigned long long *h_off = nullptr, *d_off = nullptr;
         cudaEvent_t ev_off = nullptr;                  // recorded after the offsets upload: the staging may be rewritten after it
     } slot[kSlots];
-    int cur_slot = 0, next_submit = 0, next_collect = 0;
+    int next_submit = 0, next_collect = 0, last_slot = 0;   // last_slot: given the last batch, read by stage-wise and read_*
     int sizes_h[5], sizes_w[5];          // extents: [0] input, [1..4] encoder outputs
     Geom gx[4];                          // X0..X3 (Tn = 4): inputs of enc1..enc4
     Geom gd[4];                          // D0in..D3in (Tn = 1): inputs of dec0..dec3
@@ -565,9 +566,7 @@ struct cova_pipeline {
     float *d_wraw = nullptr;
     DevLayer enc[4], dec[4];
     DevLayer encs[4];                    // blocks 2..4, weights-stationary kernel (blobnet_enc.cuh)
-    CclBuffers ccl;
     unsigned int *d_watchdog = nullptr;
-    unsigned long long *h_pinned = nullptr;   // cursor + overflow, then offsets/lens staging
     bool profiling = false;
     std::vector<cudaEvent_t> events;
     std::vector<std::string> names, last_names;
@@ -577,11 +576,8 @@ struct cova_pipeline {
     int dbg = 0;
     cova_layer_plan last_plan[8] = {};   // per layer: the plan of its last tcgen05 launch (cova_pipeline_last_plan)
 };
+using Slot = cova_pipeline::Slot;
 
-static uint32_t windows_per_stream(uint32_t fps, uint32_t T, uint32_t gamma) {
-    if (fps < T) return 0;
-    return (fps - T) / gamma + 1;
-}
 // windows of a device chain of `fps` frames whose first window has its newest frame at index `first`
 static uint32_t windows_from(uint32_t fps, uint32_t first, uint32_t gamma) { return fps > first ? (fps - 1 - first) / gamma + 1 : 0; }
 
@@ -621,6 +617,16 @@ static uint32_t chunk_streams_for(uint32_t max_streams, uint32_t max_windows, ui
     chunks = std::min(chunks, max_streams);
     return (max_streams + chunks - 1) / chunks;
 }
+static int ensure_slot(cova_pipeline *p, int k) {
+    auto &sl = p->slot[k];
+    if (!sl.d_frames) COVA_CUDA(cudaMalloc(&sl.d_frames, p->frame_bytes * p->max_streams * p->max_fps));
+    if (!sl.ccl.d_blob) {
+        sl.ccl.d_masks = p->d_mask;
+        int rc = ccl_alloc(sl.ccl, (int)p->H, (int)p->W, std::max<int>(1, (int)p->max_windows), false, p->flags);
+        if (rc) { ccl_free(sl.ccl, false); sl.ccl = CclBuffers(); return rc; }    // a later submit retries from scratch
+    }
+    return COVA_OK;
+}
 static void blobnet_geoms(int h_mb, int w_mb, int N, int F, int sizes_h[5], int sizes_w[5], Geom gx[4], Geom gd[4], Geom &gx0f);
 static int plan_blobnet(int h_mb, int w_mb, int N, int n_chains, int fps, int gamma, int dbg, int n_sms, cova_layer_plan out[8]);
 
@@ -639,12 +645,13 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
     int rc = ccl_check_flags(flags);
     if (!rc) rc = ccl_check_bands(flags, h_mb);
     if (rc) return rc;
-    const uint32_t max_windows = max_streams * windows_per_stream(max_fps, timestep, gamma);
+    const uint32_t chain_windows = windows_from(max_fps, timestep - 1, gamma);   // of a chain of max_fps frames
+    const uint32_t max_windows = max_streams * chain_windows;
     const uint32_t chunk_streams = chunk_streams_for(max_streams, max_windows, flags);
     {   // every layer must have a tile plan for a chunk of this grid (the widest grids run out of shared memory for the
         // strips of block 4 first).  Whether a plan fits does not depend on the SM count.
         cova_layer_plan plans[8];
-        rc = plan_blobnet((int)h_mb, (int)w_mb, (int)(chunk_streams * windows_per_stream(max_fps, timestep, gamma)), (int)chunk_streams,
+        rc = plan_blobnet((int)h_mb, (int)w_mb, (int)(chunk_streams * chain_windows), (int)chunk_streams,
                           (int)max_fps, (int)gamma, 0, 1, plans);
         if (rc) return rc;
     }
@@ -691,7 +698,7 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
                     return fail(set_err(COVA_E_CUDA, "event creation failed"));
         }
     }
-    const int N = (int)(p->chunk_streams * windows_per_stream(max_fps, timestep, gamma));   // windows per chunk
+    const int N = (int)(p->chunk_streams * chain_windows);                                  // windows per chunk
     const int NB = (int)p->max_windows;                                                       // windows per batch
     const int F = (int)(p->chunk_streams * max_fps);
     blobnet_geoms((int)h_mb, (int)w_mb, N, F, p->sizes_h, p->sizes_w, p->gx, p->gd, p->gx0f);
@@ -710,29 +717,22 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
     if ((rc = alloc_zero(&p->x0f, p->gx0f))) return fail(rc);
     p->packed = (flags & COVA_FLAG_INPUT_PACKED16) != 0;
     p->frame_bytes = (size_t)w_mb * h_mb * (p->packed ? 2 : 4);
-    cudaError_t e = cudaMalloc(&p->slot[0].d_frames, p->frame_bytes * max_streams * max_fps);
-    p->d_frames = p->slot[0].d_frames;
+    cudaError_t e = cudaMalloc(&p->d_mask, (size_t)std::max(1, NB) * w_mb * h_mb);
     for (auto &sl : p->slot) {
         if (e == cudaSuccess) e = cudaMallocHost(&sl.h_tab, sizeof(int2) * max_streams);
         if (e == cudaSuccess) e = cudaMalloc(&sl.d_tab, sizeof(int2) * max_streams);
         if (e == cudaSuccess) e = cudaMallocHost(&sl.h_newest, sizeof(int) * std::max(1, NB));
         if (e == cudaSuccess) e = cudaMalloc(&sl.d_newest, sizeof(int) * std::max(1, NB));
+        if (e == cudaSuccess) e = cudaMallocHost(&sl.h_cursor, sizeof(unsigned long long) * 2 * 256);
     }
-    if (e == cudaSuccess) e = cudaMalloc(&p->d_mask, (size_t)std::max(1, NB) * w_mb * h_mb);
     if (e == cudaSuccess) e = cudaMemset(p->d_mask, 0, (size_t)std::max(1, NB) * w_mb * h_mb);
     if (e == cudaSuccess && (flags & COVA_FLAG_KEEP_LOGITS)) e = cudaMalloc(&p->d_logits, sizeof(float) * (size_t)NB * w_mb * h_mb);
     if (e == cudaSuccess && (flags & COVA_FLAG_KEEP_STACKED)) e = cudaMalloc(&p->d_stacked, p->frame_bytes * timestep * (size_t)NB);
     if (e == cudaSuccess) e = cudaMalloc(&p->d_watchdog, sizeof(unsigned int));
     if (e == cudaSuccess) e = cudaMemset(p->d_watchdog, 0, sizeof(unsigned int));
-    if (e == cudaSuccess) e = cudaMallocHost(&p->h_pinned, sizeof(unsigned long long) * (2 + 2 * (size_t)std::max(1, NB) + 2 * 64));
     if (e != cudaSuccess) return fail(set_err(COVA_E_CUDA, "pipeline allocation: %s", cudaGetErrorString(e)));
-    p->slot[0].ccl.d_masks = p->d_mask;
-    if ((rc = ccl_alloc(p->slot[0].ccl, (int)h_mb, (int)w_mb, std::max(1, NB), false, flags))) return fail(rc);
-    p->slot[0].ready = true;
-    p->ccl = p->slot[0].ccl;
-    for (auto &sl : p->slot)
-        if (cudaMallocHost(&sl.h_cursor, sizeof(unsigned long long) * 2 * 256) != cudaSuccess)
-            return fail(set_err(COVA_E_CUDA, "pinned allocation failed"));
+    // slot 0 now, the others on their first submit; a CCL grid that does not fit is refused here
+    if ((rc = ensure_slot(p, 0))) return fail(rc);
 
     // weights: raw fp32 for the validation kernels, packed fp16 operand blocks for the tcgen05 path
     if ((rc = dev_upload(&p->d_wraw, p->hw.storage.data(), p->hw.storage.size() * sizeof(float)))) return fail(rc);
@@ -795,7 +795,6 @@ extern "C" void cova_pipeline_free(cova_pipeline *p) {
     if (p->d_stacked) cudaFree(p->d_stacked);
     if (p->d_wraw) cudaFree(p->d_wraw);
     if (p->d_watchdog) cudaFree(p->d_watchdog);
-    if (p->h_pinned) cudaFreeHost(p->h_pinned);
     for (auto e : p->events) cudaEventDestroy(e);
     if (p->s_in) cudaStreamDestroy(p->s_in);
     if (p->s_out) cudaStreamDestroy(p->s_out);
@@ -816,17 +815,22 @@ extern "C" int cova_pipeline_set_stream(cova_pipeline *p, void *s) {
 }
 extern "C" int cova_pipeline_n_windows(const cova_pipeline *p, uint32_t n_streams, uint32_t fps, uint32_t *n) {
     if (!p || !n) return set_err(COVA_E_INVAL, "null argument");
-    *n = n_streams * windows_per_stream(fps, p->T, p->gamma);
+    *n = n_streams * windows_from(fps, p->T - 1, p->gamma);
     return COVA_OK;
 }
 
-// Window shape of a batch of n_streams device chains of fps frames each, into the tables of slot k.  first[s] is the index
+// checked before the first device call of a submit or load_frames
+static int check_batch_bounds(const cova_pipeline *p, uint32_t n_streams, uint32_t fps) {
+    if (!n_streams || n_streams > p->max_streams || fps > p->max_fps)
+        return set_err(COVA_E_INVAL, "batch exceeds max_streams / max_frames_per_stream of the pipeline");
+    return COVA_OK;
+}
+
+// Window shape of a batch of n_streams device chains of fps frames each, into slot k.  first[s] is the index
 // (inside device chain s) of the newest frame of the chain's first window; nullptr = T - 1 for every chain, i.e. chains
 // that start with an empty window.  CONTINUED chains (submit_host2) start later, where their carried history and gamma
 // phase put them.  Lock-step and staggered batches go through the same tables and kernels.
 static int set_batch_shape(cova_pipeline *p, int k, uint32_t n_streams, uint32_t fps, const uint32_t *first = nullptr) {
-    if (!n_streams || n_streams > p->max_streams || fps > p->max_fps)
-        return set_err(COVA_E_INVAL, "batch exceeds max_streams / max_frames_per_stream of the pipeline");
     auto &sl = p->slot[k];
     const uint32_t t1 = p->T - 1, cs = p->chunk_streams;
     uint64_t total = 0;
@@ -835,7 +839,7 @@ static int set_batch_shape(cova_pipeline *p, int k, uint32_t n_streams, uint32_t
     sl.win0.resize(n_streams + 1);
     sl.win0[0] = 0;
     for (uint32_t s = 0; s < n_streams; s++) sl.win0[s + 1] = sl.win0[s] + windows_from(fps, first ? first[s] : t1, p->gamma);
-    p->cur_streams = n_streams; p->cur_fps = fps; p->cur_windows = (uint32_t)total;
+    sl.n_streams = n_streams; sl.fps = fps; sl.n_windows = (uint32_t)total;
     bool same = sl.tab_fps == fps && sl.tab_stream == p->stream && sl.tab_first.size() == n_streams;
     for (uint32_t s = 0; same && s < n_streams; s++) same = sl.tab_first[s] == (first ? first[s] : t1);
     if (same) return COVA_OK;                                      // the slot's device tables already hold this shape
@@ -858,30 +862,40 @@ static int set_batch_shape(cova_pipeline *p, int k, uint32_t n_streams, uint32_t
     return COVA_OK;
 }
 
-static void use_slot(cova_pipeline *p, int k);
-static uint32_t n_chunks_of(const cova_pipeline *p) { return (p->cur_streams + p->chunk_streams - 1) / p->chunk_streams; }
-static void select_chunk(cova_pipeline *p, uint32_t c) {
-    const std::vector<uint32_t> &win0 = p->slot[p->cur_slot].win0;
-    p->ck_stream0 = c * p->chunk_streams;
-    p->ck_n_streams = std::min(p->chunk_streams, p->cur_streams - p->ck_stream0);
-    if (!p->ck_n_streams) { p->ck_window0 = p->ck_windows = 0; return; }      // masks loaded directly: no chains
-    p->ck_window0 = win0[p->ck_stream0];
-    p->ck_windows = win0[p->ck_stream0 + p->ck_n_streams] - p->ck_window0;
+static Chunk chunk_of(const Slot &sl, uint32_t c, uint32_t chunk_streams) {
+    const uint32_t s0 = c * chunk_streams, ns = std::min(chunk_streams, sl.n_streams - s0);
+    if (!ns) return Chunk{s0, 0, 0, 0};                            // masks loaded directly: no chains
+    return Chunk{s0, ns, sl.win0[s0], sl.win0[s0 + ns] - sl.win0[s0]};
 }
-static int require_single_chunk(cova_pipeline *p) {
-    if (p->cur_streams > p->chunk_streams)
+// The stage-wise calls share the device buffers and slot 0 with the submitted batches: refused while one is in flight.
+static int require_idle(const cova_pipeline *p) {
+    for (auto &sl : p->slot)
+        if (sl.busy) return set_err(COVA_E_INVAL, "batches submitted asynchronously are still in flight");
+    return COVA_OK;
+}
+// What tensorise / blobnet / run_layer work on: the one chunk of the last batch, or ck.windows = 0 if it has no windows.
+static int stage_chunk(cova_pipeline *p, Chunk &ck) {
+    if (!p) return set_err(COVA_E_INVAL, "null handle");
+    if (int rc = require_idle(p)) return rc;
+    const Slot &sl = p->slot[p->last_slot];
+    ck = Chunk{};
+    if (!sl.n_windows) return COVA_OK;
+    COVA_CUDA(cudaSetDevice(p->device));
+    if (sl.n_streams > p->chunk_streams)
         return set_err(COVA_E_UNSUPPORTED, "stage-wise calls need a batch that fits one chunk; use cova_pipeline_run / process_host");
-    select_chunk(p, 0);
+    ck = p->last_chunk = chunk_of(sl, 0, p->chunk_streams);
     return COVA_OK;
 }
 
 extern "C" int cova_pipeline_load_frames(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, uint32_t fps, int is_device) {
     if (!p || !frames) return set_err(COVA_E_INVAL, "null argument");
-    COVA_CUDA(cudaSetDevice(p->device));
-    int rc = set_batch_shape(p, 0, n_streams, fps);
+    int rc = require_idle(p);
+    if (!rc) rc = check_batch_bounds(p, n_streams, fps);
     if (rc) return rc;
-    use_slot(p, 0);
-    COVA_CUDA(cudaMemcpyAsync(p->d_frames, frames, p->frame_bytes * n_streams * fps,
+    COVA_CUDA(cudaSetDevice(p->device));
+    if ((rc = set_batch_shape(p, 0, n_streams, fps))) return rc;
+    p->last_slot = 0;
+    COVA_CUDA(cudaMemcpyAsync(p->slot[0].d_frames, frames, p->frame_bytes * n_streams * fps,
                               is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, p->stream));
     return COVA_OK;
 }
@@ -889,21 +903,22 @@ extern "C" int cova_pipeline_load_frames(cova_pipeline *p, const uint8_t *frames
 extern "C" int cova_pipeline_load_masks(cova_pipeline *p, const uint8_t *masks, uint32_t n, int is_device) {
     if (!p || !masks) return set_err(COVA_E_INVAL, "null argument");
     if (!n || n > p->max_windows) return set_err(COVA_E_INVAL, "mask batch exceeds the pipeline's window capacity");
+    if (int rc = require_idle(p)) return rc;
     COVA_CUDA(cudaSetDevice(p->device));
-    p->cur_windows = n; p->cur_streams = 0;
-    use_slot(p, 0);
+    p->slot[0].n_streams = 0; p->slot[0].n_windows = n;
+    p->last_slot = 0;
     COVA_CUDA(cudaMemcpyAsync(p->d_mask, masks, (size_t)n * p->W * p->H, is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, p->stream));
     return COVA_OK;
 }
 
-static int tensorise_chunk(cova_pipeline *p) {
-    const int N = (int)p->ck_windows;
+static int tensorise_chunk(cova_pipeline *p, const Slot &sl, const Chunk &ck) {
+    const int N = (int)ck.windows;
     if (!N) return COVA_OK;
-    const uint8_t *frames = p->d_frames + (size_t)p->ck_stream0 * p->cur_fps * p->frame_bytes;
-    const int *newest = p->slot[p->cur_slot].d_newest + p->ck_window0;      // chunk-relative, like the frames
+    const uint8_t *frames = sl.d_frames + (size_t)ck.stream0 * sl.fps * p->frame_bytes;
+    const int *newest = sl.d_newest + ck.window0;                   // chunk-relative, like the frames
     if (p->d_stacked) {
         const size_t S = p->frame_bytes;
-        uint8_t *dst = p->d_stacked + (size_t)p->ck_window0 * p->T * S;
+        uint8_t *dst = p->d_stacked + (size_t)ck.window0 * p->T * S;
         if (S % 16 == 0) {
             long long total = (long long)N * p->T * (S / 16);
             int blocks = (int)std::min<long long>((total + 255) / 256, (long long)p->n_sms * 16);
@@ -920,7 +935,7 @@ static int tensorise_chunk(cova_pipeline *p) {
         prof_mark(p, "stack_rgba");
     }
     {   // per-frame first-conv input (tcgen05 path)
-        const int F = (int)(p->ck_n_streams * p->cur_fps);
+        const int F = (int)(ck.n_streams * sl.fps);
         long long total = (long long)F * p->H * p->gx0f.Wh;
         int blocks = (int)std::min<long long>((total + 255) / 256, (long long)p->n_sms * 32);
         if (total >= (1ll << 32)) return set_err(COVA_E_UNSUPPORTED, "chunk too large for the frame tensorisation kernel (32-bit index)");
@@ -944,11 +959,9 @@ static int tensorise_chunk(cova_pipeline *p) {
 }
 
 extern "C" int cova_pipeline_tensorise(cova_pipeline *p) {
-    if (!p) return set_err(COVA_E_INVAL, "null handle");
-    if (!p->cur_windows) return COVA_OK;
-    COVA_CUDA(cudaSetDevice(p->device));
-    int rc = require_single_chunk(p);
-    return rc ? rc : tensorise_chunk(p);
+    Chunk ck;
+    int rc = stage_chunk(p, ck);
+    return rc ? rc : tensorise_chunk(p, p->slot[p->last_slot], ck);
 }
 
 // ---- layer launchers -------------------------------------------------------------------------------
@@ -958,12 +971,12 @@ static void crop_for(int in_extent, int target, int &crop_lo) {
 }
 
 #ifndef COVA_VALIDATION
-static int simt_layer(cova_pipeline *, int) {
+static int simt_layer(cova_pipeline *, const Chunk &, int) {
     return set_err(COVA_E_UNSUPPORTED, "the validation kernels (COVA_IMPL_SIMT) are not part of this build; use libcova_b200_val.so");
 }
 #else
-static int simt_layer(cova_pipeline *p, int layer) {
-    const int N = (int)p->ck_windows;
+static int simt_layer(cova_pipeline *p, const Chunk &ck, int layer) {
+    const int N = (int)ck.windows;
     const float *w = p->d_wraw;
     if (layer == 0 && !p->x[0]) return set_err(COVA_E_UNSUPPORTED, "validation kernel of layer 0 needs a pipeline created with COVA_IMPL_SIMT");
     if (layer < 4) {
@@ -995,8 +1008,8 @@ static int simt_layer(cova_pipeline *p, int layer) {
     a.w = w + p->hw.off_dec[i][0]; a.b = w + p->hw.off_dec[i][1];
     a.gamma = w + p->hw.off_dec[i][2]; a.beta = w + p->hw.off_dec[i][3]; a.mean = w + p->hw.off_dec[i][4]; a.var = w + p->hw.off_dec[i][5];
     a.head_w = w + p->hw.off_head[0]; a.head_b = w + p->hw.off_head[1];
-    a.mask = p->d_mask + (size_t)p->ck_window0 * p->W * p->H;
-    a.logits = p->d_logits ? p->d_logits + (size_t)p->ck_window0 * p->W * p->H : nullptr;
+    a.mask = p->d_mask + (size_t)ck.window0 * p->W * p->H;
+    a.logits = p->d_logits ? p->d_logits + (size_t)ck.window0 * p->W * p->H : nullptr;
     a.Cin = kDecCin[i]; a.Cout = kDecCout[i]; a.N = N;
     a.Ht = p->sizes_h[3 - i]; a.Wt = p->sizes_w[3 - i];
     crop_for(a.gin.H, a.Ht, a.crop_t);
@@ -1193,13 +1206,13 @@ extern "C" int cova_blobnet_plan(uint32_t w_mb, uint32_t h_mb, uint32_t windows,
     return plan_blobnet((int)h_mb, (int)w_mb, (int)windows, 1, (int)windows + kT - 1, 1, debug, n_sms, out);
 }
 
-static int tc_plan(cova_pipeline *p, int layer, LayerPlan &pl) {
-    plan_input(pl, layer, p->gx, p->gd, p->gx0f, (int)p->ck_windows, (int)p->ck_n_streams, (int)p->cur_fps, (int)p->gamma);
+static int tc_plan(cova_pipeline *p, const Slot &sl, const Chunk &ck, int layer, LayerPlan &pl) {
+    plan_input(pl, layer, p->gx, p->gd, p->gx0f, (int)ck.windows, (int)ck.n_streams, (int)sl.fps, (int)p->gamma);
     return plan_layer(layer, p->dbg, p->n_sms, pl);
 }
 
 // launch a planned layer: everything but the plan's geometry and tiling fields is filled here
-static int tc_launch(cova_pipeline *p, int layer, LayerPlan &pl) {
+static int tc_launch(cova_pipeline *p, const Slot &sl, const Chunk &ck, int layer, LayerPlan &pl) {
     tc::LayerParams &lp = pl.lp;
     lp.watchdog = p->d_watchdog; lp.dbg = p->dbg;
     if (layer < 4) {
@@ -1217,7 +1230,7 @@ static int tc_launch(cova_pipeline *p, int layer, LayerPlan &pl) {
             if (!(p->hw.enc[i].gamma[c] >= 0.f)) lp.bn_nonneg = 0;
         if (i == 0) {
             lp.in = p->x0f;
-            pl.ex.tab = p->slot[p->cur_slot].d_tab + p->ck_stream0;
+            pl.ex.tab = sl.d_tab + ck.stream0;
         }
     } else {
         const int i = layer - 4;
@@ -1228,8 +1241,8 @@ static int tc_launch(cova_pipeline *p, int layer, LayerPlan &pl) {
         lp.Ht = p->sizes_h[3 - i]; lp.Wt = p->sizes_w[3 - i];
         crop_for(lp.gin.H, lp.Ht, lp.crop_t);
         crop_for(lp.gin.W, lp.Wt, lp.crop_l);
-        lp.mask = p->d_mask + (size_t)p->ck_window0 * p->W * p->H;
-        lp.logits = p->d_logits ? p->d_logits + (size_t)p->ck_window0 * p->W * p->H : nullptr;
+        lp.mask = p->d_mask + (size_t)ck.window0 * p->W * p->H;
+        lp.logits = p->d_logits ? p->d_logits + (size_t)ck.window0 * p->W * p->H : nullptr;
     }
     cudaError_t err = launch_layer(layer, pl, p->stream);
     if (err != cudaSuccess) return set_err(COVA_E_CUDA, "%s launch: %s", kLayerName[layer], cudaGetErrorString(err));
@@ -1240,27 +1253,23 @@ static int tc_launch(cova_pipeline *p, int layer, LayerPlan &pl) {
     return COVA_OK;
 }
 
-static int tc_layer(cova_pipeline *p, int layer) {
-    LayerPlan pl;
-    int rc = tc_plan(p, layer, pl);
-    return rc ? rc : tc_launch(p, layer, pl);
-}
-
 extern "C" int cova_pipeline_run_layer(cova_pipeline *p, int layer, uint32_t impl) {
     if (!p) return set_err(COVA_E_INVAL, "null handle");
     if (layer < 0 || layer > 7 || impl > COVA_IMPL_SIMT) return set_err(COVA_E_INVAL, "layer must be 0..7, impl 0 or 1");
-    if (!p->cur_windows) return COVA_OK;
-    COVA_CUDA(cudaSetDevice(p->device));
-    int rc = require_single_chunk(p);
-    if (rc) return rc;
-    return impl == COVA_IMPL_SIMT ? simt_layer(p, layer) : tc_layer(p, layer);
+    Chunk ck;
+    int rc = stage_chunk(p, ck);
+    if (rc || !ck.windows) return rc;
+    if (impl == COVA_IMPL_SIMT) return simt_layer(p, ck, layer);
+    LayerPlan pl;
+    if ((rc = tc_plan(p, p->slot[p->last_slot], ck, layer, pl))) return rc;
+    return tc_launch(p, p->slot[p->last_slot], ck, layer, pl);
 }
 
-static int blobnet_chunk(cova_pipeline *p) {
-    if (!p->ck_windows) return COVA_OK;
+static int blobnet_chunk(cova_pipeline *p, const Slot &sl, const Chunk &ck) {
+    if (!ck.windows) return COVA_OK;
     if (p->impl == COVA_IMPL_SIMT) {
         for (int layer = 0; layer < 8; layer++) {
-            int rc = simt_layer(p, layer);
+            int rc = simt_layer(p, ck, layer);
             if (rc) return rc;
         }
         return COVA_OK;
@@ -1269,42 +1278,40 @@ static int blobnet_chunk(cova_pipeline *p) {
     // refused on the host, with nothing of the chunk's network enqueued
     LayerPlan plans[8];
     for (int layer = 0; layer < 8; layer++) {
-        int rc = tc_plan(p, layer, plans[layer]);
+        int rc = tc_plan(p, sl, ck, layer, plans[layer]);
         if (rc) return rc;
     }
     for (int layer = 0; layer < 8; layer++) {
-        int rc = tc_launch(p, layer, plans[layer]);
+        int rc = tc_launch(p, sl, ck, layer, plans[layer]);
         if (rc) return rc;
     }
     return COVA_OK;
 }
 
 extern "C" int cova_pipeline_blobnet(cova_pipeline *p) {
-    if (!p) return set_err(COVA_E_INVAL, "null handle");
-    if (!p->cur_windows) return COVA_OK;
-    COVA_CUDA(cudaSetDevice(p->device));
-    int rc = require_single_chunk(p);
-    return rc ? rc : blobnet_chunk(p);
+    Chunk ck;
+    int rc = stage_chunk(p, ck);
+    return rc ? rc : blobnet_chunk(p, p->slot[p->last_slot], ck);
 }
 
-static int ccl_range(cova_pipeline *p, size_t first, int n, bool reset_cursor) {
-    int rc = ccl_launch(p->ccl, p->d_mask, n, p->cc_threshold, false, p->stream, first, reset_cursor, !(p->dbg & kDbgNoPdl));
+static int ccl_range(cova_pipeline *p, Slot &sl, size_t first, int n, bool reset_cursor) {
+    int rc = ccl_launch(sl.ccl, p->d_mask, n, p->cc_threshold, false, p->stream, first, reset_cursor, !(p->dbg & kDbgNoPdl));
     if (rc) return rc;
     if (n > 0) {
         p->launches++;
-        prof_mark(p, p->ccl.k > 1 ? "ccl_bbox_cluster" : "ccl_bbox");
+        prof_mark(p, sl.ccl.k > 1 ? "ccl_bbox_cluster" : "ccl_bbox");
     }
     return COVA_OK;
 }
 
 extern "C" int cova_pipeline_ccl(cova_pipeline *p) {
     if (!p) return set_err(COVA_E_INVAL, "null handle");
+    if (int rc = require_idle(p)) return rc;
     COVA_CUDA(cudaSetDevice(p->device));
-    if (!p->cur_windows) {
-        COVA_CUDA(cudaMemsetAsync(p->ccl.d_cursor, 0, 2 * sizeof(unsigned long long), p->stream));
-        return COVA_OK;
-    }
-    return ccl_range(p, 0, (int)p->cur_windows, true);
+    Slot &sl = p->slot[p->last_slot];
+    // ccl_range resets the box arena's cursor only when it launches
+    if (!sl.n_windows) COVA_CUDA(cudaMemsetAsync(sl.ccl.d_cursor, 0, 2 * sizeof(unsigned long long), p->stream));
+    return ccl_range(p, sl, 0, (int)sl.n_windows, true);
 }
 
 static void prof_begin(cova_pipeline *p) {
@@ -1315,31 +1322,26 @@ static void prof_begin(cova_pipeline *p) {
 }
 
 // all kernels of one chunk, on p->stream
-static int run_chunk(cova_pipeline *p, uint32_t c) {
-    select_chunk(p, c);
+static int run_chunk(cova_pipeline *p, Slot &sl, const Chunk &ck) {
+    p->last_chunk = ck;
     // the box arena's cursor is reset ahead of the batch's first kernel, not between the last layer and the CCL
     // kernel: a memset node there would break the chain of programmatic dependent launches (common.cuh)
-    if (c == 0) COVA_CUDA(cudaMemsetAsync(p->ccl.d_cursor, 0, 2 * sizeof(unsigned long long), p->stream));
-    int rc = tensorise_chunk(p);
-    if (!rc) rc = blobnet_chunk(p);
-    if (!rc) rc = ccl_range(p, p->ck_window0, (int)p->ck_windows, false);
+    if (ck.stream0 == 0) COVA_CUDA(cudaMemsetAsync(sl.ccl.d_cursor, 0, 2 * sizeof(unsigned long long), p->stream));
+    int rc = tensorise_chunk(p, sl, ck);
+    if (!rc) rc = blobnet_chunk(p, sl, ck);
+    if (!rc) rc = ccl_range(p, sl, ck.window0, (int)ck.windows, false);
     return rc;
 }
 
 extern "C" int cova_pipeline_run(cova_pipeline *p) {
     if (!p) return set_err(COVA_E_INVAL, "null handle");
+    if (int rc = require_idle(p)) return rc;
     COVA_CUDA(cudaSetDevice(p->device));
     prof_begin(p);
-    if (!p->cur_streams) return cova_pipeline_ccl(p);      // masks were loaded directly
-    if (!p->cur_windows) {
-        COVA_CUDA(cudaMemsetAsync(p->ccl.d_cursor, 0, 2 * sizeof(unsigned long long), p->stream));
-        return COVA_OK;
-    }
-    const uint32_t nc = n_chunks_of(p);
-    for (uint32_t c = 0; c < nc; c++) {
-        int rc = run_chunk(p, c);
-        if (rc) return rc;
-    }
+    Slot &sl = p->slot[p->last_slot];
+    if (!sl.n_streams || !sl.n_windows) return cova_pipeline_ccl(p);   // masks loaded directly, or no window at all
+    for (uint32_t c = 0; c * p->chunk_streams < sl.n_streams; c++)
+        if (int rc = run_chunk(p, sl, chunk_of(sl, c, p->chunk_streams))) return rc;
     return COVA_OK;
 }
 
@@ -1382,42 +1384,20 @@ extern "C" int cova_pipeline_sync(cova_pipeline *p) {
 extern "C" int cova_pipeline_fetch_boxes(cova_pipeline *p, uint8_t *blob, size_t blob_cap, size_t *blob_len, uint64_t *offsets, uint64_t *lens) {
     if (!p || !blob_len) return set_err(COVA_E_INVAL, "null argument");
     COVA_CUDA(cudaSetDevice(p->device));
-    const size_t n = p->cur_windows;
-    unsigned long long *hp = p->h_pinned;
-    COVA_CUDA(cudaMemcpyAsync(hp, p->ccl.d_cursor, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
-    if (n) {
-        COVA_CUDA(cudaMemcpyAsync(hp + 2, p->ccl.d_offsets, n * sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
-        COVA_CUDA(cudaMemcpyAsync(hp + 2 + n, p->ccl.d_lens, n * sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
-    }
+    Slot &sl = p->slot[p->last_slot];
+    const size_t n = sl.n_windows;
+    COVA_CUDA(cudaMemcpyAsync(sl.h_cursor, sl.ccl.d_cursor, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
     int rc = cova_pipeline_sync(p);
     if (rc) return rc;
-    if (hp[1]) return set_err(COVA_E_CUDA, "device box arena overflow (internal sizing error)");
-    *blob_len = (size_t)hp[0];
-    if (offsets) memcpy(offsets, hp + 2, n * sizeof(uint64_t));
-    if (lens) memcpy(lens, hp + 2 + n, n * sizeof(uint64_t));
-    if (!blob || blob_cap < hp[0]) return set_err(COVA_E_TOOSMALL, "box blob needs a larger buffer");
-    if (hp[0]) {
-        COVA_CUDA(cudaMemcpyAsync(blob, p->ccl.d_blob, (size_t)hp[0], cudaMemcpyDeviceToHost, p->stream));
-        COVA_CUDA(cudaStreamSynchronize(p->stream));
-    }
-    return COVA_OK;
-}
-
-static void use_slot(cova_pipeline *p, int k) {
-    p->cur_slot = k;
-    p->d_frames = p->slot[k].d_frames;
-    p->ccl = p->slot[k].ccl;
-}
-static int ensure_slot(cova_pipeline *p, int k) {
-    auto &sl = p->slot[k];
-    if (sl.ready) return COVA_OK;
-    if (!sl.d_frames) COVA_CUDA(cudaMalloc(&sl.d_frames, p->frame_bytes * p->max_streams * p->max_fps));
-    if (!sl.ccl.d_blob) {
-        sl.ccl.d_masks = p->d_mask;
-        int rc = ccl_alloc(sl.ccl, (int)p->H, (int)p->W, std::max<int>(1, (int)p->max_windows), false, p->flags);
-        if (rc) { ccl_free(sl.ccl, false); sl.ccl = CclBuffers(); return rc; }    // a later submit retries from scratch
-    }
-    sl.ready = true;
+    if (sl.h_cursor[1]) return set_err(COVA_E_CUDA, "device box arena overflow (internal sizing error)");
+    const unsigned long long end = sl.h_cursor[0];
+    *blob_len = (size_t)end;
+    if (offsets && n) COVA_CUDA(cudaMemcpyAsync(offsets, sl.ccl.d_offsets, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, p->stream));
+    if (lens && n) COVA_CUDA(cudaMemcpyAsync(lens, sl.ccl.d_lens, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, p->stream));
+    const bool fits = blob && blob_cap >= end;
+    if (fits && end) COVA_CUDA(cudaMemcpyAsync(blob, sl.ccl.d_blob, (size_t)end, cudaMemcpyDeviceToHost, p->stream));
+    COVA_CUDA(cudaStreamSynchronize(p->stream));
+    if (!fits) return set_err(COVA_E_TOOSMALL, "box blob needs a larger buffer");
     return COVA_OK;
 }
 
@@ -1458,18 +1438,19 @@ __global__ void __launch_bounds__(256) carry_kernel(uint32_t *__restrict__ pool,
 // the copy stage of a chunk: the host validates every record first and keeps their offsets; chunk c's records are one
 // contiguous byte range, copied as such, and sparse_expand_kernel writes them into the frame pool where the dense copy
 // would have put them.  Everything after that is shared.
-static int submit_impl(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, uint32_t fps, const uint32_t *stream_ids,
-                       const uint64_t *pts, uint32_t flags, bool stateful, const size_t *sparse_len = nullptr) {
-    if (!p || !frames) return set_err(COVA_E_INVAL, "null argument");
+
+// Argument checks and per-chain plan of a submit, before any device call: fills first_scratch, hist_scratch and
+// off_scratch, and raises lead (0 on entry) to the longest carried history
+static int plan_submit(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, uint32_t fps, const uint32_t *stream_ids,
+                       uint32_t flags, bool stateful, const size_t *sparse_len, uint32_t &lead) {
     if (flags & ~(COVA_SUBMIT_CONTINUE | COVA_SUBMIT_STAGGERED)) return set_err(COVA_E_INVAL, "unknown submit flag");
     if ((flags & COVA_SUBMIT_STAGGERED) && !(flags & COVA_SUBMIT_CONTINUE))
         return set_err(COVA_E_INVAL, "COVA_SUBMIT_STAGGERED needs COVA_SUBMIT_CONTINUE");
-    const bool sparse = sparse_len != nullptr;
-    const uint64_t n_frames = (uint64_t)n_streams * fps;
-    if (sparse) {           // the whole batch is checked before any device call
-        if (!p->packed) return set_err(COVA_E_INVAL, "sparse input needs a COVA_FLAG_INPUT_PACKED16 pipeline");
-        if (!n_streams || n_streams > p->max_streams || fps > p->max_fps)
-            return set_err(COVA_E_INVAL, "batch exceeds max_streams / max_frames_per_stream of the pipeline");
+    if (sparse_len && !p->packed) return set_err(COVA_E_INVAL, "sparse input needs a COVA_FLAG_INPUT_PACKED16 pipeline");
+    int rc = check_batch_bounds(p, n_streams, fps);
+    if (rc) return rc;
+    if (sparse_len) {
+        const uint64_t n_frames = (uint64_t)n_streams * fps;
         p->off_scratch.resize(n_frames + 1);
         uint64_t bad = 0;
         if (const char *why = sparse::validate_batch(frames, *sparse_len, n_frames, p->W * p->H, p->off_scratch.data(), &bad)) {
@@ -1478,15 +1459,7 @@ static int submit_impl(cova_pipeline *p, const uint8_t *frames, uint32_t n_strea
             return set_err(COVA_E_INVAL, "malformed sparse batch at frame %s: %s", frame, why);
         }
     }
-    COVA_CUDA(cudaSetDevice(p->device));
-    const int k = p->next_submit;
-    if (p->slot[k].busy) return set_err(COVA_E_INVAL, "four batches are already in flight: collect one first");
-    int rc = ensure_slot(p, k);
-    if (rc) return rc;
-    if (!n_streams || n_streams > p->max_streams) return set_err(COVA_E_INVAL, "batch exceeds max_streams of the pipeline");
-    auto &sl = p->slot[k];
     const uint32_t t1 = p->T - 1;
-    uint32_t lead = 0;                                              // carried frames in front of every device chain
     std::vector<uint32_t> &first = p->first_scratch, &hist = p->hist_scratch;
     first.assign(n_streams, t1);
     hist.assign(n_streams, 0);
@@ -1499,23 +1472,34 @@ static int submit_impl(cova_pipeline *p, const uint8_t *frames, uint32_t n_strea
             if (id >= p->max_streams) return set_err(COVA_E_INVAL, "stream id out of range (ids are 0 .. max_streams-1)");
             if (p->id_mark[id] == p->id_epoch) return set_err(COVA_E_INVAL, "a stream id appears twice in one batch");
             p->id_mark[id] = p->id_epoch;
+            if (!(flags & COVA_SUBMIT_CONTINUE)) continue;
+            const uint64_t seen = p->n_seen[id];
+            const uint32_t hs = (uint32_t)std::min<uint64_t>(seen, t1);
+            const uint64_t base = seen - hs;                        // frames of the stream in front of its carried ones
+            // smallest index i' >= T-1 of the unpadded chain with (base + i' - (T-1)) % gamma == 0 (imp.rs:321-330)
+            hist[s] = hs;
+            first[s] = t1 + (uint32_t)((p->gamma - base % p->gamma) % p->gamma);
+            lead = std::max(lead, hs);
+            // without COVA_SUBMIT_STAGGERED the streams of a batch advance in lock-step: same history, same gamma phase
+            if (!(flags & COVA_SUBMIT_STAGGERED) && s && (hs != hist[0] || first[s] != first[0]))
+                return set_err(COVA_E_INVAL, "streams of one CONTINUED batch must have the same history length and gamma phase "
+                                             "(or pass COVA_SUBMIT_STAGGERED)");
         }
-        if (flags & COVA_SUBMIT_CONTINUE) {
-            for (uint32_t s = 0; s < n_streams; s++) {
-                const uint64_t seen = p->n_seen[stream_ids ? stream_ids[s] : s];
-                const uint32_t hs = (uint32_t)std::min<uint64_t>(seen, t1);
-                const uint64_t base = seen - hs;                    // frames of the stream in front of its carried ones
-                // smallest index i' >= T-1 of the unpadded chain with (base + i' - (T-1)) % gamma == 0 (imp.rs:321-330)
-                hist[s] = hs;
-                first[s] = t1 + (uint32_t)((p->gamma - base % p->gamma) % p->gamma);
-                lead = std::max(lead, hs);
-                // without COVA_SUBMIT_STAGGERED the streams of a batch advance in lock-step: same history, same gamma phase
-                if (!(flags & COVA_SUBMIT_STAGGERED) && s && (hs != hist[0] || first[s] != first[0]))
-                    return set_err(COVA_E_INVAL, "streams of one CONTINUED batch must have the same history length and gamma phase "
-                                                 "(or pass COVA_SUBMIT_STAGGERED)");
-            }
-            for (uint32_t s = 0; s < n_streams; s++) first[s] += lead - hist[s];   // chain s is padded by lead - h_s frames
-        }
+        for (uint32_t s = 0; s < n_streams; s++) first[s] += lead - hist[s];   // chain s is padded by lead - h_s frames
+    }
+    if (fps + lead > p->max_fps)
+        return set_err(COVA_E_INVAL, "carried frames + new frames exceed max_frames_per_stream of the pipeline");
+    return COVA_OK;
+}
+
+// slot k takes the planned batch: buffers on first use, window shape, per-window stream ids and PTS, frames seen per stream
+static int setup_slot(cova_pipeline *p, int k, uint32_t n_streams, uint32_t fps, uint32_t lead, const uint32_t *stream_ids,
+                      const uint64_t *pts, uint32_t flags, bool stateful, bool sparse) {
+    int rc = ensure_slot(p, k);
+    if (rc) return rc;
+    auto &sl = p->slot[k];
+    const uint32_t t1 = p->T - 1;
+    if (stateful) {
         if (!p->d_carry && t1) {
             COVA_CUDA(cudaMalloc(&p->d_carry, (size_t)p->max_streams * t1 * p->frame_bytes));
             COVA_CUDA(cudaMemsetAsync(p->d_carry, 0, (size_t)p->max_streams * t1 * p->frame_bytes, p->stream));
@@ -1532,12 +1516,9 @@ static int submit_impl(cova_pipeline *p, const uint8_t *frames, uint32_t n_strea
         if (!sl.d_off) COVA_CUDA(cudaMalloc(&sl.d_off, sizeof(unsigned long long) * (max_frames + 1)));
         COVA_CUDA(cudaEventCreateWithFlags(&sl.ev_off, cudaEventDisableTiming));
     }
-    const uint32_t fps_dev = fps + lead;                            // frames per chain on the device
-    if (fps_dev > p->max_fps)
-        return set_err(COVA_E_INVAL, "carried frames + new frames exceed max_frames_per_stream of the pipeline");
-    if ((rc = set_batch_shape(p, k, n_streams, fps_dev, first.data()))) return rc;
-    use_slot(p, k);
-    sl.n_streams = n_streams; sl.fps = fps_dev; sl.n_windows = p->cur_windows;
+    const std::vector<uint32_t> &first = p->first_scratch;
+    if ((rc = set_batch_shape(p, k, n_streams, fps + lead, first.data()))) return rc;
+    p->last_slot = k;
     sl.win_pts.clear(); sl.win_ids.clear();
     if (stateful) {
         // window w of chain s has its newest frame at device index first_s + w*gamma = new-frame index first_s + w*gamma - lead
@@ -1553,68 +1534,91 @@ static int submit_impl(cova_pipeline *p, const uint8_t *frames, uint32_t n_strea
             p->n_seen[id] = ((flags & COVA_SUBMIT_CONTINUE) ? p->n_seen[id] : 0) + fps;
         }
     }
-    sl.busy = true; sl.failed = false;
-    p->next_submit = (k + 1) % kSlots;
-    if (!stateful && !p->cur_windows) return COVA_OK;              // chains shorter than a window: nothing to compute
-    // from here on a failure leaves the slot marked failed: the matching collect reports it instead of reading events that
-    // were never recorded
-    auto fail = [&](int code) { sl.failed = true; return code; };
-#define COVA_CUDA_SLOT(expr)                                                                                        \
-    do {                                                                                                            \
-        cudaError_t _e = (expr);                                                                                    \
-        if (_e != cudaSuccess) return fail(cova::set_err(COVA_E_CUDA, "%s: %s", #expr, cudaGetErrorString(_e)));    \
-    } while (0)
-    const uint32_t nc = n_chunks_of(p);
-    const size_t src_chain = p->frame_bytes * fps, dst_chain = p->frame_bytes * fps_dev, lead_bytes = p->frame_bytes * lead;
+    return COVA_OK;
+}
+
+// copy stage, on s_in: per chunk the new frames (dense, padded behind lead carried frames, or sparse records), then ev_in[c]
+static int copy_chunks(cova_pipeline *p, Slot &sl, const uint8_t *frames, uint32_t fps, uint32_t lead, bool sparse) {
     if (sparse) {
         // the slot's previous offsets upload has completed (its batch was collected); the event makes that explicit
-        COVA_CUDA_SLOT(cudaEventSynchronize(sl.ev_off));
-        memcpy(sl.h_off, p->off_scratch.data(), sizeof(unsigned long long) * (n_frames + 1));
-        COVA_CUDA_SLOT(cudaMemcpyAsync(sl.d_off, sl.h_off, sizeof(unsigned long long) * (n_frames + 1), cudaMemcpyHostToDevice, p->stream));
-        COVA_CUDA_SLOT(cudaEventRecord(sl.ev_off, p->stream));
+        const size_t n_offs = (size_t)sl.n_streams * fps + 1;
+        COVA_CUDA(cudaEventSynchronize(sl.ev_off));
+        memcpy(sl.h_off, p->off_scratch.data(), sizeof(unsigned long long) * n_offs);
+        COVA_CUDA(cudaMemcpyAsync(sl.d_off, sl.h_off, sizeof(unsigned long long) * n_offs, cudaMemcpyHostToDevice, p->stream));
+        COVA_CUDA(cudaEventRecord(sl.ev_off, p->stream));
     }
-    for (uint32_t c = 0; c < nc; c++) {
-        const size_t s0 = (size_t)c * p->chunk_streams, ns = std::min<size_t>(p->chunk_streams, n_streams - s0);
+    const size_t src_chain = p->frame_bytes * fps, dst_chain = p->frame_bytes * sl.fps, lead_bytes = p->frame_bytes * lead;
+    for (uint32_t c = 0; c * p->chunk_streams < sl.n_streams; c++) {
+        const Chunk ck = chunk_of(sl, c, p->chunk_streams);
+        const size_t s0 = ck.stream0, ns = ck.n_streams;
         if (sparse) {      // chunk c's records: one contiguous byte range, to the same offset of the staging
             const uint64_t b0 = p->off_scratch[s0 * fps], b1 = p->off_scratch[(s0 + ns) * fps];
-            COVA_CUDA_SLOT(cudaMemcpyAsync(sl.d_sparse + b0, frames + b0, b1 - b0, cudaMemcpyHostToDevice, p->s_in));
-        } else if (!lead) COVA_CUDA_SLOT(cudaMemcpyAsync(sl.d_frames + s0 * dst_chain, frames + s0 * src_chain, ns * src_chain, cudaMemcpyHostToDevice, p->s_in));
-        else COVA_CUDA_SLOT(cudaMemcpy2DAsync(sl.d_frames + s0 * dst_chain + lead_bytes, dst_chain, frames + s0 * src_chain, src_chain, src_chain, ns,
-                                              cudaMemcpyHostToDevice, p->s_in));
-        COVA_CUDA_SLOT(cudaEventRecord(sl.ev_in[c], p->s_in));
+            COVA_CUDA(cudaMemcpyAsync(sl.d_sparse + b0, frames + b0, b1 - b0, cudaMemcpyHostToDevice, p->s_in));
+        } else if (!lead) COVA_CUDA(cudaMemcpyAsync(sl.d_frames + s0 * dst_chain, frames + s0 * src_chain, ns * src_chain, cudaMemcpyHostToDevice, p->s_in));
+        else COVA_CUDA(cudaMemcpy2DAsync(sl.d_frames + s0 * dst_chain + lead_bytes, dst_chain, frames + s0 * src_chain, src_chain, src_chain, ns,
+                                         cudaMemcpyHostToDevice, p->s_in));
+        COVA_CUDA(cudaEventRecord(sl.ev_in[c], p->s_in));
     }
-    if (stateful) COVA_CUDA_SLOT(cudaMemcpyAsync(sl.d_ids, sl.h_ids, sizeof(uint32_t) * n_streams, cudaMemcpyHostToDevice, p->stream));
+    return COVA_OK;
+}
+
+// compute stage, on p->stream: per chunk after ev_in[c] sparse expansion, carry restore / save, kernels, cursor snapshot
+static int compute_chunks(cova_pipeline *p, Slot &sl, uint32_t fps, uint32_t lead, bool stateful, bool sparse) {
+    const uint32_t t1 = p->T - 1, fps_dev = sl.fps;
+    const size_t dst_chain = p->frame_bytes * fps_dev;
     const int wpf = (int)(p->frame_bytes / 4);
-    for (uint32_t c = 0; c < nc; c++) {
-        COVA_CUDA_SLOT(cudaStreamWaitEvent(p->stream, sl.ev_in[c], 0));
+    if (stateful) COVA_CUDA(cudaMemcpyAsync(sl.d_ids, sl.h_ids, sizeof(uint32_t) * sl.n_streams, cudaMemcpyHostToDevice, p->stream));
+    for (uint32_t c = 0; c * p->chunk_streams < sl.n_streams; c++) {
+        const Chunk ck = chunk_of(sl, c, p->chunk_streams);
+        COVA_CUDA(cudaStreamWaitEvent(p->stream, sl.ev_in[c], 0));
         if (sparse) {      // a plain launch: tensorise_frames_kernel waits for it (pdl_wait) before reading the pool
-            const uint32_t s0 = c * p->chunk_streams, ns = std::min(p->chunk_streams, n_streams - s0);
-            SparseExpandArgs ea{sl.d_sparse, sl.d_off, sl.d_frames, s0 * fps, fps, fps_dev, lead, p->W * p->H};
-            sparse_expand_kernel<<<ns * fps, kExpandThreads, 0, p->stream>>>(ea);
+            SparseExpandArgs ea{sl.d_sparse, sl.d_off, sl.d_frames, ck.stream0 * fps, fps, fps_dev, lead, p->W * p->H};
+            sparse_expand_kernel<<<ck.n_streams * fps, kExpandThreads, 0, p->stream>>>(ea);
             p->launches++;
-            COVA_CUDA_SLOT(cudaGetLastError());
+            COVA_CUDA(cudaGetLastError());
         }
         if (stateful && t1) {
-            const size_t s0 = (size_t)c * p->chunk_streams;
-            const int ns = (int)std::min<size_t>(p->chunk_streams, n_streams - s0);
-            uint32_t *pool = reinterpret_cast<uint32_t *>(sl.d_frames + s0 * dst_chain);
+            const int ns = (int)ck.n_streams;
+            uint32_t *pool = reinterpret_cast<uint32_t *>(sl.d_frames + ck.stream0 * dst_chain);
             const int blocks = std::min(p->n_sms * 8, std::max(1, (int)(((long long)ns * t1 * wpf + 255) / 256)));
             if (lead) {     // lead frames for every chain: a chain with less history gets older carry bytes no window reads
-                carry_kernel<<<blocks, 256, 0, p->stream>>>(pool, reinterpret_cast<uint32_t *>(p->d_carry), sl.d_ids + s0, ns, wpf, (int)fps_dev, (int)lead, (int)t1, 0);
+                carry_kernel<<<blocks, 256, 0, p->stream>>>(pool, reinterpret_cast<uint32_t *>(p->d_carry), sl.d_ids + ck.stream0, ns, wpf, (int)fps_dev, (int)lead, (int)t1, 0);
                 p->launches++;
             }
-            carry_kernel<<<blocks, 256, 0, p->stream>>>(pool, reinterpret_cast<uint32_t *>(p->d_carry), sl.d_ids + s0, ns, wpf, (int)fps_dev, (int)lead, (int)t1, 1);
+            carry_kernel<<<blocks, 256, 0, p->stream>>>(pool, reinterpret_cast<uint32_t *>(p->d_carry), sl.d_ids + ck.stream0, ns, wpf, (int)fps_dev, (int)lead, (int)t1, 1);
             p->launches++;
-            COVA_CUDA_SLOT(cudaGetLastError());
+            COVA_CUDA(cudaGetLastError());
         }
-        if (p->cur_windows) {
-            if ((rc = run_chunk(p, c))) return fail(rc);
-            COVA_CUDA_SLOT(cudaMemcpyAsync(sl.h_cursor + 2 * c, sl.ccl.d_cursor, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
+        if (sl.n_windows) {
+            int rc = run_chunk(p, sl, ck);
+            if (rc) return rc;
+            COVA_CUDA(cudaMemcpyAsync(sl.h_cursor + 2 * c, sl.ccl.d_cursor, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
         }
-        COVA_CUDA_SLOT(cudaEventRecord(sl.ev_done[c], p->stream));
+        COVA_CUDA(cudaEventRecord(sl.ev_done[c], p->stream));
     }
-#undef COVA_CUDA_SLOT
     return COVA_OK;
+}
+
+static int submit_impl(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, uint32_t fps, const uint32_t *stream_ids,
+                       const uint64_t *pts, uint32_t flags, bool stateful, const size_t *sparse_len = nullptr) {
+    if (!p || !frames) return set_err(COVA_E_INVAL, "null argument");
+    const bool sparse = sparse_len != nullptr;
+    uint32_t lead = 0;                                              // carried frames in front of every device chain
+    int rc = plan_submit(p, frames, n_streams, fps, stream_ids, flags, stateful, sparse_len, lead);
+    if (rc) return rc;
+    COVA_CUDA(cudaSetDevice(p->device));
+    const int k = p->next_submit;
+    if (p->slot[k].busy) return set_err(COVA_E_INVAL, "four batches are already in flight: collect one first");
+    if ((rc = setup_slot(p, k, n_streams, fps, lead, stream_ids, pts, flags, stateful, sparse))) return rc;
+    auto &sl = p->slot[k];
+    sl.busy = true; sl.failed = false;
+    p->next_submit = (k + 1) % kSlots;
+    if (!stateful && !sl.n_windows) return COVA_OK;                // chains shorter than a window: nothing to compute
+    // from here on a failure leaves the slot marked failed: the matching collect reports it instead of reading events that
+    // were never recorded
+    if ((rc = copy_chunks(p, sl, frames, fps, lead, sparse)) || (rc = compute_chunks(p, sl, fps, lead, stateful, sparse)))
+        sl.failed = true;
+    return rc;
 }
 
 extern "C" int cova_pipeline_submit_host(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, uint32_t fps) {
@@ -1671,8 +1675,8 @@ static int collect_impl(cova_pipeline *p, uint8_t *blob, size_t blob_cap, size_t
         if (cudaEventSynchronize(sl.ev_done[c]) != cudaSuccess) return sync_stream(p, p->stream);
         if (sl.h_cursor[2 * c + 1]) return set_err(COVA_E_CUDA, "device box arena overflow (internal sizing error)");
         const unsigned long long end = sl.h_cursor[2 * c];
-        const size_t w0 = sl.win0[c * p->chunk_streams];
-        const size_t nw = sl.win0[std::min<uint32_t>((c + 1) * p->chunk_streams, sl.n_streams)] - w0;
+        const Chunk ck = chunk_of(sl, c, p->chunk_streams);
+        const size_t w0 = ck.window0, nw = ck.windows;
         if (offsets) COVA_CUDA(cudaMemcpyAsync(offsets + w0, sl.ccl.d_offsets + w0, nw * sizeof(uint64_t), cudaMemcpyDeviceToHost, p->s_out));
         if (lens) COVA_CUDA(cudaMemcpyAsync(lens + w0, sl.ccl.d_lens + w0, nw * sizeof(uint64_t), cudaMemcpyDeviceToHost, p->s_out));
         if (blob && end <= blob_cap) {
@@ -1700,11 +1704,11 @@ extern "C" int cova_pipeline_collect_host2(cova_pipeline *p, uint8_t *blob, size
 extern "C" int cova_pipeline_process_host(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, uint32_t fps, uint8_t *blob,
                                           size_t blob_cap, size_t *blob_len, uint64_t *offsets, uint64_t *lens, uint32_t *n_windows) {
     if (!p || !frames || !blob_len) return set_err(COVA_E_INVAL, "null argument");
-    for (auto &sl : p->slot)
-        if (sl.busy) return set_err(COVA_E_INVAL, "batches submitted asynchronously are still in flight");
+    int rc = require_idle(p);
+    if (rc) return rc;
     p->next_submit = p->next_collect = 0;
     prof_begin(p);
-    int rc = cova_pipeline_submit_host(p, frames, n_streams, fps);
+    rc = cova_pipeline_submit_host(p, frames, n_streams, fps);
     if (!rc) rc = cova_pipeline_collect_host(p, blob, blob_cap, blob_len, offsets, lens, n_windows);
     else if (p->slot[0].busy) { p->slot[0].busy = false; p->slot[0].failed = false; p->next_submit = p->next_collect = 0; }
     if (!rc) rc = cova_pipeline_sync(p);
@@ -1712,34 +1716,28 @@ extern "C" int cova_pipeline_process_host(cova_pipeline *p, const uint8_t *frame
 }
 
 // ---- inspection ------------------------------------------------------------------------------------
+// the last batch's [n_windows][per_window] array of elem_bytes elements on the device -> out (cap elements)
+static int read_windows(cova_pipeline *p, const void *src, size_t per_window, size_t elem_bytes, void *out, size_t cap) {
+    const size_t n = per_window * p->slot[p->last_slot].n_windows;
+    if (cap < n) return set_err(COVA_E_TOOSMALL, "buffer too small");
+    int rc = cova_pipeline_sync(p);
+    if (rc) return rc;
+    COVA_CUDA(cudaMemcpy(out, src, n * elem_bytes, cudaMemcpyDeviceToHost));
+    return COVA_OK;
+}
 extern "C" int cova_pipeline_read_stacked(cova_pipeline *p, uint8_t *out, size_t cap) {
     if (!p || !out) return set_err(COVA_E_INVAL, "null argument");
     if (!p->d_stacked) return set_err(COVA_E_INVAL, "pipeline was created without COVA_FLAG_KEEP_STACKED");
-    size_t bytes = p->frame_bytes * p->T * p->cur_windows;
-    if (cap < bytes) return set_err(COVA_E_TOOSMALL, "buffer too small");
-    int rc = cova_pipeline_sync(p);
-    if (rc) return rc;
-    COVA_CUDA(cudaMemcpy(out, p->d_stacked, bytes, cudaMemcpyDeviceToHost));
-    return COVA_OK;
+    return read_windows(p, p->d_stacked, p->frame_bytes * p->T, 1, out, cap);
 }
 extern "C" int cova_pipeline_read_mask(cova_pipeline *p, uint8_t *out, size_t cap) {
     if (!p || !out) return set_err(COVA_E_INVAL, "null argument");
-    size_t bytes = (size_t)p->cur_windows * p->W * p->H;
-    if (cap < bytes) return set_err(COVA_E_TOOSMALL, "buffer too small");
-    int rc = cova_pipeline_sync(p);
-    if (rc) return rc;
-    COVA_CUDA(cudaMemcpy(out, p->d_mask, bytes, cudaMemcpyDeviceToHost));
-    return COVA_OK;
+    return read_windows(p, p->d_mask, (size_t)p->W * p->H, 1, out, cap);
 }
 extern "C" int cova_pipeline_read_logits(cova_pipeline *p, float *out, size_t cap_floats) {
     if (!p || !out) return set_err(COVA_E_INVAL, "null argument");
     if (!p->d_logits) return set_err(COVA_E_INVAL, "pipeline was created without COVA_FLAG_KEEP_LOGITS");
-    size_t n = (size_t)p->cur_windows * p->W * p->H;
-    if (cap_floats < n) return set_err(COVA_E_TOOSMALL, "buffer too small");
-    int rc = cova_pipeline_sync(p);
-    if (rc) return rc;
-    COVA_CUDA(cudaMemcpy(out, p->d_logits, n * sizeof(float), cudaMemcpyDeviceToHost));
-    return COVA_OK;
+    return read_windows(p, p->d_logits, (size_t)p->W * p->H, sizeof(float), out, cap_floats);
 }
 
 extern "C" int cova_pipeline_read_activation(cova_pipeline *p, int layer, float *out, size_t cap_floats, uint32_t shape[5]) {
@@ -1749,7 +1747,7 @@ extern "C" int cova_pipeline_read_activation(cova_pipeline *p, int layer, float 
     const Geom &g = enc_side ? p->gx[layer] : p->gd[layer - 4];
     const uint4 *src = enc_side ? p->x[layer] : p->d[layer - 4];
     const int C = layer == 0 ? 3 : (enc_side ? kEncCout[layer - 1] : kDecCin[layer - 4]);
-    const int N = (int)p->ck_windows, Tn = g.Tn;   // activations of the chunk processed last
+    const int N = (int)p->last_chunk.windows, Tn = g.Tn;
     shape[0] = N; shape[1] = C; shape[2] = Tn; shape[3] = g.H; shape[4] = g.W;
     size_t n = (size_t)N * C * Tn * g.H * g.W;
     if (cap_floats < n) return set_err(COVA_E_TOOSMALL, "buffer too small");
@@ -1765,7 +1763,7 @@ extern "C" int cova_pipeline_read_activation(cova_pipeline *p, int layer, float 
                 for (int t = 0; t < kT; t++)
                     for (int y = 0; y < gf.H; y++)
                         for (int x = 0; x < gf.W; x++) {
-                            const int f = p->slot[p->cur_slot].h_newest[p->ck_window0 + nn] - t;
+                            const int f = p->slot[p->last_slot].h_newest[p->last_chunk.window0 + nn] - t;
                             const Row8 &r = host[(size_t)geom_row(gf, 0, (y & 1) << 1, geom_pos(gf, f, y >> 1, x >> 1, 0))];
                             out[((((size_t)nn * 3 + c) * kT + t) * gf.H + y) * gf.W + x] = __half2float(r.v[(x & 1) * 4 + c]);
                         }

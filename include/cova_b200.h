@@ -150,7 +150,9 @@ int cova_pipeline_set_stream(cova_pipeline *p, void *cuda_stream);
 int cova_pipeline_n_windows(const cova_pipeline *p, uint32_t n_streams, uint32_t frames_per_stream, uint32_t *n);
 
 /* stage 0: put a batch of frames [n_streams][frames_per_stream][h_mb][w_mb][4] into the device frame pool.
- * is_device != 0: frames is a device pointer (device-to-device copy). Asynchronous on the stream. */
+ * is_device != 0: frames is a device pointer (device-to-device copy). Asynchronous on the stream.
+ * The stage-wise calls (load_frames, load_masks, tensorise, blobnet, run_layer, ccl, run) share the pipeline's buffers
+ * with submitted batches: while a submit waits for its collect they return COVA_E_INVAL before any device call. */
 int cova_pipeline_load_frames(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams,
                               uint32_t frames_per_stream, int is_device);
 /* stages, each asynchronous on the stream, operating on the loaded batch */

@@ -463,6 +463,28 @@ def test_async_submit_collect_batches_in_flight():
         assert got == want
 
 
+def test_stage_wise_calls_are_refused_while_a_submitted_batch_is_in_flight():
+    """The stage-wise calls share slot 0 and the device buffers with submitted batches: while one waits for its collect they
+    return E_INVAL before any device call, and the collect still returns the boxes process() gives.  After the collect
+    the stage-wise path works again, with a batch of another shape."""
+    wts = weights.random_weights(0, head_bias=-1.0)
+    frames = synth.synth_streams(3, 9, 45, 80, config_idx=12)
+    other = synth.synth_streams(2, 7, 45, 80, config_idx=13)
+    p = BlobPipeline(80, 45, weights.to_blob(wts), 3, 9)
+    want, want_other = p.process(frames), p.process(other)
+    p.submit(frames)
+    masks = np.zeros((2, 45, 80), dtype=np.uint8)
+    for call in (lambda: p.load_frames(other), p.run, lambda: p.load_masks(masks), p.tensorise, p.blobnet,
+                 lambda: p.run_layer(0, _lib.IMPL_TCGEN05), p.ccl):
+        with pytest.raises(_lib.CovaError) as e:
+            call()
+        assert e.value.code == _lib.E_INVAL
+    assert p.collect() == want
+    p.load_frames(other)
+    p.run()
+    assert p.fetch_boxes() == want_other
+
+
 def test_bind_rank_to_gpu_keeps_the_process_inside_its_cpu_set():
     """cova_bind_host_to_device: the affinity after the call is a non-empty subset of the one before (N>1 ranks of
     bench.py call it before allocating their pinned buffers)."""
