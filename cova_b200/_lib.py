@@ -91,6 +91,8 @@ SIGNATURES = {
     "cova_packer_pack": (ctypes.c_int, [_vp, _vp, _vp, ctypes.c_size_t]),
     "cova_packer_pack_sparse": (ctypes.c_int, [_vp, _vp, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32, _vp, ctypes.c_size_t, _szp]),
     "cova_pipeline_submit_sparse": (ctypes.c_int, [_vp, _vp, ctypes.c_size_t, ctypes.c_uint32, ctypes.c_uint32, _vp, _vp, ctypes.c_uint32]),
+    "cova_pipeline_submit_ragged": (ctypes.c_int, [_vp, _vp, ctypes.c_uint32, _vp, _vp, _vp, ctypes.c_uint32]),
+    "cova_pipeline_submit_sparse_ragged": (ctypes.c_int, [_vp, _vp, ctypes.c_size_t, ctypes.c_uint32, _vp, _vp, _vp, ctypes.c_uint32]),
     "cova_pipeline_load_masks": (ctypes.c_int, [_vp, _vp, ctypes.c_uint32, ctypes.c_int]),
     "cova_pipeline_read_stacked": (ctypes.c_int, [_vp, _vp, ctypes.c_size_t]),
     "cova_pipeline_read_mask": (ctypes.c_int, [_vp, _vp, ctypes.c_size_t]),

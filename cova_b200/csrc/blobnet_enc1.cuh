@@ -32,15 +32,17 @@ constexpr int kThreads1 = 64 + 32 * kEpiWarps1;
 constexpr int kPairRows = 2 * kTileM;
 
 struct Enc1Extra {
-    int n_chains, fps, gamma;               // chains of this chunk, frames per chain, sub-sampling
-    // per chain of the chunk: (index of the newest frame of its first window, index of that window in the chunk).  Chains
-    // of a staggered batch differ in both (cova_abi.cu, set_batch_shape); a chain's window n + k has its newest frame at
-    // first + k * gamma
-    const int2 *tab;
+    int n_chains, fps, gamma;               // chains of this chunk, frame stride of a chain in the pool, sub-sampling
+    // per chain of the chunk: (x = index of the newest frame of its first window, y = index of that window in the chunk,
+    // z = end: the chain's frames are [0, end), w = frames of the chunk's chains before it, sum of their ends).  Chains of a
+    // staggered batch differ in x and y, chains of a ragged batch in z (cova_abi.cu, set_batch_shape); a chain's window
+    // n + k has its newest frame at x + k * gamma
+    const int4 *tab;
     int ntp;                                // tile pairs per frame
-    int n_items;                            // (chain, tile pair) items = n_chains * ntp, each fps frame steps long
+    int n_items;                            // (chain, tile pair) items = n_chains * ntp, item (c, j) is end_c frame steps long
     int full_items;                         // items handed out whole, round-robin: a multiple of the grid size
     int total, span;                        // frame steps in all items / consecutive steps of the REMAINING items per CTA
+    int g0;                                 // frame steps of the whole items: where the remaining items' steps begin
 };
 
 struct SmemPlan1 {
@@ -60,33 +62,41 @@ __host__ __device__ inline SmemPlan1 plan_smem1(int Ls, int n_stage, int w_bytes
 struct Item {
     int chain, jp, i0, i1, start;
 };
-// Work partition.  An item = one (chain, tile pair) walked through its fps frames; consecutive items are the tile pairs
-// of one chain, and handing them out round-robin keeps the CTAs that run concurrently on the same few chains (the four
-// tile pairs of a frame read and write neighbouring DRAM pages - a flat split of the whole step sequence into 148 spans
-// balanced better and ran 12 % slower).  Only the items left over after the last whole round (items mod grid size) are
-// cut: their steps form one sequence that is split evenly, and a CTA whose piece starts inside an item re-computes the
+// Work partition.  An item = one (chain, tile pair) walked through the chain's end_c frames; consecutive items are the
+// tile pairs of one chain, and handing them out round-robin keeps the CTAs that run concurrently on the same few chains (the
+// four tile pairs of a frame read and write neighbouring DRAM pages - a flat split of the whole step sequence into 148
+// spans balanced better and ran 12 % slower).  Only the items left over after the last whole round (items mod grid size)
+// are cut: their steps form one sequence that is split evenly, and a CTA whose piece starts inside an item re-computes the
 // kT - 1 warm-up frames the register ring needs.  At the benchmark size: 3 whole items + a 31-step piece = 235 steps per
-// CTA for 232 of work (whole items only: 268; two fixed segments per item: 259).
+// CTA for 232 of work (whole items only: 268; two fixed segments per item: 259).  Item (c, j) starts at step
+// ntp * tab[c].w + j * tab[c].z of the sequence, so a piece finds its item by a binary search over the chunk's chains;
+// with equal ends this is exactly the division by the chain length it replaces.
 struct WorkIter {
     int item, g, g1;
 };
 __device__ __forceinline__ WorkIter work_begin(const Enc1Extra &ex, int cta) {
     WorkIter wi;
     wi.item = cta;
-    wi.g = ex.full_items * ex.fps + cta * ex.span;
+    wi.g = ex.g0 + cta * ex.span;
     wi.g1 = min(ex.total, wi.g + ex.span);
     return wi;
 }
 __device__ __forceinline__ bool work_next(const Enc1Extra &ex, int n_cta, WorkIter &wi, Item &it) {
     if (wi.item < ex.full_items) {                                   // a whole item
-        it.jp = wi.item % ex.ntp; it.chain = wi.item / ex.ntp; it.i0 = 0; it.i1 = ex.fps; it.start = 0;
+        it.jp = wi.item % ex.ntp; it.chain = wi.item / ex.ntp; it.i0 = 0; it.i1 = __ldg(&ex.tab[it.chain].z); it.start = 0;
         wi.item += n_cta;
         return true;
     }
     if (wi.g >= wi.g1) return false;
-    const int item = wi.g / ex.fps, i = wi.g - item * ex.fps;          // a piece of a left-over item
-    const int len = min(ex.fps - i, wi.g1 - wi.g);
-    it.jp = item % ex.ntp; it.chain = item / ex.ntp; it.i0 = i; it.i1 = i + len; it.start = max(0, i - (kT - 1));
+    int lo = 0, hi = ex.n_chains - 1;                                 // the last chain that starts at or before step g
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (ex.ntp * __ldg(&ex.tab[mid].w) <= wi.g) lo = mid; else hi = mid - 1;
+    }
+    const int end = __ldg(&ex.tab[lo].z), r = wi.g - ex.ntp * __ldg(&ex.tab[lo].w);
+    const int jp = r / end, i = r - jp * end;                         // a piece of a left-over item
+    const int len = min(end - i, wi.g1 - wi.g);
+    it.jp = jp; it.chain = lo; it.i0 = i; it.i1 = i + len; it.start = max(0, i - (kT - 1));
     wi.g += len;
     return true;
 }
@@ -190,7 +200,7 @@ __global__ void __launch_bounds__(kThreads1, 1) enc1_fused_kernel(const __grid_c
             const bool valid = r < gi.S && y2 < (gi.H >> 1) && x2 < (gi.W >> 1);
             const bool warp_live = __any_sync(0xffffffffu, valid);       // warps that only cover padding rows skip the arithmetic
             // (first, window 0) of the chain: one load per item; window 0 goes into the base addresses, only first stays live
-            const int2 cw = ex.tab[w.chain];
+            const int2 cw = *reinterpret_cast<const int2 *>(&ex.tab[w.chain]);
             const int Y = y2 + (gi.H & 1), X = x2 + (gi.W & 1);          // zero-pad top / left when odd (encoder.py:68-76)
             const int pho = ((Y & 1) << 1) | (X & 1);
             const long long base_o = (long long)(cg * 4 + pho) * p.gout.Lp + p.gout.guard + ((long long)(Y >> 1) * p.gout.P + (X >> 1)) * kT +
@@ -290,8 +300,9 @@ __global__ void __launch_bounds__(kThreads1, 1) enc1_fused_kernel(const __grid_c
     if (warp == 1) tc::tmem_dealloc(tmem_base, 512);
 }
 
-// as tc::plan / tc::launch: the ring depth is the only choice (as deep as fits, at least 2)
-inline bool plan_enc1(LayerParams &p, Enc1Extra &ex, int n_sms, tc::Grid &g) {
+// as tc::plan / tc::launch: the ring depth is the only choice (as deep as fits, at least 2).  htab: the host copy of the
+// chunk's chain table (ends and their prefix sums); nullptr = every chain ends at ex.fps.
+inline bool plan_enc1(LayerParams &p, Enc1Extra &ex, const int4 *htab, int n_sms, tc::Grid &g) {
     p.Ls = kPairRows + 2 * p.gin.halo;
     if (p.gin.P >= 16384) return false;                                            // LBO field: 14 bits of 16-byte units
     ex.ntp = (p.gin.S + kPairRows - 1) / kPairRows;
@@ -301,11 +312,15 @@ inline bool plan_enc1(LayerParams &p, Enc1Extra &ex, int n_sms, tc::Grid &g) {
     if ((p.gout.Lp & 1) || (p.gout.guard & 1)) return false;                       // 256-bit stores need 32-byte aligned rows
     p.w_bytes = C1::BLOCKS * C1::BLOCK_N * 32;
     if (F * ex.ntp >= (1ll << 31)) return false;
-    ex.total = (int)(F * ex.ntp);
+    // frames that exist: the chains' ends (every end is at most the stride, so the bounds above hold)
+    const long long frames = htab ? (long long)htab[ex.n_chains - 1].w + htab[ex.n_chains - 1].z : F;
+    ex.total = (int)(frames * ex.ntp);
     ex.n_items = ex.n_chains * ex.ntp;
     const int ctas = std::max(1, std::min(n_sms, ex.total));
     ex.full_items = (ex.n_items / ctas) * ctas;
-    ex.span = ((ex.n_items - ex.full_items) * ex.fps + ctas - 1) / ctas;
+    const int c = ex.full_items / ex.ntp, j = ex.full_items - c * ex.ntp;           // the first left-over item
+    ex.g0 = htab ? (c < ex.n_chains ? ex.ntp * htab[c].w + j * htab[c].z : ex.total) : ex.full_items * ex.fps;
+    ex.span = (ex.total - ex.g0 + ctas - 1) / ctas;
     for (p.n_stage = kMaxStage1; p.n_stage >= 2; p.n_stage--)
         if (plan_smem1(p.Ls, p.n_stage, p.w_bytes).total <= (uint32_t)tc::kSmemLimit) break;
     if (p.n_stage < 2) return false;

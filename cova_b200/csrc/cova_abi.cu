@@ -512,6 +512,7 @@ struct cova_pipeline {
     std::vector<uint64_t> n_seen, id_mark;
     uint64_t id_epoch = 0;
     std::vector<uint32_t> first_scratch, hist_scratch;   // per chain of the batch being submitted
+    std::vector<uint32_t> count_scratch;                 // new frames per chain of the batch being submitted
     std::vector<uint64_t> off_scratch;                   // record offsets of the sparse batch being submitted
     // A batch is processed in chunks of whole chains: the activation buffers are sized for ONE chunk, and
     // process_host() overlaps the H2D copy of chunk c+1, the kernels of chunk c and the D2H of chunk c-1.
@@ -533,17 +534,24 @@ struct cova_pipeline {
         uint32_t *h_ids = nullptr, *d_ids = nullptr;   // stream ids of a submit_host2 batch (pinned staging + device copy)
         std::vector<uint64_t> win_pts;                 // per window: PTS of its newest frame / stream id (submit_host2)
         std::vector<uint32_t> win_ids;
-        // Window shape of the slot's batch (set_batch_shape).  Chain s yields windows [win0[s], win0[s+1]) of the batch; its
-        // first one has its newest frame at device index first_s, the next ones follow every gamma frames.
-        //   tab[s]     = (first_s, win0[s] - win0[first chain of s's chunk])      read by enc1_fused_kernel
+        // Window shape of the slot's batch (set_batch_shape).  Device chains have one stride (fps above); chain s holds
+        // frames [0, end_s) and yields windows [win0[s], win0[s+1]) of the batch; its first one has its newest frame at
+        // device index first_s, the next ones follow every gamma frames.  Nothing reads or writes a chain at or past end_s.
+        //   tab[s]     = (first_s, win0[s] - win0[c0], end_s, fpre[s] - fpre[c0])  c0 = first chain of s's chunk;
+        //                                                                          read by enc1_fused_kernel & co.
         //   newest[w]  = index of window w's newest frame among its chunk's frames  read by the gather kernels
+        //   fmap[f]    = (ragged batches only) pool index, among its chunk's frames, of the batch's f-th existing frame
         // Each slot owns pinned staging and a device copy, uploaded on the compute stream in order with the batch's
         // kernels: batches of different shapes can be in flight together without draining the pipeline.
         std::vector<uint32_t> win0;
-        int2 *h_tab = nullptr, *d_tab = nullptr;
+        std::vector<uint32_t> fpre;                    // prefix sums of end_s: existing frames of the chains before s
+        std::vector<uint64_t> npre;                    // prefix sums of the new frames per chain (source / PTS / record index)
+        bool ragged = false;                           // some end_s differs from the stride
+        int4 *h_tab = nullptr, *d_tab = nullptr;
         int *h_newest = nullptr, *d_newest = nullptr;
+        int *h_fmap = nullptr, *d_fmap = nullptr;      // allocated on the slot's first ragged batch
         cudaEvent_t ev_tab = nullptr;                  // recorded after the upload: the staging may be rewritten after it
-        std::vector<uint32_t> tab_first;               // what the tables hold: per-chain first, frames per chain, stream
+        std::vector<uint32_t> tab_first, tab_end;      // what the tables hold: per-chain first and end, stride, stream
         uint32_t tab_fps = 0;
         cudaStream_t tab_stream = nullptr;
         // sparse input (cova_pipeline_submit_sparse), allocated on the slot's first sparse submit: the batch's records at
@@ -719,8 +727,8 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
     p->frame_bytes = (size_t)w_mb * h_mb * (p->packed ? 2 : 4);
     cudaError_t e = cudaMalloc(&p->d_mask, (size_t)std::max(1, NB) * w_mb * h_mb);
     for (auto &sl : p->slot) {
-        if (e == cudaSuccess) e = cudaMallocHost(&sl.h_tab, sizeof(int2) * max_streams);
-        if (e == cudaSuccess) e = cudaMalloc(&sl.d_tab, sizeof(int2) * max_streams);
+        if (e == cudaSuccess) e = cudaMallocHost(&sl.h_tab, sizeof(int4) * max_streams);
+        if (e == cudaSuccess) e = cudaMalloc(&sl.d_tab, sizeof(int4) * max_streams);
         if (e == cudaSuccess) e = cudaMallocHost(&sl.h_newest, sizeof(int) * std::max(1, NB));
         if (e == cudaSuccess) e = cudaMalloc(&sl.d_newest, sizeof(int) * std::max(1, NB));
         if (e == cudaSuccess) e = cudaMallocHost(&sl.h_cursor, sizeof(unsigned long long) * 2 * 256);
@@ -781,6 +789,8 @@ extern "C" void cova_pipeline_free(cova_pipeline *p) {
         if (sl.d_tab) cudaFree(sl.d_tab);
         if (sl.h_newest) cudaFreeHost(sl.h_newest);
         if (sl.d_newest) cudaFree(sl.d_newest);
+        if (sl.h_fmap) cudaFreeHost(sl.h_fmap);
+        if (sl.d_fmap) cudaFree(sl.d_fmap);
         if (sl.ev_tab) cudaEventDestroy(sl.ev_tab);
         if (sl.d_sparse) cudaFree(sl.d_sparse);
         if (sl.h_off) cudaFreeHost(sl.h_off);
@@ -826,38 +836,54 @@ static int check_batch_bounds(const cova_pipeline *p, uint32_t n_streams, uint32
     return COVA_OK;
 }
 
-// Window shape of a batch of n_streams device chains of fps frames each, into slot k.  first[s] is the index
-// (inside device chain s) of the newest frame of the chain's first window; nullptr = T - 1 for every chain, i.e. chains
-// that start with an empty window.  CONTINUED chains (submit_host2) start later, where their carried history and gamma
-// phase put them.  Lock-step and staggered batches go through the same tables and kernels.
-static int set_batch_shape(cova_pipeline *p, int k, uint32_t n_streams, uint32_t fps, const uint32_t *first = nullptr) {
+// Window shape of a batch of n_streams device chains of stride fps, into slot k.  first[s] is the index (inside device
+// chain s) of the newest frame of the chain's first window; nullptr = T - 1 for every chain, i.e. chains that start with
+// an empty window.  CONTINUED chains (submit_host2) start later, where their carried history and gamma phase put them.
+// end[s] is where chain s's frames end (ragged batches); nullptr = fps for every chain.  Lock-step, staggered and ragged
+// batches go through the same tables and kernels.
+static int set_batch_shape(cova_pipeline *p, int k, uint32_t n_streams, uint32_t fps, const uint32_t *first = nullptr,
+                           const uint32_t *end = nullptr) {
     auto &sl = p->slot[k];
     const uint32_t t1 = p->T - 1, cs = p->chunk_streams;
+    auto first_of = [&](uint32_t s) { return first ? first[s] : t1; };
+    auto end_of = [&](uint32_t s) { return end ? end[s] : fps; };
     uint64_t total = 0;
-    for (uint32_t s = 0; s < n_streams; s++) total += windows_from(fps, first ? first[s] : t1, p->gamma);
+    for (uint32_t s = 0; s < n_streams; s++) total += windows_from(end_of(s), first_of(s), p->gamma);
     if (total > p->max_windows) return set_err(COVA_E_INVAL, "batch produces more windows than the pipeline was sized for");
     sl.win0.resize(n_streams + 1);
-    sl.win0[0] = 0;
-    for (uint32_t s = 0; s < n_streams; s++) sl.win0[s + 1] = sl.win0[s] + windows_from(fps, first ? first[s] : t1, p->gamma);
+    sl.fpre.resize(n_streams + 1);
+    sl.win0[0] = 0; sl.fpre[0] = 0;
+    sl.ragged = false;
+    for (uint32_t s = 0; s < n_streams; s++) {
+        sl.win0[s + 1] = sl.win0[s] + windows_from(end_of(s), first_of(s), p->gamma);
+        sl.fpre[s + 1] = sl.fpre[s] + end_of(s);
+        sl.ragged = sl.ragged || end_of(s) != fps;
+    }
     sl.n_streams = n_streams; sl.fps = fps; sl.n_windows = (uint32_t)total;
     bool same = sl.tab_fps == fps && sl.tab_stream == p->stream && sl.tab_first.size() == n_streams;
-    for (uint32_t s = 0; same && s < n_streams; s++) same = sl.tab_first[s] == (first ? first[s] : t1);
+    for (uint32_t s = 0; same && s < n_streams; s++) same = sl.tab_first[s] == first_of(s) && sl.tab_end[s] == end_of(s);
     if (same) return COVA_OK;                                      // the slot's device tables already hold this shape
+    if (sl.ragged && !sl.h_fmap) {
+        COVA_CUDA(cudaMallocHost(&sl.h_fmap, sizeof(int) * (size_t)p->max_streams * p->max_fps));
+        COVA_CUDA(cudaMalloc(&sl.d_fmap, sizeof(int) * (size_t)p->max_streams * p->max_fps));
+    }
     // The staging may still be read by this slot's previous upload when synchronous entry points reuse slot 0 back to back.
     // On the submit path that upload has completed: the slot's previous batch was collected.
     COVA_CUDA(cudaEventSynchronize(sl.ev_tab));
-    sl.tab_first.clear();                                          // invalid until the upload below is enqueued
+    sl.tab_first.clear(); sl.tab_end.clear();                      // invalid until the upload below is enqueued
     for (uint32_t s = 0; s < n_streams; s++) {
-        const uint32_t f = first ? first[s] : t1, c0 = s / cs * cs;
-        sl.h_tab[s] = make_int2((int)f, (int)(sl.win0[s] - sl.win0[c0]));
+        const uint32_t f = first_of(s), c0 = s / cs * cs;
+        sl.h_tab[s] = make_int4((int)f, (int)(sl.win0[s] - sl.win0[c0]), (int)end_of(s), (int)(sl.fpre[s] - sl.fpre[c0]));
         for (uint32_t w = sl.win0[s]; w < sl.win0[s + 1]; w++)
             sl.h_newest[w] = (int)((s - c0) * fps + f + (w - sl.win0[s]) * p->gamma);
+        if (sl.ragged)
+            for (uint32_t i = 0; i < end_of(s); i++) sl.h_fmap[sl.fpre[s] + i] = (int)((s - c0) * fps + i);
     }
-    COVA_CUDA(cudaMemcpyAsync(sl.d_tab, sl.h_tab, sizeof(int2) * n_streams, cudaMemcpyHostToDevice, p->stream));
+    COVA_CUDA(cudaMemcpyAsync(sl.d_tab, sl.h_tab, sizeof(int4) * n_streams, cudaMemcpyHostToDevice, p->stream));
     if (total) COVA_CUDA(cudaMemcpyAsync(sl.d_newest, sl.h_newest, sizeof(int) * total, cudaMemcpyHostToDevice, p->stream));
+    if (sl.ragged) COVA_CUDA(cudaMemcpyAsync(sl.d_fmap, sl.h_fmap, sizeof(int) * sl.fpre[n_streams], cudaMemcpyHostToDevice, p->stream));
     COVA_CUDA(cudaEventRecord(sl.ev_tab, p->stream));
-    if (first) sl.tab_first.assign(first, first + n_streams);
-    else sl.tab_first.assign(n_streams, t1);
+    for (uint32_t s = 0; s < n_streams; s++) { sl.tab_first.push_back(first_of(s)); sl.tab_end.push_back(end_of(s)); }
     sl.tab_fps = fps; sl.tab_stream = p->stream;
     return COVA_OK;
 }
@@ -934,14 +960,15 @@ static int tensorise_chunk(cova_pipeline *p, const Slot &sl, const Chunk &ck) {
         p->launches++;
         prof_mark(p, "stack_rgba");
     }
-    {   // per-frame first-conv input (tcgen05 path)
-        const int F = (int)(ck.n_streams * sl.fps);
+    {   // per-frame first-conv input (tcgen05 path), of the frames that exist (a ragged chunk's chains end early)
+        const int F = (int)(sl.fpre[ck.stream0 + ck.n_streams] - sl.fpre[ck.stream0]);
+        const int *fmap = sl.ragged ? sl.d_fmap + sl.fpre[ck.stream0] : nullptr;
         long long total = (long long)F * p->H * p->gx0f.Wh;
         int blocks = (int)std::min<long long>((total + 255) / 256, (long long)p->n_sms * 32);
         if (total >= (1ll << 32)) return set_err(COVA_E_UNSUPPORTED, "chunk too large for the frame tensorisation kernel (32-bit index)");
         COVA_CUDA(launch_pdl(p->packed ? tensorise_frames_kernel<true> : tensorise_frames_kernel<false>, dim3((unsigned)blocks), dim3(256), 0,
                              p->stream, !(p->dbg & kDbgNoPdl), reinterpret_cast<const uint32_t *>(frames), p->x0f, p->gx0f, F,
-                             make_fastdiv((uint32_t)std::max(2, p->gx0f.Wh)), make_fastdiv((uint32_t)std::max<uint32_t>(2u, p->H))));
+                             make_fastdiv((uint32_t)std::max(2, p->gx0f.Wh)), make_fastdiv((uint32_t)std::max<uint32_t>(2u, p->H)), fmap));
         p->launches++;
         prof_mark(p, "tensorise_frames");
     }
@@ -1058,6 +1085,7 @@ struct LayerPlan {
     cova_layer_plan info;
     tc::LayerParams lp;
     tc1::Enc1Extra ex;        // block 1 only
+    const int4 *htab;         // block 1 of a ragged chunk: host copy of the chunk's chain table (nullptr: equal ends)
     tc::Grid grid;
 };
 
@@ -1099,9 +1127,10 @@ static cudaError_t launch_entry(Cands<Cs...>, const LayerPlan &pl, cudaStream_t 
     return launch_nth<WS, Cs...>(pl, pl.info.config, st);
 }
 
-// The geometry part of a layer's parameters, all a plan depends on: N windows (block 1: n_chains chains of fps frames).
+// The geometry part of a layer's parameters, all a plan depends on: N windows (block 1: n_chains chains of stride fps,
+// ending at htab[c].z, or all at fps when htab is nullptr).
 static void plan_input(LayerPlan &pl, int layer, const Geom gx[4], const Geom gd[4], const Geom &gx0f, int N, int n_chains,
-                       int fps, int gamma) {
+                       int fps, int gamma, const int4 *htab = nullptr) {
     memset(&pl, 0, sizeof(pl));
     tc::LayerParams &lp = pl.lp;
     lp.N = N;
@@ -1109,6 +1138,7 @@ static void plan_input(LayerPlan &pl, int layer, const Geom gx[4], const Geom gd
     if (layer == 0) {
         lp.gin = gx0f; lp.gout = gx[1]; lp.gout2 = gd[3]; lp.N = n_chains * fps;
         pl.ex.n_chains = n_chains; pl.ex.fps = fps; pl.ex.gamma = gamma;
+        pl.htab = htab;
     } else if (layer < 4) {
         const int i = layer;
         lp.gin = gx[i]; lp.gout = i < 3 ? gx[i + 1] : gx[3]; lp.gout2 = gd[3 - i];
@@ -1126,7 +1156,7 @@ static int plan_layer(int layer, int dbg, int n_sms, LayerPlan &pl) {
     bool ok = false;
     if (layer == 0) {
         // first block: frame-level conv + PointWiseTN over a register ring of 4 frames, one kernel (blobnet_enc1.cuh)
-        ok = tc1::plan_enc1(pl.lp, pl.ex, n_sms, pl.grid);
+        ok = tc1::plan_enc1(pl.lp, pl.ex, pl.htab, n_sms, pl.grid);
         pl.info.family = COVA_PLAN_ENC1; pl.info.tps = 2; pl.info.tile = kTileM;
     } else if (layer < 4) {
         const int i = layer;
@@ -1207,7 +1237,8 @@ extern "C" int cova_blobnet_plan(uint32_t w_mb, uint32_t h_mb, uint32_t windows,
 }
 
 static int tc_plan(cova_pipeline *p, const Slot &sl, const Chunk &ck, int layer, LayerPlan &pl) {
-    plan_input(pl, layer, p->gx, p->gd, p->gx0f, (int)ck.windows, (int)ck.n_streams, (int)sl.fps, (int)p->gamma);
+    plan_input(pl, layer, p->gx, p->gd, p->gx0f, (int)ck.windows, (int)ck.n_streams, (int)sl.fps, (int)p->gamma,
+               sl.ragged ? sl.h_tab + ck.stream0 : nullptr);
     return plan_layer(layer, p->dbg, p->n_sms, pl);
 }
 
@@ -1403,16 +1434,20 @@ extern "C" int cova_pipeline_fetch_boxes(cova_pipeline *p, uint8_t *blob, size_t
 
 // Per-stream carry-over for CONTINUED batches.  carry[id] holds the last T - 1 frames of stream `id`, newest last.
 //   mode 0 (restore): device chain s gets the newest h carried frames of stream ids[s] in front of its new frames;
-//   mode 1 (save):    the last min(fps_dev, T - 1) frames of device chain s become the carry of stream ids[s].
+//   mode 1 (save):    the last min(end_s, T - 1) frames of device chain s, ending at end_s, become the carry of stream
+//                     ids[s].  end_s = tab[s].z for the chunks of a ragged batch, fps_dev otherwise (tab = nullptr).
 __global__ void __launch_bounds__(256) carry_kernel(uint32_t *__restrict__ pool, uint32_t *__restrict__ carry, const uint32_t *__restrict__ ids,
-                                                    int n_streams, int words_per_frame, int fps_dev, int h, int t1, int mode) {
-    const int k = mode ? min(fps_dev, t1) : h;                     // frames moved per stream
+                                                    const int4 *__restrict__ tab, int n_streams, int words_per_frame, int fps_dev,
+                                                    int h, int t1, int mode) {
+    const int k = mode ? min(fps_dev, t1) : h;                     // frames moved per stream (at most)
     const long long per_stream = (long long)k * words_per_frame, total = per_stream * n_streams;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
         const int s = (int)(i / per_stream);
         const long long e = i - (long long)s * per_stream;
+        const int end = mode && tab ? __ldg(&tab[s].z) : fps_dev;
+        if (e < (long long)(k - end) * words_per_frame) continue;  // a chain shorter than k moves its end_s frames only
         uint32_t *c = carry + ((long long)ids[s] * t1 + (t1 - k)) * words_per_frame + e;
-        uint32_t *f = pool + ((long long)s * fps_dev + (mode ? fps_dev - k : 0)) * words_per_frame + e;
+        uint32_t *f = pool + ((long long)s * fps_dev + (mode ? end - k : 0)) * words_per_frame + e;
         if (mode) *c = *f; else *f = *c;
     }
 }
@@ -1438,19 +1473,37 @@ __global__ void __launch_bounds__(256) carry_kernel(uint32_t *__restrict__ pool,
 // the copy stage of a chunk: the host validates every record first and keeps their offsets; chunk c's records are one
 // contiguous byte range, copied as such, and sparse_expand_kernel writes them into the frame pool where the dense copy
 // would have put them.  Everything after that is shared.
+//
+// Ragged batches (submit_ragged / submit_sparse_ragged) give chain s its own count n_s of new frames.  The pool keeps one
+// stride, fps_dev = lead + max_s n_s; chain s's new frames are [lead, end_s), end_s = lead + n_s, and no kernel touches a
+// chain at or past its end.  Every other submit is the ragged plan with n_s = fps for every chain: one plan, one slot
+// set-up, one copy stage and one compute stage, which for equal counts enqueue exactly what they always did.
 
-// Argument checks and per-chain plan of a submit, before any device call: fills first_scratch, hist_scratch and
-// off_scratch, and raises lead (0 on entry) to the longest carried history
-static int plan_submit(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, uint32_t fps, const uint32_t *stream_ids,
-                       uint32_t flags, bool stateful, const size_t *sparse_len, uint32_t &lead) {
+// Argument checks and per-chain plan of a submit, before any device call: fills count_scratch (n_s: `counts`, or fps for
+// every chain when counts is nullptr), first_scratch, hist_scratch and off_scratch, and raises lead (0 on entry) to the
+// longest carried history
+static int plan_submit(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, uint32_t fps, const uint32_t *counts,
+                       const uint32_t *stream_ids, uint32_t flags, bool stateful, const size_t *sparse_len, uint32_t &lead) {
     if (flags & ~(COVA_SUBMIT_CONTINUE | COVA_SUBMIT_STAGGERED)) return set_err(COVA_E_INVAL, "unknown submit flag");
     if ((flags & COVA_SUBMIT_STAGGERED) && !(flags & COVA_SUBMIT_CONTINUE))
         return set_err(COVA_E_INVAL, "COVA_SUBMIT_STAGGERED needs COVA_SUBMIT_CONTINUE");
     if (sparse_len && !p->packed) return set_err(COVA_E_INVAL, "sparse input needs a COVA_FLAG_INPUT_PACKED16 pipeline");
-    int rc = check_batch_bounds(p, n_streams, fps);
+    uint32_t max_n = fps;
+    uint64_t n_frames = (uint64_t)n_streams * fps;
+    if (counts) {
+        if (!n_streams || n_streams > p->max_streams) return set_err(COVA_E_INVAL, "batch exceeds max_streams of the pipeline");
+        max_n = 0; n_frames = 0;
+        for (uint32_t s = 0; s < n_streams; s++) {
+            if (!counts[s]) return set_err(COVA_E_INVAL, "every stream of a ragged batch needs at least one frame (omit the stream instead)");
+            max_n = std::max(max_n, counts[s]);
+            n_frames += counts[s];
+        }
+        p->count_scratch.assign(counts, counts + n_streams);
+    }
+    int rc = check_batch_bounds(p, n_streams, max_n);
     if (rc) return rc;
+    if (!counts) p->count_scratch.assign(n_streams, fps);
     if (sparse_len) {
-        const uint64_t n_frames = (uint64_t)n_streams * fps;
         p->off_scratch.resize(n_frames + 1);
         uint64_t bad = 0;
         if (const char *why = sparse::validate_batch(frames, *sparse_len, n_frames, p->W * p->H, p->off_scratch.data(), &bad)) {
@@ -1464,7 +1517,7 @@ static int plan_submit(cova_pipeline *p, const uint8_t *frames, uint32_t n_strea
     first.assign(n_streams, t1);
     hist.assign(n_streams, 0);
     if (stateful) {
-        if (!fps) return set_err(COVA_E_INVAL, "a stream batch needs at least one frame per stream");
+        if (!max_n) return set_err(COVA_E_INVAL, "a stream batch needs at least one frame per stream");
         if (p->n_seen.empty()) { p->n_seen.assign(p->max_streams, 0); p->id_mark.assign(p->max_streams, 0); }
         p->id_epoch++;                                              // "seen in this batch" marks without clearing the array
         for (uint32_t s = 0; s < n_streams; s++) {
@@ -1487,13 +1540,13 @@ static int plan_submit(cova_pipeline *p, const uint8_t *frames, uint32_t n_strea
         }
         for (uint32_t s = 0; s < n_streams; s++) first[s] += lead - hist[s];   // chain s is padded by lead - h_s frames
     }
-    if (fps + lead > p->max_fps)
+    if (max_n + lead > p->max_fps)
         return set_err(COVA_E_INVAL, "carried frames + new frames exceed max_frames_per_stream of the pipeline");
     return COVA_OK;
 }
 
 // slot k takes the planned batch: buffers on first use, window shape, per-window stream ids and PTS, frames seen per stream
-static int setup_slot(cova_pipeline *p, int k, uint32_t n_streams, uint32_t fps, uint32_t lead, const uint32_t *stream_ids,
+static int setup_slot(cova_pipeline *p, int k, uint32_t n_streams, uint32_t lead, const uint32_t *stream_ids,
                       const uint64_t *pts, uint32_t flags, bool stateful, bool sparse) {
     int rc = ensure_slot(p, k);
     if (rc) return rc;
@@ -1516,8 +1569,18 @@ static int setup_slot(cova_pipeline *p, int k, uint32_t n_streams, uint32_t fps,
         if (!sl.d_off) COVA_CUDA(cudaMalloc(&sl.d_off, sizeof(unsigned long long) * (max_frames + 1)));
         COVA_CUDA(cudaEventCreateWithFlags(&sl.ev_off, cudaEventDisableTiming));
     }
-    const std::vector<uint32_t> &first = p->first_scratch;
-    if ((rc = set_batch_shape(p, k, n_streams, fps + lead, first.data()))) return rc;
+    const std::vector<uint32_t> &first = p->first_scratch, &cnt = p->count_scratch;
+    uint32_t max_n = 0;
+    std::vector<uint32_t> &end = p->hist_scratch;                  // the histories are no longer needed: chain ends
+    end.resize(n_streams);
+    sl.npre.resize(n_streams + 1);
+    sl.npre[0] = 0;
+    for (uint32_t s = 0; s < n_streams; s++) {
+        max_n = std::max(max_n, cnt[s]);
+        end[s] = lead + cnt[s];
+        sl.npre[s + 1] = sl.npre[s] + cnt[s];
+    }
+    if ((rc = set_batch_shape(p, k, n_streams, max_n + lead, first.data(), end.data()))) return rc;
     p->last_slot = k;
     sl.win_pts.clear(); sl.win_ids.clear();
     if (stateful) {
@@ -1529,51 +1592,67 @@ static int setup_slot(cova_pipeline *p, int k, uint32_t n_streams, uint32_t fps,
             sl.h_ids[s] = id;
             for (uint32_t w = sl.win0[s]; w < sl.win0[s + 1]; w++) {
                 sl.win_ids[w] = id;
-                if (pts) sl.win_pts[w] = pts[(size_t)s * fps + (first[s] + (w - sl.win0[s]) * p->gamma - lead)];
+                if (pts) sl.win_pts[w] = pts[sl.npre[s] + (first[s] + (w - sl.win0[s]) * p->gamma - lead)];
             }
-            p->n_seen[id] = ((flags & COVA_SUBMIT_CONTINUE) ? p->n_seen[id] : 0) + fps;
+            p->n_seen[id] = ((flags & COVA_SUBMIT_CONTINUE) ? p->n_seen[id] : 0) + cnt[s];
         }
     }
     return COVA_OK;
 }
 
-// copy stage, on s_in: per chunk the new frames (dense, padded behind lead carried frames, or sparse records), then ev_in[c]
-static int copy_chunks(cova_pipeline *p, Slot &sl, const uint8_t *frames, uint32_t fps, uint32_t lead, bool sparse) {
+// copy stage, on s_in: per chunk the new frames (dense, padded behind lead carried frames, or sparse records), then ev_in[c].
+// Dense: each run of consecutive chains with the same count is one copy - one cudaMemcpyAsync when the run is contiguous
+// in the pool too (no carried frames, chains as long as the stride), one cudaMemcpy2DAsync otherwise.  A batch of equal
+// counts is one run per chunk; all distinct counts cost one copy per chain.
+static int copy_chunks(cova_pipeline *p, Slot &sl, const uint8_t *frames, uint32_t lead, bool sparse) {
+    const std::vector<uint32_t> &cnt = p->count_scratch;
     if (sparse) {
         // the slot's previous offsets upload has completed (its batch was collected); the event makes that explicit
-        const size_t n_offs = (size_t)sl.n_streams * fps + 1;
+        const size_t n_offs = (size_t)sl.npre[sl.n_streams] + 1;
         COVA_CUDA(cudaEventSynchronize(sl.ev_off));
         memcpy(sl.h_off, p->off_scratch.data(), sizeof(unsigned long long) * n_offs);
         COVA_CUDA(cudaMemcpyAsync(sl.d_off, sl.h_off, sizeof(unsigned long long) * n_offs, cudaMemcpyHostToDevice, p->stream));
         COVA_CUDA(cudaEventRecord(sl.ev_off, p->stream));
     }
-    const size_t src_chain = p->frame_bytes * fps, dst_chain = p->frame_bytes * sl.fps, lead_bytes = p->frame_bytes * lead;
+    const size_t fb = p->frame_bytes, dst_chain = fb * sl.fps, lead_bytes = fb * lead;
     for (uint32_t c = 0; c * p->chunk_streams < sl.n_streams; c++) {
         const Chunk ck = chunk_of(sl, c, p->chunk_streams);
         const size_t s0 = ck.stream0, ns = ck.n_streams;
         if (sparse) {      // chunk c's records: one contiguous byte range, to the same offset of the staging
-            const uint64_t b0 = p->off_scratch[s0 * fps], b1 = p->off_scratch[(s0 + ns) * fps];
+            const uint64_t b0 = p->off_scratch[sl.npre[s0]], b1 = p->off_scratch[sl.npre[s0 + ns]];
             COVA_CUDA(cudaMemcpyAsync(sl.d_sparse + b0, frames + b0, b1 - b0, cudaMemcpyHostToDevice, p->s_in));
-        } else if (!lead) COVA_CUDA(cudaMemcpyAsync(sl.d_frames + s0 * dst_chain, frames + s0 * src_chain, ns * src_chain, cudaMemcpyHostToDevice, p->s_in));
-        else COVA_CUDA(cudaMemcpy2DAsync(sl.d_frames + s0 * dst_chain + lead_bytes, dst_chain, frames + s0 * src_chain, src_chain, src_chain, ns,
-                                         cudaMemcpyHostToDevice, p->s_in));
+        } else {
+            for (size_t s = s0, e; s < s0 + ns; s = e) {
+                for (e = s + 1; e < s0 + ns && cnt[e] == cnt[s];) e++;
+                const size_t src_chain = fb * cnt[s];
+                const uint8_t *src = frames + fb * sl.npre[s];
+                if (!lead && src_chain == dst_chain)
+                    COVA_CUDA(cudaMemcpyAsync(sl.d_frames + s * dst_chain, src, (e - s) * src_chain, cudaMemcpyHostToDevice, p->s_in));
+                else
+                    COVA_CUDA(cudaMemcpy2DAsync(sl.d_frames + s * dst_chain + lead_bytes, dst_chain, src, src_chain, src_chain, e - s,
+                                                cudaMemcpyHostToDevice, p->s_in));
+            }
+        }
         COVA_CUDA(cudaEventRecord(sl.ev_in[c], p->s_in));
     }
     return COVA_OK;
 }
 
 // compute stage, on p->stream: per chunk after ev_in[c] sparse expansion, carry restore / save, kernels, cursor snapshot
-static int compute_chunks(cova_pipeline *p, Slot &sl, uint32_t fps, uint32_t lead, bool stateful, bool sparse) {
+static int compute_chunks(cova_pipeline *p, Slot &sl, uint32_t lead, bool stateful, bool sparse) {
     const uint32_t t1 = p->T - 1, fps_dev = sl.fps;
     const size_t dst_chain = p->frame_bytes * fps_dev;
     const int wpf = (int)(p->frame_bytes / 4);
     if (stateful) COVA_CUDA(cudaMemcpyAsync(sl.d_ids, sl.h_ids, sizeof(uint32_t) * sl.n_streams, cudaMemcpyHostToDevice, p->stream));
     for (uint32_t c = 0; c * p->chunk_streams < sl.n_streams; c++) {
         const Chunk ck = chunk_of(sl, c, p->chunk_streams);
+        const int4 *tab = sl.ragged ? sl.d_tab + ck.stream0 : nullptr;
         COVA_CUDA(cudaStreamWaitEvent(p->stream, sl.ev_in[c], 0));
         if (sparse) {      // a plain launch: tensorise_frames_kernel waits for it (pdl_wait) before reading the pool
-            SparseExpandArgs ea{sl.d_sparse, sl.d_off, sl.d_frames, ck.stream0 * fps, fps, fps_dev, lead, p->W * p->H};
-            sparse_expand_kernel<<<ck.n_streams * fps, kExpandThreads, 0, p->stream>>>(ea);
+            const uint32_t f0 = (uint32_t)sl.npre[ck.stream0], nf = (uint32_t)(sl.npre[ck.stream0 + ck.n_streams] - f0);
+            SparseExpandArgs ea{sl.d_sparse, sl.d_off, sl.d_frames + ck.stream0 * dst_chain, f0, fps_dev - lead, fps_dev, lead,
+                                p->W * p->H, tab, ck.n_streams};
+            sparse_expand_kernel<<<nf, kExpandThreads, 0, p->stream>>>(ea);
             p->launches++;
             COVA_CUDA(cudaGetLastError());
         }
@@ -1582,10 +1661,10 @@ static int compute_chunks(cova_pipeline *p, Slot &sl, uint32_t fps, uint32_t lea
             uint32_t *pool = reinterpret_cast<uint32_t *>(sl.d_frames + ck.stream0 * dst_chain);
             const int blocks = std::min(p->n_sms * 8, std::max(1, (int)(((long long)ns * t1 * wpf + 255) / 256)));
             if (lead) {     // lead frames for every chain: a chain with less history gets older carry bytes no window reads
-                carry_kernel<<<blocks, 256, 0, p->stream>>>(pool, reinterpret_cast<uint32_t *>(p->d_carry), sl.d_ids + ck.stream0, ns, wpf, (int)fps_dev, (int)lead, (int)t1, 0);
+                carry_kernel<<<blocks, 256, 0, p->stream>>>(pool, reinterpret_cast<uint32_t *>(p->d_carry), sl.d_ids + ck.stream0, nullptr, ns, wpf, (int)fps_dev, (int)lead, (int)t1, 0);
                 p->launches++;
             }
-            carry_kernel<<<blocks, 256, 0, p->stream>>>(pool, reinterpret_cast<uint32_t *>(p->d_carry), sl.d_ids + ck.stream0, ns, wpf, (int)fps_dev, (int)lead, (int)t1, 1);
+            carry_kernel<<<blocks, 256, 0, p->stream>>>(pool, reinterpret_cast<uint32_t *>(p->d_carry), sl.d_ids + ck.stream0, tab, ns, wpf, (int)fps_dev, (int)lead, (int)t1, 1);
             p->launches++;
             COVA_CUDA(cudaGetLastError());
         }
@@ -1599,38 +1678,50 @@ static int compute_chunks(cova_pipeline *p, Slot &sl, uint32_t fps, uint32_t lea
     return COVA_OK;
 }
 
-static int submit_impl(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, uint32_t fps, const uint32_t *stream_ids,
-                       const uint64_t *pts, uint32_t flags, bool stateful, const size_t *sparse_len = nullptr) {
+// counts: n_s per chain (ragged submits), or nullptr: fps for every chain
+static int submit_impl(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, uint32_t fps, const uint32_t *counts,
+                       const uint32_t *stream_ids, const uint64_t *pts, uint32_t flags, bool stateful, const size_t *sparse_len = nullptr) {
     if (!p || !frames) return set_err(COVA_E_INVAL, "null argument");
     const bool sparse = sparse_len != nullptr;
     uint32_t lead = 0;                                              // carried frames in front of every device chain
-    int rc = plan_submit(p, frames, n_streams, fps, stream_ids, flags, stateful, sparse_len, lead);
+    int rc = plan_submit(p, frames, n_streams, fps, counts, stream_ids, flags, stateful, sparse_len, lead);
     if (rc) return rc;
     COVA_CUDA(cudaSetDevice(p->device));
     const int k = p->next_submit;
     if (p->slot[k].busy) return set_err(COVA_E_INVAL, "four batches are already in flight: collect one first");
-    if ((rc = setup_slot(p, k, n_streams, fps, lead, stream_ids, pts, flags, stateful, sparse))) return rc;
+    if ((rc = setup_slot(p, k, n_streams, lead, stream_ids, pts, flags, stateful, sparse))) return rc;
     auto &sl = p->slot[k];
     sl.busy = true; sl.failed = false;
     p->next_submit = (k + 1) % kSlots;
     if (!stateful && !sl.n_windows) return COVA_OK;                // chains shorter than a window: nothing to compute
     // from here on a failure leaves the slot marked failed: the matching collect reports it instead of reading events that
     // were never recorded
-    if ((rc = copy_chunks(p, sl, frames, fps, lead, sparse)) || (rc = compute_chunks(p, sl, fps, lead, stateful, sparse)))
+    if ((rc = copy_chunks(p, sl, frames, lead, sparse)) || (rc = compute_chunks(p, sl, lead, stateful, sparse)))
         sl.failed = true;
     return rc;
 }
 
 extern "C" int cova_pipeline_submit_host(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, uint32_t fps) {
-    return submit_impl(p, frames, n_streams, fps, nullptr, nullptr, 0, false);
+    return submit_impl(p, frames, n_streams, fps, nullptr, nullptr, nullptr, 0, false);
 }
 extern "C" int cova_pipeline_submit_host2(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, uint32_t fps,
                                           const uint32_t *stream_ids, const uint64_t *pts, uint32_t flags) {
-    return submit_impl(p, frames, n_streams, fps, stream_ids, pts, flags, true);
+    return submit_impl(p, frames, n_streams, fps, nullptr, stream_ids, pts, flags, true);
 }
 extern "C" int cova_pipeline_submit_sparse(cova_pipeline *p, const uint8_t *data, size_t data_len, uint32_t n_streams,
                                            uint32_t fps, const uint32_t *stream_ids, const uint64_t *pts, uint32_t flags) {
-    return submit_impl(p, data, n_streams, fps, stream_ids, pts, flags, true, &data_len);
+    return submit_impl(p, data, n_streams, fps, nullptr, stream_ids, pts, flags, true, &data_len);
+}
+extern "C" int cova_pipeline_submit_ragged(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, const uint32_t *n_frames,
+                                           const uint32_t *stream_ids, const uint64_t *pts, uint32_t flags) {
+    if (!n_frames) return set_err(COVA_E_INVAL, "null n_frames");
+    return submit_impl(p, frames, n_streams, 0, n_frames, stream_ids, pts, flags, true);
+}
+extern "C" int cova_pipeline_submit_sparse_ragged(cova_pipeline *p, const uint8_t *data, size_t data_len, uint32_t n_streams,
+                                                  const uint32_t *n_frames, const uint32_t *stream_ids, const uint64_t *pts,
+                                                  uint32_t flags) {
+    if (!n_frames) return set_err(COVA_E_INVAL, "null n_frames");
+    return submit_impl(p, data, n_streams, 0, n_frames, stream_ids, pts, flags, true, &data_len);
 }
 extern "C" int cova_pipeline_reset_streams(cova_pipeline *p, const uint32_t *stream_ids, uint32_t n) {
     if (!p) return set_err(COVA_E_INVAL, "null handle");

@@ -7,7 +7,9 @@
 // number of u32 (not necessarily of 16 bytes).
 //
 // Frame i = (s, f) of the batch lands at chain-relative index lead + f of device chain s, exactly where the dense H2D copy
-// puts packed16 frames: carry-over, staggering and every later kernel see the same pool.  The record offsets come from
+// puts packed16 frames: carry-over, staggering and every later kernel see the same pool.  In a ragged batch
+// (cova_pipeline_submit_sparse_ragged) chain s brings n_s frames: the CTA finds its chain by a binary search over the
+// chunk's chain table, whose prefix of chain ends minus lead per chain is the prefix of the n_s.  The record offsets come from
 // the host's validation walk; the kernel reads nothing outside [off[i], off[i+1]) even if the caller's buffer changed
 // after it was validated (a value rank past the record's end yields the background instead).
 #pragma once
@@ -22,9 +24,11 @@ constexpr int kExpandTileWords = 4 * kExpandThreads;   // 32,768 macroblocks per
 struct SparseExpandArgs {
     const uint8_t *data;                 // device copy of the batch, records at their host byte offsets
     const unsigned long long *off;       // n_frames + 1 record offsets of the batch
-    uint8_t *pool;                       // the slot's frame pool: chains of fps_dev frames of 2 * n_mb bytes
+    uint8_t *pool;                       // the chunk's part of the slot's frame pool: chains of fps_dev frames of 2 * n_mb bytes
     uint32_t frame0;                     // first batch frame of this launch (the chunk's first)
-    uint32_t fps, fps_dev, lead, n_mb;
+    uint32_t fps, fps_dev, lead, n_mb;   // fps: new frames of every chain (equal counts)
+    const int4 *tab;                     // ragged: the chunk's chain table (.w = frames of the chains before), else nullptr
+    uint32_t n_chains;                   // chains of the chunk (ragged)
 };
 
 __global__ void __launch_bounds__(kExpandThreads) sparse_expand_kernel(SparseExpandArgs a) {
@@ -34,7 +38,18 @@ __global__ void __launch_bounds__(kExpandThreads) sparse_expand_kernel(SparseExp
     __shared__ uint32_t s_tile_total;
     const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
     const uint32_t i = a.frame0 + blockIdx.x;
-    const uint32_t s = i / a.fps, f = i - s * a.fps;
+    uint32_t s, f;
+    if (a.tab) {                                                        // the last chain whose new frames start at or before i
+        const uint32_t r = blockIdx.x;                                  // chunk-relative, like s
+        uint32_t lo = 0, hi = a.n_chains - 1;
+        while (lo < hi) {
+            const uint32_t mid = (lo + hi + 1) >> 1;
+            if ((uint32_t)__ldg(&a.tab[mid].w) - mid * a.lead <= r) lo = mid; else hi = mid - 1;
+        }
+        s = lo; f = r - ((uint32_t)__ldg(&a.tab[lo].w) - lo * a.lead);
+    } else {
+        s = blockIdx.x / a.fps; f = blockIdx.x - s * a.fps;
+    }
     const unsigned long long lo = a.off[i], rec_len = a.off[i + 1] - lo;
     const uint8_t *rec = a.data + lo;
     const uint32_t nw = sparse::bitmap_words(a.n_mb), vo = sparse::values_offset(a.n_mb);

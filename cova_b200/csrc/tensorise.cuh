@@ -98,9 +98,13 @@ __device__ __forceinline__ uint2 quad_to_half4(uint32_t q) {
 // whose first operation is clip(., 0, 6) (utils/model/preprocessing.py:5-8), and half the host->device bytes.  W is even.
 __device__ __forceinline__ uint32_t unpack16(uint32_t p) { return (p & 7u) | ((p & 0x38u) << 5) | ((p & 0x1c0u) << 10); }
 
+// fmap (chunks of a ragged batch, cova_pipeline_submit_ragged): frame f of the n_frames that exist is frame fmap[f] of the
+// pool, whose chains have one stride but end at different frames; nullptr = every frame of the pool exists (fmap[f] = f).
+// The thread count scales with the frames that exist: a chain's dead tail is neither read nor written.
 template <bool PACKED>
 __global__ void __launch_bounds__(256) tensorise_frames_kernel(const uint32_t *__restrict__ frames, uint4 *__restrict__ x0f,
-                                                               Geom g, int n_frames, FastDiv div_wh, FastDiv div_h) {
+                                                               Geom g, int n_frames, FastDiv div_wh, FastDiv div_h,
+                                                               const int *__restrict__ fmap) {
     pdl_launch_dependents();
     pdl_wait();              // x0f is still being read by the previous batch's first block until that batch has completed
     const uint32_t Wh = (uint32_t)g.Wh, H = (uint32_t)g.H, W = (uint32_t)g.W;
@@ -117,7 +121,12 @@ __global__ void __launch_bounds__(256) tensorise_frames_kernel(const uint32_t *_
             const uint32_t i = i0 + (uint32_t)k * stride;
             q0[k] = q1[k] = 0u; rr[k] = xx[k] = 0u;
             if (i < total) {
-                const uint32_t r = Wh > 1 ? fast_div(i, div_wh) : i, x2 = i - r * Wh;      // r = f * H + y
+                uint32_t r = Wh > 1 ? fast_div(i, div_wh) : i;                           // r = f * H + y
+                const uint32_t x2 = i - r * Wh;
+                if (fmap) {                                                                  // -> row of the pool
+                    const uint32_t f = H > 1 ? fast_div(r, div_h) : r;
+                    r += ((uint32_t)__ldg(fmap + f) - f) * H;
+                }
                 const uint32_t *src = frames + ((size_t)r * W + 2 * x2);
                 rr[k] = r; xx[k] = x2;
                 if constexpr (PACKED) {

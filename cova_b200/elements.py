@@ -66,12 +66,14 @@ class PinnedBuffer:
 class SparseBatch:
     """A batch in the sparse input format (include/cova_b200.h, COVA_SPARSE_MAX_FRAME_BYTES): the records of
     n_streams x frames_per_stream frames, stream-major.  `data` is u8 and exactly the batch's bytes (it may be a view of
-    a PinnedBuffer array).  BlobPipeline(packed_input=True).submit() takes it like a dense frames array."""
+    a PinnedBuffer array).  BlobPipeline(packed_input=True).submit() takes it like a dense frames array.  A ragged batch
+    (pack_sparse(..., counts=)) holds counts[s] frames of stream s instead; frames_per_stream is then 0."""
     data: np.ndarray
     n_streams: int
     frames_per_stream: int
     h_mb: int
     w_mb: int
+    counts: np.ndarray | None = None
 
 
 class FramePacker:
@@ -92,11 +94,16 @@ class FramePacker:
         check(_lib.load().cova_packer_pack(self._h, _ptr(a), _ptr(out), out.size))
         return out
 
-    def pack_sparse(self, quads: np.ndarray, out: np.ndarray | None = None) -> SparseBatch:
+    def pack_sparse(self, quads: np.ndarray, out: np.ndarray | None = None, counts=None) -> SparseBatch:
         """quads [n_streams, frames, h, w, 4] u8 -> SparseBatch (cova_packer_pack_sparse).  `out`: a u8 array to encode
         into (e.g. PinnedBuffer(...).array); data is then a view of its first bytes.  Raises CovaError(E_TOOSMALL) when
-        it is too small."""
+        it is too small.  With `counts` (frames per stream) quads is [sum(counts), h, w, 4], stream-major, and the batch
+        is ragged (BlobPipeline.submit sends it through cova_pipeline_submit_sparse_ragged)."""
         a = np.ascontiguousarray(quads, dtype=np.uint8)
+        if counts is not None:
+            counts = np.ascontiguousarray(counts, dtype=np.uint32)
+            assert a.ndim == 4 and a.shape[-1] == 4 and counts.ndim == 1 and a.shape[0] == int(counts.sum()), (a.shape, counts)
+            a = a.reshape(1, *a.shape)
         assert a.ndim == 5 and a.shape[-1] == 4, a.shape
         n_streams, fps, h_mb, w_mb = a.shape[:4]
         n_frames = n_streams * fps
@@ -105,6 +112,8 @@ class FramePacker:
         assert out.dtype == np.uint8 and out.flags.c_contiguous
         ln = ctypes.c_size_t()
         check(_lib.load().cova_packer_pack_sparse(self._h, _ptr(a), n_frames, w_mb, h_mb, _ptr(out), out.size, ctypes.byref(ln)))
+        if counts is not None:
+            return SparseBatch(out.reshape(-1)[: ln.value], counts.size, 0, h_mb, w_mb, counts)
         return SparseBatch(out.reshape(-1)[: ln.value], n_streams, fps, h_mb, w_mb)
 
     def close(self):
@@ -437,13 +446,14 @@ class BlobPipeline:
         self._check(self._L.cova_pipeline_n_windows(self._h, n_streams, frames_per_stream, ctypes.byref(n)))
         return n.value
 
-    def _frames(self, frames) -> np.ndarray:
+    def _frames(self, frames, lead: int = 2) -> np.ndarray:
+        # lead: leading dimensions before the frame ([n_streams, frames] or, for ragged batches, [sum(counts)])
         if self.packed_input:
             a = np.ascontiguousarray(frames, dtype=np.uint16)
-            assert a.shape[2:] == (self.h_mb, self.w_mb), a.shape
+            assert a.shape[lead:] == (self.h_mb, self.w_mb), a.shape
         else:
             a = np.ascontiguousarray(frames, dtype=np.uint8)
-            assert a.shape[2:] == (self.h_mb, self.w_mb, 4), a.shape
+            assert a.shape[lead:] == (self.h_mb, self.w_mb, 4), a.shape
         return a
 
     # ---- stages
@@ -510,7 +520,7 @@ class BlobPipeline:
 
     # ---- asynchronous streaming form: at most four batches in flight
     def submit(self, frames: np.ndarray, blob_cap: int | None = None, stream_ids=None, pts=None, cont: bool | None = None,
-               staggered: bool = False):
+               staggered: bool = False, counts=None):
         """Enqueue one batch (copies + kernels) and return immediately.  `frames` should live in page-locked
         memory (PinnedBuffer) and must stay untouched until the matching collect().
 
@@ -520,10 +530,19 @@ class BlobPipeline:
         element would.  staggered=True (with cont=True) lets those streams differ in history and gamma phase: each continues
         from its own state, so chains may yield different numbers of windows (collect(meta=True) maps them to streams).
 
-        `frames` may be a SparseBatch (packed_input pipelines): it goes through cova_pipeline_submit_sparse with the same
-        stream semantics as cova_pipeline_submit_host2."""
+        With `counts` (new frames per stream, each >= 1) the batch is ragged and goes through cova_pipeline_submit_ragged:
+        `frames` is [sum(counts), h, w(, 4)], stream-major, and `pts` is 1-D with one entry per frame; everything else is
+        as above.
+
+        `frames` may be a SparseBatch (packed_input pipelines): it goes through cova_pipeline_submit_sparse (or
+        cova_pipeline_submit_sparse_ragged, when it carries counts) with the same stream semantics as
+        cova_pipeline_submit_host2."""
         if isinstance(frames, SparseBatch):
+            assert counts is None, "a SparseBatch carries its own counts"
             self._submit_sparse(frames, blob_cap, stream_ids, pts, cont, staggered)
+            return
+        if counts is not None:
+            self._submit_ragged(frames, counts, blob_cap, stream_ids, pts, cont, staggered)
             return
         a = self._frames(frames)
         if stream_ids is None and pts is None and cont is None and not staggered:
@@ -541,18 +560,43 @@ class BlobPipeline:
                                                          (_lib.SUBMIT_CONTINUE if cont else 0) | (_lib.SUBMIT_STAGGERED if staggered else 0)))
         self._inflight = getattr(self, "_inflight", []) + [a]
 
+    @staticmethod
+    def _submit_flags(cont, staggered) -> int:
+        return (_lib.SUBMIT_CONTINUE if cont else 0) | (_lib.SUBMIT_STAGGERED if staggered else 0)
+
+    def _submit_ragged(self, frames, counts, blob_cap, stream_ids, pts, cont, staggered):
+        a = self._frames(frames, lead=1)
+        c = np.ascontiguousarray(counts, dtype=np.uint32)
+        assert c.ndim == 1 and a.shape[0] == int(c.sum()), (a.shape, c)
+        # a continued chain can emit one window per new frame
+        self._ensure_out(blob_cap or self._worst_case_cap(int(c.sum())))
+        ids = None if stream_ids is None else np.ascontiguousarray(stream_ids, dtype=np.uint32)
+        p = None if pts is None else np.ascontiguousarray(pts, dtype=np.uint64)
+        assert ids is None or ids.shape == c.shape
+        assert p is None or p.shape == (a.shape[0],)
+        self._check(self._L.cova_pipeline_submit_ragged(self._h, _ptr(a), c.size, _ptr(c), None if ids is None else _ptr(ids),
+                                                        None if p is None else _ptr(p), self._submit_flags(cont, staggered)))
+        self._inflight = getattr(self, "_inflight", []) + [a]
+
     def _submit_sparse(self, b: SparseBatch, blob_cap, stream_ids, pts, cont, staggered):
         assert (b.h_mb, b.w_mb) == (self.h_mb, self.w_mb), (b.h_mb, b.w_mb)
         d = b.data
         assert d.dtype == np.uint8 and d.ndim == 1 and d.flags.c_contiguous
-        self._ensure_out(blob_cap or self._worst_case_cap(b.n_streams * b.frames_per_stream))
+        n_frames = int(b.counts.sum()) if b.counts is not None else b.n_streams * b.frames_per_stream
+        self._ensure_out(blob_cap or self._worst_case_cap(n_frames))
         ids = None if stream_ids is None else np.ascontiguousarray(stream_ids, dtype=np.uint32)
         p = None if pts is None else np.ascontiguousarray(pts, dtype=np.uint64)
         assert ids is None or ids.shape == (b.n_streams,)
-        assert p is None or p.shape == (b.n_streams, b.frames_per_stream)
-        self._check(self._L.cova_pipeline_submit_sparse(self._h, _ptr(d), d.size, b.n_streams, b.frames_per_stream,
-                                                        None if ids is None else _ptr(ids), None if p is None else _ptr(p),
-                                                        (_lib.SUBMIT_CONTINUE if cont else 0) | (_lib.SUBMIT_STAGGERED if staggered else 0)))
+        flags = self._submit_flags(cont, staggered)
+        if b.counts is not None:
+            c = np.ascontiguousarray(b.counts, dtype=np.uint32)
+            assert p is None or p.shape == (n_frames,)
+            self._check(self._L.cova_pipeline_submit_sparse_ragged(self._h, _ptr(d), d.size, b.n_streams, _ptr(c),
+                                                                   None if ids is None else _ptr(ids), None if p is None else _ptr(p), flags))
+        else:
+            assert p is None or p.shape == (b.n_streams, b.frames_per_stream)
+            self._check(self._L.cova_pipeline_submit_sparse(self._h, _ptr(d), d.size, b.n_streams, b.frames_per_stream,
+                                                            None if ids is None else _ptr(ids), None if p is None else _ptr(p), flags))
         self._inflight = getattr(self, "_inflight", []) + [d]
 
     def reset_streams(self, stream_ids=None):

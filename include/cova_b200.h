@@ -198,8 +198,8 @@ int cova_pipeline_collect_host(cova_pipeline *p, uint8_t *blob, size_t blob_cap,
  *          Any other flag bit, or STAGGERED without CONTINUE: COVA_E_INVAL before any device call.
  * Constraints: without COVA_SUBMIT_STAGGERED the streams of one CONTINUED batch must advance in lock-step (same history
  * length min(seen, timestep-1) and same gamma phase) - COVA_E_INVAL otherwise; pass COVA_SUBMIT_STAGGERED to lift this
- * rule.  frames_per_stream is the same for every stream of a call, and frames_per_stream + max_s h_s must fit
- * max_frames_per_stream.  Window order stays stream-major, time-minor.
+ * rule.  frames_per_stream is the same for every stream of a call (cova_pipeline_submit_ragged below lifts this), and
+ * frames_per_stream + max_s h_s must fit max_frames_per_stream.  Window order stays stream-major, time-minor.
  * collect_host2: as collect_host, plus per window the stream id and the PTS of its newest frame (the PTS the
  * reference's metapreprocess output buffer carries, BaseTransform default; cova/imp.rs:110-112 requires it).
  * Both arrays have n_windows entries; win_pts is only written when the submit passed pts. */
@@ -209,6 +209,16 @@ int cova_pipeline_submit_host2(cova_pipeline *p, const uint8_t *frames, uint32_t
                                const uint32_t *stream_ids, const uint64_t *pts, uint32_t flags);
 int cova_pipeline_collect_host2(cova_pipeline *p, uint8_t *blob, size_t blob_cap, size_t *blob_len, uint64_t *offsets,
                                 uint64_t *lens, uint32_t *n_windows, uint32_t *win_stream_ids, uint64_t *win_pts);
+/* As cova_pipeline_submit_host2, but stream s brings n_frames[s] >= 1 new frames (GoP shards of different lengths, live
+ * flushes with a different frame count per camera).  frames = the sum of n_frames[] frames, stream-major and time-minor,
+ * without gaps, in the pipeline's input format (quads, or u16 with COVA_FLAG_INPUT_PACKED16); pts (optional) has one entry
+ * per frame in the same order.  Stream ids, COVA_SUBMIT_CONTINUE / _STAGGERED, the lock-step rule without STAGGERED, PTS
+ * echo and collect_host2 are exactly submit_host2's.  Chain s yields exactly the windows its uncut stream yields for its
+ * n_frames[s] frames.  Bound: lead + max_s n_frames[s] <= max_frames_per_stream, where lead is the longest carried
+ * history of the batch (with equal counts this is submit_host2's rule).  COVA_E_INVAL before any device call: n_frames
+ * NULL, a count of 0, the bound broken, and everything submit_host2 refuses. */
+int cova_pipeline_submit_ragged(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, const uint32_t *n_frames,
+                                const uint32_t *stream_ids, const uint64_t *pts, uint32_t flags);
 /* forget the state of the given streams (NULL = all): their next CONTINUED batch starts with an empty window */
 int cova_pipeline_reset_streams(cova_pipeline *p, const uint32_t *stream_ids, uint32_t n);
 
@@ -244,6 +254,11 @@ int cova_packer_pack_sparse(cova_packer *pk, const uint8_t *quads, uint32_t n_fr
  * data_len - and a malformed batch is COVA_E_INVAL with nothing in flight.  data must stay valid until the collect. */
 int cova_pipeline_submit_sparse(cova_pipeline *p, const uint8_t *data, size_t data_len, uint32_t n_streams,
                                 uint32_t frames_per_stream, const uint32_t *stream_ids, const uint64_t *pts, uint32_t flags);
+/* cova_pipeline_submit_ragged with the frames as a sparse batch of data_len bytes: the records of sum(n_frames) frames in
+ * the same order, checked as submit_sparse checks them (data_len must end exactly at the last record). */
+int cova_pipeline_submit_sparse_ragged(cova_pipeline *p, const uint8_t *data, size_t data_len, uint32_t n_streams,
+                                       const uint32_t *n_frames, const uint32_t *stream_ids, const uint64_t *pts,
+                                       uint32_t flags);
 
 /* feed a mask batch straight to the CCL stage (u8 [n][h_mb][w_mb]; is_device as above) */
 int cova_pipeline_load_masks(cova_pipeline *p, const uint8_t *masks, uint32_t n, int is_device);
