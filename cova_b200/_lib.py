@@ -86,6 +86,8 @@ SIGNATURES = {
     "cova_pipeline_submit_host2": (ctypes.c_int, [_vp, _vp, ctypes.c_uint32, ctypes.c_uint32, _vp, _vp, ctypes.c_uint32]),
     "cova_pipeline_collect_host2": (ctypes.c_int, [_vp, _vp, ctypes.c_size_t, _szp, _vp, _vp, _u32p, _vp, _vp]),
     "cova_pipeline_reset_streams": (ctypes.c_int, [_vp, _vp, ctypes.c_uint32]),
+    "cova_pipeline_set_stream_property": (ctypes.c_int, [_vp, _vp, ctypes.c_uint32, ctypes.c_char_p, ctypes.c_uint32]),
+    "cova_pipeline_get_stream_property": (ctypes.c_int, [_vp, ctypes.c_uint32, ctypes.c_char_p, _u32p]),
     "cova_packer_new": (ctypes.c_int, [_vpp, ctypes.c_uint32]),
     "cova_packer_free": (None, [_vp]),
     "cova_packer_pack": (ctypes.c_int, [_vp, _vp, _vp, ctypes.c_size_t]),

@@ -36,8 +36,9 @@ struct Enc1Extra {
     // per chain of the chunk: (x = index of the newest frame of its first window, y = index of that window in the chunk,
     // z = end: the chain's frames are [0, end), w = frames of the chunk's chains before it, sum of their ends).  Chains of a
     // staggered batch differ in x and y, chains of a ragged batch in z (cova_abi.cu, set_batch_shape); a chain's window
-    // n + k has its newest frame at x + k * gamma
+    // n + k has its newest frame at x + k * gamma, with the chain's own gamma when `gam` is given
     const int4 *tab;
+    const int *gam;                         // per chain of the chunk: its gamma (nullptr: every chain has `gamma`)
     int ntp;                                // tile pairs per frame
     int n_items;                            // (chain, tile pair) items = n_chains * ntp, item (c, j) is end_c frame steps long
     int full_items;                         // items handed out whole, round-robin: a multiple of the grid size
@@ -208,6 +209,7 @@ __global__ void __launch_bounds__(kThreads1, 1) enc1_fused_kernel(const __grid_c
             const long long base_s = (long long)((p.out2_cb + cg) * 4 + pho) * p.gout2.Lp + p.gout2.guard + (long long)(Y >> 1) * p.gout2.P + (X >> 1) +
                                    (long long)cw.y * p.gout2.S;
             const int first = cw.x;
+            const int gam = ex.gam ? __ldg(&ex.gam[w.chain]) : ex.gamma;
             // Ring of the last four pooled frames: ring[s][k] = channel pair (2k, 2k+1) of the frame whose index is s mod 4,
             // as fp32 values already rounded to fp16 (the pooled activation is an fp16 tensor).  The frame loop is
             // unrolled four times over the ring phase R, so "frame i - t" is the compile-time slot (R - t) & 3: no
@@ -257,9 +259,9 @@ __global__ void __launch_bounds__(kThreads1, 1) enc1_fused_kernel(const __grid_c
                     }
                 }
                 const int rel = i - first;
-                const bool emit = i >= w.i0 && rel >= 0 && (ex.gamma == 1 || rel % ex.gamma == 0);   // warp-uniform
+                const bool emit = i >= w.i0 && rel >= 0 && (gam == 1 || rel % gam == 0);   // warp-uniform
                 if (emit && valid) {
-                    const long long n = ex.gamma == 1 ? rel : rel / ex.gamma;           // window of the chain
+                    const long long n = gam == 1 ? rel : rel / gam;                     // window of the chain
                     uint32_t o32[4][4];
 #pragma unroll
                     for (int k = 0; k < 4; k++) {                        // channel pair (2k, 2k+1) in the two packed fp32 lanes

@@ -26,6 +26,7 @@ struct CclArgs {
     const uint8_t *masks;     // [n][H][W]
     int H, W, nbx, nby;       // nbx = ceil(W/2), nby = ceil(H/2)
     int area_thresh;          // u32 property reinterpreted as i32 like imp.rs:248
+    const int *thresh;        // optional [n]: per-mask area_thresh (a batch whose streams have their own cc-threshold)
     uint8_t *blob;            // bincode output arena
     unsigned long long blob_cap;
     unsigned long long *cursor;   // [0] bytes reserved so far, [1] overflow flag
@@ -402,6 +403,7 @@ __global__ void ccl_bbox_kernel(CclArgs A) {
     pdl_launch_dependents();
     pdl_wait();              // the mask comes from the preceding kernel of the stream (common.cuh, "Programmatic dependent launch")
     const uint8_t *m = A.masks + (size_t)frame * A.H * A.W;
+    const int thresh = A.thresh ? __ldg(A.thresh + frame) : A.area_thresh;
 
     unsigned short *my_list;
     const int n_fg = ccl_codes_and_merge<COMPACT>(A, M, m, nb, my_list);
@@ -448,7 +450,7 @@ __global__ void ccl_bbox_kernel(CclArgs A) {
     const int b0 = min(tid * ipt, nb), b1 = min(b0 + ipt, nb);
     int cnt = 0;
     for (int b = b0; b < b1; b++)
-        if ((int)M.parent[b] == b) cnt += 0x10000 + (M.stat_area(b) >= A.area_thresh ? 1 : 0);
+        if ((int)M.parent[b] == b) cnt += 0x10000 + (M.stat_area(b) >= thresh ? 1 : 0);
     int incl = cnt;
     const int wid = tid >> 5;
 #pragma unroll
@@ -503,7 +505,7 @@ __global__ void ccl_bbox_kernel(CclArgs A) {
             int32_t *s5 = st + (size_t)rank_all * 5;
             s5[0] = x0; s5[1] = y0; s5[2] = w; s5[3] = h; s5[4] = ar;
         }
-        if (ar >= A.area_thresh) {
+        if (ar >= thresh) {
             if (fits) {
                 uint32_t *rec = reinterpret_cast<uint32_t *>(A.blob + off + 8 + 24ull * rank_keep);
                 float fw = (float)w, fh = (float)h;
@@ -631,6 +633,7 @@ __global__ void ccl_cluster_kernel(const __grid_constant__ CclClusterArgs C) {
     pdl_launch_dependents();
     pdl_wait();
     const uint8_t *m = A.masks + (size_t)frame * C.H * A.W + (size_t)2 * row0 * A.W;
+    const int thresh = A.thresh ? __ldg(A.thresh + frame) : A.area_thresh;
 
     // 1-2. codes, runs and merge inside the band, on band-local indices (in-band links never leave the band)
     unsigned short *my_list;
@@ -689,7 +692,7 @@ __global__ void ccl_cluster_kernel(const __grid_constant__ CclClusterArgs C) {
     const int b0 = min(tid * ipt, nb), b1 = min(b0 + ipt, nb);
     int cnt = 0;
     for (int b = b0; b < b1; b++)
-        if (M.parent[b] == off + b) cnt += 0x10000 + (M.stat[5 * b + 4] >= A.area_thresh ? 1 : 0);
+        if (M.parent[b] == off + b) cnt += 0x10000 + (M.stat[5 * b + 4] >= thresh ? 1 : 0);
     int incl = cnt;
     const int wid = tid >> 5;
 #pragma unroll
@@ -752,7 +755,7 @@ __global__ void ccl_cluster_kernel(const __grid_constant__ CclClusterArgs C) {
             int32_t *s5 = st + (size_t)rank_all * 5;
             s5[0] = x0; s5[1] = y0; s5[2] = w; s5[3] = h; s5[4] = ar;
         }
-        if (ar >= A.area_thresh) {
+        if (ar >= thresh) {
             if (fits) {
                 uint32_t *rec = reinterpret_cast<uint32_t *>(A.blob + off_out + 8 + 24ull * rank_keep);
                 float fw = (float)w, fh = (float)h;

@@ -345,12 +345,14 @@ static void ccl_grid_args(CclArgs &a, int nby, int threads) {
     a.div_tile_rows = make_fastdiv((uint32_t)std::max(2, a.tile_rows));
 }
 
+// d_thresh: optional per-mask thresholds of masks [0, first + n) (i32, like cc_threshold), nullptr = cc_threshold for all
 static int ccl_launch(CclBuffers &b, const uint8_t *d_masks, int n, uint32_t cc_threshold, bool want_labels, cudaStream_t st,
-                      size_t first = 0, bool reset_cursor = true, bool pdl = true) {
+                      size_t first = 0, bool reset_cursor = true, bool pdl = true, const int *d_thresh = nullptr) {
     if (n <= 0) return COVA_OK;
     CclArgs a;
     a.masks = d_masks + first * (size_t)b.H * b.W; a.H = b.H; a.W = b.W; a.nbx = b.nbx;
     a.area_thresh = (int)cc_threshold;   // `settings.cc_threshold as i32` (imp.rs:248)
+    a.thresh = d_thresh ? d_thresh + first : nullptr;
     a.blob = b.d_blob; a.blob_cap = b.blob_cap; a.cursor = b.d_cursor; a.offsets = b.d_offsets + first; a.lens = b.d_lens + first;
     a.labels = want_labels ? b.d_labels : nullptr;
     a.stats = want_labels ? b.d_stats : nullptr;
@@ -510,8 +512,15 @@ struct cova_pipeline {
     // stream): the last T - 1 frames of every stream id on the device, frames seen so far on the host
     uint8_t *d_carry = nullptr;
     std::vector<uint64_t> n_seen, id_mark;
+    std::vector<uint32_t> gamma_idx;     // per stream id: the element's countdown to its next window (imp.rs:321-330)
     uint64_t id_epoch = 0;
+    // Per-stream element properties (cova_pipeline_set_stream_property), by stream id: gamma (0 = the creation gamma) and
+    // cc-threshold (used when thr_set; the pipeline's cc_threshold otherwise).  Read by the submits that name streams.
+    std::vector<uint32_t> s_gamma, s_thr;
+    std::vector<uint8_t> s_thr_set;
     std::vector<uint32_t> first_scratch, hist_scratch;   // per chain of the batch being submitted
+    std::vector<uint32_t> gam_scratch, thr_scratch;      // gamma and cc-threshold per chain of the batch being submitted
+    std::vector<uint32_t> cd_scratch;                    // countdown per chain after the batch being submitted
     std::vector<uint32_t> count_scratch;                 // new frames per chain of the batch being submitted
     std::vector<uint64_t> off_scratch;                   // record offsets of the sparse batch being submitted
     // A batch is processed in chunks of whole chains: the activation buffers are sized for ONE chunk, and
@@ -550,8 +559,15 @@ struct cova_pipeline {
         int4 *h_tab = nullptr, *d_tab = nullptr;
         int *h_newest = nullptr, *d_newest = nullptr;
         int *h_fmap = nullptr, *d_fmap = nullptr;      // allocated on the slot's first ragged batch
+        // per-stream properties (set_stream_property), allocated on the slot's first batch that needs them:
+        //   gam[s]  = chain s's gamma, when some chain's differs from the creation gamma     read by enc1_fused_kernel
+        //   thr[w]  = window w's cc-threshold, when some differs from the pipeline's value   read by the CCL kernels
+        int *h_gam = nullptr, *d_gam = nullptr;
+        int *h_thr = nullptr, *d_thr = nullptr;
+        bool gam_on = false, thr_on = false;           // the batch in the slot uses gam / thr
         cudaEvent_t ev_tab = nullptr;                  // recorded after the upload: the staging may be rewritten after it
-        std::vector<uint32_t> tab_first, tab_end;      // what the tables hold: per-chain first and end, stride, stream
+        std::vector<uint32_t> tab_first, tab_end;      // what the tables hold: per-chain first and end, stride, stream,
+        std::vector<uint32_t> tab_gam, tab_thr;        // per-chain gamma, per-chain threshold (empty: thr not uploaded)
         uint32_t tab_fps = 0;
         cudaStream_t tab_stream = nullptr;
         // sparse input (cova_pipeline_submit_sparse), allocated on the slot's first sparse submit: the batch's records at
@@ -680,6 +696,7 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
     p->max_streams = max_streams; p->max_fps = max_fps; p->flags = flags; p->impl = flags & 0xffu;
     p->cc_threshold = cc_threshold;
     p->max_windows = max_windows;
+    p->s_gamma.assign(max_streams, 0); p->s_thr.assign(max_streams, 0); p->s_thr_set.assign(max_streams, 0);
     auto fail = [&](int code) { cova_pipeline_free(p); return code; };
     if ((rc = parse_weights(weights, weights_len, p->hw))) return fail(rc);
     cudaDeviceProp prop;
@@ -791,6 +808,10 @@ extern "C" void cova_pipeline_free(cova_pipeline *p) {
         if (sl.d_newest) cudaFree(sl.d_newest);
         if (sl.h_fmap) cudaFreeHost(sl.h_fmap);
         if (sl.d_fmap) cudaFree(sl.d_fmap);
+        if (sl.h_gam) cudaFreeHost(sl.h_gam);
+        if (sl.d_gam) cudaFree(sl.d_gam);
+        if (sl.h_thr) cudaFreeHost(sl.h_thr);
+        if (sl.d_thr) cudaFree(sl.d_thr);
         if (sl.ev_tab) cudaEventDestroy(sl.ev_tab);
         if (sl.d_sparse) cudaFree(sl.d_sparse);
         if (sl.h_off) cudaFreeHost(sl.h_off);
@@ -839,51 +860,75 @@ static int check_batch_bounds(const cova_pipeline *p, uint32_t n_streams, uint32
 // Window shape of a batch of n_streams device chains of stride fps, into slot k.  first[s] is the index (inside device
 // chain s) of the newest frame of the chain's first window; nullptr = T - 1 for every chain, i.e. chains that start with
 // an empty window.  CONTINUED chains (submit_host2) start later, where their carried history and gamma phase put them.
-// end[s] is where chain s's frames end (ragged batches); nullptr = fps for every chain.  Lock-step, staggered and ragged
-// batches go through the same tables and kernels.
+// end[s] is where chain s's frames end (ragged batches); nullptr = fps for every chain.  gam[s] is chain s's gamma, nullptr
+// = the creation gamma for every chain; thr[s] is chain s's cc-threshold, nullptr = the pipeline's value at CCL launch
+// (stream properties, cova_pipeline_set_stream_property).  Lock-step, staggered, ragged and mixed-property batches go
+// through the same tables and kernels.
 static int set_batch_shape(cova_pipeline *p, int k, uint32_t n_streams, uint32_t fps, const uint32_t *first = nullptr,
-                           const uint32_t *end = nullptr) {
+                           const uint32_t *end = nullptr, const uint32_t *gam = nullptr, const uint32_t *thr = nullptr) {
     auto &sl = p->slot[k];
     const uint32_t t1 = p->T - 1, cs = p->chunk_streams;
     auto first_of = [&](uint32_t s) { return first ? first[s] : t1; };
     auto end_of = [&](uint32_t s) { return end ? end[s] : fps; };
+    auto gam_of = [&](uint32_t s) { return gam ? gam[s] : p->gamma; };
     uint64_t total = 0;
-    for (uint32_t s = 0; s < n_streams; s++) total += windows_from(end_of(s), first_of(s), p->gamma);
+    for (uint32_t s = 0; s < n_streams; s++) total += windows_from(end_of(s), first_of(s), gam_of(s));
     if (total > p->max_windows) return set_err(COVA_E_INVAL, "batch produces more windows than the pipeline was sized for");
     sl.win0.resize(n_streams + 1);
     sl.fpre.resize(n_streams + 1);
     sl.win0[0] = 0; sl.fpre[0] = 0;
     sl.ragged = false;
+    sl.gam_on = false;
     for (uint32_t s = 0; s < n_streams; s++) {
-        sl.win0[s + 1] = sl.win0[s] + windows_from(end_of(s), first_of(s), p->gamma);
+        sl.win0[s + 1] = sl.win0[s] + windows_from(end_of(s), first_of(s), gam_of(s));
         sl.fpre[s + 1] = sl.fpre[s] + end_of(s);
         sl.ragged = sl.ragged || end_of(s) != fps;
+        sl.gam_on = sl.gam_on || gam_of(s) != p->gamma;
     }
+    sl.thr_on = thr != nullptr;
     sl.n_streams = n_streams; sl.fps = fps; sl.n_windows = (uint32_t)total;
-    bool same = sl.tab_fps == fps && sl.tab_stream == p->stream && sl.tab_first.size() == n_streams;
-    for (uint32_t s = 0; same && s < n_streams; s++) same = sl.tab_first[s] == first_of(s) && sl.tab_end[s] == end_of(s);
+    bool same = sl.tab_fps == fps && sl.tab_stream == p->stream && sl.tab_first.size() == n_streams &&
+                sl.tab_thr.size() == (thr ? n_streams : 0);
+    for (uint32_t s = 0; same && s < n_streams; s++)
+        same = sl.tab_first[s] == first_of(s) && sl.tab_end[s] == end_of(s) && sl.tab_gam[s] == gam_of(s) && (!thr || sl.tab_thr[s] == thr[s]);
     if (same) return COVA_OK;                                      // the slot's device tables already hold this shape
     if (sl.ragged && !sl.h_fmap) {
         COVA_CUDA(cudaMallocHost(&sl.h_fmap, sizeof(int) * (size_t)p->max_streams * p->max_fps));
         COVA_CUDA(cudaMalloc(&sl.d_fmap, sizeof(int) * (size_t)p->max_streams * p->max_fps));
     }
+    if (sl.gam_on && !sl.h_gam) {
+        COVA_CUDA(cudaMallocHost(&sl.h_gam, sizeof(int) * p->max_streams));
+        COVA_CUDA(cudaMalloc(&sl.d_gam, sizeof(int) * p->max_streams));
+    }
+    if (thr && !sl.h_thr) {
+        COVA_CUDA(cudaMallocHost(&sl.h_thr, sizeof(int) * std::max<size_t>(1, p->max_windows)));
+        COVA_CUDA(cudaMalloc(&sl.d_thr, sizeof(int) * std::max<size_t>(1, p->max_windows)));
+    }
     // The staging may still be read by this slot's previous upload when synchronous entry points reuse slot 0 back to back.
     // On the submit path that upload has completed: the slot's previous batch was collected.
     COVA_CUDA(cudaEventSynchronize(sl.ev_tab));
-    sl.tab_first.clear(); sl.tab_end.clear();                      // invalid until the upload below is enqueued
+    sl.tab_first.clear(); sl.tab_end.clear(); sl.tab_gam.clear(); sl.tab_thr.clear();   // invalid until the upload below is enqueued
     for (uint32_t s = 0; s < n_streams; s++) {
         const uint32_t f = first_of(s), c0 = s / cs * cs;
         sl.h_tab[s] = make_int4((int)f, (int)(sl.win0[s] - sl.win0[c0]), (int)end_of(s), (int)(sl.fpre[s] - sl.fpre[c0]));
-        for (uint32_t w = sl.win0[s]; w < sl.win0[s + 1]; w++)
-            sl.h_newest[w] = (int)((s - c0) * fps + f + (w - sl.win0[s]) * p->gamma);
+        if (sl.gam_on) sl.h_gam[s] = (int)gam_of(s);
+        for (uint32_t w = sl.win0[s]; w < sl.win0[s + 1]; w++) {
+            sl.h_newest[w] = (int)((s - c0) * fps + f + (w - sl.win0[s]) * gam_of(s));
+            if (thr) sl.h_thr[w] = (int)thr[s];                    // `cc_threshold as i32` (bboxcc/imp.rs:248)
+        }
         if (sl.ragged)
             for (uint32_t i = 0; i < end_of(s); i++) sl.h_fmap[sl.fpre[s] + i] = (int)((s - c0) * fps + i);
     }
     COVA_CUDA(cudaMemcpyAsync(sl.d_tab, sl.h_tab, sizeof(int4) * n_streams, cudaMemcpyHostToDevice, p->stream));
     if (total) COVA_CUDA(cudaMemcpyAsync(sl.d_newest, sl.h_newest, sizeof(int) * total, cudaMemcpyHostToDevice, p->stream));
     if (sl.ragged) COVA_CUDA(cudaMemcpyAsync(sl.d_fmap, sl.h_fmap, sizeof(int) * sl.fpre[n_streams], cudaMemcpyHostToDevice, p->stream));
+    if (sl.gam_on) COVA_CUDA(cudaMemcpyAsync(sl.d_gam, sl.h_gam, sizeof(int) * n_streams, cudaMemcpyHostToDevice, p->stream));
+    if (thr && total) COVA_CUDA(cudaMemcpyAsync(sl.d_thr, sl.h_thr, sizeof(int) * total, cudaMemcpyHostToDevice, p->stream));
     COVA_CUDA(cudaEventRecord(sl.ev_tab, p->stream));
-    for (uint32_t s = 0; s < n_streams; s++) { sl.tab_first.push_back(first_of(s)); sl.tab_end.push_back(end_of(s)); }
+    for (uint32_t s = 0; s < n_streams; s++) {
+        sl.tab_first.push_back(first_of(s)); sl.tab_end.push_back(end_of(s)); sl.tab_gam.push_back(gam_of(s));
+        if (thr) sl.tab_thr.push_back(thr[s]);
+    }
     sl.tab_fps = fps; sl.tab_stream = p->stream;
     return COVA_OK;
 }
@@ -931,7 +976,7 @@ extern "C" int cova_pipeline_load_masks(cova_pipeline *p, const uint8_t *masks, 
     if (!n || n > p->max_windows) return set_err(COVA_E_INVAL, "mask batch exceeds the pipeline's window capacity");
     if (int rc = require_idle(p)) return rc;
     COVA_CUDA(cudaSetDevice(p->device));
-    p->slot[0].n_streams = 0; p->slot[0].n_windows = n;
+    p->slot[0].n_streams = 0; p->slot[0].n_windows = n; p->slot[0].thr_on = false;
     p->last_slot = 0;
     COVA_CUDA(cudaMemcpyAsync(p->d_mask, masks, (size_t)n * p->W * p->H, is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, p->stream));
     return COVA_OK;
@@ -1262,6 +1307,7 @@ static int tc_launch(cova_pipeline *p, const Slot &sl, const Chunk &ck, int laye
         if (i == 0) {
             lp.in = p->x0f;
             pl.ex.tab = sl.d_tab + ck.stream0;
+            pl.ex.gam = sl.gam_on ? sl.d_gam + ck.stream0 : nullptr;
         }
     } else {
         const int i = layer - 4;
@@ -1326,7 +1372,8 @@ extern "C" int cova_pipeline_blobnet(cova_pipeline *p) {
 }
 
 static int ccl_range(cova_pipeline *p, Slot &sl, size_t first, int n, bool reset_cursor) {
-    int rc = ccl_launch(sl.ccl, p->d_mask, n, p->cc_threshold, false, p->stream, first, reset_cursor, !(p->dbg & kDbgNoPdl));
+    int rc = ccl_launch(sl.ccl, p->d_mask, n, p->cc_threshold, false, p->stream, first, reset_cursor, !(p->dbg & kDbgNoPdl),
+                        sl.thr_on ? sl.d_thr : nullptr);
     if (rc) return rc;
     if (n > 0) {
         p->launches++;
@@ -1480,8 +1527,9 @@ __global__ void __launch_bounds__(256) carry_kernel(uint32_t *__restrict__ pool,
 // set-up, one copy stage and one compute stage, which for equal counts enqueue exactly what they always did.
 
 // Argument checks and per-chain plan of a submit, before any device call: fills count_scratch (n_s: `counts`, or fps for
-// every chain when counts is nullptr), first_scratch, hist_scratch and off_scratch, and raises lead (0 on entry) to the
-// longest carried history
+// every chain when counts is nullptr), first_scratch, hist_scratch and off_scratch, for stream batches also gam_scratch,
+// thr_scratch (the streams' properties now) and cd_scratch (their countdowns after the batch), and raises lead (0 on entry)
+// to the longest carried history
 static int plan_submit(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, uint32_t fps, const uint32_t *counts,
                        const uint32_t *stream_ids, uint32_t flags, bool stateful, const size_t *sparse_len, uint32_t &lead) {
     if (flags & ~(COVA_SUBMIT_CONTINUE | COVA_SUBMIT_STAGGERED)) return set_err(COVA_E_INVAL, "unknown submit flag");
@@ -1518,25 +1566,40 @@ static int plan_submit(cova_pipeline *p, const uint8_t *frames, uint32_t n_strea
     hist.assign(n_streams, 0);
     if (stateful) {
         if (!max_n) return set_err(COVA_E_INVAL, "a stream batch needs at least one frame per stream");
-        if (p->n_seen.empty()) { p->n_seen.assign(p->max_streams, 0); p->id_mark.assign(p->max_streams, 0); }
+        if (p->n_seen.empty()) {
+            p->n_seen.assign(p->max_streams, 0); p->id_mark.assign(p->max_streams, 0); p->gamma_idx.assign(p->max_streams, 0);
+        }
         p->id_epoch++;                                              // "seen in this batch" marks without clearing the array
+        std::vector<uint32_t> &gam = p->gam_scratch, &thr = p->thr_scratch, &cd = p->cd_scratch;
+        gam.resize(n_streams); thr.resize(n_streams); cd.resize(n_streams);
         for (uint32_t s = 0; s < n_streams; s++) {
             const uint32_t id = stream_ids ? stream_ids[s] : s;
             if (id >= p->max_streams) return set_err(COVA_E_INVAL, "stream id out of range (ids are 0 .. max_streams-1)");
             if (p->id_mark[id] == p->id_epoch) return set_err(COVA_E_INVAL, "a stream id appears twice in one batch");
             p->id_mark[id] = p->id_epoch;
-            if (!(flags & COVA_SUBMIT_CONTINUE)) continue;
-            const uint64_t seen = p->n_seen[id];
-            const uint32_t hs = (uint32_t)std::min<uint64_t>(seen, t1);
-            const uint64_t base = seen - hs;                        // frames of the stream in front of its carried ones
-            // smallest index i' >= T-1 of the unpadded chain with (base + i' - (T-1)) % gamma == 0 (imp.rs:321-330)
+            gam[s] = p->s_gamma[id] ? p->s_gamma[id] : p->gamma;
+            thr[s] = p->s_thr_set[id] ? p->s_thr[id] : p->cc_threshold;
+            // In the unpadded chain (hs carried frames, then the new ones) index T-1 is the first new frame whose window is
+            // full; from there the element emits when its countdown gamma_idx is 0 and then restarts it at gamma - 1
+            // (imp.rs:321-330).  A fresh chain starts with an empty window and a countdown of 0.
+            uint32_t hs = 0, idx = 0;
+            if (flags & COVA_SUBMIT_CONTINUE) {
+                hs = (uint32_t)std::min<uint64_t>(p->n_seen[id], t1);
+                idx = p->gamma_idx[id];
+            }
             hist[s] = hs;
-            first[s] = t1 + (uint32_t)((p->gamma - base % p->gamma) % p->gamma);
+            first[s] = t1 + idx;
+            // countdown after the batch: the next emitting index past the chain's end (hs + n_s), less the frames from
+            // T-1 on that the batch brings
+            const uint32_t e = hs + p->count_scratch[s];
+            cd[s] = first[s] + windows_from(e, first[s], gam[s]) * gam[s] - std::max(e, t1);
             lead = std::max(lead, hs);
-            // without COVA_SUBMIT_STAGGERED the streams of a batch advance in lock-step: same history, same gamma phase
-            if (!(flags & COVA_SUBMIT_STAGGERED) && s && (hs != hist[0] || first[s] != first[0]))
-                return set_err(COVA_E_INVAL, "streams of one CONTINUED batch must have the same history length and gamma phase "
-                                             "(or pass COVA_SUBMIT_STAGGERED)");
+            // without COVA_SUBMIT_STAGGERED the streams of a CONTINUED batch advance in lock-step: same history, countdown
+            // and gamma
+            if ((flags & COVA_SUBMIT_CONTINUE) && !(flags & COVA_SUBMIT_STAGGERED) && s &&
+                (hs != hist[0] || first[s] != first[0] || gam[s] != gam[0]))
+                return set_err(COVA_E_INVAL, "streams of one CONTINUED batch must have the same history length, gamma countdown "
+                                             "and gamma (or pass COVA_SUBMIT_STAGGERED)");
         }
         for (uint32_t s = 0; s < n_streams; s++) first[s] += lead - hist[s];   // chain s is padded by lead - h_s frames
     }
@@ -1580,11 +1643,18 @@ static int setup_slot(cova_pipeline *p, int k, uint32_t n_streams, uint32_t lead
         end[s] = lead + cnt[s];
         sl.npre[s + 1] = sl.npre[s] + cnt[s];
     }
-    if ((rc = set_batch_shape(p, k, n_streams, max_n + lead, first.data(), end.data()))) return rc;
+    // stream properties: a table only for a batch that does not run entirely on the pipeline's values
+    const uint32_t *gam = nullptr, *thr = nullptr;
+    for (uint32_t s = 0; stateful && s < n_streams; s++) {
+        if (p->gam_scratch[s] != p->gamma) gam = p->gam_scratch.data();
+        if (p->thr_scratch[s] != p->cc_threshold) thr = p->thr_scratch.data();
+    }
+    if ((rc = set_batch_shape(p, k, n_streams, max_n + lead, first.data(), end.data(), gam, thr))) return rc;
     p->last_slot = k;
     sl.win_pts.clear(); sl.win_ids.clear();
     if (stateful) {
-        // window w of chain s has its newest frame at device index first_s + w*gamma = new-frame index first_s + w*gamma - lead
+        // window w of chain s has its newest frame at device index first_s + w*gamma_s = new-frame index
+        // first_s + w*gamma_s - lead
         sl.win_ids.resize(sl.n_windows);
         if (pts) sl.win_pts.resize(sl.n_windows);
         for (uint32_t s = 0; s < n_streams; s++) {
@@ -1592,9 +1662,10 @@ static int setup_slot(cova_pipeline *p, int k, uint32_t n_streams, uint32_t lead
             sl.h_ids[s] = id;
             for (uint32_t w = sl.win0[s]; w < sl.win0[s + 1]; w++) {
                 sl.win_ids[w] = id;
-                if (pts) sl.win_pts[w] = pts[sl.npre[s] + (first[s] + (w - sl.win0[s]) * p->gamma - lead)];
+                if (pts) sl.win_pts[w] = pts[sl.npre[s] + (first[s] + (w - sl.win0[s]) * p->gam_scratch[s] - lead)];
             }
             p->n_seen[id] = ((flags & COVA_SUBMIT_CONTINUE) ? p->n_seen[id] : 0) + cnt[s];
+            p->gamma_idx[id] = p->cd_scratch[s];
         }
     }
     return COVA_OK;
@@ -1726,11 +1797,48 @@ extern "C" int cova_pipeline_submit_sparse_ragged(cova_pipeline *p, const uint8_
 extern "C" int cova_pipeline_reset_streams(cova_pipeline *p, const uint32_t *stream_ids, uint32_t n) {
     if (!p) return set_err(COVA_E_INVAL, "null handle");
     if (p->n_seen.empty()) return COVA_OK;
-    if (!stream_ids) { std::fill(p->n_seen.begin(), p->n_seen.end(), 0); return COVA_OK; }
+    if (!stream_ids) {
+        std::fill(p->n_seen.begin(), p->n_seen.end(), 0);
+        std::fill(p->gamma_idx.begin(), p->gamma_idx.end(), 0);
+        return COVA_OK;
+    }
     for (uint32_t i = 0; i < n; i++) {
         if (stream_ids[i] >= p->max_streams) return set_err(COVA_E_INVAL, "stream id out of range");
         p->n_seen[stream_ids[i]] = 0;
+        p->gamma_idx[stream_ids[i]] = 0;
     }
+    return COVA_OK;
+}
+
+// 0: "gamma", 1: "cc-threshold", -1: no such stream property
+static int stream_property(const char *name) {
+    return !strcmp(name, "gamma") ? 0 : !strcmp(name, "cc-threshold") ? 1 : -1;
+}
+extern "C" int cova_pipeline_set_stream_property(cova_pipeline *p, const uint32_t *stream_ids, uint32_t n, const char *name,
+                                                 uint32_t value) {
+    if (!p || !name) return set_err(COVA_E_INVAL, "null argument");
+    const int prop = stream_property(name);
+    if (prop < 0) return set_err(COVA_E_INVAL, "unknown stream property (\"gamma\" or \"cc-threshold\")");
+    if (prop == 0 && value < 1) return set_err(COVA_E_INVAL, "gamma is a u32 >= 1");
+    // the window buffers and the max_windows bound were sized for the creation gamma; a larger one yields fewer windows
+    if (prop == 0 && value < p->gamma) return set_err(COVA_E_INVAL, "a stream's gamma cannot be below the pipeline's creation gamma");
+    const uint32_t m = stream_ids ? n : p->max_streams;
+    for (uint32_t i = 0; stream_ids && i < m; i++)                 // the whole list before anything changes
+        if (stream_ids[i] >= p->max_streams) return set_err(COVA_E_INVAL, "stream id out of range (ids are 0 .. max_streams-1)");
+    for (uint32_t i = 0; i < m; i++) {
+        const uint32_t id = stream_ids ? stream_ids[i] : i;
+        if (prop == 0) p->s_gamma[id] = value;
+        else { p->s_thr[id] = value; p->s_thr_set[id] = 1; }
+    }
+    return COVA_OK;
+}
+extern "C" int cova_pipeline_get_stream_property(const cova_pipeline *p, uint32_t stream_id, const char *name, uint32_t *value) {
+    if (!p || !name || !value) return set_err(COVA_E_INVAL, "null argument");
+    const int prop = stream_property(name);
+    if (prop < 0) return set_err(COVA_E_INVAL, "unknown stream property (\"gamma\" or \"cc-threshold\")");
+    if (stream_id >= p->max_streams) return set_err(COVA_E_INVAL, "stream id out of range (ids are 0 .. max_streams-1)");
+    if (prop == 0) *value = p->s_gamma[stream_id] ? p->s_gamma[stream_id] : p->gamma;
+    else *value = p->s_thr_set[stream_id] ? p->s_thr[stream_id] : p->cc_threshold;
     return COVA_OK;
 }
 

@@ -606,6 +606,19 @@ class BlobPipeline:
             ids = np.ascontiguousarray(stream_ids, dtype=np.uint32)
             self._check(self._L.cova_pipeline_reset_streams(self._h, _ptr(ids), ids.size))
 
+    def set_stream_property(self, name: str, value: int, stream_ids=None):
+        """cova_pipeline_set_stream_property: "gamma" (>= the creation gamma) or "cc-threshold" of the given stream ids
+        (None = every stream), used by the submits that name streams from the next one on."""
+        ids = None if stream_ids is None else np.ascontiguousarray(stream_ids, dtype=np.uint32).reshape(-1)
+        self._check(self._L.cova_pipeline_set_stream_property(self._h, None if ids is None else _ptr(ids),
+                                                              0 if ids is None else ids.size, name.encode(), value))
+
+    def get_stream_property(self, name: str, stream_id: int) -> int:
+        """The value a batch submitted now would use for this stream (its own, or the pipeline's)."""
+        v = ctypes.c_uint32()
+        self._check(self._L.cova_pipeline_get_stream_property(self._h, stream_id, name.encode(), ctypes.byref(v)))
+        return v.value
+
     def collect(self, raw: bool = False, meta: bool = False):
         """Wait for the oldest submitted batch; same return value as process().  meta=True (batches submitted with
         stream_ids / pts): returns (result, window_stream_ids, window_pts) through cova_pipeline_collect_host2."""

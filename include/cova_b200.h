@@ -146,7 +146,8 @@ void cova_pipeline_free(cova_pipeline *p);
 int cova_pipeline_set_cc_threshold(cova_pipeline *p, uint32_t cc_threshold);
 /* run all kernels on this stream (a cudaStream_t / CUstream as void*); NULL = the pipeline's own */
 int cova_pipeline_set_stream(cova_pipeline *p, void *cuda_stream);
-/* number of windows a batch of this shape produces */
+/* number of windows a batch of this shape produces, at the creation gamma (a stream batch with per-stream gammas,
+ * cova_pipeline_set_stream_property: read the per-stream counts from collect_host2's n_windows / win_stream_ids) */
 int cova_pipeline_n_windows(const cova_pipeline *p, uint32_t n_streams, uint32_t frames_per_stream, uint32_t *n);
 
 /* stage 0: put a batch of frames [n_streams][frames_per_stream][h_mb][w_mb][4] into the device frame pool.
@@ -221,6 +222,27 @@ int cova_pipeline_submit_ragged(cova_pipeline *p, const uint8_t *frames, uint32_
                                 const uint32_t *stream_ids, const uint64_t *pts, uint32_t flags);
 /* forget the state of the given streams (NULL = all): their next CONTINUED batch starts with an empty window */
 int cova_pipeline_reset_streams(cova_pipeline *p, const uint32_t *stream_ids, uint32_t n);
+/* Per-stream element properties of a batch pipeline, by name like the GObject properties they replace:
+ *   "gamma"         u32 >= 1      metapreprocess/imp.rs:57-133   (sub-sampling of windows)
+ *   "cc-threshold"  u32           bboxcc/imp.rs:16,51-101        (reinterpreted as i32, imp.rs:248, as today)
+ * stream_ids[n]: ids in [0, max_streams); NULL = every stream of the pipeline (n ignored), like reset_streams.
+ * The submits that name streams (submit_host2, submit_ragged, submit_sparse, submit_sparse_ragged) use the values in
+ * effect when they are called; batches already in flight keep theirs, and a set is allowed while batches are in flight.
+ * A stream that never had a property set follows the pipeline: its creation gamma, and the current
+ * cova_pipeline_set_cc_threshold value; once set, a stream keeps its own value (a later set_cc_threshold does not move it).
+ * The anonymous entry points (process_host, submit_host, load_frames / load_masks + run / ccl) ignore stream properties.
+ * Properties survive reset_streams.  Each stream keeps the element's countdown gamma_idx: once its window is full a frame
+ * emits a window when the countdown is 0 and restarts it at gamma - 1, so a new gamma takes effect after the stream's next
+ * emitted window, as with cova_metapreprocess_set_gamma.  A fresh (non-CONTINUE) batch and reset_streams restart the
+ * countdown at 0.  The window buffers are sized at creation for the creation gamma, so a stream gamma below it is refused;
+ * a pipeline created with gamma 1 (the default, and the reference's effective value) accepts every gamma.  Without
+ * COVA_SUBMIT_STAGGERED the streams of a CONTINUED batch must also share their gamma and countdown.
+ * COVA_E_INVAL, with nothing changed (the whole id list is checked first): a null handle or name, an unknown name, gamma 0
+ * or below the creation gamma, an id >= max_streams. */
+int cova_pipeline_set_stream_property(cova_pipeline *p, const uint32_t *stream_ids, uint32_t n, const char *name,
+                                      uint32_t value);
+/* the value a batch submitted now would use for this stream: its own, or the pipeline's if it never had one */
+int cova_pipeline_get_stream_property(const cova_pipeline *p, uint32_t stream_id, const char *name, uint32_t *value);
 
 /* Host-side packer for COVA_FLAG_INPUT_PACKED16: n_mb macroblock quads (the decoder's [mb_weight, |mv_x|, |mv_y|, stale]
  * bytes, h264_mb.c:822-855) -> n_mb u16.  A packer owns n_threads worker threads (0 = one per online CPU, at most 64);
