@@ -71,6 +71,7 @@ SIGNATURES = {
                                         ctypes.c_uint32, ctypes.c_uint32, _vp, ctypes.c_size_t, ctypes.c_uint32, ctypes.c_uint32]),
     "cova_pipeline_free": (None, [_vp]),
     "cova_pipeline_set_cc_threshold": (ctypes.c_int, [_vp, ctypes.c_uint32]),
+    "cova_pipeline_set_segmentation_threshold": (ctypes.c_int, [_vp, ctypes.c_float]),
     "cova_pipeline_set_stream": (ctypes.c_int, [_vp, _vp]),
     "cova_pipeline_n_windows": (ctypes.c_int, [_vp, ctypes.c_uint32, ctypes.c_uint32, _u32p]),
     "cova_pipeline_load_frames": (ctypes.c_int, [_vp, _vp, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_int]),
@@ -88,6 +89,8 @@ SIGNATURES = {
     "cova_pipeline_reset_streams": (ctypes.c_int, [_vp, _vp, ctypes.c_uint32]),
     "cova_pipeline_set_stream_property": (ctypes.c_int, [_vp, _vp, ctypes.c_uint32, ctypes.c_char_p, ctypes.c_uint32]),
     "cova_pipeline_get_stream_property": (ctypes.c_int, [_vp, ctypes.c_uint32, ctypes.c_char_p, _u32p]),
+    "cova_pipeline_set_stream_property_f32": (ctypes.c_int, [_vp, _vp, ctypes.c_uint32, ctypes.c_char_p, ctypes.c_float]),
+    "cova_pipeline_get_stream_property_f32": (ctypes.c_int, [_vp, ctypes.c_uint32, ctypes.c_char_p, _f32p]),
     "cova_packer_new": (ctypes.c_int, [_vpp, ctypes.c_uint32]),
     "cova_packer_free": (None, [_vp]),
     "cova_packer_pack": (ctypes.c_int, [_vp, _vp, _vp, ctypes.c_size_t]),

@@ -84,6 +84,7 @@ struct SimtDecArgs {
     const float *w, *b, *gamma, *beta, *mean, *var;   // convt_w [Cin][Cout][4][4]
     const float *head_w, *head_b;  // last layer only
     uint8_t *mask; float *logits;  // last layer only: [N][Ht][Wt]
+    const float *seg; float seg_tau;   // last layer only: foreground when logit > (seg ? seg[n] : seg_tau), as tc epilogue_head
     int Cin, Cout, N, Ht, Wt, crop_t, crop_l;
 };
 
@@ -148,7 +149,7 @@ __global__ void __launch_bounds__(128) simt_head_kernel(SimtDecArgs A) {
     float z = A.head_b[0];
     for (int j = 0; j < 16; j++) z = fmaf(acc[j], A.head_w[j], z);
     size_t o = ((size_t)n * A.Ht + Y) * A.Wt + X;
-    A.mask[o] = z > 0.f ? 1 : 0;     // sigmoid(z) > 0.5 <=> z > 0; maskcopy's class_map + 1
+    A.mask[o] = z > (A.seg ? A.seg[n] : A.seg_tau) ? 1 : 0;   // sigmoid(z) > segmentation-threshold; maskcopy's class_map + 1
     if (A.logits) A.logits[o] = z;
 }
 

@@ -46,6 +46,7 @@ struct LayerParams {
     int nsplit;                        // DEC: N split over CTAs (dec0: 2)
     int Ht, Wt, crop_t, crop_l;        // DEC/HEAD: target extent and crop
     uint8_t *mask; float *logits;      // HEAD
+    const float *seg; float seg_tau;   // HEAD: pixel is foreground when logit > (seg ? seg[n] : seg_tau), n = window of the chunk
     unsigned int *watchdog;            // set to a non-zero code if a barrier wait times out
     int bn_nonneg;                     // ENC: every BatchNorm scale of the layer is >= 0 (skips the min-pool path)
     int dbg;                           // experiments only: bit0 = skip the MMAs, bit1 = skip the epilogue math (results are garbage)
@@ -510,13 +511,15 @@ __device__ __forceinline__ void epilogue_head(const LayerParams &p, const float 
     tmem_wait_ld();
     const int oy = 2 * y2 + (ph >> 1), ox = 2 * x2 + (ph & 1);
     const bool vpos = n < p.N && oy <= gi.H && ox <= gi.W;
+    // tau = logit(segmentation-threshold), 0 at the default 0.5; per window only for a batch whose streams set their own
+    const float tau = vpos && p.seg ? __ldg(p.seg + n) : p.seg_tau;
 #pragma unroll
     for (int par = 0; par < 4; par++) {
         const int Y = 2 * oy + (par >> 1) - p.crop_t, X = 2 * ox + (par & 1) - p.crop_l;
         if (vpos && Y >= 0 && Y < p.Ht && X >= 0 && X < p.Wt) {
             const float z = __uint_as_float(v[par]) + c0;
             const size_t o = ((size_t)n * p.Ht + Y) * p.Wt + X;
-            p.mask[o] = z > 0.f ? 1 : 0;      // sigmoid(z) > 0.5 (nvinfer threshold), +1 of maskcopy folded
+            p.mask[o] = z > tau ? 1 : 0;      // sigmoid(z) > segmentation-threshold (nvinfer), +1 of maskcopy folded
             if (p.logits) p.logits[o] = z;
         }
     }

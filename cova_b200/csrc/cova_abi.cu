@@ -505,6 +505,7 @@ struct cova_pipeline {
     int device = 0, n_sms = 0;
     uint32_t W = 0, H = 0, T = 0, gamma = 1, max_streams = 0, max_fps = 0, max_windows = 0, flags = 0, impl = 0;
     uint32_t cc_threshold = 0;
+    float seg_t = 0.5f, seg_tau = 0.f;   // segmentation-threshold and its logit (seg_tau_of), read when BlobNet is enqueued
     cudaStream_t own_stream = nullptr, stream = nullptr;
     size_t frame_bytes = 0;              // bytes of one frame in the pool: 4 per macroblock, or 2 with COVA_FLAG_INPUT_PACKED16
     bool packed = false;
@@ -514,12 +515,16 @@ struct cova_pipeline {
     std::vector<uint64_t> n_seen, id_mark;
     std::vector<uint32_t> gamma_idx;     // per stream id: the element's countdown to its next window (imp.rs:321-330)
     uint64_t id_epoch = 0;
-    // Per-stream element properties (cova_pipeline_set_stream_property), by stream id: gamma (0 = the creation gamma) and
-    // cc-threshold (used when thr_set; the pipeline's cc_threshold otherwise).  Read by the submits that name streams.
+    // Per-stream element properties (cova_pipeline_set_stream_property / _f32), by stream id: gamma (0 = the creation
+    // gamma), cc-threshold (used when thr_set; the pipeline's cc_threshold otherwise) and segmentation-threshold (used when
+    // seg_set; seg_t otherwise).  Read by the submits that name streams.
     std::vector<uint32_t> s_gamma, s_thr;
     std::vector<uint8_t> s_thr_set;
+    std::vector<float> s_seg;
+    std::vector<uint8_t> s_seg_set;
     std::vector<uint32_t> first_scratch, hist_scratch;   // per chain of the batch being submitted
     std::vector<uint32_t> gam_scratch, thr_scratch;      // gamma and cc-threshold per chain of the batch being submitted
+    std::vector<float> seg_scratch;                      // segmentation-threshold per chain of the batch being submitted
     std::vector<uint32_t> cd_scratch;                    // countdown per chain after the batch being submitted
     std::vector<uint32_t> count_scratch;                 // new frames per chain of the batch being submitted
     std::vector<uint64_t> off_scratch;                   // record offsets of the sparse batch being submitted
@@ -562,12 +567,16 @@ struct cova_pipeline {
         // per-stream properties (set_stream_property), allocated on the slot's first batch that needs them:
         //   gam[s]  = chain s's gamma, when some chain's differs from the creation gamma     read by enc1_fused_kernel
         //   thr[w]  = window w's cc-threshold, when some differs from the pipeline's value   read by the CCL kernels
+        //   seg[w]  = logit of window w's segmentation-threshold, when some threshold differs from the pipeline's value
+        //                                                                          read by the BlobNet head's epilogue
         int *h_gam = nullptr, *d_gam = nullptr;
         int *h_thr = nullptr, *d_thr = nullptr;
-        bool gam_on = false, thr_on = false;           // the batch in the slot uses gam / thr
+        float *h_seg = nullptr, *d_seg = nullptr;
+        bool gam_on = false, thr_on = false, seg_on = false;   // the batch in the slot uses gam / thr / seg
         cudaEvent_t ev_tab = nullptr;                  // recorded after the upload: the staging may be rewritten after it
         std::vector<uint32_t> tab_first, tab_end;      // what the tables hold: per-chain first and end, stride, stream,
-        std::vector<uint32_t> tab_gam, tab_thr;        // per-chain gamma, per-chain threshold (empty: thr not uploaded)
+        std::vector<uint32_t> tab_gam, tab_thr;        // per-chain gamma, per-chain threshold (empty: thr not uploaded),
+        std::vector<float> tab_seg;                    // per-chain segmentation-threshold (empty: seg not uploaded)
         uint32_t tab_fps = 0;
         cudaStream_t tab_stream = nullptr;
         // sparse input (cova_pipeline_submit_sparse), allocated on the slot's first sparse submit: the batch's records at
@@ -601,6 +610,10 @@ struct cova_pipeline {
     cova_layer_plan last_plan[8] = {};   // per layer: the plan of its last tcgen05 launch (cova_pipeline_last_plan)
 };
 using Slot = cova_pipeline::Slot;
+
+// The mask contract: a pixel is foreground when sigmoid(logit) > t (nvinfer's segmentation-threshold), evaluated as
+// logit > tau with tau computed here once, in double, and rounded once to fp32.  t = 0.5 gives tau = 0.0f exactly.
+static float seg_tau_of(float t) { return (float)log((double)t / (1.0 - (double)t)); }
 
 // windows of a device chain of `fps` frames whose first window has its newest frame at index `first`
 static uint32_t windows_from(uint32_t fps, uint32_t first, uint32_t gamma) { return fps > first ? (fps - 1 - first) / gamma + 1 : 0; }
@@ -697,6 +710,7 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
     p->cc_threshold = cc_threshold;
     p->max_windows = max_windows;
     p->s_gamma.assign(max_streams, 0); p->s_thr.assign(max_streams, 0); p->s_thr_set.assign(max_streams, 0);
+    p->s_seg.assign(max_streams, 0.5f); p->s_seg_set.assign(max_streams, 0);
     auto fail = [&](int code) { cova_pipeline_free(p); return code; };
     if ((rc = parse_weights(weights, weights_len, p->hw))) return fail(rc);
     cudaDeviceProp prop;
@@ -812,6 +826,8 @@ extern "C" void cova_pipeline_free(cova_pipeline *p) {
         if (sl.d_gam) cudaFree(sl.d_gam);
         if (sl.h_thr) cudaFreeHost(sl.h_thr);
         if (sl.d_thr) cudaFree(sl.d_thr);
+        if (sl.h_seg) cudaFreeHost(sl.h_seg);
+        if (sl.d_seg) cudaFree(sl.d_seg);
         if (sl.ev_tab) cudaEventDestroy(sl.ev_tab);
         if (sl.d_sparse) cudaFree(sl.d_sparse);
         if (sl.h_off) cudaFreeHost(sl.h_off);
@@ -839,6 +855,14 @@ extern "C" int cova_pipeline_set_cc_threshold(cova_pipeline *p, uint32_t t) {
     p->cc_threshold = t;
     return COVA_OK;
 }
+// nvinfer's segmentation-threshold: a float in (0, 1)
+static bool seg_threshold_ok(float t) { return t > 0.f && t < 1.f; }
+extern "C" int cova_pipeline_set_segmentation_threshold(cova_pipeline *p, float t) {
+    if (!p) return set_err(COVA_E_INVAL, "null handle");
+    if (!seg_threshold_ok(t)) return set_err(COVA_E_INVAL, "segmentation-threshold must be finite and inside (0, 1)");
+    p->seg_t = t; p->seg_tau = seg_tau_of(t);
+    return COVA_OK;
+}
 extern "C" int cova_pipeline_set_stream(cova_pipeline *p, void *s) {
     if (!p) return set_err(COVA_E_INVAL, "null handle");
     p->stream = s ? reinterpret_cast<cudaStream_t>(s) : p->own_stream;
@@ -861,11 +885,13 @@ static int check_batch_bounds(const cova_pipeline *p, uint32_t n_streams, uint32
 // chain s) of the newest frame of the chain's first window; nullptr = T - 1 for every chain, i.e. chains that start with
 // an empty window.  CONTINUED chains (submit_host2) start later, where their carried history and gamma phase put them.
 // end[s] is where chain s's frames end (ragged batches); nullptr = fps for every chain.  gam[s] is chain s's gamma, nullptr
-// = the creation gamma for every chain; thr[s] is chain s's cc-threshold, nullptr = the pipeline's value at CCL launch
-// (stream properties, cova_pipeline_set_stream_property).  Lock-step, staggered, ragged and mixed-property batches go
-// through the same tables and kernels.
+// = the creation gamma for every chain; thr[s] is chain s's cc-threshold, nullptr = the pipeline's value at CCL launch;
+// seg[s] is chain s's segmentation-threshold, nullptr = the pipeline's value at BlobNet launch (stream properties,
+// cova_pipeline_set_stream_property / _f32).  Lock-step, staggered, ragged and mixed-property batches go through the same
+// tables and kernels.
 static int set_batch_shape(cova_pipeline *p, int k, uint32_t n_streams, uint32_t fps, const uint32_t *first = nullptr,
-                           const uint32_t *end = nullptr, const uint32_t *gam = nullptr, const uint32_t *thr = nullptr) {
+                           const uint32_t *end = nullptr, const uint32_t *gam = nullptr, const uint32_t *thr = nullptr,
+                           const float *seg = nullptr) {
     auto &sl = p->slot[k];
     const uint32_t t1 = p->T - 1, cs = p->chunk_streams;
     auto first_of = [&](uint32_t s) { return first ? first[s] : t1; };
@@ -886,11 +912,13 @@ static int set_batch_shape(cova_pipeline *p, int k, uint32_t n_streams, uint32_t
         sl.gam_on = sl.gam_on || gam_of(s) != p->gamma;
     }
     sl.thr_on = thr != nullptr;
+    sl.seg_on = seg != nullptr;
     sl.n_streams = n_streams; sl.fps = fps; sl.n_windows = (uint32_t)total;
     bool same = sl.tab_fps == fps && sl.tab_stream == p->stream && sl.tab_first.size() == n_streams &&
-                sl.tab_thr.size() == (thr ? n_streams : 0);
+                sl.tab_thr.size() == (thr ? n_streams : 0) && sl.tab_seg.size() == (seg ? n_streams : 0);
     for (uint32_t s = 0; same && s < n_streams; s++)
-        same = sl.tab_first[s] == first_of(s) && sl.tab_end[s] == end_of(s) && sl.tab_gam[s] == gam_of(s) && (!thr || sl.tab_thr[s] == thr[s]);
+        same = sl.tab_first[s] == first_of(s) && sl.tab_end[s] == end_of(s) && sl.tab_gam[s] == gam_of(s) &&
+               (!thr || sl.tab_thr[s] == thr[s]) && (!seg || sl.tab_seg[s] == seg[s]);
     if (same) return COVA_OK;                                      // the slot's device tables already hold this shape
     if (sl.ragged && !sl.h_fmap) {
         COVA_CUDA(cudaMallocHost(&sl.h_fmap, sizeof(int) * (size_t)p->max_streams * p->max_fps));
@@ -904,17 +932,24 @@ static int set_batch_shape(cova_pipeline *p, int k, uint32_t n_streams, uint32_t
         COVA_CUDA(cudaMallocHost(&sl.h_thr, sizeof(int) * std::max<size_t>(1, p->max_windows)));
         COVA_CUDA(cudaMalloc(&sl.d_thr, sizeof(int) * std::max<size_t>(1, p->max_windows)));
     }
+    if (seg && !sl.h_seg) {
+        COVA_CUDA(cudaMallocHost(&sl.h_seg, sizeof(float) * std::max<size_t>(1, p->max_windows)));
+        COVA_CUDA(cudaMalloc(&sl.d_seg, sizeof(float) * std::max<size_t>(1, p->max_windows)));
+    }
     // The staging may still be read by this slot's previous upload when synchronous entry points reuse slot 0 back to back.
     // On the submit path that upload has completed: the slot's previous batch was collected.
     COVA_CUDA(cudaEventSynchronize(sl.ev_tab));
     sl.tab_first.clear(); sl.tab_end.clear(); sl.tab_gam.clear(); sl.tab_thr.clear();   // invalid until the upload below is enqueued
+    sl.tab_seg.clear();
     for (uint32_t s = 0; s < n_streams; s++) {
         const uint32_t f = first_of(s), c0 = s / cs * cs;
+        const float tau = seg ? seg_tau_of(seg[s]) : 0.f;
         sl.h_tab[s] = make_int4((int)f, (int)(sl.win0[s] - sl.win0[c0]), (int)end_of(s), (int)(sl.fpre[s] - sl.fpre[c0]));
         if (sl.gam_on) sl.h_gam[s] = (int)gam_of(s);
         for (uint32_t w = sl.win0[s]; w < sl.win0[s + 1]; w++) {
             sl.h_newest[w] = (int)((s - c0) * fps + f + (w - sl.win0[s]) * gam_of(s));
             if (thr) sl.h_thr[w] = (int)thr[s];                    // `cc_threshold as i32` (bboxcc/imp.rs:248)
+            if (seg) sl.h_seg[w] = tau;
         }
         if (sl.ragged)
             for (uint32_t i = 0; i < end_of(s); i++) sl.h_fmap[sl.fpre[s] + i] = (int)((s - c0) * fps + i);
@@ -924,10 +959,12 @@ static int set_batch_shape(cova_pipeline *p, int k, uint32_t n_streams, uint32_t
     if (sl.ragged) COVA_CUDA(cudaMemcpyAsync(sl.d_fmap, sl.h_fmap, sizeof(int) * sl.fpre[n_streams], cudaMemcpyHostToDevice, p->stream));
     if (sl.gam_on) COVA_CUDA(cudaMemcpyAsync(sl.d_gam, sl.h_gam, sizeof(int) * n_streams, cudaMemcpyHostToDevice, p->stream));
     if (thr && total) COVA_CUDA(cudaMemcpyAsync(sl.d_thr, sl.h_thr, sizeof(int) * total, cudaMemcpyHostToDevice, p->stream));
+    if (seg && total) COVA_CUDA(cudaMemcpyAsync(sl.d_seg, sl.h_seg, sizeof(float) * total, cudaMemcpyHostToDevice, p->stream));
     COVA_CUDA(cudaEventRecord(sl.ev_tab, p->stream));
     for (uint32_t s = 0; s < n_streams; s++) {
         sl.tab_first.push_back(first_of(s)); sl.tab_end.push_back(end_of(s)); sl.tab_gam.push_back(gam_of(s));
         if (thr) sl.tab_thr.push_back(thr[s]);
+        if (seg) sl.tab_seg.push_back(seg[s]);
     }
     sl.tab_fps = fps; sl.tab_stream = p->stream;
     return COVA_OK;
@@ -976,7 +1013,7 @@ extern "C" int cova_pipeline_load_masks(cova_pipeline *p, const uint8_t *masks, 
     if (!n || n > p->max_windows) return set_err(COVA_E_INVAL, "mask batch exceeds the pipeline's window capacity");
     if (int rc = require_idle(p)) return rc;
     COVA_CUDA(cudaSetDevice(p->device));
-    p->slot[0].n_streams = 0; p->slot[0].n_windows = n; p->slot[0].thr_on = false;
+    p->slot[0].n_streams = 0; p->slot[0].n_windows = n; p->slot[0].thr_on = false; p->slot[0].seg_on = false;
     p->last_slot = 0;
     COVA_CUDA(cudaMemcpyAsync(p->d_mask, masks, (size_t)n * p->W * p->H, is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, p->stream));
     return COVA_OK;
@@ -1043,11 +1080,11 @@ static void crop_for(int in_extent, int target, int &crop_lo) {
 }
 
 #ifndef COVA_VALIDATION
-static int simt_layer(cova_pipeline *, const Chunk &, int) {
+static int simt_layer(cova_pipeline *, const Slot &, const Chunk &, int) {
     return set_err(COVA_E_UNSUPPORTED, "the validation kernels (COVA_IMPL_SIMT) are not part of this build; use libcova_b200_val.so");
 }
 #else
-static int simt_layer(cova_pipeline *p, const Chunk &ck, int layer) {
+static int simt_layer(cova_pipeline *p, const Slot &sl, const Chunk &ck, int layer) {
     const int N = (int)ck.windows;
     const float *w = p->d_wraw;
     if (layer == 0 && !p->x[0]) return set_err(COVA_E_UNSUPPORTED, "validation kernel of layer 0 needs a pipeline created with COVA_IMPL_SIMT");
@@ -1082,6 +1119,7 @@ static int simt_layer(cova_pipeline *p, const Chunk &ck, int layer) {
     a.head_w = w + p->hw.off_head[0]; a.head_b = w + p->hw.off_head[1];
     a.mask = p->d_mask + (size_t)ck.window0 * p->W * p->H;
     a.logits = p->d_logits ? p->d_logits + (size_t)ck.window0 * p->W * p->H : nullptr;
+    a.seg = sl.seg_on ? sl.d_seg + ck.window0 : nullptr; a.seg_tau = p->seg_tau;
     a.Cin = kDecCin[i]; a.Cout = kDecCout[i]; a.N = N;
     a.Ht = p->sizes_h[3 - i]; a.Wt = p->sizes_w[3 - i];
     crop_for(a.gin.H, a.Ht, a.crop_t);
@@ -1320,6 +1358,7 @@ static int tc_launch(cova_pipeline *p, const Slot &sl, const Chunk &ck, int laye
         crop_for(lp.gin.W, lp.Wt, lp.crop_l);
         lp.mask = p->d_mask + (size_t)ck.window0 * p->W * p->H;
         lp.logits = p->d_logits ? p->d_logits + (size_t)ck.window0 * p->W * p->H : nullptr;
+        lp.seg = sl.seg_on ? sl.d_seg + ck.window0 : nullptr; lp.seg_tau = p->seg_tau;
     }
     cudaError_t err = launch_layer(layer, pl, p->stream);
     if (err != cudaSuccess) return set_err(COVA_E_CUDA, "%s launch: %s", kLayerName[layer], cudaGetErrorString(err));
@@ -1336,7 +1375,7 @@ extern "C" int cova_pipeline_run_layer(cova_pipeline *p, int layer, uint32_t imp
     Chunk ck;
     int rc = stage_chunk(p, ck);
     if (rc || !ck.windows) return rc;
-    if (impl == COVA_IMPL_SIMT) return simt_layer(p, ck, layer);
+    if (impl == COVA_IMPL_SIMT) return simt_layer(p, p->slot[p->last_slot], ck, layer);
     LayerPlan pl;
     if ((rc = tc_plan(p, p->slot[p->last_slot], ck, layer, pl))) return rc;
     return tc_launch(p, p->slot[p->last_slot], ck, layer, pl);
@@ -1346,7 +1385,7 @@ static int blobnet_chunk(cova_pipeline *p, const Slot &sl, const Chunk &ck) {
     if (!ck.windows) return COVA_OK;
     if (p->impl == COVA_IMPL_SIMT) {
         for (int layer = 0; layer < 8; layer++) {
-            int rc = simt_layer(p, ck, layer);
+            int rc = simt_layer(p, sl, ck, layer);
             if (rc) return rc;
         }
         return COVA_OK;
@@ -1528,8 +1567,8 @@ __global__ void __launch_bounds__(256) carry_kernel(uint32_t *__restrict__ pool,
 
 // Argument checks and per-chain plan of a submit, before any device call: fills count_scratch (n_s: `counts`, or fps for
 // every chain when counts is nullptr), first_scratch, hist_scratch and off_scratch, for stream batches also gam_scratch,
-// thr_scratch (the streams' properties now) and cd_scratch (their countdowns after the batch), and raises lead (0 on entry)
-// to the longest carried history
+// thr_scratch, seg_scratch (the streams' properties now) and cd_scratch (their countdowns after the batch), and raises
+// lead (0 on entry) to the longest carried history
 static int plan_submit(cova_pipeline *p, const uint8_t *frames, uint32_t n_streams, uint32_t fps, const uint32_t *counts,
                        const uint32_t *stream_ids, uint32_t flags, bool stateful, const size_t *sparse_len, uint32_t &lead) {
     if (flags & ~(COVA_SUBMIT_CONTINUE | COVA_SUBMIT_STAGGERED)) return set_err(COVA_E_INVAL, "unknown submit flag");
@@ -1571,7 +1610,7 @@ static int plan_submit(cova_pipeline *p, const uint8_t *frames, uint32_t n_strea
         }
         p->id_epoch++;                                              // "seen in this batch" marks without clearing the array
         std::vector<uint32_t> &gam = p->gam_scratch, &thr = p->thr_scratch, &cd = p->cd_scratch;
-        gam.resize(n_streams); thr.resize(n_streams); cd.resize(n_streams);
+        gam.resize(n_streams); thr.resize(n_streams); cd.resize(n_streams); p->seg_scratch.resize(n_streams);
         for (uint32_t s = 0; s < n_streams; s++) {
             const uint32_t id = stream_ids ? stream_ids[s] : s;
             if (id >= p->max_streams) return set_err(COVA_E_INVAL, "stream id out of range (ids are 0 .. max_streams-1)");
@@ -1579,6 +1618,7 @@ static int plan_submit(cova_pipeline *p, const uint8_t *frames, uint32_t n_strea
             p->id_mark[id] = p->id_epoch;
             gam[s] = p->s_gamma[id] ? p->s_gamma[id] : p->gamma;
             thr[s] = p->s_thr_set[id] ? p->s_thr[id] : p->cc_threshold;
+            p->seg_scratch[s] = p->s_seg_set[id] ? p->s_seg[id] : p->seg_t;
             // In the unpadded chain (hs carried frames, then the new ones) index T-1 is the first new frame whose window is
             // full; from there the element emits when its countdown gamma_idx is 0 and then restarts it at gamma - 1
             // (imp.rs:321-330).  A fresh chain starts with an empty window and a countdown of 0.
@@ -1645,11 +1685,13 @@ static int setup_slot(cova_pipeline *p, int k, uint32_t n_streams, uint32_t lead
     }
     // stream properties: a table only for a batch that does not run entirely on the pipeline's values
     const uint32_t *gam = nullptr, *thr = nullptr;
+    const float *seg = nullptr;
     for (uint32_t s = 0; stateful && s < n_streams; s++) {
         if (p->gam_scratch[s] != p->gamma) gam = p->gam_scratch.data();
         if (p->thr_scratch[s] != p->cc_threshold) thr = p->thr_scratch.data();
+        if (p->seg_scratch[s] != p->seg_t) seg = p->seg_scratch.data();
     }
-    if ((rc = set_batch_shape(p, k, n_streams, max_n + lead, first.data(), end.data(), gam, thr))) return rc;
+    if ((rc = set_batch_shape(p, k, n_streams, max_n + lead, first.data(), end.data(), gam, thr, seg))) return rc;
     p->last_slot = k;
     sl.win_pts.clear(); sl.win_ids.clear();
     if (stateful) {
@@ -1810,21 +1852,39 @@ extern "C" int cova_pipeline_reset_streams(cova_pipeline *p, const uint32_t *str
     return COVA_OK;
 }
 
-// 0: "gamma", 1: "cc-threshold", -1: no such stream property
+// u32 properties 0: "gamma", 1: "cc-threshold"; f32 property 2: "segmentation-threshold"; -1: no such stream property
 static int stream_property(const char *name) {
-    return !strcmp(name, "gamma") ? 0 : !strcmp(name, "cc-threshold") ? 1 : -1;
+    return !strcmp(name, "gamma") ? 0 : !strcmp(name, "cc-threshold") ? 1 : !strcmp(name, "segmentation-threshold") ? 2 : -1;
+}
+// the property of a u32 / f32 call, or -1 with the error set
+static int u32_property(const char *name) {
+    const int prop = stream_property(name);
+    if (prop == 2) set_err(COVA_E_INVAL, "segmentation-threshold is a float: use cova_pipeline_set/get_stream_property_f32");
+    else if (prop < 0) set_err(COVA_E_INVAL, "unknown stream property (\"gamma\" or \"cc-threshold\")");
+    return prop == 2 ? -1 : prop;
+}
+static int f32_property(const char *name) {
+    const int prop = stream_property(name);
+    if (prop == 0 || prop == 1) set_err(COVA_E_INVAL, "%s is a u32: use cova_pipeline_set/get_stream_property", name);
+    else if (prop < 0) set_err(COVA_E_INVAL, "unknown float stream property (\"segmentation-threshold\")");
+    return prop == 2 ? prop : -1;
+}
+// the whole id list before anything changes
+static int check_stream_ids(const cova_pipeline *p, const uint32_t *stream_ids, uint32_t n) {
+    for (uint32_t i = 0; stream_ids && i < n; i++)
+        if (stream_ids[i] >= p->max_streams) return set_err(COVA_E_INVAL, "stream id out of range (ids are 0 .. max_streams-1)");
+    return COVA_OK;
 }
 extern "C" int cova_pipeline_set_stream_property(cova_pipeline *p, const uint32_t *stream_ids, uint32_t n, const char *name,
                                                  uint32_t value) {
     if (!p || !name) return set_err(COVA_E_INVAL, "null argument");
-    const int prop = stream_property(name);
-    if (prop < 0) return set_err(COVA_E_INVAL, "unknown stream property (\"gamma\" or \"cc-threshold\")");
+    const int prop = u32_property(name);
+    if (prop < 0) return COVA_E_INVAL;
     if (prop == 0 && value < 1) return set_err(COVA_E_INVAL, "gamma is a u32 >= 1");
     // the window buffers and the max_windows bound were sized for the creation gamma; a larger one yields fewer windows
     if (prop == 0 && value < p->gamma) return set_err(COVA_E_INVAL, "a stream's gamma cannot be below the pipeline's creation gamma");
     const uint32_t m = stream_ids ? n : p->max_streams;
-    for (uint32_t i = 0; stream_ids && i < m; i++)                 // the whole list before anything changes
-        if (stream_ids[i] >= p->max_streams) return set_err(COVA_E_INVAL, "stream id out of range (ids are 0 .. max_streams-1)");
+    if (int rc = check_stream_ids(p, stream_ids, m)) return rc;
     for (uint32_t i = 0; i < m; i++) {
         const uint32_t id = stream_ids ? stream_ids[i] : i;
         if (prop == 0) p->s_gamma[id] = value;
@@ -1834,11 +1894,31 @@ extern "C" int cova_pipeline_set_stream_property(cova_pipeline *p, const uint32_
 }
 extern "C" int cova_pipeline_get_stream_property(const cova_pipeline *p, uint32_t stream_id, const char *name, uint32_t *value) {
     if (!p || !name || !value) return set_err(COVA_E_INVAL, "null argument");
-    const int prop = stream_property(name);
-    if (prop < 0) return set_err(COVA_E_INVAL, "unknown stream property (\"gamma\" or \"cc-threshold\")");
+    const int prop = u32_property(name);
+    if (prop < 0) return COVA_E_INVAL;
     if (stream_id >= p->max_streams) return set_err(COVA_E_INVAL, "stream id out of range (ids are 0 .. max_streams-1)");
     if (prop == 0) *value = p->s_gamma[stream_id] ? p->s_gamma[stream_id] : p->gamma;
     else *value = p->s_thr_set[stream_id] ? p->s_thr[stream_id] : p->cc_threshold;
+    return COVA_OK;
+}
+extern "C" int cova_pipeline_set_stream_property_f32(cova_pipeline *p, const uint32_t *stream_ids, uint32_t n, const char *name,
+                                                     float value) {
+    if (!p || !name) return set_err(COVA_E_INVAL, "null argument");
+    if (f32_property(name) < 0) return COVA_E_INVAL;
+    if (!seg_threshold_ok(value)) return set_err(COVA_E_INVAL, "segmentation-threshold must be finite and inside (0, 1)");
+    const uint32_t m = stream_ids ? n : p->max_streams;
+    if (int rc = check_stream_ids(p, stream_ids, m)) return rc;
+    for (uint32_t i = 0; i < m; i++) {
+        const uint32_t id = stream_ids ? stream_ids[i] : i;
+        p->s_seg[id] = value; p->s_seg_set[id] = 1;
+    }
+    return COVA_OK;
+}
+extern "C" int cova_pipeline_get_stream_property_f32(const cova_pipeline *p, uint32_t stream_id, const char *name, float *value) {
+    if (!p || !name || !value) return set_err(COVA_E_INVAL, "null argument");
+    if (f32_property(name) < 0) return COVA_E_INVAL;
+    if (stream_id >= p->max_streams) return set_err(COVA_E_INVAL, "stream id out of range (ids are 0 .. max_streams-1)");
+    *value = p->s_seg_set[stream_id] ? p->s_seg[stream_id] : p->seg_t;
     return COVA_OK;
 }
 

@@ -433,10 +433,14 @@ class BlobPipeline:
         return check(rc, self._L)
 
     # ---- configuration
-    def set_property(self, name: str, value: int):
-        if name != "cc-threshold":
+    def set_property(self, name: str, value):
+        """"cc-threshold" (u32, bboxcc) or "segmentation-threshold" (float in (0, 1), nvinfer) of the whole pipeline."""
+        if name == "cc-threshold":
+            self._check(self._L.cova_pipeline_set_cc_threshold(self._h, value))
+        elif name == "segmentation-threshold":
+            self._check(self._L.cova_pipeline_set_segmentation_threshold(self._h, value))
+        else:
             raise KeyError(name)
-        self._check(self._L.cova_pipeline_set_cc_threshold(self._h, value))
 
     def set_stream(self, cuda_stream: int | None):
         self._check(self._L.cova_pipeline_set_stream(self._h, ctypes.c_void_p(cuda_stream or 0)))
@@ -606,17 +610,23 @@ class BlobPipeline:
             ids = np.ascontiguousarray(stream_ids, dtype=np.uint32)
             self._check(self._L.cova_pipeline_reset_streams(self._h, _ptr(ids), ids.size))
 
-    def set_stream_property(self, name: str, value: int, stream_ids=None):
+    def set_stream_property(self, name: str, value, stream_ids=None):
         """cova_pipeline_set_stream_property: "gamma" (>= the creation gamma) or "cc-threshold" of the given stream ids
-        (None = every stream), used by the submits that name streams from the next one on."""
+        (None = every stream), used by the submits that name streams from the next one on.  "segmentation-threshold"
+        (a float in (0, 1)) goes through cova_pipeline_set_stream_property_f32."""
         ids = None if stream_ids is None else np.ascontiguousarray(stream_ids, dtype=np.uint32).reshape(-1)
-        self._check(self._L.cova_pipeline_set_stream_property(self._h, None if ids is None else _ptr(ids),
-                                                              0 if ids is None else ids.size, name.encode(), value))
+        fn = (self._L.cova_pipeline_set_stream_property_f32 if name == "segmentation-threshold"
+              else self._L.cova_pipeline_set_stream_property)
+        self._check(fn(self._h, None if ids is None else _ptr(ids), 0 if ids is None else ids.size, name.encode(), value))
 
-    def get_stream_property(self, name: str, stream_id: int) -> int:
-        """The value a batch submitted now would use for this stream (its own, or the pipeline's)."""
-        v = ctypes.c_uint32()
-        self._check(self._L.cova_pipeline_get_stream_property(self._h, stream_id, name.encode(), ctypes.byref(v)))
+    def get_stream_property(self, name: str, stream_id: int):
+        """The value a batch submitted now would use for this stream (its own, or the pipeline's): an int, or a float for
+        "segmentation-threshold"."""
+        if name == "segmentation-threshold":
+            v, fn = ctypes.c_float(), self._L.cova_pipeline_get_stream_property_f32
+        else:
+            v, fn = ctypes.c_uint32(), self._L.cova_pipeline_get_stream_property
+        self._check(fn(self._h, stream_id, name.encode(), ctypes.byref(v)))
         return v.value
 
     def collect(self, raw: bool = False, meta: bool = False):

@@ -144,6 +144,16 @@ int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb, uint32_t h
                       size_t weights_len, uint32_t cc_threshold, uint32_t flags);
 void cova_pipeline_free(cova_pipeline *p);
 int cova_pipeline_set_cc_threshold(cova_pipeline *p, uint32_t cc_threshold);
+/* nvinfer's segmentation-threshold (config/blobnet/amsterdam_b128.txt:26, `class_map = prob > threshold`): a pixel of a
+ * window's mask is foreground when sigmoid(logit) > t, for a float t with 0 < t < 1; the default is 0.5.  Contract: the
+ * library evaluates this as logit > tau, tau = (float)log((double)t / (1.0 - (double)t)), computed once on the host in
+ * double and rounded once to fp32 (t = 0.5 gives tau = 0.0f exactly, the compare every earlier release made).  So the
+ * mask can differ from an fp32 `sigmoid(z) > t` only for logits within a rounding of tau.  Logits kept with
+ * COVA_FLAG_KEEP_LOGITS are unchanged by t.  The value is read when a BlobNet stage is enqueued (submit time for the
+ * submits, call time for blobnet / run / process_host); batches already in flight keep theirs, and a set is allowed
+ * while batches are in flight.  Per stream: cova_pipeline_set_stream_property_f32.  COVA_E_INVAL, with nothing
+ * changed: a null handle, a t that is not finite or not inside (0, 1). */
+int cova_pipeline_set_segmentation_threshold(cova_pipeline *p, float t);
 /* run all kernels on this stream (a cudaStream_t / CUstream as void*); NULL = the pipeline's own */
 int cova_pipeline_set_stream(cova_pipeline *p, void *cuda_stream);
 /* number of windows a batch of this shape produces, at the creation gamma (a stream batch with per-stream gammas,
@@ -243,6 +253,17 @@ int cova_pipeline_set_stream_property(cova_pipeline *p, const uint32_t *stream_i
                                       uint32_t value);
 /* the value a batch submitted now would use for this stream: its own, or the pipeline's if it never had one */
 int cova_pipeline_get_stream_property(const cova_pipeline *p, uint32_t stream_id, const char *name, uint32_t *value);
+/* The float stream property, with the rules of cova_pipeline_set_stream_property (NULL ids = every stream; read by the
+ * submits that name streams, at submit; a stream never set follows the current cova_pipeline_set_segmentation_threshold
+ * value, and once set keeps its own; values survive reset_streams; the anonymous and stage-wise entry points ignore it):
+ *   "segmentation-threshold"  float, 0 < t < 1, default 0.5   nvinfer config/blobnet/amsterdam_b128.txt:26
+ * It changes neither the windows nor the lock-step rule, only which pixels are foreground.  COVA_E_INVAL, with nothing
+ * changed (the whole id list is checked first): a null handle or name, an unknown name, "gamma" or "cc-threshold" (u32:
+ * the calls above, which in turn refuse "segmentation-threshold"), a value that is not finite or not inside (0, 1), an
+ * id >= max_streams.  The getter returns the value a batch submitted now would use for this stream. */
+int cova_pipeline_set_stream_property_f32(cova_pipeline *p, const uint32_t *stream_ids, uint32_t n, const char *name,
+                                          float value);
+int cova_pipeline_get_stream_property_f32(const cova_pipeline *p, uint32_t stream_id, const char *name, float *value);
 
 /* Host-side packer for COVA_FLAG_INPUT_PACKED16: n_mb macroblock quads (the decoder's [mb_weight, |mv_x|, |mv_y|, stale]
  * bytes, h264_mb.c:822-855) -> n_mb u16.  A packer owns n_threads worker threads (0 = one per online CPU, at most 64);
