@@ -105,6 +105,7 @@ SIGNATURES = {
     "cova_pipeline_read_activation": (ctypes.c_int, [_vp, ctypes.c_int, _vp, ctypes.c_size_t, _u32p]),
     "cova_pipeline_run_layer": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_uint32]),
     "cova_pipeline_set_debug": (ctypes.c_int, [_vp, ctypes.c_int]),
+    "cova_pipeline_set_sm_limit": (ctypes.c_int, [_vp, ctypes.c_int]),
     "cova_blobnet_plan": (ctypes.c_int, [ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_int, ctypes.c_int, _vp]),
     "cova_pipeline_last_plan": (ctypes.c_int, [_vp, _vp]),
     "cova_pipeline_launch_count": (ctypes.c_int, [_vp, _u64p]),

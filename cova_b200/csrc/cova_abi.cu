@@ -502,7 +502,8 @@ constexpr int kSlots = 4;
 struct Chunk { uint32_t stream0, n_streams, window0, windows; };
 
 struct cova_pipeline {
-    int device = 0, n_sms = 0;
+    int device = 0, n_sms = 0;           // n_sms: what the grids are sized for, the device's SMs unless capped (set_sm_limit)
+    int dev_sms = 0;                     // the device's SMs
     uint32_t W = 0, H = 0, T = 0, gamma = 1, max_streams = 0, max_fps = 0, max_windows = 0, flags = 0, impl = 0;
     uint32_t cc_threshold = 0;
     float seg_t = 0.5f, seg_tau = 0.f;   // segmentation-threshold and its logit (seg_tau_of), read when BlobNet is enqueued
@@ -715,7 +716,7 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
     if ((rc = parse_weights(weights, weights_len, p->hw))) return fail(rc);
     cudaDeviceProp prop;
     if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return fail(set_err(COVA_E_CUDA, "cudaGetDeviceProperties failed"));
-    p->n_sms = prop.multiProcessorCount;
+    p->n_sms = p->dev_sms = prop.multiProcessorCount;
     if (p->impl == COVA_IMPL_TCGEN05 && prop.major != 10)
         return fail(set_err(COVA_E_UNSUPPORTED, "the tcgen05 path needs an sm_100 device"));
     if (cudaStreamCreateWithFlags(&p->own_stream, cudaStreamNonBlocking) != cudaSuccess) return fail(set_err(COVA_E_CUDA, "stream creation failed"));
@@ -2066,6 +2067,13 @@ extern "C" int cova_pipeline_set_debug(cova_pipeline *p, int flags) {
     if (!p) return set_err(COVA_E_INVAL, "null handle");
     p->dbg = flags;
     // bit 5 (kDbgNoPdl): plain stream-ordered launches instead of programmatic dependent launch, for THIS handle only
+    return COVA_OK;
+}
+extern "C" int cova_pipeline_set_sm_limit(cova_pipeline *p, int n_sms) {
+    if (!p) return set_err(COVA_E_INVAL, "null handle");
+    if (n_sms < 0 || n_sms > p->dev_sms) return set_err(COVA_E_INVAL, "need 0 <= n_sms <= the device's SM count");
+    if (int rc = require_idle(p)) return rc;
+    p->n_sms = n_sms ? n_sms : p->dev_sms;
     return COVA_OK;
 }
 extern "C" int cova_pipeline_last_plan(const cova_pipeline *p, cova_layer_plan out[8]) {

@@ -698,6 +698,10 @@ class BlobPipeline:
     def set_debug(self, flags: int):
         self._check(self._L.cova_pipeline_set_debug(self._h, flags))
 
+    def set_sm_limit(self, n_sms: int):
+        """cova_pipeline_set_sm_limit: size this handle's grids for n_sms SMs (0 = the device's); results do not change."""
+        self._check(self._L.cova_pipeline_set_sm_limit(self._h, n_sms))
+
     def last_plan(self) -> list[dict]:
         """cova_pipeline_last_plan: per layer the launch plan of its last tcgen05 launch (family 0: not launched yet)."""
         out = (_lib.LayerPlan * _lib.N_LAYERS)()

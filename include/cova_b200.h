@@ -323,6 +323,11 @@ int cova_pipeline_run_layer(cova_pipeline *p, int layer, uint32_t impl);
  * stream-ordered launches instead of programmatic dependent launch (this handle only), bit 6 whole-tile accumulators for
  * dec0 / dec1 */
 int cova_pipeline_set_debug(cova_pipeline *p, int flags);
+/* Size every grid of this handle (the BlobNet layers, tensorisation, the carry of continued streams) as on a device of
+ * n_sms SMs; 0 restores the device's count.  Results do not depend on it: each persistent CTA then walks more tile groups,
+ * which lets the tests reach the state carried between groups at small shapes.  COVA_E_INVAL for a null handle, n_sms < 0
+ * or above the device's count, and while submitted batches are in flight; a refused call changes nothing. */
+int cova_pipeline_set_sm_limit(cova_pipeline *p, int n_sms);
 
 /* Diagnostics: the launch plan of each tcgen05 BlobNet layer, out[layer] for the layers of cova_pipeline_run_layer.  Each
  * layer picks its plan at run time from a list of candidate tile configurations, by what fits shared memory for the
