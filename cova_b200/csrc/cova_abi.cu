@@ -702,6 +702,8 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
     if ((flags & 0xffu) == COVA_IMPL_SIMT)
         return set_err(COVA_E_UNSUPPORTED, "the validation kernels (COVA_IMPL_SIMT) are not part of this build; use libcova_b200_val.so");
 #endif
+    HostWeights hw;                  // parsed and checked before the device is touched: a CPU-only caller sees the refusal
+    if ((rc = parse_weights(weights, weights_len, hw))) return rc;
     rc = check_device(device);
     if (rc) return rc;
     auto *p = new (std::nothrow) cova_pipeline();
@@ -713,7 +715,7 @@ extern "C" int cova_pipeline_new(cova_pipeline **out, int device, uint32_t w_mb,
     p->s_gamma.assign(max_streams, 0); p->s_thr.assign(max_streams, 0); p->s_thr_set.assign(max_streams, 0);
     p->s_seg.assign(max_streams, 0.5f); p->s_seg_set.assign(max_streams, 0);
     auto fail = [&](int code) { cova_pipeline_free(p); return code; };
-    if ((rc = parse_weights(weights, weights_len, p->hw))) return fail(rc);
+    p->hw = std::move(hw);           // moves the storage the tensor pointers of hw point into
     cudaDeviceProp prop;
     if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return fail(set_err(COVA_E_CUDA, "cudaGetDeviceProperties failed"));
     p->n_sms = p->dev_sms = prop.multiProcessorCount;

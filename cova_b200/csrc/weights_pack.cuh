@@ -22,6 +22,68 @@ struct HostWeights {
     size_t off_enc[4][8], off_dec[4][6], off_head[2];   // float offsets into storage (mirrored on device)
 };
 
+// Finite values the kernels still cannot represent, refused instead of turning into NaN / Inf outputs: a negative
+// variance (NaN BatchNorm scale), a BatchNorm scale, shift or offset that overflows fp32, and a weight whose fp16 image
+// overflows (|v| >= 65520 rounds to Inf): W / 6 in block 1, W in the other layers, the head folded into dec3.  Each
+// value is computed by the expression the packing (below) uses.  Keras never leaves a negative moving variance.
+inline int check_weights(const HostWeights &hw) {
+    char name[32];
+    auto bad = [&](const char *what) { return set_err(COVA_E_WEIGHTS, "CVBN %s: %s", name, what); };
+    auto fp16_ok = [](float v) { return fabsf(v) < 65520.f; };
+    auto scale_ok = [&](const float *gamma, const float *var, int c, float &s) {
+        s = gamma[c] / sqrtf(var[c] + kBnEps);
+        return std::isfinite(s);
+    };
+    for (int i = 0; i < 4; i++) {
+        const auto &e = hw.enc[i];
+        const size_t co_n = kEncCout[i], n_w = co_n * kEncCin[i] * 9;
+        snprintf(name, sizeof(name), "enc%d.conv_w", i);
+        for (size_t k = 0; k < n_w; k++)
+            if (!fp16_ok(i == 0 ? e.conv_w[k] / 6.0f : e.conv_w[k]))
+                return bad(i == 0 ? "a weight / 6 overflows fp16" : "a weight overflows fp16");
+        for (size_t c = 0; c < co_n; c++) {
+            float s;
+            snprintf(name, sizeof(name), "enc%d.bn_var", i);
+            if (e.var[c] < 0.f) return bad("negative variance");
+            snprintf(name, sizeof(name), "enc%d.bn_gamma", i);
+            if (!scale_ok(e.gamma, e.var, (int)c, s)) return bad("the BatchNorm scale overflows fp32");
+            snprintf(name, sizeof(name), "enc%d.bn_mean", i);
+            if (!std::isfinite(e.beta[c] - e.mean[c] * s)) return bad("the BatchNorm shift overflows fp32");
+        }
+    }
+    for (int i = 0; i < 4; i++) {
+        const auto &d = hw.dec[i];
+        const size_t co_n = kDecCout[i], n_w = co_n * kDecCin[i] * 16;
+        snprintf(name, sizeof(name), "dec%d.convt_w", i);
+        if (i < 3)
+            for (size_t k = 0; k < n_w; k++)
+                if (!fp16_ok(d.convt_w[k])) return bad("a weight overflows fp16");
+        for (size_t c = 0; i < 3 && c < co_n; c++) {
+            float s;
+            snprintf(name, sizeof(name), "dec%d.bn_var", i);
+            if (d.var[c] < 0.f) return bad("negative variance");
+            snprintf(name, sizeof(name), "dec%d.bn_gamma", i);
+            if (!scale_ok(d.gamma, d.var, (int)c, s)) return bad("the BatchNorm scale overflows fp32");
+            snprintf(name, sizeof(name), "dec%d.bn_mean", i);
+            if (!std::isfinite((d.convt_b[c] - d.mean[c]) * s + d.beta[c])) return bad("the BatchNorm offset overflows fp32");
+        }
+    }
+    // dec3 + head: fold[ci][ky][kx] = sum_co W[ci][co][ky][kx] * head_w[co] in double, rounded to fp32 then fp16
+    const int ci_n = kDecCin[3], co_n = kDecCout[3];
+    snprintf(name, sizeof(name), "head_w");
+    for (int ci = 0; ci < ci_n; ci++)
+        for (int k = 0; k < 16; k++) {
+            double acc = 0;
+            for (int co = 0; co < co_n; co++) acc += (double)hw.dec[3].convt_w[((size_t)ci * co_n + co) * 16 + k] * hw.head_w[co];
+            if (!fp16_ok((float)acc)) return bad("dec3.convt_w folded with the head overflows fp16");
+        }
+    double c0 = hw.head_b[0];
+    for (int co = 0; co < co_n; co++) c0 += (double)hw.head_w[co] * hw.dec[3].convt_b[co];
+    snprintf(name, sizeof(name), "head_b");
+    if (!std::isfinite((float)c0)) return bad("head_b + head_w . dec3.convt_b overflows fp32");
+    return COVA_OK;
+}
+
 inline int parse_weights(const void *blob, size_t len, HostWeights &hw) {
     if (!blob || len < 16) return set_err(COVA_E_WEIGHTS, "weight blob too short");
     const uint32_t *h = static_cast<const uint32_t *>(blob);
@@ -65,7 +127,7 @@ inline int parse_weights(const void *blob, size_t len, HostWeights &hw) {
     hw.head_b = take(1, hw.off_head[1]);
     for (float v : hw.storage)
         if (!(v == v) || v > 3e38f || v < -3e38f) return set_err(COVA_E_WEIGHTS, "CVBN container holds NaN/Inf");
-    return COVA_OK;
+    return check_weights(hw);
 }
 
 inline int floor_div2(int v) { return v >= 0 ? v / 2 : -((-v + 1) / 2); }

@@ -28,7 +28,9 @@ extern "C" {
 #define COVA_E_CUDA (-2)        /* a CUDA call failed; see cova_last_error() */
 #define COVA_E_NOMEM (-3)
 #define COVA_E_TOOSMALL (-4)    /* output buffer too small; the required size is reported */
-#define COVA_E_WEIGHTS (-5)     /* not a CVBN v1 weight container */
+#define COVA_E_WEIGHTS (-5)     /* not a CVBN v1 weight container, or one the kernels cannot represent: NaN/Inf, a negative
+                                   BatchNorm variance, a BatchNorm scale / shift that overflows fp32, a weight whose fp16
+                                   image overflows (cova_last_error() names the tensor); checked before any device use */
 #define COVA_E_UNSUPPORTED (-6) /* e.g. timestep != 4 for BlobNet, grid too large for the CCL kernel (see COVA_FLAG_CCL_CLUSTER) */
 #define COVA_E_NODEVICE (-7)    /* no CUDA device: there is no CPU fallback */
 #define COVA_E_NUMERIC (-8)     /* host tracker: Kalman innovation covariance not positive definite */
